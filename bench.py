@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path (through the C ABI)
   python bench.py --impl reference --gpus N --steps K ...  # the reference's algorithm on the host CPU (oracle port)
+  python bench.py ... --dump-outputs DIR                   # + the latents of the last timed step, DIR/*.npy (float32)
 
 Workload (BASELINE.json configs[1], SURVEY cfg-2): conditional_dm3d U-Net (F=32, widths 64/128/256, cross-attention at
 8^3), DDPM, batch 8 per GPU, 32^3 x 256 latent, class-id context, random-init weights, synthetic latents.
@@ -188,6 +189,22 @@ def ncu_traffic():
         return None
 
 
+DUMP_ELEMS = 1 << 23   # 32 MB of fp32 per rank
+
+
+def dump_outputs(out_dir, lat, rank, world):
+    """Write the fp32 latents the timed steps left in the step state (what generate() returns to its caller) to
+    <out_dir>/latents.npy, or, when larger than DUMP_ELEMS, DUMP_ELEMS of them at flat indices drawn once from a seed-0 CPU
+    generator and sorted (latents_sample.npy), so that two builds can be compared output for output."""
+    flat = lat.reshape(-1)
+    name = "latents"
+    if flat.numel() > DUMP_ELEMS:
+        idx = torch.randint(0, flat.numel(), (DUMP_ELEMS,), generator=torch.Generator().manual_seed(0)).sort().values
+        flat, name = flat[idx.to(flat.device)], "latents_sample"
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, name + (f"_rank{rank}" if world > 1 else "") + ".npy"), flat.float().cpu().numpy())
+
+
 def event_time(fn, iters, warm=1):
     for _ in range(warm):
         fn()
@@ -252,6 +269,8 @@ def run_ours(args):
     ms = max_over_ranks(e0.elapsed_time(e1), world, dev)
     clk = clocks.stop()
     value = world * B * K / (ms * 1e-3)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, st["x"], rank, world)
 
     # ---- end to end through the public API with HOST buffers: pinned x_T -> H2D -> K steps -> D2H latents
     x_host = torch.randn(shape, generator=torch.Generator().manual_seed(rank)).pin_memory()
@@ -519,7 +538,13 @@ def main():
     ap.add_argument("--no-cfg3", action="store_true", help="skip the cfg-3 (quantize + decode) leg (tuning runs)")
     ap.add_argument("--batch", type=int, default=None, help="tuning aid: per-GPU batch other than the cfg-2 value (8); not a bench line")
     ap.add_argument("--dump-ops", default=None, help="write per-op (kind,name,work,ms) CSV of one step")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the latents of the last timed step to DIR as float32 .npy (a fixed, seeded sample when larger than 32 MB)")
     args = ap.parse_args()
+    if not 1 <= args.steps <= CFG["T"] - max(args.warmup, 3):
+        ap.error(f"--steps must be in [1, {CFG['T']} - max(--warmup, 3)]: the timed steps walk one T={CFG['T']} timestep sequence")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the CUDA path's latents (--impl ours)")
     if args.batch:
         CFG["B"] = args.batch
     try:

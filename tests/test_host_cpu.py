@@ -202,7 +202,7 @@ def test_tuning_switches_need_the_tuning_gate(monkeypatch):
     assert L.tuning_env("B200DM_CHAINS", "1") == "4"
 
 
-def test_test_dm_script_flags():
+def test_test_dm_script_flags(tmp_path):
     """tools/test_dm.py mirrors the --test_dm invocation of main.py:428-448 / main_conditional_dm.py:195-215: the reference's flag
     names parse with the reference's defaults, the modes outside the sampling path are accepted by the parser and refused at run
     time (no GPU needed for either)."""
@@ -218,8 +218,7 @@ def test_test_dm_script_flags():
     with pytest.raises(SystemExit, match="--test_dm only"):
         mod.run(b)
     img = np.arange(12, dtype=np.float32).reshape(3, 4)
-    path = os.path.join(os.environ.get("TMPDIR", "/tmp"), "b200dm_slice_test.pgm")
+    path = str(tmp_path / "slice.pgm")
     mod.write_pgm(path, img)
     raw = open(path, "rb").read()
     assert raw.startswith(b"P5\n4 3\n255\n") and len(raw) == len(b"P5\n4 3\n255\n") + 12 and raw[-1] == 255 and raw[len(b"P5\n4 3\n255\n")] == 0
-    os.remove(path)

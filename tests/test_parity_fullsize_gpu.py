@@ -31,7 +31,12 @@ from oracle.unet import UNet as OUNet
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GOLD = os.path.join(ROOT, "tests", "golden")
-CACHE = os.environ.get("B200DM_ORACLE_CACHE", "/tmp/b200dm_oracle_cache")   # fp32-oracle results shared with the fp16 child run
+
+
+@pytest.fixture(scope="session")
+def oracle_cache(tmp_path_factory):
+    """fp32-oracle results of this session; the fp16 child run is pointed at its parent's (B200DM_ORACLE_CACHE)."""
+    return os.environ.get("B200DM_ORACLE_CACHE") or str(tmp_path_factory.mktemp("oracle_cache"))
 
 
 def prec():
@@ -56,9 +61,8 @@ def maxabs(a, b):
     return (a.float().cpu() - b.float()).abs().max().item()
 
 
-def cached(name, fn):
-    os.makedirs(CACHE, exist_ok=True)
-    p = os.path.join(CACHE, name + ".pt")
+def cached(cache, name, fn):
+    p = os.path.join(cache, name + ".pt")
     if os.path.exists(p):
         return torch.load(p)
     v = fn()
@@ -85,7 +89,7 @@ def _cfg2():
     return net, ou, P
 
 
-def test_cfg2_eps_forward_full_batch(cuda):
+def test_cfg2_eps_forward_full_batch(cuda, oracle_cache):
     """eps_hat = network([x, t, ctx]) at B=8, 32^3 x 256, t=500, per-sample class ids: CUDA vs the fp32 oracle (the
     reference's arithmetic) and vs the oracle that rounds where the CUDA path stores 16-bit values."""
     torch.set_num_threads(os.cpu_count() or 1)
@@ -99,7 +103,7 @@ def test_cfg2_eps_forward_full_batch(cuda):
     y = net([x.to(cuda), tt, ctx]).cpu()
     flag_ok()
     with torch.no_grad():
-        ref = cached("cfg2_eps_B8_t500", lambda: ou.forward(P, x, tt, ctx=ctx))
+        ref = cached(oracle_cache, "cfg2_eps_B8_t500", lambda: ou.forward(P, x, tt, ctx=ctx))
         ref_e = ou.forward(P, x[:2], tt[:2], ctx=ctx[:2], emu=emu16())
     r_x, r_e = rel(y, ref), rel(y[:2], ref_e)
     report("cfg-2 eps_hat B=8 32^3x256 t=500", rel_l2_vs_fp32_oracle=r_x, rel_l2_vs_emulating_oracle=r_e,
@@ -108,7 +112,7 @@ def test_cfg2_eps_forward_full_batch(cuda):
     assert r_e <= tol(2.5e-2, 4e-3), r_e
 
 
-def test_cfg2_last_50_steps_of_the_chain(cuda):
+def test_cfg2_last_50_steps_of_the_chain(cuda, oracle_cache):
     """The last 50 reverse steps (t = 49 .. 0) of the T=1000 DDPM chain, B=2, same x and per-step noise on both sides."""
     import b200dm
     torch.set_num_threads(os.cpu_count() or 1)
@@ -132,7 +136,7 @@ def test_cfg2_last_50_steps_of_the_chain(cuda):
                 x = OS.ddpm_step(b, x, eps, i, noises.get(i))
         return x
 
-    ref = cached("cfg2_chain50_B2", oracle_chain)
+    ref = cached(oracle_cache, "cfg2_chain50_B2", oracle_chain)
     r, ma = rel(lat, ref), maxabs(lat, ref)
     report("cfg-2 last 50 DDPM steps B=2 32^3x256", rel_l2=r, max_abs=ma, north_star_rel=1e-3, north_star_maxabs=1e-2)
     assert r <= tol(1e-2, 1.5e-3) and ma <= tol(1e-1, 2e-2), (r, ma)
@@ -170,7 +174,7 @@ def test_cfg1_full_1000_step_chain_production_path(cuda):
 
 
 # ------------------------------------------------------------------------------------------------ cfg-3
-def test_cfg3_vq_and_attn_cp_decoder_fullsize(cuda):
+def test_cfg3_vq_and_attn_cp_decoder_fullsize(cuda, oracle_cache):
     """quantize (K=1024, D=256, 32^3 rows) + vqgan_attn_cp Decoder (32,64,128): 32^3 -> 128^3, B=1, vs the oracle."""
     import b200dm
     torch.set_num_threads(os.cpu_count() or 1)
@@ -197,13 +201,13 @@ def test_cfg3_vq_and_attn_cp_decoder_fullsize(cuda):
     flag_ok()
     assert tuple(vol.shape) == (1, 128, 128, 128, 1)
     with torch.no_grad():
-        ref = cached("cfg3_attncp_B1", lambda: od.forward(P, q_ref))
+        ref = cached(oracle_cache, "cfg3_attncp_B1", lambda: od.forward(P, q_ref))
     r, ma = rel(vol, ref), maxabs(vol, ref)
     report("cfg-3 attn_cp decoder 32^3->128^3 B=1", rel_l2=r, max_abs=ma, ref_absmax=ref.abs().max().item())
     assert r <= tol(2e-2, 3e-3), r
 
 
-def test_cfg3_monai_decoder_fullsize(cuda):
+def test_cfg3_monai_decoder_fullsize(cuda, oracle_cache):
     """The DM's own first stage (dm3d.py:386-404): monai decoder 8^3 x 256 -> 128^3, channels (32,64,128,256), R=5, B=1."""
     import b200dm
     torch.set_num_threads(os.cpu_count() or 1)
@@ -217,7 +221,7 @@ def test_cfg3_monai_decoder_fullsize(cuda):
     flag_ok()
     assert tuple(vol.shape) == (1, 128, 128, 128, 1)
     with torch.no_grad():
-        ref = cached("cfg3_monai_B1", lambda: od.forward(P, z))
+        ref = cached(oracle_cache, "cfg3_monai_B1", lambda: od.forward(P, z))
     r, ma = rel(vol, ref), maxabs(vol, ref)
     report("cfg-3 monai decoder 8^3->128^3 R=5 B=1", rel_l2=r, max_abs=ma, ref_absmax=ref.abs().max().item())
     assert r <= tol(3e-2, 5e-3), r
@@ -385,10 +389,10 @@ def test_set_weights_invalidates_compiled_step(cuda):
 
 # ------------------------------------------------------------------------------------------------ the fp16 build
 @pytest.mark.skipif(os.environ.get("B200DM_PRECISION", "bf16") != "bf16", reason="already the child run")
-def test_fp16_build_meets_chain_tolerances(cuda):
+def test_fp16_build_meets_chain_tolerances(cuda, oracle_cache):
     """libb200dm_f16.so (same sources, IEEE fp16 as the 16-bit storage type): the cfg-2 / cfg-1 / cfg-3 parity tests of this file in a
     child process; their fp16 tolerances are north_star's chain targets (rel-L2 <= 1e-3 x 1.5-3 margin, max-abs <= 2e-2)."""
-    env = dict(os.environ, B200DM_PRECISION="fp16", B200DM_ORACLE_CACHE=CACHE)
+    env = dict(os.environ, B200DM_PRECISION="fp16", B200DM_ORACLE_CACHE=oracle_cache)
     sel = "cfg2 or cfg1 or cfg3 or cfg4 or per_sample"
     r = subprocess.run([sys.executable, "-m", "pytest", os.path.abspath(__file__), "-m", "gpu", "-x", "-q", "-s", "-k", sel],
                        env=env, cwd=ROOT, capture_output=True, text=True)
