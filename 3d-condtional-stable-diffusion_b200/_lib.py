@@ -129,11 +129,8 @@ _SIGS = {
     "b200dm_conv_plan_flops": (C.c_double, [C.c_void_p]),
     "b200dm_conv_plan_set_trace": (C.c_int, [C.c_void_p, C.c_void_p]),
     "b200dm_conv_plan_set_out_affine": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
-    "b200dm_conv_plan_add_output": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32]),
-    "b200dm_conv_plan_set_side_norm": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32]),
     "b200dm_conv_plan_set_fused_update": (C.c_int, [C.c_void_p, C.POINTER(UpdateDesc), C.c_void_p, C.c_void_p, C.c_void_p]),
     "b200dm_conv_plan_info": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
-    "b200dm_conv_plan_set_input_norm": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32]),
     "b200dm_conv_plan_gn_partials_bytes": (C.c_size_t, [C.c_void_p, C.POINTER(C.c_int32)]),
     "b200dm_conv_plan_set_gn_partials": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t]),
     "b200dm_gn_finalize": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int64, C.c_float, C.c_void_p, C.c_void_p]),
@@ -183,8 +180,8 @@ def lib():
 
 
 def tuning_env(name: str, default: str) -> str:
-    """Experiment switches (B200DM_CHAINS, B200DM_LANES, B200DM_SHADOW, ...) are honoured only when B200DM_TUNING=1 is also set, like
-    the native library's: a production process's environment cannot reconfigure the program by accident."""
+    """Experiment switches (B200DM_CHAINS) are honoured only when B200DM_TUNING=1 is also set: a production process's environment
+    cannot reconfigure the program by accident."""
     return os.environ.get(name, default) if os.environ.get("B200DM_TUNING") == "1" else default
 
 

@@ -19,19 +19,10 @@
 // Warp roles (192 threads): warp 0 = TMA producer, warp 1 = TMEM owner + MMA issuer, warps 2-5 = epilogue.
 #include <cuda.h>
 #include <string.h>
-#include <stdlib.h>
 #include <math.h>
 #include <new>
 #include <vector>
 #include "conv_common.cuh"
-
-// Tuning / experiment switches (B200DM_NO_PAIR, B200DM_CLUSTER, B200DM_KSPLIT, ...) are read only when the process also sets
-// B200DM_TUNING=1: a production process's environment cannot reconfigure the kernels by accident.
-static const char* tuning_env(const char* name) {
-  static int on = -1;
-  if (on < 0) { const char* e = getenv("B200DM_TUNING"); on = (e && e[0] == '1') ? 1 : 0; }
-  return on ? getenv(name) : nullptr;
-}
 
 #include "conv_halo.cuh"
 #include "conv_halo_up.cuh"
@@ -43,10 +34,10 @@ namespace {
 constexpr int kThreads = 192;
 constexpr int kABytes = 128 * 128;  // 128 rows x 64 bf16
 
-// CMODE 0: plain; 1: cluster with TMA-multicast operands (experiment); 2: split-K cluster (K range per CTA, partial
-// accumulators reduced through distributed shared memory by the cluster's first CTA).
+// KSPLIT: split-K cluster (K range per CTA, partial accumulators reduced through distributed shared memory by the cluster's
+// first CTA); four-stage instantiations only.
 // (two-stage instantiations: registers capped so that four CTAs share an SM -- see conv_plan_create)
-template <int BLOCK_N, int NSTAGE, int CMODE>
+template <int BLOCK_N, int NSTAGE, bool KSPLIT>
 __global__ void __launch_bounds__(kThreads, NSTAGE == 2 ? 4 : 1)
 conv_igemm_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant__ CUtensorMap mapA1,
                   const __grid_constant__ CUtensorMap mapB, const __grid_constant__ ConvOutMaps om, const ConvParams p) {
@@ -56,13 +47,10 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_consta
   constexpr int kResBytes = BLOCK_N >= 64 ? BLOCK_N * 256 : 0;   // staged epilogue: 128 rows x BLOCK_N bf16 residual tile
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  const bool staged = BLOCK_N >= 64 && CMODE != 1 && p.tma_epi != 0;
+  const bool staged = BLOCK_N >= 64 && p.tma_epi != 0;
   const bool staged_res = staged && p.residual != nullptr;
   uint8_t* res_smem = smem + NSTAGE * kStageBytes;
-  const bool side_on = BLOCK_N >= 64 && CMODE == 0 && p.side != 0 && blockIdx.y == 0;   // n-tile 0 writes the side output
-  uint8_t* side_smem = res_smem + (staged_res ? kResBytes : 0);                         // [128 rows][128 B] staging + affine table
-  float* side_tab = reinterpret_cast<float*>(side_smem + 16384);                        // [2][side_c]
-  uint64_t* bars = reinterpret_cast<uint64_t*>(side_smem + (p.side ? 16384 + 2 * p.side_c * 4 : 0));
+  uint64_t* bars = reinterpret_cast<uint64_t*>(res_smem + (staged_res ? kResBytes : 0));
   // bars[0..NSTAGE) full, [NSTAGE..2NSTAGE) empty, [2NSTAGE] tmem_full, [2NSTAGE+1] residual tile; then tmem ptr
   uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(bars + 2 * NSTAGE + 3);   // (+3 keeps bias_s 16-byte aligned)
   float* bias_s = reinterpret_cast<float*>(tmem_ptr_smem + 2);   // [2][BLOCK_N]: bias (+temb), output-affine scale
@@ -79,8 +67,6 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_consta
   pdl_launch_dependents();
   int tix = 0;   // timeline index of this thread's region (tuning aid: b200dm_conv_plan_set_trace)
   if (threadIdx.x == 0) trace_ev(p, 3, tix, 40);
-  constexpr bool CLUSTER = CMODE == 1;
-  constexpr bool KSPLIT = CMODE == 2;
   const int ks = KSPLIT ? p.ksplit : 1;
   const int krank = KSPLIT ? (int)ptx::cluster_ctaid_x() : 0;
   int bx = KSPLIT ? blockIdx.x / ks : blockIdx.x;
@@ -96,15 +82,8 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_consta
   const int kb0 = KSPLIT ? (int)((long long)krank * nkb_all / ks) : 0;            // this CTA's K range
   const int kb1 = KSPLIT ? (int)((long long)(krank + 1) * nkb_all / ks) : nkb_all;
 
-  // Cluster of cl_m x cl_n CTAs (x = m-tiles, y = n-tiles): the cl_n CTAs of one m-tile each fetch 1/cl_n of the A tile and
-  // TMA-multicast it to all of them; the cl_m CTAs of one n-tile do the same with the B tile.  A stage may be refilled
-  // only when EVERY CTA of the cluster has consumed it (their tcgen05.commit multicasts onto all empty barriers).
-  // Why: one SM's TMA path sustains ~35 B/cycle (measured), a 128x128 tile wants 128 B/cycle of operands.
-  const uint32_t cl_m = CLUSTER ? (uint32_t)p.cl_m : 1u, cl_n = CLUSTER ? (uint32_t)p.cl_n : 1u;
-  const uint32_t rank_m = CLUSTER ? ptx::cluster_ctaid_x() : 0u, rank_n = CLUSTER ? ptx::cluster_ctaid_y() : 0u;
-
   if (threadIdx.x == 0) {
-    for (int s = 0; s < NSTAGE; ++s) { ptx::mbar_init(full_bar(s), 1); ptx::mbar_init(empty_bar(s), cl_m * cl_n + (side_on ? 1u : 0u)); }
+    for (int s = 0; s < NSTAGE; ++s) { ptx::mbar_init(full_bar(s), 1); ptx::mbar_init(empty_bar(s), 1); }
     ptx::mbar_init(tmem_full_bar, 1);
     ptx::mbar_init(res_bar, 1);
     ptx::fence_barrier_init();
@@ -118,7 +97,6 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_consta
   }
   ptx::tc_fence_before();
   __syncthreads();
-  if (CLUSTER) ptx::cluster_sync_all();   // peers' barriers are initialised before any multicast / remote arrive
   bool mid_synced = false;                // split-K: every thread of the cluster passes ONE mid-kernel cluster barrier
   ptx::tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr_smem;
@@ -158,23 +136,8 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_consta
           ptx::mbar_expect_tx(full_bar(s), kStageBytes);
           const CUtensorMap* mapA = chunk < p.nch0 ? &mapA0 : &mapA1;
           const int cch = (chunk < p.nch0 ? chunk : chunk - p.nch0) * 64;
-          int cw = w0 * p.stride + ow, chh = h0 * p.stride + oh, cd = d0 * p.stride + od, cn = n0;
-          if (CLUSTER && cl_n > 1) {
-            const int off = (int)rank_n * p.a_split_ext;
-            if (p.a_split_dim == 1) cw += off; else if (p.a_split_dim == 2) chh += off; else if (p.a_split_dim == 3) cd += off; else cn += off;
-            uint16_t mask = 0;
-            for (uint32_t j = 0; j < cl_n; ++j) mask |= (uint16_t)(1u << (rank_m + j * cl_m));
-            ptx::tma_load_5d_mc(a_dst + rank_n * (kABytes / cl_n), mapA, full_bar(s), cch, cw, chh, cd, cn, mask);
-          } else {
-            ptx::tma_load_5d(a_dst, mapA, full_bar(s), cch, cw, chh, cd, cn);
-          }
-          if (CLUSTER && cl_m > 1) {
-            uint16_t mask = 0;
-            for (uint32_t i = 0; i < cl_m; ++i) mask |= (uint16_t)(1u << (i + rank_n * cl_m));
-            ptx::tma_load_2d_mc(b_dst + rank_m * (kBBytes / cl_m), &mapB, full_bar(s), kb * 64, b_row + (int)rank_m * (BLOCK_N / (int)cl_m), mask);
-          } else {
-            ptx::tma_load_2d(b_dst, &mapB, full_bar(s), kb * 64, b_row);
-          }
+          ptx::tma_load_5d(a_dst, mapA, full_bar(s), cch, w0 * p.stride + ow, h0 * p.stride + oh, d0 * p.stride + od, n0);
+          ptx::tma_load_2d(b_dst, &mapB, full_bar(s), kb * 64, b_row);
         }
         __syncwarp();
         if (++s == NSTAGE) { s = 0; phase ^= 1; }
@@ -205,8 +168,7 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_consta
           if (ksn > 1) ptx::tc_mma_f16(tmem_base, da + 2, db + 2, idesc, 1u);
           if (ksn > 2) ptx::tc_mma_f16(tmem_base, da + 4, db + 4, idesc, 1u);
           if (ksn > 3) ptx::tc_mma_f16(tmem_base, da + 6, db + 6, idesc, 1u);
-          if (CLUSTER) ptx::tc_commit_mc(empty_bar(s), (uint16_t)((1u << (cl_m * cl_n)) - 1u));
-          else ptx::tc_commit(empty_bar(s));
+          ptx::tc_commit(empty_bar(s));
         }
         __syncwarp();
         if (++s == NSTAGE) { s = 0; phase ^= 1; }
@@ -246,50 +208,6 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_consta
     if (has_bs) {
       stage_bias(p, bias_s, scale_s, n_tile * BLOCK_N, BLOCK_N, cbrow, threadIdx.x - 64);
       epilogue_bar_sync();
-    }
-    if (BLOCK_N >= 64 && CMODE == 0 && side_on) {
-      // ---- side output: every A tile (one 64-channel chunk of x or skip, 1^3 conv => k-block == chunk) is read back from
-      // shared memory, normalised (+ swish) and TMA-stored at its channel offset of the concatenated tensor; the stage is
-      // released to the producer only after these 128 threads are done with it (empty barrier count 2)
-      const int et = threadIdx.x - 64;
-      for (int c = et; c < p.side_c; c += 128) { side_tab[c] = __ldg(p.side_scale + c); side_tab[p.side_c + c] = __ldg(p.side_shift + c); }
-      epilogue_bar_sync();
-      uint32_t ss = 0, sph = 0;
-      for (int kb = 0; kb < nkb_all; ++kb) {
-        if (!ptx::mbar_wait(full_bar(ss), sph, p.dbg, 5)) break;
-        const int cbase = kb < p.nch0 ? kb * 64 : p.nch0 * 64 + (kb - p.nch0) * 64;   // (c0 % 64 == 0 whenever c1 > 0)
-        if (kb > 0) {   // the previous chunk's store has finished reading the staging tile
-          if (et == 0) ptx::bulk_wait_read_all();
-          epilogue_bar_sync();
-        }
-        const uint8_t* arow = smem + ss * kStageBytes + (uint32_t)r * 128u;
-        uint8_t* srow = side_smem + (uint32_t)r * 128u;
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-          const uint32_t o = (uint32_t)((j ^ (r & 7)) << 4);
-          float f[8];
-          unpack8(*reinterpret_cast<const bf16x8*>(arow + o), f);
-          const int c = cbase + j * 8;
-          if (c < p.side_c) {   // (side_c % 8 == 0)
-            const float4 a0 = *reinterpret_cast<const float4*>(side_tab + c), a1 = *reinterpret_cast<const float4*>(side_tab + c + 4);
-            const float4 b0 = *reinterpret_cast<const float4*>(side_tab + p.side_c + c), b1 = *reinterpret_cast<const float4*>(side_tab + p.side_c + c + 4);
-            f[0] = apply_act(fmaf(f[0], a0.x, b0.x), p.side_act); f[1] = apply_act(fmaf(f[1], a0.y, b0.y), p.side_act);
-            f[2] = apply_act(fmaf(f[2], a0.z, b0.z), p.side_act); f[3] = apply_act(fmaf(f[3], a0.w, b0.w), p.side_act);
-            f[4] = apply_act(fmaf(f[4], a1.x, b1.x), p.side_act); f[5] = apply_act(fmaf(f[5], a1.y, b1.y), p.side_act);
-            f[6] = apply_act(fmaf(f[6], a1.z, b1.z), p.side_act); f[7] = apply_act(fmaf(f[7], a1.w, b1.w), p.side_act);
-          }
-          *reinterpret_cast<bf16x8*>(srow + o) = pack8(f);
-        }
-        ptx::fence_proxy_async();
-        epilogue_bar_sync();
-        if (et == 0) {
-          ptx::tma_store_5d(&om.s, ptx::smem_u32(side_smem), cbase, w0, h0, d0, n0);
-          ptx::bulk_commit_group();
-          ptx::mbar_arrive(empty_bar(ss));
-        }
-        if (++ss == NSTAGE) { ss = 0; sph ^= 1; }
-      }
-      if (et == 0) ptx::bulk_wait_read_all();
     }
     if (warp == 2 && lane == 0) trace_ev(p, 1, tix, 45);
     const bool ok = ptx::mbar_wait(tmem_full_bar, 0, p.dbg, 3);
@@ -401,11 +319,8 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_consta
           const int col0 = n_tile * BLOCK_N + c0;
           if (col0 >= p.c_out) break;  // warp-uniform
           uint32_t rr[16];
-          if (p.epi_dbg < 2) {
-            ptx::tc_ld_32x32b_x16(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)c0, rr);
-            ptx::tc_wait_ld();
-          }
-          if (p.epi_dbg != 0) continue;
+          ptx::tc_ld_32x32b_x16(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)c0, rr);
+          ptx::tc_wait_ld();
           if (KSPLIT) {
             for (int pr = 1; pr < ks; ++pr) {
               const uint32_t remote = ptx::mapa_shared(ptx::smem_u32(stage_f + c0 * 128 + r * 4), (uint32_t)pr);
@@ -432,7 +347,7 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_consta
     ptx::tc_fence_after();
     ptx::tmem_dealloc(tmem_base, kTmemCols);
   }
-  if (CLUSTER || KSPLIT) ptx::cluster_sync_all();   // no CTA exits while a peer may still write / read its shared memory
+  if (KSPLIT) ptx::cluster_sync_all();   // no CTA exits while a peer may still write / read its shared memory
   if (threadIdx.x == 0) trace_ev(p, 3, tix, 48);
 }
 
@@ -505,11 +420,6 @@ int compute_geometry(const b200dm_conv_desc* d, Geometry* g) {
   else if (d->c_out <= 64) g->n_pad = 64;
   else g->n_pad = ((d->c_out + 127) / 128) * 128;
   g->block_n = g->n_pad < 128 ? g->n_pad : 128;
-  if (const char* e = tuning_env("B200DM_IGEMM_BN")) {   // tuning aid: narrower N tiles (more CTAs, shorter epilogues)
-    const int v = atoi(e);
-    if ((v == 64 || v == 32) && g->n_pad >= 128 && !(d->mode == B200DM_CONV_DIRECT && d->ksize == 3 && d->stride == 1 && d->in_w >= 8 && d->in_h >= 16))
-      g->block_n = v;
-  }
   g->ktot = (size_t)(g->nch0 + g->nch1) * g->ntaps * 64;
   // M tile box, product 128
   if (d->mode == B200DM_CONV_BATCHED_GEMM) {
@@ -648,25 +558,26 @@ extern "C" int b200dm_conv_pack_weights(const b200dm_conv_desc* d, const float* 
   return B200DM_OK;
 }
 
-static size_t conv_smem_bytes(int block_n, int nstage, bool staged_res, int side_c = 0) {
+static size_t conv_smem_bytes(int block_n, int nstage, bool staged_res) {
   return 1024 + (size_t)nstage * (kABytes + block_n * 128) + (staged_res ? (size_t)block_n * 256 : 0) +
-         (side_c > 0 ? 16384 + (size_t)2 * side_c * 4 : 0) + (2 * nstage + 3) * 8 + 16 + 2 * block_n * 4;
+         (2 * nstage + 3) * 8 + 16 + 2 * block_n * 4;
 }
 
 static size_t conv_smem_attr(int block_n, int nstage) {   // opt-in ceiling of one kernel instantiation
-  const size_t v = conv_smem_bytes(block_n, nstage, true, 1024);
+  const size_t v = conv_smem_bytes(block_n, nstage, true);
   return v > 232448 ? 232448 : v;
 }
 
-template <int BLOCK_N, int NSTAGE>
+template <int BLOCK_N, int NSTAGE, bool KSPLIT>
 static int launch_conv(const b200dm_conv_plan* pl, cudaStream_t s) {
-  if (pl->p.ksplit > 1) {
-    auto kern = conv_igemm_kernel<BLOCK_N, NSTAGE, 2>;
-    static bool attr_set = false;
-    if (!attr_set) {
-      B2_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)conv_smem_attr(BLOCK_N, NSTAGE)));
-      attr_set = true;
-    }
+  static_assert(!KSPLIT || NSTAGE == 4, "split-K runs four stages only");
+  auto kern = conv_igemm_kernel<BLOCK_N, NSTAGE, KSPLIT>;
+  static bool attr_set = false;
+  if (!attr_set) {
+    B2_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)conv_smem_attr(BLOCK_N, NSTAGE)));
+    attr_set = true;
+  }
+  if constexpr (KSPLIT) {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = pl->grid; cfg.blockDim = dim3(kThreads); cfg.dynamicSmemBytes = pl->smem; cfg.stream = s;
     cudaLaunchAttribute at[2];
@@ -676,33 +587,9 @@ static int launch_conv(const b200dm_conv_plan* pl, cudaStream_t s) {
     at[1].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = at; cfg.numAttrs = b200dm_pdl_enabled() ? 2 : 1;
     B2_CHECK_CUDA(cudaLaunchKernelEx(&cfg, kern, pl->mapA0, pl->mapA1, pl->mapB, pl->om, pl->p));
-    return B200DM_OK;
+  } else {
+    B2_CHECK_CUDA(b2_launch(kern, pl->grid, dim3(kThreads), pl->smem, s, pl->mapA0, pl->mapA1, pl->mapB, pl->om, pl->p));
   }
-  if (pl->p.cl_m * pl->p.cl_n > 1) {
-    auto kern = conv_igemm_kernel<BLOCK_N, NSTAGE, 1>;
-    static bool attr_set = false;
-    if (!attr_set) {
-      B2_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)conv_smem_attr(BLOCK_N, NSTAGE)));
-      attr_set = true;
-    }
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = pl->grid; cfg.blockDim = dim3(kThreads); cfg.dynamicSmemBytes = pl->smem; cfg.stream = s;
-    cudaLaunchAttribute at[2];
-    at[0].id = cudaLaunchAttributeClusterDimension;
-    at[0].val.clusterDim.x = pl->p.cl_m; at[0].val.clusterDim.y = pl->p.cl_n; at[0].val.clusterDim.z = 1;
-    at[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[1].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = at; cfg.numAttrs = b200dm_pdl_enabled() ? 2 : 1;
-    B2_CHECK_CUDA(cudaLaunchKernelEx(&cfg, kern, pl->mapA0, pl->mapA1, pl->mapB, pl->om, pl->p));
-    return B200DM_OK;
-  }
-  auto kern = conv_igemm_kernel<BLOCK_N, NSTAGE, 0>;
-  static bool attr_set = false;
-  if (!attr_set) {
-    B2_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)conv_smem_attr(BLOCK_N, NSTAGE)));
-    attr_set = true;
-  }
-  B2_CHECK_CUDA(b2_launch(kern, pl->grid, dim3(kThreads), pl->smem, s, pl->mapA0, pl->mapA1, pl->mapB, pl->om, pl->p));
   return B200DM_OK;
 }
 
@@ -861,8 +748,7 @@ extern "C" int b200dm_conv_plan_create(const b200dm_conv_desc* d, const void* x0
   // C_out = 1, C_in = 32, 3^3 stride 1 (the vqgan_attn_cp decoder's head): HBM-bound stencil-reduce kernel instead of an
   // N = 16 tensor-core tile (conv_stencil.cuh); bias + activation epilogue only
   if (d->mode == B200DM_CONV_DIRECT && d->ksize == 3 && d->stride == 1 && d->c_out == 1 && d->c0 == stencil::kC && d->c1 == 0 &&
-      !chan_bias && !residual && !prelu_alpha && d->reserved[0] == B200DM_ACT_NONE && d->reserved[1] == 0 && d->use_halo >= 0 &&
-      !tuning_env("B200DM_NO_STENCIL")) {
+      !chan_bias && !residual && !prelu_alpha && d->reserved[0] == B200DM_ACT_NONE && d->reserved[1] == 0 && d->use_halo >= 0) {
     cuuint64_t dims[5] = {(cuuint64_t)d->c0, (cuuint64_t)d->in_w, (cuuint64_t)d->in_h, (cuuint64_t)d->in_d, (cuuint64_t)d->batch};
     cuuint64_t strides[4] = {(cuuint64_t)d->c0 * 2, (cuuint64_t)d->in_w * d->c0 * 2, (cuuint64_t)d->in_h * d->in_w * d->c0 * 2,
                              (cuuint64_t)d->in_d * d->in_h * d->in_w * d->c0 * 2};
@@ -894,7 +780,7 @@ extern "C" int b200dm_conv_plan_create(const b200dm_conv_desc* d, const void* x0
   // kd taps of an input plane as one N = 96 MMA and the weight set resident in shared memory (conv_sweep.cuh)
   if (d->mode == B200DM_CONV_DIRECT && d->ksize == 3 && d->stride == 1 && d->c_out == 32 && d->c0 == 32 && d->c1 == 0 &&
       d->y_dtype == B200DM_BF16 && !chan_bias && !prelu_alpha && d->reserved[1] == 0 && d->use_halo >= 0 && g.n_pad == 32 &&
-      g.ktot == 27 * 64 && d->in_w >= 8 && d->in_h >= 16 && d->in_d >= 2 && !tuning_env("B200DM_NO_SWEEP")) {
+      g.ktot == 27 * 64 && d->in_w >= 8 && d->in_h >= 16 && d->in_d >= 2) {
     const cuuint64_t C = 32;
     cuuint64_t dims[5] = {C, (cuuint64_t)d->in_w, (cuuint64_t)d->in_h, (cuuint64_t)d->in_d, (cuuint64_t)d->batch};
     cuuint64_t strides[4] = {C * 2, (cuuint64_t)d->in_w * C * 2, (cuuint64_t)d->in_h * d->in_w * C * 2,
@@ -942,49 +828,23 @@ extern "C" int b200dm_conv_plan_create(const b200dm_conv_desc* d, const void* x0
   // weight stream; bf16 staged output only
   pl->pair = !pl->halo && d->mode == B200DM_CONV_DIRECT && d->ksize == 3 && d->stride == 1 && d->in_w == 8 && d->in_h == 8 &&
              d->in_d >= 2 && d->reserved[1] == 0 && d->use_halo >= 0 && d->y_dtype == B200DM_BF16 && d->c_out % 64 == 0 &&
-             !prelu_alpha && !(tuning_env("B200DM_TMA_EPI") && atoi(tuning_env("B200DM_TMA_EPI")) == 0) && !tuning_env("B200DM_NO_PAIR");
+             !prelu_alpha;
   if (pl->pair) { pl->halo = true; g.block_n = 64; pl->g.block_n = 64; }
   // x2 up-convolutions (nearest-upsample + conv3, ConvT k4 s2) on low-resolution planes that fill the 8 x 16 halo tile
   {
     const long long per_up = (long long)((d->in_w + 7) / 8) * ((d->in_h + 15) / 16) * ((d->in_d + 1) / 2) * d->batch;
     // (C_out = 32 -- the decoders' last ConvT, 64 -> 32 at 64^3 -> 128^3 -- runs N = 32 tiles with 64-byte staged rows)
-    const bool up32 = d->c_out == 32 && g.block_n == 32 && !tuning_env("B200DM_NO_UP32");
+    const bool up32 = d->c_out == 32 && g.block_n == 32;
     pl->ups = d->mode == B200DM_CONV_PARITY && d->in_w >= 8 && d->in_h >= 16 && d->in_d >= 2 && (d->c_out % 64 == 0 || up32) &&
               d->y_dtype == B200DM_BF16 && !residual && !prelu_alpha && d->reserved[1] == 0 && d->use_halo >= 0 && per_up % 2 == 0 &&
-              (g.block_n == 64 || g.block_n == 128 || up32) && !(tuning_env("B200DM_TMA_EPI") && atoi(tuning_env("B200DM_TMA_EPI")) == 0) &&
-              !(tuning_env("B200DM_CG2") && atoi(tuning_env("B200DM_CG2")) == 0) && !tuning_env("B200DM_NO_UPS");
+              (g.block_n == 64 || g.block_n == 128 || up32);
     if (pl->ups) pl->halo = true;
     // the same on 8 x 8 low-resolution planes (8^3 -> 16^3): pair-slab tiles
     const long long per_pair = (long long)((d->in_d + 1) / 2) * d->batch;
     if (!pl->ups && d->mode == B200DM_CONV_PARITY && d->in_w == 8 && d->in_h == 8 && d->in_d >= 2 && d->in_d % 2 == 0 && d->c_out % 64 == 0 &&
         d->y_dtype == B200DM_BF16 && !residual && !prelu_alpha && d->reserved[1] == 0 && d->use_halo >= 0 && per_pair % 2 == 0 &&
-        (g.block_n == 64 || g.block_n == 128) && !(tuning_env("B200DM_TMA_EPI") && atoi(tuning_env("B200DM_TMA_EPI")) == 0) &&
-        !(tuning_env("B200DM_CG2") && atoi(tuning_env("B200DM_CG2")) == 0) && !tuning_env("B200DM_NO_UPS")) {
+        (g.block_n == 64 || g.block_n == 128)) {
       pl->ups = true; pl->pair = true; pl->halo = true;
-    }
-  }
-  // igemm cluster (see the kernel): cl_n n-tiles share A, cl_m m-tiles share B; B200DM_CLUSTER="m,n" switches it on.
-  int cl_m = 1, cl_n = 1, a_split_dim = 0, a_split_ext = 0;
-  if (!pl->halo && st == 1) {
-    const long long mt = (long long)((g.m_w + g.box_w - 1) / g.box_w) * ((g.m_h + g.box_h - 1) / g.box_h) *
-                         ((g.m_d + g.box_d - 1) / g.box_d) * ((d->batch + g.box_n - 1) / g.box_n);
-    const int nt = d->mode == B200DM_CONV_BATCHED_GEMM ? (d->c_out + g.block_n - 1) / g.block_n : g.n_pad / g.block_n;
-    // Default OFF: measured on B200 (8^3 256->256 conv, 47 us unclustered) 2x1 68 us, 1x2 72 us, 2x2 91 us, 4x2 97 us --
-    // the operand stream is capped by what ONE SM can take from L2 (~40 B/clk), which multicast does not raise at
-    // cluster sizes <= 4, and the cluster-wide stage hand-shake adds latency.  Kept for experiments and tests.
-    int want_m = 1, want_n = 1;
-    if (const char* e = tuning_env("B200DM_CLUSTER")) { if (sscanf(e, "%d,%d", &want_m, &want_n) != 2) { want_m = 1; want_n = 1; } }
-    // B is shared by m-tiles of the same sample only in GEMM mode (x = tile within sample fastest)
-    const long long m_share = d->mode == B200DM_CONV_BATCHED_GEMM ? (g.m_w + g.box_w - 1) / g.box_w : mt;
-    for (cl_m = want_m; cl_m > 1 && (m_share % cl_m != 0 || mt % cl_m != 0 || g.block_n / cl_m < 8); cl_m >>= 1) {}
-    for (cl_n = want_n; cl_n > 1 && nt % cl_n != 0; cl_n >>= 1) {}
-    if (cl_m < 1) cl_m = 1;
-    if (cl_n < 1) cl_n = 1;
-    if (cl_n > 1) {  // split the outermost non-unit box dim of the A tile between the sharers
-      int ext[5] = {0, g.box_w, g.box_h, g.box_d, g.box_n};
-      for (int dim = 4; dim >= 1; --dim)
-        if (ext[dim] > 1) { if (ext[dim] % cl_n == 0) { a_split_dim = dim; a_split_ext = ext[dim] / cl_n; } break; }
-      if (a_split_dim == 0) cl_n = 1;
     }
   }
   auto encodeA = [&](CUtensorMap* m, const void* ptr, int C) -> int {
@@ -998,7 +858,6 @@ extern "C" int b200dm_conv_plan_create(const b200dm_conv_desc* d, const void* x0
       strides[1] = sd; strides[2] = sh;
       box[1] = 10; box[2] = 2; box[3] = 10; box[4] = 1;
     } else if (pl->halo) { box[1] = 10; box[2] = 18; box[3] = 1; box[4] = 1; }   // one halo d-plane slab
-    else if (cl_n > 1) box[a_split_dim] = (cuuint32_t)a_split_ext;          // this CTA's share of the multicast A tile
 
     cuuint32_t es[5] = {1, (cuuint32_t)st, (cuuint32_t)st, (cuuint32_t)st, 1};
     CUresult r = enc(m, kTmapAct16, 5, const_cast<void*>(ptr), dims, strides, box, es,
@@ -1019,7 +878,7 @@ extern "C" int b200dm_conv_plan_create(const b200dm_conv_desc* d, const void* x0
       // (masked by the epilogue's col < c_out), K beyond c0 is zero-filled by TMA.
       dims[0] = (cuuint64_t)d->c0; dims[1] = (cuuint64_t)d->batch * d->c_out; strides[0] = (cuuint64_t)d->c0 * 2;
     }
-    cuuint32_t box[2] = {64, (cuuint32_t)(g.block_n / cl_m)};   // this CTA's share of the multicast B tile
+    cuuint32_t box[2] = {64, (cuuint32_t)g.block_n};
     cuuint32_t es[3] = {1, 1, 1};
     CUresult r;
     if (pl->halo) {
@@ -1064,8 +923,6 @@ extern "C" int b200dm_conv_plan_create(const b200dm_conv_desc* d, const void* x0
   p.bias = bias; p.chan_bias = chan_bias; p.t_dev = t_dev;
   p.residual = (const act_t*)residual; p.prelu_alpha = (const act_t*)prelu_alpha;
   p.y = y; p.dbg = g_dbg_flag;
-  if (const char* e = tuning_env("B200DM_EPI_DBG")) p.epi_dbg = atoi(e);
-  p.cl_m = cl_m; p.cl_n = cl_n; p.a_split_dim = a_split_dim; p.a_split_ext = a_split_ext;
   const long long mtiles = (long long)p.tiles_w * p.tiles_h * p.tiles_d * p.tiles_n;
   if (mtiles > 0x7fffffffLL) { delete pl; b200dm_set_error("conv_plan_create: too many tiles"); return B200DM_ERR_INVALID; }
   const int ntiles = d->mode == B200DM_CONV_BATCHED_GEMM ? (d->c_out + g.block_n - 1) / g.block_n : g.n_pad / g.block_n;
@@ -1073,12 +930,11 @@ extern "C" int b200dm_conv_plan_create(const b200dm_conv_desc* d, const void* x0
   // split-K: when the tile grid leaves most SMs idle and K is long, ksplit CTAs (one cluster) share a tile.  Each CTA
   // streams its K range at the per-SM operand rate (~40 B/clk), so an under-filled grid is K-latency-bound otherwise.
   p.ksplit = 1;
-  if (!pl->halo && cl_m * cl_n == 1 && d->reserved[1] == 0) {
+  if (!pl->halo && d->reserved[1] == 0) {
     const long long ctas = mtiles * ntiles * (d->mode == B200DM_CONV_PARITY ? 8 : 1);
     const int nkb = (g.nch0 + g.nch1) * g.ntaps;
     int ksp = 1;
     while (ksp < 8 && ctas * (ksp * 2) <= b2_num_sms() && nkb / (ksp * 2) >= 13) ksp *= 2;   // >= 13 k-blocks per CTA: 3^3 convs only
-    if (const char* e = tuning_env("B200DM_KSPLIT")) { const int v = atoi(e); if (v >= 1 && v <= 8 && (v & (v - 1)) == 0 && nkb / v >= 1) ksp = v; }
     if (ksp > 1) { p.ksplit = ksp; pl->grid.x = (unsigned)(mtiles * ksp); }
   }
   // pipeline depth 4; measured on B200: a deeper ring (6 stages at BLOCK_N=128, 8 below) does not help at BLOCK_N=128 (the
@@ -1086,23 +942,24 @@ extern "C" int b200dm_conv_plan_create(const b200dm_conv_desc* d, const void* x0
   pl->nstage = 4;
   // short K loops (1^3 convs: 1-3 k-blocks) never fill four stages; two stages let 3-4 CTAs share an SM, which hides the
   // per-CTA prologue / TMA latency / epilogue of these HBM-bound launches
-  if ((g.nch0 + g.nch1) * g.ntaps <= 3 && g.block_n >= 64 && cl_m * cl_n == 1 && !tuning_env("B200DM_IGEMM_NO2")) pl->nstage = 2;
+  if ((g.nch0 + g.nch1) * g.ntaps <= 3 && g.block_n >= 64) pl->nstage = 2;
   // grids of several waves: two stages x three co-resident CTAs keep more operand bytes in flight per SM than one CTA with
   // four stages, and hide every CTA's prologue / epilogue (measured: 16^3 128->128 parity conv 123 -> 77 us, 8^3 MLP GEMM
   // 17.5 -> 12.7 us; a single-wave split-K grid gets slower, so it keeps four stages)
-  if (!pl->halo && (long long)pl->grid.x * pl->grid.y * pl->grid.z >= 2LL * b2_num_sms() && g.block_n >= 64 && p.ksplit <= 1 &&
-      cl_m * cl_n == 1 && !tuning_env("B200DM_IGEMM_NO2"))
+  if (!pl->halo && (long long)pl->grid.x * pl->grid.y * pl->grid.z >= 2LL * b2_num_sms() && g.block_n >= 64 && p.ksplit <= 1)
     pl->nstage = 2;
-  if (const char* e = tuning_env("B200DM_IGEMM_STAGES")) { if (atoi(e) == 2 && g.block_n >= 64 && cl_m * cl_n == 1) pl->nstage = 2; if (atoi(e) == 4) pl->nstage = 4; }
+  // split-K needs >= 26 k-blocks, the first two-stage rule <= 3: the split-K kernel is instantiated with four stages only
+  if (p.ksplit > 1 && pl->nstage != 4) {
+    delete pl; b200dm_set_error("conv_plan_create: internal: split-K plan with two stages"); return B200DM_ERR_UNSUPPORTED;
+  }
   // staged (TMA-store) epilogue of the per-tap GEMM kernel: bf16 NDHWC output with whole 64-channel groups
   memset(&pl->om, 0, sizeof(pl->om));
   {
     const bool f32 = d->y_dtype == B200DM_F32;   // fp32 output (the U-Net's eps): halo kernel only, 32-column groups
     // (halo kernel, C_out = 32: one 32-channel group of 64-byte rows, SWIZZLE_64B -- the decoders' 128^3 convs)
     const bool n32 = pl->halo && !pl->pair && d->c_out == 32 && g.block_n == 32 && !f32 && (pl->ups || d->mode == B200DM_CONV_DIRECT);
-    bool want = cl_m * cl_n == 1 && (!f32 || pl->halo) && d->reserved[1] == 0 && !prelu_alpha &&
-                ((d->c_out % 64 == 0 && g.block_n >= 64) || n32) && !(d->mode == B200DM_CONV_PARITY && residual);
-    if (const char* e = tuning_env("B200DM_TMA_EPI")) { if (atoi(e) == 0) want = false; }
+    const bool want = (!f32 || pl->halo) && d->reserved[1] == 0 && !prelu_alpha &&
+                      ((d->c_out % 64 == 0 && g.block_n >= 64) || n32) && !(d->mode == B200DM_CONV_PARITY && residual);
     if (want) {
       const int par = d->mode == B200DM_CONV_PARITY ? 8 : 1;
       const int ps = d->mode == B200DM_CONV_PARITY ? 2 : 1;   // output voxel stride of one M-space step
@@ -1136,10 +993,9 @@ extern "C" int b200dm_conv_plan_create(const b200dm_conv_desc* d, const void* x0
     }
   }
   // per-sample transposed store by operand swap (see the kernel): tiles of whole planes inside one sample, bias only
-  if (d->reserved[1] != 0 && !pl->halo && cl_m * cl_n == 1 && d->mode == B200DM_CONV_DIRECT && d->ksize == 1 && st == 1 &&
+  if (d->reserved[1] != 0 && !pl->halo && d->mode == B200DM_CONV_DIRECT && d->ksize == 1 && st == 1 &&
       d->y_dtype == B200DM_BF16 && g.block_n == 128 && g.box_n == 1 && g.box_w == g.m_w && g.box_h == g.m_h && g.m_d % g.box_d == 0 &&
-      !residual && !prelu_alpha && !chan_bias && d->act == B200DM_ACT_NONE && d->reserved[0] == B200DM_ACT_NONE &&
-      !(tuning_env("B200DM_TMA_EPI") && atoi(tuning_env("B200DM_TMA_EPI")) == 0)) {
+      !residual && !prelu_alpha && !chan_bias && d->act == B200DM_ACT_NONE && d->reserved[0] == B200DM_ACT_NONE) {
     const cuuint64_t Lv = (cuuint64_t)g.m_w * g.m_h * g.m_d;
     cuuint64_t dims[5] = {Lv, (cuuint64_t)d->c_out, 1, 1, (cuuint64_t)d->batch};
     cuuint64_t strides[4] = {Lv * 2, Lv * d->c_out * 2, Lv * d->c_out * 2, Lv * d->c_out * 2};
@@ -1156,7 +1012,7 @@ extern "C" int b200dm_conv_plan_create(const b200dm_conv_desc* d, const void* x0
   // BLOCK_N = 128 with the staged epilogue: one-tap weight stages hold only 8 MMAs (4 per issuer warp) and the per-stage
   // barrier round trip (~200 cycles) made those convs issue-bound (45 % of the MMA floor); 3-tap stages x 2 fit once the
   // slab ring is the 4 slabs a channel chunk needs (the next chunk's slab i reloads as soon as slab i is released).
-  if (pl->halo && !pl->pair && g.block_n == 128 && p.tma_epi && !tuning_env("B200DM_NO_WIDE")) {
+  if (pl->halo && !pl->pair && g.block_n == 128 && p.tma_epi) {
     cuuint64_t dims3[3] = {64, (cuuint64_t)g.n_pad, (cuuint64_t)(g.ktot / 64)};
     cuuint64_t strides3[2] = {(cuuint64_t)g.ktot * 2, 128};
     cuuint32_t box3[3] = {64, 128, 3};
@@ -1166,15 +1022,12 @@ extern "C" int b200dm_conv_plan_create(const b200dm_conv_desc* d, const void* x0
             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS) { delete pl; b200dm_set_error("cuTensorMapEncodeTiled(B wide) failed"); return B200DM_ERR_CUDA; }
     pl->wide = true; pl->halo_nb = 2; pl->halo_tps = 3;
   }
-  // CTA pairs (cta_group::2) for every staged halo configuration with 64- or 128-channel tiles: needs an even tile count per
-  // n-tile so that the two CTAs of a pair always work on the same n-tile and run the same number of tiles
-  // the U-Net's input conv (256 -> 32, direct stores).  Short-K N=32 convs (the decoder's 32 -> 32 at 128^3) are bound by their
-  // direct-store epilogue; pairing them only couples two epilogues (measured 4.18 -> 4.79 ms), so they stay single-CTA.
-  // With the SWIZZLE_64B staged epilogue (n32 above) those convs run 3.78 ms, paired or not gated on tma_epi any more.
-  const bool cg2_short = p.tma_epi && tuning_env("B200DM_CG2_N32S") && atoi(tuning_env("B200DM_CG2_N32S")) != 0;   // experiment: pair short-K staged N=32 convs too
-  const bool cg2_n32 = g.block_n == 32 && !pl->pair && !pl->ups && pl->halo_td == 2 && !p.y2 && (g.nch0 + g.nch1 >= 2 || cg2_short);
-  if (pl->halo && (((g.block_n == 64 || g.block_n == 128) && p.tma_epi && (pl->pair || pl->halo_td == 2 || g.block_n == 128)) || cg2_n32) &&
-      !(tuning_env("B200DM_CG2") && atoi(tuning_env("B200DM_CG2")) == 0)) {
+  // CTA pairs (cta_group::2) for every staged halo configuration with 64- or 128-channel tiles, and for N = 32 convs with at
+  // least two channel chunks (the U-Net's input conv, 256 -> 32, direct stores): needs an even tile count per n-tile so that the
+  // two CTAs of a pair always work on the same n-tile and run the same number of tiles.  Short-K N = 32 convs (one channel chunk)
+  // stay single-CTA: with direct stores pairing couples two epilogues (measured 4.18 -> 4.79 ms), staged it gained 3.79 -> 3.74 ms only.
+  const bool cg2_n32 = g.block_n == 32 && !pl->pair && !pl->ups && pl->halo_td == 2 && g.nch0 + g.nch1 >= 2;
+  if (pl->halo && (((g.block_n == 64 || g.block_n == 128) && p.tma_epi && (pl->pair || pl->halo_td == 2 || g.block_n == 128)) || cg2_n32)) {
     const int td = pl->halo_td;   // (pair: d step 2)
     const long long per = (long long)((d->in_w + 7) / 8) * (pl->pair ? (d->in_h + 7) / 8 : (d->in_h + 15) / 16) * ((d->in_d + td - 1) / td) * d->batch;
     if (per % 2 == 0) {
@@ -1270,15 +1123,23 @@ extern "C" int b200dm_conv_plan_run(b200dm_conv_plan* pl, void* stream) {
   }
   if (pl->nstage == 2) {
     switch (pl->g.block_n) {
-      case 64: return launch_conv<64, 2>(pl, s);
-      case 128: return launch_conv<128, 2>(pl, s);
+      case 64: return launch_conv<64, 2, false>(pl, s);
+      case 128: return launch_conv<128, 2, false>(pl, s);
     }
-  }
-  switch (pl->g.block_n) {
-    case 16: return launch_conv<16, 4>(pl, s);
-    case 32: return launch_conv<32, 4>(pl, s);
-    case 64: return launch_conv<64, 4>(pl, s);
-    case 128: return launch_conv<128, 4>(pl, s);
+  } else if (pl->p.ksplit > 1) {
+    switch (pl->g.block_n) {
+      case 16: return launch_conv<16, 4, true>(pl, s);
+      case 32: return launch_conv<32, 4, true>(pl, s);
+      case 64: return launch_conv<64, 4, true>(pl, s);
+      case 128: return launch_conv<128, 4, true>(pl, s);
+    }
+  } else {
+    switch (pl->g.block_n) {
+      case 16: return launch_conv<16, 4, false>(pl, s);
+      case 32: return launch_conv<32, 4, false>(pl, s);
+      case 64: return launch_conv<64, 4, false>(pl, s);
+      case 128: return launch_conv<128, 4, false>(pl, s);
+    }
   }
   b200dm_set_error("conv_plan_run: unsupported BLOCK_N %d", pl->g.block_n);
   return B200DM_ERR_UNSUPPORTED;
@@ -1295,18 +1156,6 @@ extern "C" int b200dm_conv_plan_set_trace(b200dm_conv_plan* p, void* trace) {
 
 extern "C" double b200dm_conv_plan_flops(const b200dm_conv_plan* p) { return p ? p->flops : 0.0; }
 
-extern "C" int b200dm_conv_plan_add_output(b200dm_conv_plan* p, void* y_extra, const float* scale, const float* shift, int32_t act) {
-  B2_CHECK_ARG(p && y_extra && scale && shift, "conv_plan_add_output: null argument");
-  B2_CHECK_ARG(p->desc.c_out % 16 == 0 && p->desc.reserved[1] == 0, "conv_plan_add_output: needs c_out %% 16 == 0 and a plain (non-transposed) store");
-  B2_CHECK_ARG(((uintptr_t)y_extra & 15) == 0 && ((uintptr_t)scale & 15) == 0 && ((uintptr_t)shift & 15) == 0, "conv_plan_add_output: pointers must be 16-byte aligned");
-  if (p->pair || p->wide || p->cg2 || p->stencil || p->sweep) { b200dm_set_error("conv_plan_add_output: not available on pair-slab / wide-stage halo / stencil plans"); return B200DM_ERR_UNSUPPORTED; }
-  if (p->p.tma_epi) { p->p.tma_epi = 0; p->smem = p->halo ? halo_smem_bytes(p) : conv_smem_bytes(p->g.block_n, p->nstage, false); }
-  if (!p->p.y2) { p->p.y2 = (act_t*)y_extra; p->p.scale2 = scale; p->p.shift2 = shift; p->p.act2 = act; }
-  else if (!p->p.y3) { p->p.y3 = (act_t*)y_extra; p->p.scale3 = scale; p->p.shift3 = shift; p->p.act3 = act; }
-  else { b200dm_set_error("conv_plan_add_output: at most two extra outputs"); return B200DM_ERR_UNSUPPORTED; }
-  return B200DM_OK;
-}
-
 extern "C" int b200dm_conv_plan_set_fused_update(b200dm_conv_plan* pl, const b200dm_update_desc* u, const float* x_t, float* x_prev,
                                                  void* x_prev_16) {
   B2_CHECK_ARG(pl && u && x_t && x_prev && x_prev_16, "conv_plan_set_fused_update: null argument");
@@ -1314,7 +1163,7 @@ extern "C" int b200dm_conv_plan_set_fused_update(b200dm_conv_plan* pl, const b20
   const ConvParams& p = pl->p;
   // the CTA-pair N = 128 halo kernel with the fp32 staged epilogue, no other epilogue term
   if (!(pl->halo && pl->cg2 && !pl->pair && !pl->ups && !pl->sweep && !pl->stencil && pl->g.block_n == 128 &&
-        p.y_f32 && p.tma_epi && d->c_out % 128 == 0 && !p.residual && !p.prelu_alpha && !p.y2 && p.act == B200DM_ACT_NONE &&
+        p.y_f32 && p.tma_epi && d->c_out % 128 == 0 && !p.residual && !p.prelu_alpha && p.act == B200DM_ACT_NONE &&
         p.post_act == B200DM_ACT_NONE)) {
     b200dm_set_error("conv_plan_set_fused_update: only on the CTA-pair fp32-output 3^3 conv with C_out %% 128 == 0");
     return B200DM_ERR_UNSUPPORTED;
@@ -1348,34 +1197,6 @@ extern "C" int b200dm_conv_plan_set_fused_update(b200dm_conv_plan* pl, const b20
   pl->fuse = true;
   pl->smem = halo_smem_bytes(pl);
   if (pl->smem > 232448) { b200dm_set_error("conv_plan_set_fused_update: shared memory"); return B200DM_ERR_UNSUPPORTED; }
-  return B200DM_OK;
-}
-
-extern "C" int b200dm_conv_plan_set_side_norm(b200dm_conv_plan* pl, void* y_side, const float* scale, const float* shift, int32_t act) {
-  B2_CHECK_ARG(pl && y_side && scale && shift, "conv_plan_set_side_norm: null argument");
-  const b200dm_conv_desc* d = &pl->desc;
-  const int C = d->c0 + d->c1;
-  if (pl->halo || pl->stencil || !pl->p.tma_epi || pl->p.swap_ab || pl->p.ksplit > 1 || pl->p.cl_m * pl->p.cl_n != 1 || d->mode != B200DM_CONV_DIRECT ||
-      d->ksize != 1 || d->stride != 1 || pl->g.block_n < 64 || (d->c1 > 0 && d->c0 % 64 != 0) || C % 8 != 0 || C > 1024 ||
-      ((uintptr_t)y_side & 15) != 0) {
-    b200dm_set_error("conv_plan_set_side_norm: only on staged 1^3 stride-1 convs (c0 %% 64 == 0 when c1 > 0)");
-    return B200DM_ERR_UNSUPPORTED;
-  }
-  EncodeTiledFn enc = get_encode_fn();
-  cuuint64_t dims[5] = {(cuuint64_t)C, (cuuint64_t)d->in_w, (cuuint64_t)d->in_h, (cuuint64_t)d->in_d, (cuuint64_t)d->batch};
-  cuuint64_t strides[4] = {(cuuint64_t)C * 2, (cuuint64_t)d->in_w * C * 2, (cuuint64_t)d->in_h * d->in_w * C * 2,
-                           (cuuint64_t)d->in_d * d->in_h * d->in_w * C * 2};
-  cuuint32_t box[5] = {64, (cuuint32_t)pl->g.box_w, (cuuint32_t)pl->g.box_h, (cuuint32_t)pl->g.box_d, (cuuint32_t)pl->g.box_n};
-  cuuint32_t es[5] = {1, 1, 1, 1, 1};
-  if (!enc || enc(&pl->om.s, kTmapAct16, 5, y_side, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                  CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS) {
-    b200dm_set_error("conv_plan_set_side_norm: cuTensorMapEncodeTiled failed");
-    return B200DM_ERR_CUDA;
-  }
-  const size_t smem = conv_smem_bytes(pl->g.block_n, pl->nstage, pl->p.residual != nullptr, C);
-  if (smem > conv_smem_attr(pl->g.block_n, pl->nstage)) { b200dm_set_error("conv_plan_set_side_norm: shared memory"); return B200DM_ERR_UNSUPPORTED; }
-  pl->smem = smem;
-  pl->p.side = 1; pl->p.side_act = act; pl->p.side_c = C; pl->p.side_scale = scale; pl->p.side_shift = shift;
   return B200DM_OK;
 }
 
@@ -1423,16 +1244,5 @@ extern "C" int b200dm_gn_finalize(const float* partials, int32_t batch, int32_t 
   const double count = (double)voxels_per_sample * (c / groups);
   B2_CHECK_CUDA(b2_launch(sweep::gn_finalize_kernel, dim3((unsigned)(batch * groups)), dim3(128), 0, (cudaStream_t)stream, partials,
                           rows_per_sample, 1, c, groups, count, eps, mean_rstd));
-  return B200DM_OK;
-}
-
-// Fold the consumer-side GroupNorm + activation into the conv's operand path (d-sweeping kernel only): the conv then computes
-// conv(act(gamma * (x - mean) * rstd + beta)) from the RAW x, mean / rstd per (sample, group) read from `mean_rstd` at run time.
-extern "C" int b200dm_conv_plan_set_input_norm(b200dm_conv_plan* p, const float* mean_rstd, const float* gamma, const float* beta,
-                                               int32_t groups, int32_t act) {
-  B2_CHECK_ARG(p && mean_rstd && gamma && beta, "conv_plan_set_input_norm: null argument");
-  if (!p->sweep) { b200dm_set_error("conv_plan_set_input_norm: this plan's kernel has no input transform"); return B200DM_ERR_UNSUPPORTED; }
-  B2_CHECK_ARG(groups > 0 && 32 % groups == 0, "conv_plan_set_input_norm: groups must divide 32");
-  p->wp.in_mr = mean_rstd; p->wp.in_gamma = gamma; p->wp.in_beta = beta; p->wp.in_groups = groups; p->wp.in_act = act;
   return B200DM_OK;
 }

@@ -18,16 +18,8 @@ struct ConvParams {
   int chan_bias_rows;
   int halo_td, halo_tiles_per_ntile, halo_ntn, halo_total_tiles;   // halo kernel only
   int tma_epi;                       // staged epilogue: bf16 tile -> swizzled smem -> TMA store (residual tile TMA-loaded)
-  // side output of a 1^3 conv (ResidualBlock shortcut): act(side_scale[c] * x + side_shift[c]) of the conv's own INPUT
-  // channels (both K segments, concatenated), written while the A tiles sit in shared memory -- the block's norm1 +
-  // swish pass (dm3d.py:235-236) without a second read of x / skip
-  int side, side_act, side_c;
-  const float* side_scale; const float* side_shift;
   int swap_ab;                       // transposed store by operand swap: D^T = W X^T (TMEM lane = channel, column = voxel)
-  int epi_dbg;                       // tuning aid (B200DM_EPI_DBG): 1 = skip global stores, 2 = skip TMEM loads too
   int ksplit;                        // igemm split-K: cluster of ksplit CTAs per tile, each owns a K range (0/1 = off)
-  int cl_m, cl_n;                    // igemm cluster: cl_m m-tiles share every B tile, cl_n n-tiles share every A tile
-  int a_split_dim, a_split_ext;      // A box is split over the cl_n sharers along box dim a_split_dim (1=w..4=n), ext per part
   const float* bias;
   const float* out_scale;            // optional per-channel affine applied after the bias adds (a folded BatchNorm of the
   const float* out_shift;            // CONSUMER: y = act(scale * (acc + bias + temb) + shift)), fp32[c_out]
@@ -36,11 +28,6 @@ struct ConvParams {
   const act_t* residual;
   const act_t* prelu_alpha;  // (d,h,w,c) bf16, no batch dim
   void* y;
-  // up to two EXTRA bf16 outputs of the same shape: y_k = act_k(scale_k[co] * v + shift_k[co]) of the final value v --
-  // the folded BatchNorm (+ swish) of the tensor's consumers, written by the producer so that no separate
-  // normalisation pass ever re-reads the tensor
-  act_t* y2; const float* scale2; const float* shift2; int act2;
-  act_t* y3; const float* scale3; const float* shift3; int act3;
   int* dbg;
   long long* trace;                  // optional per-role clock64 timeline of CTA 0 (tuning aid), else nullptr
   // fused reverse-diffusion update (the U-Net's output conv on the sampling graph, b200dm_conv_plan_set_fused_update): the
@@ -55,7 +42,6 @@ struct ConvParams {
 struct ConvOutMaps {
   CUtensorMap y[8];
   CUtensorMap r;
-  CUtensorMap s;   // side output (see ConvParams::side)
 };
 
 // timeline regions (each kTraceRegion entries): 0 = MMA issuer, 1 = epilogue warp 4, 2 = slab producer, 3 = weight producer
@@ -68,21 +54,6 @@ __device__ __forceinline__ void trace_ev(const ConvParams& p, int region, int& i
 }
 
 __device__ __forceinline__ float bf(const act_t v) { return act_to_float(v); }
-
-// one extra normalised copy of 16 channels: act(scale * v + shift) -> bf16
-__device__ __forceinline__ void extra_output16(const float (&v)[16], act_t* yo, const float* sc, const float* sh, int act) {
-  float w[16];
-#pragma unroll
-  for (int j = 0; j < 16; j += 4) {
-    const float4 a = __ldg(reinterpret_cast<const float4*>(sc + j)), b = __ldg(reinterpret_cast<const float4*>(sh + j));
-    w[j] = fmaf(a.x, v[j], b.x); w[j + 1] = fmaf(a.y, v[j + 1], b.y); w[j + 2] = fmaf(a.z, v[j + 2], b.z); w[j + 3] = fmaf(a.w, v[j + 3], b.w);
-  }
-  if (act != B200DM_ACT_NONE) {
-    apply_act_vec(w, act);
-  }
-  *reinterpret_cast<bf16x8*>(yo) = pack8(*reinterpret_cast<float(*)[8]>(&w[0]));
-  *reinterpret_cast<bf16x8*>(yo + 8) = pack8(*reinterpret_cast<float(*)[8]>(&w[8]));
-}
 
 // Epilogue for 16 consecutive accumulator columns of one output voxel (thread = TMEM lane = GEMM row):
 //   + bias[co] + chan_bias[t][n][co]  ->  * out_scale[co] + out_shift[co]  ->  PReLU(alpha[voxel][co])  ->  act  ->
@@ -157,8 +128,6 @@ __device__ __forceinline__ void conv_epilogue16(const ConvParams& p, const uint3
       *reinterpret_cast<bf16x8*>(yo) = pack8(*reinterpret_cast<float(*)[8]>(&v[0]));
       *reinterpret_cast<bf16x8*>(yo + 8) = pack8(*reinterpret_cast<float(*)[8]>(&v[8]));
     }
-    if (p.y2) extra_output16(v, p.y2 + row_off + col0, p.scale2 + col0, p.shift2 + col0, p.act2);
-    if (p.y3) extra_output16(v, p.y3 + row_off + col0, p.scale3 + col0, p.shift3 + col0, p.act3);
   } else {
     // scalar path: ragged channel tail (e.g. C_out = 1) or per-sample transposed store
 #pragma unroll

@@ -509,12 +509,10 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constan
             const int col0 = colt + c * 16;
             if (col0 >= p.c_out) break;
             uint32_t ra[16], rb[16];
-            if (p.epi_dbg < 2) {
-              ptx::tc_ld_32x32b_x16(taddr + c * 16, ra);
-              if (c + 1 < kChunks) ptx::tc_ld_32x32b_x16(taddr + c * 16 + 16, rb);
-              ptx::tc_wait_ld();
-            }
-            if (valid && p.epi_dbg == 0) {
+            ptx::tc_ld_32x32b_x16(taddr + c * 16, ra);
+            if (c + 1 < kChunks) ptx::tc_ld_32x32b_x16(taddr + c * 16 + 16, rb);
+            ptx::tc_wait_ld();
+            if (valid) {
               conv_epilogue16(p, ra, col0, t.n, vox, vox_per, row_off, has_bs ? bs + cbase + c * 16 : nullptr, nullptr,
                               has_sc ? scs + cbase + c * 16 : nullptr, pre ? rpre[pl][c] : nullptr);
               if (c + 1 < kChunks && col0 + 16 < p.c_out)

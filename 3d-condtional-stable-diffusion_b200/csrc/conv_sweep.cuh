@@ -15,9 +15,9 @@
 // window {p+1, p, p-1} is ascending and contiguous except when it wraps (2 of R planes: two MMAs then).  A plane's first
 // contribution (kd = 0, tap 0, k-step 0) is issued with accumulate = 0 on its own, so no slot is ever zeroed by hand.
 //
-// Warps (768 threads): 0 slab producer, 1 weight loader, 1 + 3 optional input transform (GroupNorm apply + SiLU on the landed
-// slab, in place; warps 20-23 help), 2 TMEM owner + MMA issuer, 4-11 / 12-19 two epilogue
-// groups that take alternate planes (an epilogue pass is ~1.5 k cycles of latency, the MMAs of a plane ~1.0 k).
+// Warps (640 threads): 0 slab producer, 1 weight loader, 2 TMEM owner + MMA issuer, 3 idle (the epilogue warps must start at 4:
+// TMEM lane quarter = warp % 4), 4-11 / 12-19 two epilogue groups that take alternate planes (an epilogue pass is ~1.5 k cycles of
+// latency, the MMAs of a plane ~1.0 k).
 // Input planes are staged and issued in PAIRS (one TMA box of two planes): the issuing thread's per-iteration bookkeeping
 // (barrier waits, commits, index arithmetic: ~600 cycles, not overlapped because the tcgen05 queue is shallow) is paid once per two planes.
 #pragma once
@@ -25,7 +25,7 @@
 
 namespace sweep {
 
-constexpr int kThreads = 768;               // 24 warps: 80 registers per thread
+constexpr int kThreads = 640;               // 20 warps
 constexpr int kC = 32;
 constexpr int kPlaneBytes = 180 * 64;       // one input plane of the column: 10 x 18 voxels x 64 B
 constexpr int kSlabTx = 2 * kPlaneBytes;    // a slab = TWO consecutive input planes (one TMA box {32, 10, 18, 2, 1}): one barrier round
@@ -34,19 +34,13 @@ constexpr int kNS = 3;                      // slab ring
 constexpr int kR = 16;                      // TMEM ring: 16 slots x 32 columns = 512 columns
 constexpr int kWBytes = 27 * 2048;          // [kh*3+kw][kd][32 co][32 ci] bf16, one 2 KB SWIZZLE_64B tile per tap
 constexpr int kStgBytes = 8192;             // one plane tile: 128 rows x 64 B
-constexpr size_t kSmem = 1024 + (size_t)kNS * kSlabBytes + kWBytes + 4 * kStgBytes + (3 * kNS + 1 + 2 * kR + 2) * 8 + 16 + 2 * 32 * 4 +
+constexpr size_t kSmem = 1024 + (size_t)kNS * kSlabBytes + kWBytes + 4 * kStgBytes + (2 * kNS + 1 + 2 * kR + 2) * 8 + 8 + 2 * 32 * 4 +
                          2 * 4 * 2 * 32 * 4;
 
 struct Params {
   int D, H, W, batch;
   int tiles_w, tiles_h, dsplit, dlen, items;
   float* gn_part;   // optional [items][2 groups][32 channels][2] partial (sum, sum of squares) of the STORED values, else null
-  // optional input transform: the conv reads act(GroupNorm(x)) -- x stays raw in HBM, the normalisation runs on the slab in shared
-  // memory (vqgan_attn_cp.py:262-270: GN -> SiLU -> Conv3D), so the separate normalisation pass over the tensor disappears
-  const float* in_mr;      // (batch, in_groups, 2) mean / rstd, else null
-  const float* in_gamma;   // (32)
-  const float* in_beta;    // (32)
-  int in_groups, in_act;
 };
 
 struct Item { int n, h0, w0, d0, d1; };
@@ -70,21 +64,6 @@ __device__ __forceinline__ void tma_load_3d(uint32_t dst, const CUtensorMap* m, 
 __device__ __forceinline__ void group_bar_sync(int g) { asm volatile("bar.sync %0, 256;" ::"r"(g + 1) : "memory"); }
 
 constexpr uint64_t kLayoutSw64 = 4;
-
-// activation of the input transform.  bf16 storage: SiLU as h + h * tanh(h), h = x / 2 -- ONE MUFU op (tanh.approx, relative error
-// 2^-11, a quarter of a bf16 ulp) instead of ex2 + rcp: the transform is MUFU-bound.  fp16 storage keeps the exact form.
-__device__ __forceinline__ float xform_act(float x, int act) {
-#ifndef B200DM_ACT_FP16
-  if (act == B200DM_ACT_SILU) {
-    const float h = 0.5f * x;
-    float t;
-    asm("tanh.approx.f32 %0, %1;" : "=f"(t) : "f"(h));
-    return fmaf(h, t, h);
-  }
-#endif
-  return apply_act(x, act);
-}
-
 
 constexpr uint32_t kIdesc32 = ptx::make_idesc_act(128, 32), kIdesc64 = ptx::make_idesc_act(128, 64), kIdesc96 = ptx::make_idesc_act(128, 96);
 __host__ __device__ constexpr uint32_t idesc_of(int nkd) { return nkd == 1 ? kIdesc32 : (nkd == 2 ? kIdesc64 : kIdesc96); }
@@ -132,8 +111,8 @@ conv_sweep32_kernel(const __grid_constant__ CUtensorMap mapX, const __grid_const
   uint8_t* w_s = smem + kNS * kSlabBytes;
   uint8_t* stg_base = w_s + kWBytes;                     // [group][2 buffers][8 KB]
   uint64_t* bars = reinterpret_cast<uint64_t*>(stg_base + 4 * kStgBytes);
-  uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(bars + 3 * kNS + 1 + 2 * kR + 2);
-  float* bias_s = reinterpret_cast<float*>(tmem_ptr_smem + 4);   // [bias | scale][32]
+  uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(bars + 2 * kNS + 1 + 2 * kR + 2);
+  float* bias_s = reinterpret_cast<float*>(tmem_ptr_smem + 2);   // [bias | scale][32] (16-byte aligned)
   float* red_s = bias_s + 64;                                     // [group][quarter][half][16 columns][2]
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -143,16 +122,13 @@ conv_sweep32_kernel(const __grid_constant__ CUtensorMap mapX, const __grid_const
   const uint32_t w_full = bar_base + 8u * (2 * kNS);
   auto acc_full = [&](int s) { return bar_base + 8u * (2 * kNS + 1 + s); };
   auto acc_empty = [&](int s) { return bar_base + 8u * (2 * kNS + 1 + kR + s); };
-  auto slab_ready = [&](int s) { return bar_base + 8u * (2 * kNS + 1 + 2 * kR + s); };   // input transform done (6 warps)
-  auto res_bar = [&](int g) { return bar_base + 8u * (3 * kNS + 1 + 2 * kR + g); };   // residual tile of epilogue group g has landed
-  const bool xform = q.in_mr != nullptr;
+  auto res_bar = [&](int g) { return bar_base + 8u * (2 * kNS + 1 + 2 * kR + g); };   // residual tile of epilogue group g has landed
 
   pdl_launch_dependents();
   if (threadIdx.x == 0) {
     for (int s = 0; s < kNS; ++s) { ptx::mbar_init(slab_full(s), 1); ptx::mbar_init(slab_empty(s), 1); }
     ptx::mbar_init(w_full, 1);
     for (int s = 0; s < kR; ++s) { ptx::mbar_init(acc_full(s), 1); ptx::mbar_init(acc_empty(s), 8); }
-    for (int s = 0; s < kNS; ++s) ptx::mbar_init(slab_ready(s), 6);
     ptx::mbar_init(res_bar(0), 1); ptx::mbar_init(res_bar(1), 1);
     ptx::fence_barrier_init();
     ptx::prefetch_tmap(&mapX);
@@ -192,89 +168,14 @@ conv_sweep32_kernel(const __grid_constant__ CUtensorMap mapX, const __grid_const
         if (++s == kNS) { s = 0; ph ^= 1; }
       }
     }
-  } else if (warp == 1 || warp == 3 || warp >= 20) {
+  } else if (warp == 1) {
     // ===================== weights: 27 tiles of [32 co][32 ci], resident for the whole launch =====================
-    if (warp == 1) {
-      if (ptx::elect_one()) {
-        ptx::mbar_expect_tx(w_full, kWBytes);
-        for (int kd = 0; kd < 3; ++kd)
-          for (int k9 = 0; k9 < 9; ++k9) tma_load_3d(w_base + (k9 * 3 + kd) * 2048, &mapW, w_full, 0, 0, kd * 9 + k9);
-      }
-      __syncwarp();
+    if (ptx::elect_one()) {
+      ptx::mbar_expect_tx(w_full, kWBytes);
+      for (int kd = 0; kd < 3; ++kd)
+        for (int k9 = 0; k9 < 9; ++k9) tma_load_3d(w_base + (k9 * 3 + kd) * 2048, &mapW, w_full, 0, 0, kd * 9 + k9);
     }
-    // ===================== input transform (optional): act(a[c] * x + b[c]) on every landed slab, in place =====================
-    // 192 threads (warps 1, 3, 20-23); thread = (row group, 16-byte chunk): it keeps ONE channel octet, so its 16 coefficients live
-    // in registers; 8 rows per thread and slab, loads issued before any use (the per-row chain LDS -> FMA -> ex2 -> rcp -> STS is
-    // ~500 cycles of latency: two warps working row by row made the conv 2.7x slower).  Rows outside the volume stay zero ('same'
-    // padding pads the NORMALISED tensor).  Same arithmetic as norm_act_kernel.
-    if (xform) {
-      // 8 virtual warps of work, dealt so that every SM sub-partition (warp % 4) carries a quarter: the MUFU unit (ex2 / rcp / tanh,
-      // 4 lanes per clock and sub-partition) is the transform's bottleneck.  Warps 20 / 22 are alone on sub-partitions 0 / 2 and take
-      // two virtual warps each; 1 + 21 and 3 + 23 share sub-partitions 1 / 3.  ch (the channel octet) = lane & 3 for all of them.
-      const int v_lo = warp == 20 ? 0 : (warp == 22 ? 2 : (warp == 1 ? 4 : (warp == 21 ? 5 : (warp == 3 ? 6 : 7))));
-      const int v_hi = v_lo + ((warp == 20 || warp == 22) ? 2 : 1);
-      const int ch = lane & 3;
-      uint32_t s = 0, ph = 0;
-      bool ok = true;
-      int cur_n = -1, tix = 0;
-      float a[8], b[8];
-      for (int item = blockIdx.x; item < q.items && ok; item += gridDim.x) {
-        const Item it = decode(q, item);
-        if (it.n != cur_n) {
-          cur_n = it.n;
-          const int cpg = kC / q.in_groups;
-#pragma unroll
-          for (int j = 0; j < 8; ++j) {
-            const int c = ch * 8 + j, g = c / cpg;
-            const float m = __ldg(q.in_mr + ((size_t)it.n * q.in_groups + g) * 2), r = __ldg(q.in_mr + ((size_t)it.n * q.in_groups + g) * 2 + 1);
-            a[j] = r * __ldg(q.in_gamma + c);
-            b[j] = __ldg(q.in_beta + c) - m * a[j];
-          }
-        }
-        for (int pl = it.d0 - 1; pl <= it.d1 && ok; pl += 2) {
-          if (warp == 1 && lane == 0) trace_ev(p, 3, tix, 30);
-          ok = ptx::mbar_wait_sleep(slab_full(s), ph, p.dbg, 0x5306);
-          if (!ok) break;
-          if (warp == 1 && lane == 0) trace_ev(p, 3, tix, 31);
-          const uint32_t sb = slab_base + s * kSlabBytes;
-#pragma unroll 1
-          for (int vk = v_lo * 6; vk < v_hi * 6; vk += 2) {   // (virtual warp, 64-row step); two rows in flight per thread: more would
-            uint32_t addr[2];                                 // not leave registers for the per-element chains
-            uint4 u[2];
-#pragma unroll
-            for (int k = 0; k < 2; ++k) {
-              const int v = (vk + k) / 6, rr = v * 8 + (lane >> 2) + 64 * ((vk + k) - v * 6);
-              const int pp = rr >= 180 ? 1 : 0, r = rr - pp * 180, hh = r / 10, ww = r - hh * 10;
-              const int d = pl + pp, h = it.h0 - 1 + hh, w = it.w0 - 1 + ww;
-              const bool live = rr < 360 && d >= 0 && d < q.D && h >= 0 && h < q.H && w >= 0 && w < q.W;
-              const uint32_t row = sb + pp * kPlaneBytes + r * 64;
-              addr[k] = live ? row + (((uint32_t)ch ^ ((row >> 7) & 3u)) << 4) : 0u;   // SWIZZLE_64B on the absolute address
-              if (live) asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(u[k].x), "=r"(u[k].y), "=r"(u[k].z), "=r"(u[k].w) : "r"(addr[k]));
-            }
-#pragma unroll
-            for (int k = 0; k < 2; ++k) {
-              if (addr[k] == 0u) continue;
-              bf16x8 v8;
-              memcpy(&v8, &u[k], 16);
-              float f[8];
-              unpack8(v8, f);
-#pragma unroll
-              for (int j = 0; j < 8; ++j) f[j] = xform_act(fmaf(f[j], a[j], b[j]), q.in_act);
-              v8 = pack8(f);
-              uint4 o;
-              memcpy(&o, &v8, 16);
-              asm volatile("st.shared.v4.u32 [%4], {%0, %1, %2, %3};" ::"r"(o.x), "r"(o.y), "r"(o.z), "r"(o.w), "r"(addr[k]) : "memory");
-            }
-          }
-          if (warp == 1 && lane == 0) trace_ev(p, 3, tix, 32);
-          ptx::fence_proxy_async();   // generic-proxy writes -> visible to the tensor core's (async proxy) operand reads
-          __syncwarp();
-          if (lane == 0) ptx::mbar_arrive(slab_ready(s));
-          if (warp == 1 && lane == 0) trace_ev(p, 3, tix, 33);
-          if (++s == kNS) { s = 0; ph ^= 1; }
-        }
-      }
-    }
+    __syncwarp();
   } else if (warp == 2) {
     // ===================== MMA issuer =====================
     if (ptx::elect_one()) {
@@ -328,7 +229,7 @@ conv_sweep32_kernel(const __grid_constant__ CUtensorMap mapX, const __grid_const
             drained = T;
             trace_ev(p, 0, ti, 2);
           }
-          ok = ptx::mbar_wait(xform ? slab_ready(s) : slab_full(s), ph, p.dbg, 0x5304);
+          ok = ptx::mbar_wait(slab_full(s), ph, p.dbg, 0x5304);
           if (!ok) break;
           trace_ev(p, 0, ti, 3);
           ptx::tc_fence_after();
@@ -418,7 +319,7 @@ conv_sweep32_kernel(const __grid_constant__ CUtensorMap mapX, const __grid_const
         if (q.gn_part) {
           // GroupNorm statistics of the tensor as STORED (rounded).  32 values per row (16 sums, 16 squares) are reduce-SCATTERED
           // over the warp's 32 rows: after 5 exchange steps (16 + 8 + 4 + 2 + 1 shuffles) lane L holds the total of value L, so the
-          // running sums take ONE register per thread instead of 32 (the kernel runs 768 threads at 80 registers).
+          // running sums take ONE register per thread instead of 32 (640 threads share the register file).
           float w[32];
           unpack8(o0, *reinterpret_cast<float(*)[8]>(&w[0]));
           unpack8(o1, *reinterpret_cast<float(*)[8]>(&w[8]));

@@ -102,9 +102,8 @@ __device__ __forceinline__ void bulk_wait_read_all() { asm volatile("cp.async.bu
 
 __device__ __forceinline__ void bulk_wait_read_1() { asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory"); }
 
-// ---------------------------------------------------------------- thread-block clusters + TMA multicast
+// ---------------------------------------------------------------- thread-block clusters
 __device__ __forceinline__ uint32_t cluster_ctaid_x() { uint32_t r; asm volatile("mov.u32 %0, %%cluster_ctaid.x;" : "=r"(r)); return r; }
-__device__ __forceinline__ uint32_t cluster_ctaid_y() { uint32_t r; asm volatile("mov.u32 %0, %%cluster_ctaid.y;" : "=r"(r)); return r; }
 __device__ __forceinline__ void cluster_sync_all() {  // every thread of every CTA of the cluster
   asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
 }
@@ -131,27 +130,6 @@ __device__ __forceinline__ float4 ld_dsmem_f32x4(uint32_t cluster_addr) {
   asm volatile("ld.shared::cluster.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(cluster_addr) : "memory");
   return v;
 }
-// Multicast loads: the box lands at the same CTA-relative smem offset in every CTA of `mask`, and each of those CTAs'
-// mbarrier (same offset) receives the complete_tx.
-__device__ __forceinline__ void tma_load_2d_mc(uint32_t dst, const CUtensorMap* m, uint32_t bar, int c0, int c1, uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4}], [%2], %5;" ::
-          "r"(dst), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1), "h"(mask)
-      : "memory");
-}
-__device__ __forceinline__ void tma_load_5d_mc(uint32_t dst, const CUtensorMap* m, uint32_t bar, int c0, int c1, int c2, int c3,
-                                               int c4, uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.5d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4, %5, %6, %7}], [%2], %8;" ::
-          "r"(dst), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(c4), "h"(mask)
-      : "memory");
-}
-// tcgen05.commit arriving on the mbarrier at the same offset in every CTA of `mask`
-__device__ __forceinline__ void tc_commit_mc(uint32_t bar, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar), "h"(mask)
-               : "memory");
-}
-
 // ---------------------------------------------------------------- tcgen05 / TMEM
 __device__ __forceinline__ void tmem_alloc(uint32_t smem_dst, uint32_t ncols) {  // whole warp
   asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_dst), "r"(ncols) : "memory");

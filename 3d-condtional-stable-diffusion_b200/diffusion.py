@@ -199,8 +199,8 @@ class DiffusionModel:
         if seed is None:
             seed = int.from_bytes(os.urandom(7), "little")
         self.last_seed = seed
-        if fuse_update is None:   # default: on whenever nothing needs eps_hat in HBM (B200DM_FUSE_UPDATE=0 under B200DM_TUNING=1: off)
-            fuse_update = noise is None and on_step is None and L.tuning_env("B200DM_FUSE_UPDATE", "1") != "0"
+        if fuse_update is None:   # default: on whenever nothing needs eps_hat in HBM
+            fuse_update = noise is None and on_step is None
         assert not (fuse_update and (noise is not None or on_step is not None)), "fuse_update: no injected noise / eps callback"
         st = self._compile(B, sampler, noise is not None, seed, sample_id0, fuse_update)
         dev, nets, cb = st["dev"], st["nets"], st["chain_batch"]

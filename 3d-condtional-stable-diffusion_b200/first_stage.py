@@ -109,15 +109,14 @@ class _DecoderBase:
         return sum(int(np.prod(s)) for _, s, _ in self.spec)
 
     def _conv(self, pr, x0, kernel, bias, cout, k=3, mode=L.CONV_DIRECT, act=None, post_act=None, residual=None,
-              prelu_alpha=None, y_dtype=torch.bfloat16, transposed=False, note="", stride=1, in_norm=None):
-        """``in_norm``: see Program.conv; returns None when the conv's kernel cannot fold the input normalisation."""
+              prelu_alpha=None, y_dtype=torch.bfloat16, transposed=False, note="", stride=1):
         B, D, H, W, c0 = x0.shape
         desc = ops.make_conv_desc(mode, B, (D, H, W), c0, 0, cout, k, stride, act, post_act, y_dtype)
         wp = ops.pack_conv_weights(desc, kernel, transposed).to(self.device)
         od, oh, ow = ops.conv_out_shape(mode, (D, H, W), stride)
         y = pr.buf((B, od, oh, ow, cout), y_dtype)
         return pr.conv(desc, x0, wp, y, bias=bias.to(self.device).contiguous(), residual=residual,
-                       prelu_alpha=prelu_alpha, note=note, in_norm=in_norm)
+                       prelu_alpha=prelu_alpha, note=note)
 
     def __call__(self, latents):
         """decoder(latents (B,s,s,s,D) fp32|bf16) -> volumes (B,S,S,S,out) fp32."""
@@ -299,20 +298,9 @@ class AttnCpDecoder(_DecoderBase):
                            note=f"level.{i}.up")
             def norm_conv(t, norm, conv, residual=None):
                 """Conv3(SiLU(GN(t))) (vqgan_attn_cp.py:262-270) = GroupNorm statistics (from the producing conv's epilogue when its
-                kernel accumulates them) -> fused GN + SiLU pass -> conv.  The d-sweeping kernel can also normalise its input slabs in
-                shared memory (set_input_norm), which deletes the pass -- measured at 128^3, B=16: 3.0 ms against 1.61 ms (conv) +
-                0.72 ms (pass): that kernel's MMAs already use the whole shared-memory bandwidth, so the transform's loads see
-                ~1000-cycle latencies.  Kept behind B200DM_TUNING=1 B200DM_FOLD_GN=1."""
-                if L.tuning_env("B200DM_FOLD_GN", "0") == "1":
-                    mr = pr.gn_stats(t, grp, 1e-6, note=f"{norm}.stats")
-                    y = self._conv(pr, t, P[f"{conv}.kernel"], P[f"{conv}.bias"], c, residual=residual, note=f"{norm}+{conv.rsplit('.', 1)[-1]}",
-                                   in_norm=(mr, g(f"{norm}.gamma"), g(f"{norm}.beta"), grp, "silu"))
-                    if y is not None:
-                        return y
-                    hh = pr.norm_act(t, g(f"{norm}.gamma"), g(f"{norm}.beta"), pr.buf(t.shape), act="silu", kind=1, groups=grp, mean_rstd=mr, note=norm)
-                else:
-                    hh = gn_silu(t, norm, grp)
-                return self._conv(pr, hh, P[f"{conv}.kernel"], P[f"{conv}.bias"], c, residual=residual, note=conv)
+                kernel accumulates them) -> fused GN + SiLU pass -> conv.  (Normalising the slabs inside the d-sweeping conv instead
+                of the pass measured slower: 3.0 ms against 1.61 + 0.72 ms at 128^3, B=16.)"""
+                return self._conv(pr, gn_silu(t, norm, grp), P[f"{conv}.kernel"], P[f"{conv}.bias"], c, residual=residual, note=conv)
 
             for j in range(2):
                 n = f"level.{i}.res.{j}"

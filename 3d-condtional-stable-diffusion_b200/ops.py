@@ -254,22 +254,6 @@ class ConvPlan:
         check(lib().b200dm_conv_plan_info(self.h, C.byref(halo), C.byref(bn), C.byref(ks)))
         return dict(halo=halo.value, block_n=bn.value, ksplit=ks.value)   # halo: 0 per-tap GEMM, 1 halo kernel, 2 C_out=1 stencil
 
-    def add_output(self, y_extra, scale, shift, act=None):
-        """Extra bf16 output act(scale*v + shift) of the final value (the consumer's folded BatchNorm), same shape as y."""
-        assert y_extra.shape == self.y.shape and y_extra.dtype == L.ACT_DTYPE
-        check(lib().b200dm_conv_plan_add_output(self.h, ptr(y_extra), ptr(scale), ptr(shift), L.ACT[act]))
-        self.keep = self.keep + (y_extra, scale, shift)
-        return y_extra
-
-    def set_side_norm(self, y_side, scale, shift, act=None):
-        """1^3 conv only: also write act(scale*x + shift) of the conv's own input channels (x0|x1) to ``y_side``.
-        Returns False when the plan cannot (caller runs a norm pass instead)."""
-        rc = lib().b200dm_conv_plan_set_side_norm(self.h, ptr(y_side), ptr(scale), ptr(shift), L.ACT[act])
-        if rc != 0:
-            return False
-        self.keep = self.keep + (y_side, scale, shift)
-        return True
-
     def set_fused_update(self, upd_desc, x_t, x_prev, x_prev_16):
         """Output conv of the U-Net only: the epilogue applies the reverse-diffusion update to its eps tile and stores
         x_{t-1} (fp32 -> ``x_prev`` = ``x_t``, in place; 16-bit copy -> ``x_prev_16``) instead of eps.  False when the plan's
@@ -284,16 +268,6 @@ class ConvPlan:
     def run(self):
         check(lib().b200dm_conv_plan_run(self.h, stream()))
         return self.y
-
-    def set_input_norm(self, mean_rstd, gamma, beta, groups, act=None):
-        """Fold act(GroupNorm(x)) of the conv's INPUT into its operand path (x stays raw in HBM).  False when the plan's kernel has
-        no input transform (the caller then runs a normalisation pass)."""
-        rc = lib().b200dm_conv_plan_set_input_norm(self.h, ptr(mean_rstd), ptr(gamma), ptr(beta), groups, L.ACT[act])
-        if rc == L.ERR_UNSUPPORTED:
-            return False
-        check(rc)
-        self.keep = self.keep + (mean_rstd, gamma, beta)
-        return True
 
     def gn_partials(self):
         """GroupNorm partial sums as a by-product of this conv: -> (workspace fp32 (B * rows, C, 2), rows per sample), or None

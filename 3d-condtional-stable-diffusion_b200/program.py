@@ -24,7 +24,7 @@ class Program:
         self.bytes = 0.0     # algorithmic HBM bytes of the elementwise ops per run
         self.log = []        # (kind, note) per op, for profiles / debugging
         self.outputs = {}    # note -> output tensor (layer-by-layer parity debugging)
-        self.producers = {}  # data_ptr of a conv output -> its ConvPlan (extra normalised outputs are attached there)
+        self.producers = {}  # data_ptr of a conv output -> its ConvPlan (gn_stats asks it for GroupNorm partial sums)
         self.op_bytes = {}   # note -> algorithmic HBM bytes of that conv launch
 
     # -- allocation helper
@@ -41,14 +41,9 @@ class Program:
 
     # -- ops
     def conv(self, desc, x0, w_packed, y, x1=None, bias=None, chan_bias=None, t_dev=None, residual=None,
-             prelu_alpha=None, out_affine=None, note="", side=None, in_norm=None):
-        """``in_norm`` = (mean_rstd, gamma, beta, groups, act): the conv reads act(GroupNorm(x0)) with the normalisation folded
-        into its operand path; returns None (nothing recorded) when the plan's kernel cannot do that."""
+             prelu_alpha=None, out_affine=None, note=""):
         plan = ops.ConvPlan(desc, x0, w_packed, y, x1=x1, bias=bias, chan_bias=chan_bias, t_dev=t_dev,
                             residual=residual, prelu_alpha=prelu_alpha, out_affine=out_affine)
-        if in_norm is not None and not plan.set_input_norm(*in_norm):
-            return None
-        self.side_ok = side is not None and plan.set_side_norm(*side)   # (y_side, scale, shift, act)
         check(lib().b200dm_program_add_conv(self.h, plan.h))
         plan.release()
         self.keep.extend(t for t in plan.keep if t is not None)
@@ -63,22 +58,6 @@ class Program:
             self.log.append(("conv_halo" if kind else "conv", note, plan.flops))
         self.outputs[note] = y
         self.producers[y.data_ptr()] = plan
-        return y
-
-    def normalized_by_producer(self, t, scale, shift, act=None, note=""):
-        """act(scale*t + shift) as an extra output of the conv that produces ``t``; None if ``t`` is not a conv output or
-        the producer has no free output slot (the caller then runs a norm pass)."""
-        plan = self.producers.get(t.data_ptr())
-        if plan is None or t.dtype != L.ACT_DTYPE or t.shape[-1] % 16 != 0:
-            return None
-        y = self.buf(t.shape)
-        try:
-            plan.add_output(y, scale, shift, act)
-        except L.B200dmError:
-            return None
-        self.hold(scale, shift)
-        if note:
-            self.outputs[note] = y
         return y
 
     def norm_act(self, x0, a, b, y, act=None, x1=None, kind=0, groups=1, mean_rstd=None, note=""):
@@ -96,7 +75,7 @@ class Program:
         accumulate the sums in its epilogue (d-sweeping 32 -> 32 kernel), only a tiny fixed-order reduction is recorded;
         otherwise a statistics pass re-reads x."""
         plan = self.producers.get(x.data_ptr())
-        part = plan.gn_partials() if plan is not None and x.dtype == L.ACT_DTYPE and L.tuning_env("B200DM_GN_PASS", "0") != "1" else None
+        part = plan.gn_partials() if plan is not None and x.dtype == L.ACT_DTYPE else None
         if part is not None:
             ws, rows = part
             mr = self.buf((x.shape[0], groups, 2), torch.float32)

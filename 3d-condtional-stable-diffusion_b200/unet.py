@@ -169,17 +169,6 @@ class UNet:
         F, B, S = cfg.first_conv_channels, batch, cfg.img_size
         pr = Program(dev)
         self.prog = pr
-        # Producer-side normalisation (conv epilogues write the consumers' BN(+swish) copies as extra outputs) removes every
-        # norm pass, but measured SLOWER on B200 (cfg-2: 5.47 vs 5.08 ms/step): the extra stores lengthen the conv
-        # epilogues, which are on the critical path, by more than the streaming pass costs.  Off unless B200DM_FUSE_NORMS=1.
-        self._wcache = {}
-        self._lane_base, self._half = 0, (0, batch)
-        self.fuse_norms = L.tuning_env("B200DM_FUSE_NORMS", "0") == "1"
-        # norm1 as a side output of the 1^3 shortcut conv (b200dm_conv_plan_set_side_norm): measured SLOWER on B200 (cfg-2:
-        # 3.35 vs 3.15 ms/step) -- one-tile CTAs serialise load -> transform -> store, while the stand-alone pass is a
-        # pipelined HBM stream at 4.9 TB/s.  Off unless B200DM_SIDE_NORM=1 (kept, tested, for a persistent variant).
-        self.side_norm = L.tuning_env("B200DM_SIDE_NORM", "0") == "1"
-        self.lanes = L.tuning_env("B200DM_LANES", "1") != "0"   # branch-parallel CrossAttentionBlock (program lanes)
         self.t_dev = t_dev if t_dev is not None else torch.zeros(4, dtype=torch.int32, device=dev)   # [t, t_prev, seq idx, -]
         self.per_sample_t, self._temb_rows = bool(per_sample_t), []
         g = lambda n: P[n].to(dev).contiguous()  # noqa: E731
@@ -195,29 +184,24 @@ class UNet:
 
         def conv(x0, kname, cout, y=None, x1=None, k=3, stride=1, mode=L.CONV_DIRECT, act=None, bias=True, chan_bias=None,
                  residual=None, y_dtype=torch.bfloat16, transposed_store=False, dense=False, out_affine=None, note="",
-                 kern=None, bias_t=None, side=None):
+                 kern=None, bias_t=None):
             Bx, D, H, Wd, c0 = x0.shape
             c1 = x1.shape[-1] if x1 is not None else 0
             desc = ops.make_conv_desc(mode, Bx, (D, H, Wd), c0, c1, cout, k, stride, act, None, y_dtype,
                                       chan_bias_rows=(batch if self.per_sample_t else 1) if chan_bias is not None else 0,
                                       transposed_store=transposed_store)
-            kern_key = None if kern is None else "override"
             if kern is None:
                 kern = P[f"{kname}.kernel"]
             if dense:  # Dense on voxels == 1^3 conv: (in,out) -> (1,1,1,in,out)
                 kern = kern.reshape(1, 1, 1, *kern.shape)
-            wkey = (kname, mode, k, stride, c0, c1, cout, transposed_store, dense, kern_key)
-            wp = self._wcache.get(wkey)
-            if wp is None:   # (the two batch halves of the deep phase share one packed copy)
-                wp = self._wcache[wkey] = ops.pack_conv_weights(desc, kern).to(dev)
+            wp = ops.pack_conv_weights(desc, kern).to(dev)
             if y is None:
                 od, oh, ow = ops.conv_out_shape(mode, (D, H, Wd), stride)
                 y = pr.buf((Bx, cout, od * oh * ow) if transposed_store else (Bx, od, oh, ow, cout), y_dtype)
             bias_dev = None if not bias else (bias_t.to(dev).contiguous() if bias_t is not None else g(f"{kname}.bias"))
             return pr.conv(desc, x0, wp, y, x1=x1, bias=bias_dev, chan_bias=chan_bias,
                            t_dev=self.t_dev if (chan_bias is not None and not self.per_sample_t) else None, residual=residual,
-                           out_affine=out_affine,
-                           note=note or kname, side=side)
+                           out_affine=out_affine, note=note or kname)
 
         def bgemm(a, b, y_dtype, residual=None, note=""):
             Bx, M, K = a.shape
@@ -228,8 +212,9 @@ class UNet:
 
         def bn_act(x0, name, act, x1=None, note=""):
             """BatchNorm(inference) [+ swish] of x0 (or of the concat [x0, x1]) -> (y0, y1|None): the conv that reads it takes
-            the two channel segments separately.  When the sources are conv outputs the normalised copies are written by
-            the PRODUCERS' epilogues (extra outputs) and no pass runs here; otherwise one fused norm(+concat) pass."""
+            the two channel segments separately.  One fused norm(+concat) pass, or the x half only when the skip half was
+            normalised in the shadow of the 8^3 phase.  (Writing the normalised copies from the producers' epilogues instead
+            measured slower: 5.47 vs 5.08 ms/step on cfg-2, the conv epilogues are on the critical path.)"""
             sc, sh = ops.bn_fold(g(f"{name}.gamma"), g(f"{name}.beta"), g(f"{name}.mean"), g(f"{name}.var"), 1e-3)
             c0 = x0.shape[-1]
             if x1 is not None and id(x1) in self.shadow_norms:
@@ -242,14 +227,6 @@ class UNet:
                 assert hs["name"] == name
                 y0 = pr.norm_act(x0, sc[:c0].contiguous(), sh[:c0].contiguous(), pr.buf(x0.shape), act=act, note=f"{note or name}.x")
                 return y0, hs["y"]
-            if self.fuse_norms:
-                y0 = pr.normalized_by_producer(x0, sc[:c0], sh[:c0], act, note=(note or name) if x1 is None else "")
-                if y0 is not None and x1 is None:
-                    return y0, None
-                if y0 is not None:
-                    y1 = pr.normalized_by_producer(x1, sc[c0:], sh[c0:], act)
-                    if y1 is not None:
-                        return y0, y1
             C = c0 + (x1.shape[-1] if x1 is not None else 0)
             y = pr.buf((*x0.shape[:-1], C))
             return pr.norm_act(x0, sc, sh, y, act=act, x1=x1, note=note or name), None
@@ -257,16 +234,10 @@ class UNet:
         def resblock(b, x, skip):
             n, w = b["name"], b["cout"]
             cin = b["cin"] + b["cskip"]
-            h = None
             if cin != w:
-                # the 1^3 shortcut conv reads exactly the tensor(s) norm1 normalises: it writes swish(BN(x|skip)) from its
-                # A tiles as a side output, so the block needs no separate norm pass (falls back to one if the plan cannot)
-                sc1, sh1 = ops.bn_fold(g(f"{n}.norm1.gamma"), g(f"{n}.norm1.beta"), g(f"{n}.norm1.mean"), g(f"{n}.norm1.var"), 1e-3)
-                hbuf = pr.buf((*x.shape[:-1], cin))
-                res = conv(x, f"{n}.shortcut", w, x1=skip, k=1, side=(hbuf, sc1, sh1, "silu") if self.side_norm else None)
-                if pr.side_ok:
-                    h, h1 = hbuf, None
-                    pr.outputs[f"{n}.norm1"] = hbuf
+                # (norm1 as a side output of this conv, written from its A tiles, measured slower than the norm pass: 3.35 vs
+                # 3.15 ms/step on cfg-2 -- one-tile CTAs serialise load -> transform -> store)
+                res = conv(x, f"{n}.shortcut", w, x1=skip, k=1)
             elif skip is None:
                 res = x
             else:  # concat whose width equals w: materialise it once (identity affine)
@@ -277,8 +248,7 @@ class UNet:
                 rows = torch.zeros(x.shape[0], w, dtype=torch.float32, device=dev)
                 self._temb_rows.append((pr.hold(table), rows))
                 table = rows
-            if h is None:
-                h, h1 = bn_act(x, f"{n}.norm1", "silu", x1=skip)
+            h, h1 = bn_act(x, f"{n}.norm1", "silu", x1=skip)
             # conv1 + temb -> BN(norm2) -> swish (dm3d.py:237-244): conv1's output has no other reader, so norm2 and the
             # activation run in conv1's epilogue on the fp32 accumulator (one HBM pass and one bf16 rounding fewer)
             sc2, sh2 = ops.bn_fold(g(f"{n}.norm2.gamma"), g(f"{n}.norm2.beta"), g(f"{n}.norm2.mean"), g(f"{n}.norm2.var"), 1e-3)
@@ -306,19 +276,17 @@ class UNet:
         sites = {}
 
         def ctx_site(n, c, s):
-            """K_ctx / V_ctx^T buffers of one attention site for the WHOLE batch (filled by set_context); the caller gets
-            the rows of the batch range it is building."""
+            """K_ctx / V_ctx^T buffers of one attention site for the whole batch (filled by set_context)."""
             if n not in sites:
                 Lq = s ** 3
                 sites[n] = dict(name=n, c=c, s=s, kc=pr.buf((batch, Lq, c)), vcT=pr.buf((batch, c, Lq)))
                 self.ctx_sites.append(sites[n])
-            lo, hi = self._half
-            return sites[n]["kc"][lo:hi], sites[n]["vcT"][lo:hi]
+            return sites[n]["kc"], sites[n]["vcT"]
 
         def xattn_block(b, x):  # CrossAttentionBlock.call (conditional_dm3d.py:186-195)
             n, c, s = b["name"], b["c"], b["s"]
             Lq = s ** 3
-            B, lb = x.shape[0], self._lane_base
+            B = x.shape[0]
             scale = float(c) ** -0.5
             # inference BatchNorm followed by the 1^3 proj_in conv is one affine map: fold it into proj_in's kernel and bias
             # (W' = diag(a) W, b' = b + shift . W; conditional_dm3d.py:187-188) -- no normalisation pass
@@ -332,43 +300,32 @@ class UNet:
             ln = pr.layernorm(h, gam, bet, [pr.buf(h.shape) for _ in range(3)], 1e-3, note=f"{n}.ln")
             hf = h.view(B, Lq, c)
             kc, vcT = ctx_site(n, c, s)
-            if not self.lanes:
-                q1 = conv(ln[0], f"{n}.query", c, k=1, dense=True).view(B, Lq, c)
-                k1 = conv(ln[0], f"{n}.key", c, k=1, dense=True).view(B, Lq, c)
-                v1T = conv(ln[0], f"{n}.value", c, k=1, dense=True, transposed_store=True)
-                t1 = attention_core(q1, k1, v1T, scale, hf, f"{n}.self")
-                q2 = conv(ln[1], f"{n}.query", c, k=1, dense=True).view(B, Lq, c)
-                t2 = attention_core(q2, kc, vcT, scale, t1, f"{n}.cross")
-                m = conv(ln[2], f"{n}.mlp0", 4 * c, k=1, dense=True, act="relu")
-                xs = conv(m, f"{n}.mlp1", c, k=1, dense=True, residual=t2.view(B, s, s, s, c))
-                # relu(proj_out(x)) + residual: act before the residual add
-                return conv(xs, f"{n}.proj_out", c, k=1, act="relu", residual=x)
             # The three branches all read h (conditional_dm3d.py:190-192): self-attention on the caller's stream, cross
             # attention on lane 1, the MLP on lane 2 (its second GEMM adds the cross branch), and proj_out sums the two
             # partial results inside its K loop: proj_out(t1 + xs) = [t1 | xs] . [W; W]  (two K segments, no add pass).
-            pr.sync(lb, lb + 1)
-            pr.sync(lb, lb + 2)
-            pr.sync(lb, lb + 3)
+            pr.sync(0, 1)
+            pr.sync(0, 2)
+            pr.sync(0, 3)
             # query(LN1(h)) and key(LN1(h)) read the same tensor: one Dense with the kernels side by side, [q | k] = x [Wq | Wk];
             # the attention kernel reads q and k as column blocks (row stride 2C) of its output
             wqk = torch.cat([P[f"{n}.query.kernel"], P[f"{n}.key.kernel"]], dim=1)
             bqk = torch.cat([P[f"{n}.query.bias"], P[f"{n}.key.bias"]])
             qk = conv(ln[0], f"{n}.query+key", 2 * c, k=1, dense=True, kern=wqk, bias_t=bqk).view(B, Lq, 2 * c)
             q1, k1 = qk[..., :c], qk[..., c:]
-            pr.set_lane(lb + 3)
+            pr.set_lane(3)
             v1T = conv(ln[0], f"{n}.value", c, k=1, dense=True, transposed_store=True)
-            pr.set_lane(lb)
-            pr.sync(lb + 3, lb)
+            pr.set_lane(0)
+            pr.sync(3, 0)
             t1 = attention_core(q1, k1, v1T, scale, hf, f"{n}.self")
-            pr.set_lane(lb + 1)
+            pr.set_lane(1)
             q2 = conv(ln[1], f"{n}.query", c, k=1, dense=True).view(B, Lq, c)
             c2 = attention_core(q2, kc, vcT, scale, None, f"{n}.cross")
-            pr.set_lane(lb + 2)
+            pr.set_lane(2)
             m = conv(ln[2], f"{n}.mlp0", 4 * c, k=1, dense=True, act="relu")
-            pr.sync(lb + 1, lb + 2)
+            pr.sync(1, 2)
             xs = conv(m, f"{n}.mlp1", c, k=1, dense=True, residual=c2.view(B, s, s, s, c))
-            pr.set_lane(lb)
-            pr.sync(lb + 2, lb)
+            pr.set_lane(0)
+            pr.sync(2, 0)
             w2 = torch.cat([P[f"{n}.proj_out.kernel"]] * 2, dim=3)
             return conv(t1.view(B, s, s, s, c), f"{n}.proj_out", c, x1=xs, k=1, act="relu", residual=x, kern=w2)
 
@@ -379,7 +336,7 @@ class UNet:
         # (BN + swish with the CONSUMER block's parameters, dm3d.py:235-236) are therefore run on lane 4 while the 8^3 phase
         # executes on the other lanes, and the up-path passes shrink to the x half.
         self.shadow_norms, self.shadow_joined = {}, False
-        use_shadow = L.tuning_env("B200DM_SHADOW", "1") != "0" and len(cfg.widths) >= 2
+        use_shadow = len(cfg.widths) >= 2
         consumer, stack = {}, []          # push index -> the up-path ResidualBlock that pops it
         npush = 0
         for b in self.blocks:
@@ -404,70 +361,33 @@ class UNet:
                 self.shadow_norms[id(t)] = dict(name=nm, y=y)
             pr.set_lane(0)
 
-        st = dict(x=None, skips=[], ids=[])
-        self._npush = 1   # push index 0 is the input conv's output
-
-        def do_block(b, st, y_out=None):
+        x, skips, ids = None, [], []
+        next_id = 1   # push index 0 is the input conv's output
+        for b in self.blocks:
             k = b["kind"]
+            if not shadow_done and k == "res" and b["s"] == deepest:
+                shadow_pass(skips, ids)
+                shadow_done = True
             if k == "in":
-                st["x"] = conv(self.x_in, "in", b["cout"])
-                st["skips"].append(st["x"]); st["ids"].append(0)
+                x = conv(self.x_in, "in", b["cout"])
+                skips.append(x); ids.append(0)
             elif k == "res":
                 skip = None
                 if b.get("pop"):
-                    st["ids"].pop()
-                    skip = st["skips"].pop()
-                st["x"] = resblock(b, st["x"], skip)
+                    ids.pop()
+                    skip = skips.pop()
+                x = resblock(b, x, skip)
             elif k == "attn":
-                st["x"] = xattn_block(b, st["x"]) if cfg.conditional else attn_block(b, st["x"])
+                x = xattn_block(b, x) if cfg.conditional else attn_block(b, x)
             elif k == "push":
-                st["skips"].append(st["x"]); st["ids"].append(self._npush); self._npush += 1
+                skips.append(x); ids.append(next_id); next_id += 1
             elif k == "down":
-                st["x"] = conv(st["x"], b["name"], b["c"], stride=2)
+                x = conv(x, b["name"], b["c"], stride=2)
             elif k == "up":
-                st["x"] = conv(st["x"], b["name"], b["c"], mode=L.CONV_PARITY, y=y_out)
+                x = conv(x, b["name"], b["c"], mode=L.CONV_PARITY)
             elif k == "out":
-                h, _ = bn_act(st["x"], "out.norm", "silu")
+                h, _ = bn_act(x, "out.norm", "silu")
                 conv(h, "out.conv", b["cout"], y=self.eps, y_dtype=torch.float32)
-
-        # Deep phase = the blocks at the coarsest resolution (8^3 in cfg-2) up to and including the upsample conv that leaves it.
-        # B200DM_SPLIT_DEEP=1 records it twice, once per half of the batch, on two independent lane sets (0-3 and 5-8), as
-        # parallel branches of the step graph.  Measured on B200 (cfg-2): 3.23 vs 3.09 ms/step -- SLOWER: the phase's kernels
-        # are bound by their own latency (one tile per CTA either way), so halving the batch halves no kernel's duration and
-        # doubles the launches.  Off by default; kept (and parity-tested) because it is the scaffold for per-sample
-        # persistent kernels at this level.
-        blocks = self.blocks
-        deep = [i for i, b in enumerate(blocks) if b.get("s") == deepest and b["kind"] in ("res", "attn", "up")]
-        i0, i1 = (deep[0], deep[-1] + 1) if deep else (len(blocks), len(blocks))
-        split = (L.tuning_env("B200DM_SPLIT_DEEP", "0") == "1" and self.lanes and batch >= 4 and batch % 2 == 0 and deep
-                 and blocks[i1 - 1]["kind"] == "up")
-        i = 0
-        while i < len(blocks):
-            b = blocks[i]
-            if not shadow_done and b["kind"] == "res" and b["s"] == deepest:
-                shadow_pass(st["skips"], st["ids"])
-                shadow_done = True
-            if split and i == i0:
-                up = blocks[i1 - 1]
-                s_out = 2 * up["s"]
-                full = pr.buf((batch, s_out, s_out, s_out, up["c"]))
-                npush0, after = self._npush, None
-                pr.sync(0, 5)
-                for (lo, hi), lb in (((0, batch // 2), 0), ((batch // 2, batch), 5)):
-                    self._lane_base, self._half, self._npush = lb, (lo, hi), npush0
-                    pr.set_lane(lb)
-                    sh = dict(x=st["x"][lo:hi], skips=[t[lo:hi] for t in st["skips"]], ids=list(st["ids"]))
-                    for j in range(i0, i1):
-                        do_block(blocks[j], sh, y_out=full[lo:hi] if j == i1 - 1 else None)
-                    after = sh
-                self._lane_base, self._half = 0, (0, batch)
-                pr.set_lane(0)
-                pr.sync(5, 0)
-                st = dict(x=full, skips=st["skips"][:len(after["skips"])], ids=after["ids"])
-                i = i1
-                continue
-            do_block(b, st)
-            i += 1
         torch.cuda.synchronize(dev)
         return self
 

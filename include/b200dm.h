@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define B200DM_VERSION 100
+#define B200DM_VERSION 101
 
 #define B200DM_OK 0
 #define B200DM_ERR_INVALID (-1)
@@ -257,16 +257,6 @@ double b200dm_conv_plan_flops(const b200dm_conv_plan* p);
  * ResidualBlock conv1 -> BN -> swish (dm3d.py:237-244) when the un-normalised tensor has no other reader.
  * NULL, NULL switches it off. */
 int b200dm_conv_plan_set_out_affine(b200dm_conv_plan* p, const float* scale, const float* shift);
-/* Up to two EXTRA bf16 outputs with the shape of y: y_extra = act(scale[co] * v + shift[co]) of the final value v
- * (after residual / post-act).  The producer writes the BatchNorm(+swish) its consumers would apply
- * (dm3d.py:235-236 norm1 of the next ResidualBlock, the skip-connection half of an up-path norm1, dm3d.py:46 the
- * attention block's norm, dm3d.py:371-372 the output norm), so those tensors are never re-read by a separate pass. */
-int b200dm_conv_plan_add_output(b200dm_conv_plan* p, void* y_extra, const float* scale, const float* shift, int32_t act);
-/* Side output of a 1^3 stride-1 conv (the ResidualBlock shortcut, dm3d.py:226-227,250): y_side = act(scale[c] * x[c] + shift[c])
- * over the conv's own INPUT channels (x0 | x1 concatenated, bf16, same voxel grid), written from the A tiles while they sit
- * in shared memory -- the block's norm1 + swish (dm3d.py:235-236) without a second pass over x / skip.  Returns
- * B200DM_ERR_UNSUPPORTED when the plan cannot do it (the caller then runs b200dm_norm_act_fwd). */
-int b200dm_conv_plan_set_side_norm(b200dm_conv_plan* p, void* y_side, const float* scale, const float* shift, int32_t act);
 /* Fuse the reverse-diffusion update (b200dm_ddpm_update: DiffusionModel.sample + the loop body of generate, networks/dm3d.py:
  * 477-508, 516-530) into the epilogue of the U-Net's output conv (dm3d.py:373-374, the fp32 eps_hat): the conv then stores
  * x_{t-1} = step(x_t, eps_hat, Philox noise) to x_prev (fp32; must alias x_t: updated in place) and a copy in the 16-bit storage type to x_prev_16
@@ -281,11 +271,6 @@ int b200dm_conv_plan_info(const b200dm_conv_plan* p, int32_t* halo, int32_t* blo
  * accumulate per-(work item, channel) partial sums of the STORED values into `workspace` = float[batch * rows_per_sample][C][2];
  * b200dm_gn_finalize reduces them in a fixed order (bit-reproducible) to (mean, rstd) per (sample, group).
  * _bytes returns 0 when the plan cannot produce partials. */
-/* The consumer-side GroupNorm + activation folded into the conv's operand path (tfa GroupNormalization -> swish -> Conv3D,
- * vqgan_attn_cp.py:262-270): the plan then reads the RAW tensor and normalises each tile in shared memory with the (mean, rstd)
- * found in `mean_rstd` (batch, groups, 2) at run time.  B200DM_ERR_UNSUPPORTED when the plan's kernel has no input transform. */
-int b200dm_conv_plan_set_input_norm(b200dm_conv_plan* plan, const float* mean_rstd, const float* gamma, const float* beta,
-                                    int32_t groups, int32_t act);
 size_t b200dm_conv_plan_gn_partials_bytes(const b200dm_conv_plan* plan, int32_t* rows_per_sample);
 int b200dm_conv_plan_set_gn_partials(b200dm_conv_plan* plan, float* workspace, size_t ws_bytes);
 int b200dm_gn_finalize(const float* partials, int32_t batch, int32_t rows_per_sample, int32_t c, int32_t groups,

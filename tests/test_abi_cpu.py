@@ -50,7 +50,7 @@ def test_dynamic_symbol_table_has_c_linkage(L):
 
 def test_version_and_error_string(L):
     lib = L.lib()
-    assert lib.b200dm_version() == 100
+    assert lib.b200dm_version() == 101
     assert isinstance(lib.b200dm_last_error(), bytes)
 
 

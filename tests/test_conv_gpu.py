@@ -92,28 +92,6 @@ def test_conv3_pair_slab_tiles(cuda):
         _close(y, ref, tol=6e-3, what=f"pair-slab conv3 B{B} D{D} {c0}+{c1}->{cout}")
 
 
-def test_conv1_side_norm_output(cuda):
-    """1^3 shortcut conv with the block's norm1 + swish written as a side output from the A tiles (two K segments)."""
-    from b200dm import ops, _lib
-    B, S, c0, c1, cout = 2, 8, 64, 32, 64
-    x0, x1 = _rand((B, S, S, S, c0), 1), _rand((B, S, S, S, c1), 2)
-    w = _rand((1, 1, 1, c0 + c1, cout), 3, 1.0 / np.sqrt(c0 + c1))
-    b = torch.randn(cout, generator=torch.Generator().manual_seed(4))
-    sc = torch.rand(c0 + c1, generator=torch.Generator().manual_seed(5)) + 0.5
-    sh = torch.randn(c0 + c1, generator=torch.Generator().manual_seed(6)) * 0.1
-    desc = ops.make_conv_desc(_lib.CONV_DIRECT, B, (S, S, S), c0, c1, cout, 1, 1)
-    y = torch.empty(B, S, S, S, cout, dtype=torch.bfloat16, device=cuda)
-    hs = torch.zeros(B, S, S, S, c0 + c1, dtype=torch.bfloat16, device=cuda)
-    plan = ops.ConvPlan(desc, x0.to(cuda, torch.bfloat16), ops.pack_conv_weights(desc, w).to(cuda), y, x1=x1.to(cuda, torch.bfloat16),
-                        bias=b.to(cuda))
-    assert plan.set_side_norm(hs, sc.to(cuda), sh.to(cuda), "silu")
-    plan.run()
-    _check_flag()
-    xin = torch.cat([x0, x1], -1)
-    _close(y, O.conv3d(xin, w, b), tol=6e-3, what="1^3 conv with side output")
-    _close(hs, O.swish(xin * sc + sh), tol=6e-3, what="side output swish(scale*x+shift)")
-
-
 def test_conv3_two_segments(cuda):
     from b200dm import ops
     B, S, c0, c1, cout = 2, 8, 64, 32, 64
@@ -319,31 +297,6 @@ def test_conv_out_affine_fuses_consumer_batchnorm(cuda, B, S, cin, cout, halo):
     _close(y, ref, what=f"conv3 + temb + BN + swish fused, B{B} S{S} {cin}->{cout}")
 
 
-@pytest.mark.parametrize("B,S,cin,cout,halo", [(2, 8, 64, 128, -1), (1, 16, 64, 64, 0)])
-def test_conv_extra_normalised_outputs(cuda, B, S, cin, cout, halo):
-    """b200dm_conv_plan_add_output: the producer also writes act(scale*y + shift) copies (its consumers' folded BatchNorm)."""
-    from b200dm import ops, _lib
-    g = torch.Generator().manual_seed(11)
-    x = _rand((B, S, S, S, cin), 1)
-    w = _rand((3, 3, 3, cin, cout), 2, 1.0 / np.sqrt(27 * cin))
-    b = torch.randn(cout, generator=g)
-    res = _rand((B, S, S, S, cout), 5)
-    s2, h2 = torch.rand(cout, generator=g) + 0.5, torch.randn(cout, generator=g) * 0.1
-    s3, h3 = torch.rand(cout, generator=g) + 0.5, torch.randn(cout, generator=g) * 0.1
-    ref = O.conv3d(x, w, b) + res
-    desc = ops.make_conv_desc(_lib.CONV_DIRECT, B, (S, S, S), cin, 0, cout, 3, 1, use_halo=halo)
-    wp = ops.pack_conv_weights(desc, w).to(cuda)
-    y = torch.empty(B, S, S, S, cout, dtype=torch.bfloat16, device=cuda)
-    plan = ops.ConvPlan(desc, x.to(cuda, torch.bfloat16), wp, y, bias=b.to(cuda), residual=res.to(cuda, torch.bfloat16))
-    y2 = plan.add_output(torch.empty_like(y), s2.to(cuda), h2.to(cuda), "silu")
-    y3 = plan.add_output(torch.empty_like(y), s3.to(cuda), h3.to(cuda), None)
-    plan.run()
-    _check_flag()
-    _close(y, ref, tol=6e-3, what="main output")
-    _close(y2, O.swish(ref * s2 + h2), tol=8e-3, what="extra output 1 (BN + swish)")
-    _close(y3, ref * s3 + h3, tol=8e-3, what="extra output 2 (BN)")
-
-
 @pytest.mark.parametrize("shape", [(2, 9, 13, 40), (1, 16, 16, 16), (1, 3, 8, 32), (2, 33, 24, 70)])
 def test_conv3_head_stencil_kernel(cuda, shape):
     """C_in = 32 -> C_out = 1 (vqgan_attn_cp.py:424-427, the decoder's head): the HBM-bound stencil-reduce kernel
@@ -410,38 +363,3 @@ def test_conv3_sweep32_kernel(cuda, shape, extras):
     var = yf.var(dim=(1, 3), unbiased=False)
     assert torch.allclose(mr[..., 0].cpu().double(), mean, rtol=1e-4, atol=1e-5)
     assert torch.allclose(mr[..., 1].cpu().double(), 1.0 / torch.sqrt(var + 1e-6), rtol=1e-4)
-
-
-@pytest.mark.parametrize("shape,groups", [((2, 20, 16, 8), 32), ((1, 35, 24, 12), 8), ((2, 7, 40, 24), 32)])
-def test_conv3_sweep32_input_groupnorm_fold(cuda, shape, groups):
-    """Conv3D(SiLU(GroupNorm(x))) (vqgan_attn_cp.py:262-270) with the normalisation folded into the conv's operand path: the
-    kernel normalises every landed slab in shared memory, halo voxels outside the volume stay zero ('same' padding pads the
-    NORMALISED tensor).  Reference: the separate GN + SiLU pass (rounded to the 16-bit storage type) followed by the conv."""
-    from b200dm import ops, _lib as L
-    B, D, H, W = shape
-    x = _rand((B, D, H, W, 32), 1) * 1.7 + 0.3
-    x = _r(x)
-    w = _rand((3, 3, 3, 32, 32), 2, 1.0 / np.sqrt(27 * 32))
-    b = torch.randn(32, generator=torch.Generator().manual_seed(3))
-    gamma = torch.rand(32, generator=torch.Generator().manual_seed(8)) + 0.5
-    beta = torch.randn(32, generator=torch.Generator().manual_seed(9)) * 0.2
-    xg = x.reshape(B, -1, groups, 32 // groups).double()
-    mean, var = xg.mean(dim=(1, 3)), xg.var(dim=(1, 3), unbiased=False)
-    mr = torch.stack([mean, 1.0 / torch.sqrt(var + 1e-6)], -1).float()           # (B, groups, 2)
-    a = mr[..., 1].repeat_interleave(32 // groups, 1) * gamma                   # (B, 32)
-    sh = beta - mr[..., 0].repeat_interleave(32 // groups, 1) * a
-    h = O.swish(x * a[:, None, None, None, :] + sh[:, None, None, None, :]).to(L.ACT_DTYPE).float()
-    ref = O.conv3d(h, w, b)
-    xd = x.to(cuda, L.ACT_DTYPE)
-    desc = ops.make_conv_desc(L.CONV_DIRECT, B, (D, H, W), 32, 0, 32, 3, 1, None, None)
-    y = torch.empty(B, D, H, W, 32, dtype=L.ACT_DTYPE, device=cuda)
-    plan = ops.ConvPlan(desc, xd, ops.pack_conv_weights(desc, w, False).to(cuda), y, bias=b.to(cuda))
-    assert plan.set_input_norm(mr.to(cuda), gamma.to(cuda), beta.to(cuda), groups, "silu")
-    plan.run()
-    _check_flag()
-    _close(y, ref, tol=8e-3, what=f"sweep32 with folded GN+SiLU {shape}")
-    # a plan without an input transform says so instead of silently ignoring the request
-    desc2 = ops.make_conv_desc(L.CONV_DIRECT, B, (D, H, W), 32, 0, 64, 3, 1, None, None)
-    w2 = _rand((3, 3, 3, 32, 64), 2, 0.05)
-    plan2 = ops.ConvPlan(desc2, xd, ops.pack_conv_weights(desc2, w2, False).to(cuda), torch.empty(B, D, H, W, 64, dtype=L.ACT_DTYPE, device=cuda))
-    assert not plan2.set_input_norm(mr.to(cuda), gamma.to(cuda), beta.to(cuda), groups, "silu")

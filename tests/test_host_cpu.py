@@ -193,7 +193,7 @@ def test_sharded_generate_world2_gloo_matches_single_process(total):
 
 
 def test_tuning_switches_need_the_tuning_gate(monkeypatch):
-    """Experiment switches of the Python layer (and of the native library: conv.cu tuning_env) are ignored unless B200DM_TUNING=1."""
+    """Experiment switches of the Python layer are ignored unless B200DM_TUNING=1."""
     from b200dm import _lib as L
     monkeypatch.delenv("B200DM_TUNING", raising=False)
     monkeypatch.setenv("B200DM_CHAINS", "4")

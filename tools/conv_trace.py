@@ -32,9 +32,6 @@ if os.environ.get("FUSE"):           # ... with the reverse-diffusion update in 
     xb = torch.empty(B, D, H, W, cout, device=dev, dtype=torch.bfloat16)
     ud = ops.make_update_desc(betas, xt[0].numel(), B, 500, 499, 1 if os.environ["FUSE"] == "ddim" else 0, 7, 0, _lib.F32)
     assert plan.set_fused_update(ud, xt, xt, xb)
-if os.environ.get("XFORM") == "1":   # d-sweeping kernel: folded input GroupNorm + SiLU
-    mr = torch.stack([torch.zeros(B, 32), torch.ones(B, 32)], -1).to(dev)
-    assert plan.set_input_norm(mr, torch.ones(32, device=dev), torch.zeros(32, device=dev), 32, "silu")
 for _ in range(3):
     plan.run()
 tr = torch.zeros(4 * 2048, dtype=torch.int64, device=dev)
@@ -44,7 +41,7 @@ torch.cuda.synchronize()
 t = tr.cpu().view(4, 2048)
 names = {1: "tile:begin", 2: "tile:tmem_empty ok", 3: "kd:slabs ready", 4: "kd:issued", 5: "b?", 6: "b:waited", 7: "b:pre", 10: "epi:wait", 11: "epi:tmem_full ok", 12: "epi:done", 13: "epi:buf free", 14: "epi:tile written", 15: "epi:synced", 16: "epi:acc in regs", 17: "epi:half done", 18: "epi:loop top", 19: "epi:tile decoded", 20: "epi:bias staged"}
 t0 = min(int(v) >> 8 for v in t[0] if int(v) != 0)
-names.update({30: "tail:roles done", 31: "tail:block synced", 32: "tail:cluster synced", 33: "xf:signalled"})
+names.update({30: "tail:roles done", 31: "tail:block synced", 32: "tail:cluster synced"})
 for region, label in ((0, "MMA"), (1, "EPI"), (2, "SLAB"), (3, "TAIL")):
     prev = None
     out = []

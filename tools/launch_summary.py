@@ -37,7 +37,7 @@ for n, u in seq:
     a = agg.setdefault(n, [0, 0.0]); a[0] += 1; a[1] += u
 with open(f"profiles/{tag}_launches_{what}_summary.csv", "w") as f:
     f.write(f"# {tag}: per-kernel totals of one " + ("cfg-3 quantize + decode pass" if what == "decode" else "cfg-2 step") + " under ncu (cold-cache, serialised; compare SHARES)\n")
-    f.write("# conv_halo_kernel<BLOCK_N, TD, NS, NB, TPS, STAGED, PAIR, CG2, FUSE_UPD>; conv_halo_up_kernel<BLOCK_N, NS, NB, PAIR>; conv_igemm_kernel<BLOCK_N, NSTAGE, CMODE>\n")
+    f.write("# conv_halo_kernel<BLOCK_N, TD, NS, NB, TPS, STAGED, PAIR, CG2, FUSE_UPD>; conv_halo_up_kernel<BLOCK_N, NS, NB, PAIR>; conv_igemm_kernel<BLOCK_N, NSTAGE, KSPLIT>\n")
     f.write("kernel,launches,total_us,share\n")
     for n, (c, u) in sorted(agg.items(), key=lambda kv: -kv[1][1]):
         f.write(f'"{n}",{c},{u:.1f},{u / tot:.4f}\n')

@@ -1,5 +1,5 @@
-"""Time the d-sweeping 32 -> 32 conv kernel at the cfg-3 shape (B=16, 128^3) in its four configurations (GPU box):
-plain | + GroupNorm partial sums in the epilogue | + folded input GN+SiLU | both (+ residual)."""
+"""Time the d-sweeping 32 -> 32 conv kernel at the cfg-3 shape (B=16, 128^3) in three configurations (GPU box):
+plain | + GroupNorm partial sums in the epilogue | both + residual."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -13,8 +13,7 @@ res = torch.randn(B, S, S, S, 32, device=dev).to(L.ACT_DTYPE)
 w = torch.randn(3, 3, 3, 32, 32) * 0.03
 desc = ops.make_conv_desc(L.CONV_DIRECT, B, (S, S, S), 32, 0, 32, 3, 1, None, None)
 wp = ops.pack_conv_weights(desc, w, False).to(dev)
-mr = torch.stack([torch.zeros(B, 32), torch.ones(B, 32)], -1).to(dev)
-gamma, beta, bias = torch.ones(32, device=dev), torch.zeros(32, device=dev), torch.zeros(32, device=dev)
+bias = torch.zeros(32, device=dev)
 
 
 def timed(plan, n=5):
@@ -30,14 +29,12 @@ def timed(plan, n=5):
     return e0.elapsed_time(e1) / n
 
 
-for name, gn, xf, rs in (("plain", 0, 0, 0), ("gn partials", 1, 0, 0), ("input GN+SiLU", 0, 1, 0), ("both", 1, 1, 0), ("both + residual", 1, 1, 1)):
+for name, gn, rs in (("plain", 0, 0), ("gn partials", 1, 0), ("gn partials + residual", 1, 1)):
     y = torch.empty_like(x)
     plan = ops.ConvPlan(desc, x, wp, y, bias=bias, residual=res if rs else None)
     assert plan.info["halo"] == 3
     if gn:
         plan.gn_partials()
-    if xf:
-        assert plan.set_input_norm(mr, gamma, beta, 32, "silu")
     ms = timed(plan)
     fl = 2.0 * 27 * 32 * 32 * B * S ** 3
-    print(f"{name:18s} {ms:7.3f} ms  {fl / ms / 1e9:7.1f} TFLOP/s   flag {L.debug_flag()}")
+    print(f"{name:22s} {ms:7.3f} ms  {fl / ms / 1e9:7.1f} TFLOP/s   flag {L.debug_flag()}")
