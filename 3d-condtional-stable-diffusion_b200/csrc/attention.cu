@@ -363,23 +363,9 @@ flash_attn_kernel(const __grid_constant__ CUtensorMap mapQ, const __grid_constan
   }
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* f = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &f, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(f);
-  }
-  return fn;
-}
-
 // ld = row stride in elements (0 = d0: contiguous rows); lets Q / K be column blocks of one wider projection output
 int encode3(CUtensorMap* m, const void* ptr, uint64_t d0, uint64_t d1, uint64_t d2, uint32_t b0, uint32_t b1, uint64_t ld = 0) {
-  EncodeTiledFn enc = encode_fn();
+  EncodeTiledFn enc = b2_encode_tiled_fn();
   if (!enc) { b200dm_set_error("attention: cuTensorMapEncodeTiled unavailable"); return B200DM_ERR_CUDA; }
   if (ld == 0) ld = d0;
   cuuint64_t dims[3] = {d0, d1, d2};

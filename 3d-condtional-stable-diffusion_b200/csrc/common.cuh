@@ -1,5 +1,6 @@
 // Shared helpers for libb200dm (sm_100a only).
 #pragma once
+#include <cuda.h>
 #include <cuda_runtime.h>
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
@@ -70,15 +71,50 @@ __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;"
 
 bool b200dm_pdl_enabled();
 
+// cluster: CTAs per thread-block cluster along x (1 = no cluster)
 template <typename... KArgs, typename... Args>
-static inline cudaError_t b2_launch(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, Args... args) {
+static inline cudaError_t b2_launch_cluster(void (*kern)(KArgs...), dim3 grid, dim3 block, unsigned cluster, size_t smem, cudaStream_t s,
+                                            Args... args) {
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = s;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at; cfg.numAttrs = b200dm_pdl_enabled() ? 1 : 0;
+  cudaLaunchAttribute at[2];
+  unsigned n = 0;
+  if (cluster > 1) {
+    at[n].id = cudaLaunchAttributeClusterDimension;
+    at[n].val.clusterDim.x = cluster; at[n].val.clusterDim.y = 1; at[n].val.clusterDim.z = 1;
+    ++n;
+  }
+  if (b200dm_pdl_enabled()) {
+    at[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    at[n].val.programmaticStreamSerializationAllowed = 1;
+    ++n;
+  }
+  cfg.attrs = at; cfg.numAttrs = n;
   return cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
+}
+
+template <typename... KArgs, typename... Args>
+static inline cudaError_t b2_launch(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, Args... args) {
+  return b2_launch_cluster(kern, grid, block, 1u, smem, s, args...);
+}
+
+// ---- TMA descriptors ----------------------------------------------------------------------------------------------
+// Opt-in limit of one block's dynamic shared memory on sm_100 (227 KB).
+constexpr size_t kMaxDynamicSmem = 232448;
+
+// cuTensorMapEncodeTiled through the runtime's driver entry point (the library does not link libcuda); nullptr without a driver.
+typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
+                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
+                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+inline EncodeTiledFn b2_encode_tiled_fn() {
+  static EncodeTiledFn fn = nullptr;
+  if (!fn) {
+    void* f = nullptr;
+    cudaDriverEntryPointQueryResult q;
+    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &f, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
+      fn = reinterpret_cast<EncodeTiledFn>(f);
+  }
+  return fn;
 }
 
 // ---- small device helpers ------------------------------------------------------------------

@@ -20,8 +20,9 @@
 #include <cuda.h>
 #include <string.h>
 #include <math.h>
+#include <memory>
 #include <new>
-#include <vector>
+#include <utility>
 #include "conv_common.cuh"
 
 #include "conv_halo.cuh"
@@ -34,26 +35,41 @@ namespace {
 constexpr int kThreads = 192;
 constexpr int kABytes = 128 * 128;  // 128 rows x 64 bf16
 
+// Shared-memory layout of conv_igemm_kernel, offsets from the 1024-aligned base: NSTAGE x (A tile | B tile) | staged residual
+// tile (plans with a residual and the staged epilogue only) | barriers | TMEM address | bias + scale [2][BLOCK_N].
+template <int BLOCK_N, int NSTAGE>
+struct GemmSmem {
+  static constexpr int kStageBytes = kABytes + BLOCK_N * 128;
+  static constexpr int kResBytes = BLOCK_N >= 64 ? BLOCK_N * 256 : 0;   // 128 rows x BLOCK_N bf16 residual tile
+  // [0..NSTAGE) full, [NSTAGE..2NSTAGE) empty, [2NSTAGE] tmem_full, [2NSTAGE+1] residual tile (+1 keeps the bias 16-byte aligned)
+  static constexpr int kBars = 2 * NSTAGE + 3;
+  static constexpr size_t kRes = (size_t)NSTAGE * kStageBytes;
+  static constexpr size_t kTmemPtr = kBars * 8;       // from the barriers, as is the bias
+  static constexpr size_t kBias = kTmemPtr + 8;
+  __host__ __device__ static constexpr size_t bar_off(bool staged_res) { return kRes + (staged_res ? kResBytes : 0); }
+  // with the alignment slack; 16 bytes are reserved for the 8-byte TMEM address
+  static constexpr size_t bytes(bool staged_res) { return 1024 + bar_off(staged_res) + kTmemPtr + 16 + 2 * BLOCK_N * 4; }
+};
+
 // KSPLIT: split-K cluster (K range per CTA, partial accumulators reduced through distributed shared memory by the cluster's
 // first CTA); four-stage instantiations only.
-// (two-stage instantiations: registers capped so that four CTAs share an SM -- see conv_plan_create)
+// (two-stage instantiations: registers capped so that four CTAs share an SM -- see select_variant)
 template <int BLOCK_N, int NSTAGE, bool KSPLIT>
 __global__ void __launch_bounds__(kThreads, NSTAGE == 2 ? 4 : 1)
 conv_igemm_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant__ CUtensorMap mapA1,
                   const __grid_constant__ CUtensorMap mapB, const __grid_constant__ ConvOutMaps om, const ConvParams p) {
-  constexpr int kBBytes = BLOCK_N * 128;
-  constexpr int kStageBytes = kABytes + kBBytes;
+  using L = GemmSmem<BLOCK_N, NSTAGE>;
+  constexpr int kStageBytes = L::kStageBytes;
   constexpr uint32_t kTmemCols = BLOCK_N < 32 ? 32 : BLOCK_N;
-  constexpr int kResBytes = BLOCK_N >= 64 ? BLOCK_N * 256 : 0;   // staged epilogue: 128 rows x BLOCK_N bf16 residual tile
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   const bool staged = BLOCK_N >= 64 && p.tma_epi != 0;
   const bool staged_res = staged && p.residual != nullptr;
-  uint8_t* res_smem = smem + NSTAGE * kStageBytes;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(res_smem + (staged_res ? kResBytes : 0));
-  // bars[0..NSTAGE) full, [NSTAGE..2NSTAGE) empty, [2NSTAGE] tmem_full, [2NSTAGE+1] residual tile; then tmem ptr
-  uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(bars + 2 * NSTAGE + 3);   // (+3 keeps bias_s 16-byte aligned)
-  float* bias_s = reinterpret_cast<float*>(tmem_ptr_smem + 2);   // [2][BLOCK_N]: bias (+temb), output-affine scale
+  uint8_t* res_smem = smem + L::kRes;
+  uint8_t* bar_smem = smem + L::bar_off(staged_res);
+  uint64_t* bars = reinterpret_cast<uint64_t*>(bar_smem);
+  uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(bar_smem + L::kTmemPtr);
+  float* bias_s = reinterpret_cast<float*>(bar_smem + L::kBias);   // [2][BLOCK_N]: bias (+temb), output-affine scale
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const uint32_t smem_base = ptx::smem_u32(smem);
@@ -352,28 +368,14 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_consta
 }
 
 // ------------------------------------------------------------------------------------------ host side
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-EncodeTiledFn get_encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* f = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &f, cudaEnableDefault, &q) == cudaSuccess &&
-        q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(f);
-  }
-  return fn;
-}
-
 int pow2_ceil(int v) { int r = 1; while (r < v) r <<= 1; return r; }
 
 struct Geometry {
   int ntaps, pad, groups, nch0, nch1, n_pad, block_n;
   int out_d, out_h, out_w, m_d, m_h, m_w;
   int box_w, box_h, box_d, box_n;
+  int tiles_w, tiles_h, tiles_d, tiles_n;   // M tiles of the per-tap GEMM kernel
+  long long mtiles;
   size_t ktot;
 };
 
@@ -431,6 +433,9 @@ int compute_geometry(const b200dm_conv_desc* d, Geometry* g) {
     int bn = 128 / (bw * bh * bd);
     g->box_w = bw; g->box_h = bh; g->box_d = bd; g->box_n = bn;
   }
+  g->tiles_w = (g->m_w + g->box_w - 1) / g->box_w; g->tiles_h = (g->m_h + g->box_h - 1) / g->box_h;
+  g->tiles_d = (g->m_d + g->box_d - 1) / g->box_d; g->tiles_n = (d->batch + g->box_n - 1) / g->box_n;
+  g->mtiles = (long long)g->tiles_w * g->tiles_h * g->tiles_d * g->tiles_n;
   return B200DM_OK;
 }
 
@@ -448,32 +453,228 @@ uint16_t f32_to_bf16_rne(float f) {   // fp32 -> the library's 16-bit storage ty
   return (uint16_t)(u >> 16);
 }
 
+// ------------------------------------------------------------------------------------------ kernel selection
+enum class Family { kGemm, kHalo, kHaloUp, kSweep, kStencil };   // per-tap GEMM, conv_halo.cuh, conv_halo_up.cuh, conv_sweep.cuh, conv_stencil.cuh
+
+// Template arguments of one kernel instantiation (fields a family does not have stay 0 / false).
+struct KernelKey {
+  Family family;
+  int block_n;                           // BLOCK_N (sweep, stencil: 0)
+  int td, ns, nb, tps;                   // halo kernels: TD, slab ring depth NS, weight ring depth NB, taps per weight stage TPS
+  int nstage;                            // per-tap GEMM: NSTAGE
+  bool staged, pair, cg2, fuse, ksplit;  // halo kernels: STAGED, PAIR, CG2, FUSE_UPD; per-tap GEMM: KSPLIT
+};
+constexpr bool operator==(const KernelKey& a, const KernelKey& b) {
+  return a.family == b.family && a.block_n == b.block_n && a.td == b.td && a.ns == b.ns && a.nb == b.nb && a.tps == b.tps &&
+         a.nstage == b.nstage && a.staged == b.staged && a.pair == b.pair && a.cg2 == b.cg2 && a.fuse == b.fuse && a.ksplit == b.ksplit;
+}
+
+// What a plan runs: the instantiation and the runtime choices that go with it.
+struct Variant {
+  KernelKey key;
+  bool staged_epi;   // staged epilogue: 16-bit or fp32 tile -> swizzled smem -> TMA store (halo kernels: = key.staged)
+  bool swap_ab;      // per-tap GEMM: transposed store by operand swap (D^T = W X^T)
+  int ksplit;        // per-tap GEMM: CTAs (one cluster) per tile, each owning a K range; 1 = off
+  int dstep;         // halo kernels: output planes per tile (the pair tiles' d step is 2 with TD = 1)
+  int wbox[3];       // weight-map box {channels, rows, k-blocks}; k-blocks = 0: 2-D map; channels = 0: no map
+};
+
+constexpr int kHaloNS = 6;         // slab ring depth, direct-store epilogue
+constexpr int kHaloNSStaged = 5;   // staged epilogue: one slab less, the room holds the output staging tiles
+// N <= 32 tiles have small weight stages and 16 KB of staging: room for the 6th slab.  With 5 (4 live per 2-plane tile) the
+// issuers waited ~1000 cycles per 8000-cycle tile for the first two slabs of the next tile (tools/conv_trace.py, 128^3 32 -> 32).
+constexpr int halo_ns_for(int block_n, bool staged) { return staged && block_n > 32 ? kHaloNSStaged : kHaloNS; }
+constexpr int kHaloNSPair = 4;    // pair slabs are 25 KB; three per channel chunk are live
+constexpr int kHaloNSWide = 4;
+constexpr int kHaloNSFused = 4;   // the 16-bit staging tiles of the fused update take the room of the fifth slab
+
+// tiles of tw x th x td voxels over the input volume, all samples
+long long halo_tiles(const b200dm_conv_desc* d, int tw, int th, int td) {
+  return (long long)((d->in_w + tw - 1) / tw) * ((d->in_h + th - 1) / th) * ((d->in_d + td - 1) / td) * d->batch;
+}
+
+// The kernel choice, as one ordered list of rules.  Pure: reads the descriptor, the geometry, which operands are present and
+// the SM count; encodes no map and allocates nothing.
+Variant select_variant(const b200dm_conv_desc* d, const Geometry& g, bool residual, bool prelu, bool chan_bias) {
+  const int post_act = d->reserved[0];
+  const bool transposed_store = d->reserved[1] != 0;
+  const bool f32 = d->y_dtype == B200DM_F32;   // (else the 16-bit storage type)
+  const bool parity = d->mode == B200DM_CONV_PARITY;
+  const bool conv3 = d->mode == B200DM_CONV_DIRECT && d->ksize == 3 && d->stride == 1;
+  const bool halo_ok = d->use_halo >= 0 && !transposed_store;   // use_halo = -1: per-tap GEMM kernel only
+  const bool plane_8x16 = d->in_w >= 8 && d->in_h >= 16;          // planes that fill the halo kernels' 8w x 16h tile
+  const bool plane_8x8 = d->in_w == 8 && d->in_h == 8;
+  Variant v = {};
+  KernelKey& k = v.key;
+  v.ksplit = 1;
+  // 1. C_out = 1, C_in = 32, 3^3 stride 1 (the vqgan_attn_cp decoder's head): HBM-bound stencil-reduce kernel instead of an
+  //    N = 16 tensor-core tile (conv_stencil.cuh); bias + activation epilogue only
+  if (halo_ok && conv3 && d->c_out == 1 && d->c0 == stencil::kC && d->c1 == 0 && !chan_bias && !residual && !prelu &&
+      post_act == B200DM_ACT_NONE) {
+    k.family = Family::kStencil;
+    return v;
+  }
+  // 2. C_in = C_out = 32, 3^3 stride 1, 16-bit output (the decoders' 128^3 / 64^3 residual units): d-sweeping kernel with the
+  //    three kd taps of an input plane as one N = 96 MMA and the weight set resident in shared memory (conv_sweep.cuh)
+  if (halo_ok && conv3 && d->c_out == 32 && d->c0 == 32 && d->c1 == 0 && !f32 && !chan_bias && !prelu && plane_8x16 && d->in_d >= 2) {
+    k.family = Family::kSweep;
+    v.staged_epi = true;
+    v.wbox[0] = 32; v.wbox[1] = 32; v.wbox[2] = 1;
+    return v;
+  }
+  k.family = Family::kGemm;
+  k.block_n = g.block_n;
+  // 3. halo-reuse kernel: 3^3 stride-1 convs on volumes that fill its 8w x 16h tile
+  if (halo_ok && conv3 && plane_8x16) {
+    k.family = Family::kHalo;
+  // 4. 8 x 8 planes (the U-Net's deepest level): pair-slab tiles, 64 output channels per CTA so that >= 128 CTAs share the
+  //    weight stream; 16-bit staged output only
+  } else if (halo_ok && conv3 && plane_8x8 && d->in_d >= 2 && !f32 && d->c_out % 64 == 0 && !prelu) {
+    k.family = Family::kHalo;
+    k.pair = true;
+    k.block_n = 64;
+  // 5. x2 up-convolutions (nearest-upsample + conv3, ConvT k4 s2) on low-resolution planes that fill the 8 x 16 halo tile, with an
+  //    even tile count (CTA pairs).  C_out = 32 (the decoders' last ConvT, 64 -> 32 at 64^3 -> 128^3) runs N = 32 tiles with
+  //    64-byte staged rows
+  } else if (halo_ok && parity && plane_8x16 && d->in_d >= 2 && (d->c_out % 64 == 0 || d->c_out == 32) && !f32 && !residual &&
+             !prelu && halo_tiles(d, 8, 16, 2) % 2 == 0) {
+    k.family = Family::kHaloUp;
+  // 6. the same on 8 x 8 low-resolution planes (8^3 -> 16^3): pair-slab tiles
+  } else if (halo_ok && parity && plane_8x8 && d->in_d >= 2 && d->in_d % 2 == 0 && d->c_out % 64 == 0 && !f32 && !residual &&
+             !prelu && halo_tiles(d, 8, 8, 2) % 2 == 0) {
+    k.family = Family::kHaloUp;
+    k.pair = true;
+  }
+  const bool halo = k.family != Family::kGemm;
+  // 7. staged (TMA-store) epilogue: whole 64-channel groups; fp32 output (the U-Net's eps) on the halo kernels only, in 32-column
+  //    groups; on the halo kernels also C_out = 32 as one 32-channel group of 64-byte rows, SWIZZLE_64B (the decoders' 128^3 convs)
+  const bool n32 = halo && !k.pair && d->c_out == 32 && !f32;
+  v.staged_epi = (!f32 || halo) && !transposed_store && !prelu && (d->c_out % 64 == 0 || n32) && !(parity && residual);
+  // 8. per-sample transposed store by operand swap (see the kernel): tiles of whole planes inside one sample, bias only
+  if (transposed_store && d->mode == B200DM_CONV_DIRECT && d->ksize == 1 && d->stride == 1 && !f32 && g.block_n == 128 &&
+      g.box_n == 1 && g.box_w == g.m_w && g.box_h == g.m_h && g.m_d % g.box_d == 0 && ((long long)g.m_w * g.m_h * g.m_d) % 8 == 0 &&
+      !residual && !prelu && !chan_bias && d->act == B200DM_ACT_NONE && post_act == B200DM_ACT_NONE) {
+    v.swap_ab = true;
+    v.staged_epi = true;
+  }
+  const long long sms = b2_num_sms();
+  const int ntiles = g.n_pad / k.block_n;
+  if (k.family == Family::kGemm) {
+    const int nkb = (g.nch0 + g.nch1) * g.ntaps;
+    const long long ctas = g.mtiles * (d->mode == B200DM_CONV_BATCHED_GEMM ? (d->c_out + k.block_n - 1) / k.block_n : ntiles) *
+                           (parity ? 8 : 1);
+    // 9. split-K: when the tile grid leaves most SMs idle and K is long, ksplit CTAs (one cluster) share a tile.  Each CTA
+    //    streams its K range at the per-SM operand rate (~40 B/clk), so an under-filled grid is K-latency-bound otherwise.
+    if (!transposed_store)
+      while (v.ksplit < 8 && ctas * (v.ksplit * 2) <= sms && nkb / (v.ksplit * 2) >= 13) v.ksplit *= 2;   // >= 13 k-blocks per CTA: 3^3 convs only
+    k.ksplit = v.ksplit > 1;
+    // 10. pipeline depth 4; measured on B200: a deeper ring (6 stages at BLOCK_N=128, 8 below) does not help at BLOCK_N=128 (the
+    //     operand stream is bandwidth-, not latency-bound) and hurts below 128, where 4 stages let two CTAs share an SM
+    k.nstage = 4;
+    // 11. short K loops (1^3 convs: 1-3 k-blocks) never fill four stages; two stages let 3-4 CTAs share an SM, which hides the
+    //     per-CTA prologue / TMA latency / epilogue of these HBM-bound launches
+    if (nkb <= 3 && k.block_n >= 64) k.nstage = 2;
+    // 12. grids of several waves: two stages x three co-resident CTAs keep more operand bytes in flight per SM than one CTA with
+    //     four stages, and hide every CTA's prologue / epilogue (measured: 16^3 128->128 parity conv 123 -> 77 us, 8^3 MLP GEMM
+    //     17.5 -> 12.7 us; a single-wave split-K grid gets slower, so it keeps four stages)
+    if (ctas >= 2 * sms && k.block_n >= 64 && v.ksplit <= 1) k.nstage = 2;
+    // (split-K needs >= 26 k-blocks, rule 11 <= 3: no split-K plan has two stages, and no such kernel is instantiated)
+    v.wbox[0] = 64; v.wbox[1] = k.block_n; v.wbox[2] = 0;
+    return v;
+  }
+  k.staged = v.staged_epi;
+  if (k.family == Family::kHaloUp) {
+    // 13. up-convolutions: CTA pairs, two planes per tile, 4-tap weight stages; ring depths by BLOCK_N
+    k.cg2 = true;
+    v.dstep = 2;
+    k.ns = k.pair ? 4 : 5;
+    k.nb = k.block_n == 32 ? 4 : (k.block_n == 64 ? 3 : 2);
+    k.tps = 4;
+  } else {
+    // 14. planes per tile: 2 (weight stage shared by two planes, two MMA issuer warps) unless that costs a wave
+    const long long cost2 = (halo_tiles(d, 8, 16, 2) * ntiles + sms - 1) / sms * 2, cost1 = (halo_tiles(d, 8, 16, 1) * ntiles + sms - 1) / sms;
+    const int td = d->in_d >= 2 && cost2 <= cost1 ? 2 : 1;
+    v.dstep = k.pair ? 2 : td;   // (pair tiles: d step 2, one accumulator)
+    k.td = k.pair ? 1 : td;
+    // 15. weight-ring depth / taps per stage by BLOCK_N (smem: 6 slabs x 23 KB + NB x TPS x BLOCK_N x 128 B <= 227 KB)
+    k.nb = k.block_n == 64 ? 3 : 4;
+    k.tps = k.block_n >= 128 ? 1 : 3;
+    k.ns = k.pair ? kHaloNSPair : halo_ns_for(k.block_n, k.staged);
+    // 16. BLOCK_N = 128 with the staged epilogue: one-tap weight stages hold only 8 MMAs (4 per issuer warp) and the per-stage
+    //     barrier round trip (~200 cycles) made those convs issue-bound (45 % of the MMA floor); 3-tap stages x 2 fit once the
+    //     slab ring is the 4 slabs a channel chunk needs (the next chunk's slab i reloads as soon as slab i is released).
+    if (!k.pair && k.block_n == 128 && k.staged) { k.nb = 2; k.tps = 3; k.ns = kHaloNSWide; }
+    // 17. CTA pairs (cta_group::2) for every staged halo configuration with 64- or 128-channel tiles, and for N = 32 convs with at
+    //     least two channel chunks (the U-Net's input conv, 256 -> 32, direct stores): needs an even tile count per n-tile so that
+    //     the two CTAs of a pair always work on the same n-tile and run the same number of tiles.  Short-K N = 32 convs (one
+    //     channel chunk) stay single-CTA: with direct stores pairing couples two epilogues (measured 4.18 -> 4.79 ms), staged it
+    //     gained 3.79 -> 3.74 ms only.
+    const bool cg2_n32 = k.block_n == 32 && !k.pair && td == 2 && g.nch0 + g.nch1 >= 2;
+    const bool cg2_wide = (k.block_n == 64 || k.block_n == 128) && k.staged && (k.pair || td == 2 || k.block_n == 128);
+    if ((cg2_wide || cg2_n32) && halo_tiles(d, 8, k.pair ? 8 : 16, v.dstep) % 2 == 0) {
+      k.cg2 = true;
+      k.nb = cg2_n32 ? 4 : 3;
+      k.tps = 3;
+      k.ns = k.pair ? kHaloNSPair : halo_ns_for(k.block_n, k.staged);
+    }
+  }
+  // packed weights viewed as {64, rows, k-blocks}: one box = TPS consecutive taps of this CTA's rows (a CTA pair: half each)
+  v.wbox[0] = 64; v.wbox[1] = k.cg2 ? k.block_n / 2 : k.block_n; v.wbox[2] = k.tps;
+  return v;
+}
+
+// NDHWC tensor of c channels and extent (w, h, d, n) as a 5-D TMA map.  step: voxels per map coordinate along W, H, D (2: one
+// output parity of a x2 up-convolution, the map spans half the extent); estride: TMA element stride (a stride-2 conv's
+// input); dh_order: dims listed (C, W, D, H, N), so that a box lands as rows [h][d][w] (pair slabs).
+int encode_act(EncodeTiledFn enc, CUtensorMap* m, const char* what, const void* base, CUtensorMapDataType dt, int c, int w, int h,
+               int d, int n, const cuuint32_t (&box)[5], CUtensorMapSwizzle swz, int step = 1, cuuint32_t estride = 1,
+               bool dh_order = false) {
+  const cuuint64_t sw = (cuuint64_t)c * (dt == CU_TENSOR_MAP_DATA_TYPE_FLOAT32 ? 4 : 2), sh = sw * w, sd = sh * h, sn = sd * d;
+  cuuint64_t dims[5] = {(cuuint64_t)c, (cuuint64_t)(w / step), (cuuint64_t)(h / step), (cuuint64_t)(d / step), (cuuint64_t)n};
+  cuuint64_t strides[4] = {sw * step, sh * step, sd * step, sn};
+  if (dh_order) { std::swap(dims[2], dims[3]); std::swap(strides[1], strides[2]); }
+  const cuuint32_t es[5] = {1, estride, estride, estride, 1};
+  const CUresult r = enc(m, dt, 5, const_cast<void*>(base), dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE, swz,
+                         CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) {
+    b200dm_set_error("cuTensorMapEncodeTiled(%s) failed: %d (C=%d dims %d,%d,%d,%d box %u,%u,%u,%u)", what, (int)r, c, w, h, d, n,
+                     box[1], box[2], box[3], box[4]);
+    return B200DM_ERR_CUDA;
+  }
+  return B200DM_OK;
+}
+
+// packed weights [groups * n_pad rows][ktot / 64 k-blocks][64] as the 3-D view {64, rows, k-blocks}; a box row of 64 (32)
+// channels is one 128-byte (64-byte) swizzle span
+int encode_weights3(EncodeTiledFn enc, CUtensorMap* m, const void* w, const Geometry& g, const int (&box)[3]) {
+  const cuuint64_t dims[3] = {64, (cuuint64_t)g.groups * g.n_pad, (cuuint64_t)(g.ktot / 64)};
+  const cuuint64_t strides[2] = {(cuuint64_t)g.ktot * 2, 128};
+  const cuuint32_t b[3] = {(cuuint32_t)box[0], (cuuint32_t)box[1], (cuuint32_t)box[2]}, es[3] = {1, 1, 1};
+  const CUresult r = enc(m, kTmapAct16, 3, const_cast<void*>(w), dims, strides, b, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                         box[0] == 64 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                         CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) { b200dm_set_error("cuTensorMapEncodeTiled(B) failed: %d (box %d,%d,%d)", (int)r, box[0], box[1], box[2]); return B200DM_ERR_CUDA; }
+  return B200DM_OK;
+}
+
+struct Instance;
+
 }  // namespace
 
 struct b200dm_conv_plan {
   b200dm_conv_desc desc;
   Geometry g;
+  Variant v;
+  const Instance* inst;   // the instantiation v.key names
   ConvParams p;
   CUtensorMap mapA0, mapA1, mapB;
   ConvOutMaps om;
+  CUtensorMap mapS;       // stencil / sweep kernels: the input (mapB = the sweep kernel's weights, om.y[0] its output)
+  stencil::Params sp;
+  sweep::Params wp;
   dim3 grid;
   size_t smem;
-  int nstage;
   double flops;
-  bool halo = false;
-  bool ups = false;    // x2 up-convolution (PARITY mode) on the halo / CTA-pair machinery (conv_halo_up.cuh)
-  bool cg2 = false;    // halo kernel, BLOCK_N = 64, two planes, staged: CTA pairs (cta_group::2), see conv_halo.cuh
-  bool wide = false;   // halo kernel, BLOCK_N = 128, staged: 3-tap weight stages x 2, 4 slabs (see conv_plan_create)
-  bool pair = false;   // halo kernel on 8 x 8 planes: 8w x 8h x 2d tiles from pair slabs (conv_halo.cuh)
-  int halo_td = 1, halo_nb = 4, halo_tps = 1;
-  int halo_ns = 0;     // slab ring depth when a variant fixes it (0 = by epilogue kind)
-  const CUtensorMap& residual_map() const { return p.residual ? om.r : om.y[0]; }   // (a valid map either way: unused without a residual)
-  bool fuse = false;   // CTA-pair N = 128 fp32 conv with the reverse-diffusion update fused into its epilogue (set_fused_update)
-  bool stencil = false;   // C_out = 1, C_in = 32 3^3 conv: HBM-bound stencil-reduce kernel (conv_stencil.cuh)
-  stencil::Params sp;
-  CUtensorMap mapS;
-  bool sweep = false;     // C_in = C_out = 32 3^3 conv: d-sweeping N = 96 kernel (conv_sweep.cuh); mapS = input, mapB = weights, om.y[0] = output
-  sweep::Params wp;
 };
 
 static int* g_dbg_flag = nullptr;
@@ -558,169 +759,257 @@ extern "C" int b200dm_conv_pack_weights(const b200dm_conv_desc* d, const float* 
   return B200DM_OK;
 }
 
-static size_t conv_smem_bytes(int block_n, int nstage, bool staged_res) {
-  return 1024 + (size_t)nstage * (kABytes + block_n * 128) + (staged_res ? (size_t)block_n * 256 : 0) +
-         (2 * nstage + 3) * 8 + 16 + 2 * block_n * 4;
+namespace {
+
+// ------------------------------------------------------------------------------------------ kernel instantiations
+// Kernel arguments, by kernel signature.
+template <typename... KArgs, typename... Args>
+cudaError_t launch_plan(void (*k)(KArgs...), const b200dm_conv_plan* pl, unsigned threads, cudaStream_t s, Args... args) {
+  const unsigned cluster = pl->v.key.cg2 ? 2u : (unsigned)pl->v.ksplit;
+  return b2_launch_cluster(k, pl->grid, dim3(threads), cluster, pl->smem, s, args...);
+}
+// per-tap GEMM, halo up-convolution
+cudaError_t launch_args(void (*k)(CUtensorMap, CUtensorMap, CUtensorMap, ConvOutMaps, ConvParams), const b200dm_conv_plan* pl,
+                        unsigned threads, cudaStream_t s) {
+  return launch_plan(k, pl, threads, s, pl->mapA0, pl->mapA1, pl->mapB, pl->om, pl->p);
+}
+// halo kernel: output map (the fused update: x_{t-1}) and its 16-bit copy
+cudaError_t launch_args(void (*k)(CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, ConvParams),
+                        const b200dm_conv_plan* pl, unsigned threads, cudaStream_t s) {
+  return launch_plan(k, pl, threads, s, pl->mapA0, pl->mapA1, pl->mapB, pl->om.y[0], pl->om.y[1], pl->p);
+}
+// sweep kernel: input, weights, output, residual (a valid map either way: unused without a residual)
+cudaError_t launch_args(void (*k)(CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, ConvParams, sweep::Params),
+                        const b200dm_conv_plan* pl, unsigned threads, cudaStream_t s) {
+  return launch_plan(k, pl, threads, s, pl->mapS, pl->mapB, pl->om.y[0], pl->p.residual ? pl->om.r : pl->om.y[0], pl->p, pl->wp);
+}
+cudaError_t launch_args(void (*k)(CUtensorMap, stencil::Params), const b200dm_conv_plan* pl, unsigned threads, cudaStream_t s) {
+  return launch_plan(k, pl, threads, s, pl->mapS, pl->sp);
 }
 
-static size_t conv_smem_attr(int block_n, int nstage) {   // opt-in ceiling of one kernel instantiation
-  const size_t v = conv_smem_bytes(block_n, nstage, true);
-  return v > 232448 ? 232448 : v;
-}
+struct Instance {
+  KernelKey key;
+  unsigned threads;
+  size_t smem, smem_res;   // dynamic shared memory; smem_res: with the per-tap GEMM kernel's staged residual tile
+  int (*launch)(const b200dm_conv_plan*, cudaStream_t);
+  cudaError_t (*set_max_smem)(int bytes);
+};
 
+template <auto K>
+int launch(const b200dm_conv_plan* pl, cudaStream_t s) {
+  B2_CHECK_CUDA(launch_args(K, pl, pl->inst->threads, s));
+  return B200DM_OK;
+}
+template <auto K>
+cudaError_t set_max_smem(int bytes) { return cudaFuncSetAttribute(K, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes); }
+
+template <auto K>
+constexpr Instance instance(KernelKey key, unsigned threads, size_t smem, size_t smem_res) {
+  return {key, threads, smem, smem_res, &launch<K>, &set_max_smem<K>};
+}
 template <int BLOCK_N, int NSTAGE, bool KSPLIT>
-static int launch_conv(const b200dm_conv_plan* pl, cudaStream_t s) {
-  static_assert(!KSPLIT || NSTAGE == 4, "split-K runs four stages only");
-  auto kern = conv_igemm_kernel<BLOCK_N, NSTAGE, KSPLIT>;
-  static bool attr_set = false;
-  if (!attr_set) {
-    B2_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)conv_smem_attr(BLOCK_N, NSTAGE)));
-    attr_set = true;
-  }
-  if constexpr (KSPLIT) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = pl->grid; cfg.blockDim = dim3(kThreads); cfg.dynamicSmemBytes = pl->smem; cfg.stream = s;
-    cudaLaunchAttribute at[2];
-    at[0].id = cudaLaunchAttributeClusterDimension;
-    at[0].val.clusterDim.x = pl->p.ksplit; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-    at[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[1].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = at; cfg.numAttrs = b200dm_pdl_enabled() ? 2 : 1;
-    B2_CHECK_CUDA(cudaLaunchKernelEx(&cfg, kern, pl->mapA0, pl->mapA1, pl->mapB, pl->om, pl->p));
-  } else {
-    B2_CHECK_CUDA(b2_launch(kern, pl->grid, dim3(kThreads), pl->smem, s, pl->mapA0, pl->mapA1, pl->mapB, pl->om, pl->p));
-  }
-  return B200DM_OK;
+constexpr Instance gemm() {
+  using L = GemmSmem<BLOCK_N, NSTAGE>;
+  return instance<conv_igemm_kernel<BLOCK_N, NSTAGE, KSPLIT>>(
+      {Family::kGemm, BLOCK_N, 0, 0, 0, 0, NSTAGE, false, false, false, false, KSPLIT}, kThreads, L::bytes(false), L::bytes(true));
 }
-
-constexpr int kHaloNS = 6;         // slab ring depth, direct-store epilogue
-constexpr int kHaloNSStaged = 5;   // staged epilogue: one slab less, the room holds the output staging tiles
-// N <= 32 tiles have small weight stages and 16 KB of staging: room for the 6th slab.  With 5 (4 live per 2-plane tile) the
-// issuers waited ~1000 cycles per 8000-cycle tile for the first two slabs of the next tile (tools/conv_trace.py, 128^3 32 -> 32).
-constexpr int halo_ns_for(int block_n, bool staged) { return staged && block_n > 32 ? kHaloNSStaged : kHaloNS; }
-
-template <int BLOCK_N, int TD, int NB, int TPS, bool STAGED>
-static int launch_halo(const b200dm_conv_plan* pl, cudaStream_t s) {
-  auto kern = halo::conv_halo_kernel<BLOCK_N, TD, halo_ns_for(BLOCK_N, STAGED), NB, TPS, STAGED>;
-  static bool attr_set = false;
-  if (!attr_set) {
-    B2_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl->smem));
-    attr_set = true;
-  }
-  B2_CHECK_CUDA(b2_launch(kern, pl->grid, dim3(halo::kThreads), pl->smem, s, pl->mapA0, pl->mapA1, pl->mapB, pl->om.y[0], pl->om.y[1], pl->p));
-  return B200DM_OK;
+template <int BLOCK_N, int TD, int NS, int NB, int TPS, bool STAGED, bool PAIR = false, bool CG2 = false, bool FUSE_UPD = false>
+constexpr Instance halo_conv() {
+  constexpr size_t kBytes = halo::Smem<BLOCK_N, NS, NB, TPS, STAGED, PAIR, CG2, FUSE_UPD>::kBytes;
+  return instance<halo::conv_halo_kernel<BLOCK_N, TD, NS, NB, TPS, STAGED, PAIR, CG2, FUSE_UPD>>(
+      {Family::kHalo, BLOCK_N, TD, NS, NB, TPS, 0, STAGED, PAIR, CG2, FUSE_UPD, false}, FUSE_UPD ? halo::kThreadsFused : halo::kThreads,
+      kBytes, kBytes);
 }
-
 template <int BLOCK_N, int NS, int NB, bool PAIR = false>
-static int launch_halo_up(const b200dm_conv_plan* pl, cudaStream_t s) {
-  auto kern = halo::conv_halo_up_kernel<BLOCK_N, NS, NB, PAIR>;
-  static bool attr_set = false;
-  if (!attr_set) {
-    B2_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl->smem));
-    attr_set = true;
+constexpr Instance halo_up() {
+  constexpr size_t kBytes = halo::UpSmem<BLOCK_N, NS, NB, PAIR>::kBytes;
+  return instance<halo::conv_halo_up_kernel<BLOCK_N, NS, NB, PAIR>>(
+      {Family::kHaloUp, BLOCK_N, 0, NS, NB, 4, 0, true, PAIR, true, false, false}, halo::kThreads, kBytes, kBytes);
+}
+
+// Every conv kernel instantiation, each a configuration select_variant can return.  A key without an entry is an error.
+constexpr Instance kInstances[] = {
+    instance<stencil::conv_stencil_c1_kernel>({Family::kStencil}, stencil::kThreads, stencil::kSmem, stencil::kSmem),
+    instance<sweep::conv_sweep32_kernel>({Family::kSweep}, sweep::kThreads, sweep::kSmem, sweep::kSmem),
+    gemm<16, 4, false>(), gemm<32, 4, false>(), gemm<64, 4, false>(), gemm<128, 4, false>(),
+    gemm<64, 2, false>(), gemm<128, 2, false>(),
+    gemm<16, 4, true>(), gemm<32, 4, true>(), gemm<64, 4, true>(), gemm<128, 4, true>(),
+    // one CTA per tile
+    halo_conv<16, 1, kHaloNS, 4, 3, false>(), halo_conv<16, 2, kHaloNS, 4, 3, false>(),
+    halo_conv<32, 1, kHaloNS, 4, 3, false>(), halo_conv<32, 2, kHaloNS, 4, 3, false>(),
+    halo_conv<32, 1, kHaloNS, 4, 3, true>(), halo_conv<32, 2, kHaloNS, 4, 3, true>(),
+    halo_conv<64, 1, kHaloNS, 3, 3, false>(), halo_conv<64, 2, kHaloNS, 3, 3, false>(),
+    halo_conv<64, 1, kHaloNSStaged, 3, 3, true>(), halo_conv<64, 2, kHaloNSStaged, 3, 3, true>(),
+    halo_conv<128, 1, kHaloNS, 4, 1, false>(), halo_conv<128, 2, kHaloNS, 4, 1, false>(),
+    halo_conv<128, 1, kHaloNSWide, 2, 3, true>(), halo_conv<128, 2, kHaloNSWide, 2, 3, true>(),
+    halo_conv<64, 1, kHaloNSPair, 3, 3, true, true>(),
+    // CTA pairs
+    halo_conv<32, 2, kHaloNS, 4, 3, false, false, true>(), halo_conv<32, 2, kHaloNS, 4, 3, true, false, true>(),
+    halo_conv<64, 2, kHaloNSStaged, 3, 3, true, false, true>(),
+    halo_conv<128, 1, kHaloNSStaged, 3, 3, true, false, true>(), halo_conv<128, 2, kHaloNSStaged, 3, 3, true, false, true>(),
+    halo_conv<64, 1, kHaloNSPair, 3, 3, true, true, true>(),
+    halo_conv<128, 1, kHaloNSFused, 3, 3, true, false, true, true>(), halo_conv<128, 2, kHaloNSFused, 3, 3, true, false, true, true>(),
+    halo_up<32, 5, 4>(), halo_up<64, 5, 3>(), halo_up<128, 5, 2>(), halo_up<64, 4, 3, true>(), halo_up<128, 4, 2, true>(),
+};
+
+// Binds the instantiation of `v` to the plan: its launcher and shared-memory size, and the kernel's opt-in shared-memory limit.
+// The plan is left unchanged on failure.
+int bind_kernel(b200dm_conv_plan* pl, const Variant& v) {
+  const Instance* inst = nullptr;
+  for (const Instance& i : kInstances)
+    if (i.key == v.key) { inst = &i; break; }
+  if (!inst) {
+    b200dm_set_error("conv_plan: no kernel instantiation for family %d, BLOCK_N %d", (int)v.key.family, v.key.block_n);
+    return B200DM_ERR_UNSUPPORTED;
   }
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = pl->grid; cfg.blockDim = dim3(halo::kThreads); cfg.dynamicSmemBytes = pl->smem; cfg.stream = s;
-  cudaLaunchAttribute at[2];
-  at[0].id = cudaLaunchAttributeClusterDimension;
-  at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-  at[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[1].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at; cfg.numAttrs = b200dm_pdl_enabled() ? 2 : 1;
-  B2_CHECK_CUDA(cudaLaunchKernelEx(&cfg, kern, pl->mapA0, pl->mapA1, pl->mapB, pl->om, pl->p));
+  if (inst->smem_res > kMaxDynamicSmem) { b200dm_set_error("conv_plan: %zu bytes of shared memory", inst->smem_res); return B200DM_ERR_UNSUPPORTED; }
+  B2_CHECK_CUDA(inst->set_max_smem((int)inst->smem_res));
+  pl->v = v;
+  pl->inst = inst;
+  pl->smem = v.staged_epi && pl->p.residual ? inst->smem_res : inst->smem;
   return B200DM_OK;
 }
 
-constexpr int kHaloNSPair = 4;   // pair slabs are 25 KB; three per channel chunk are live
-constexpr int kHaloNSWide = 4;
-
-template <int BLOCK_N, int TD, int NS, int NB, bool PAIR, bool STAGED = true>
-static int launch_halo_cg2(const b200dm_conv_plan* pl, cudaStream_t s) {
-  auto kern = halo::conv_halo_kernel<BLOCK_N, TD, NS, NB, 3, STAGED, PAIR, true>;
-  static bool attr_set = false;
-  if (!attr_set) {
-    B2_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl->smem));
-    attr_set = true;
+// Tensor maps and launch parameters of a plan whose pl->v is selected.
+int setup_plan(b200dm_conv_plan* pl, EncodeTiledFn enc, const void* x0, const void* x1, const void* w_packed, const float* bias,
+               const float* chan_bias, const int32_t* t_dev, const void* residual, const void* prelu_alpha, void* y) {
+  const b200dm_conv_desc* d = &pl->desc;
+  const Geometry& g = pl->g;
+  Variant& v = pl->v;
+  const KernelKey& k = v.key;
+  ConvParams& p = pl->p;
+  const long long sms = b2_num_sms();
+  int rc;
+  if (k.family == Family::kStencil) {
+    rc = encode_act(enc, &pl->mapS, "stencil X", x0, kTmapAct16, d->c0, d->in_w, d->in_h, d->in_d, d->batch,
+                    {(cuuint32_t)stencil::kC, (cuuint32_t)stencil::kHW, (cuuint32_t)stencil::kHH, 1, 1}, CU_TENSOR_MAP_SWIZZLE_64B);
+    if (rc) return rc;
+    stencil::Params& sp = pl->sp;
+    sp.batch = d->batch; sp.D = d->in_d; sp.H = d->in_h; sp.W = d->in_w;
+    sp.tiles_h = (d->in_h + stencil::kTH - 1) / stencil::kTH; sp.tiles_w = (d->in_w + stencil::kTW - 1) / stencil::kTW;
+    // d ranges: enough work items for ~6 per resident CTA (two CTAs per SM), each range >= 8 planes (2 halo planes per range)
+    const long long cols = (long long)d->batch * sp.tiles_h * sp.tiles_w, ctas = 2 * sms;
+    int dsplit = 1;
+    while (cols * dsplit < 6 * ctas && d->in_d / (dsplit * 2) >= 8) dsplit *= 2;
+    sp.dlen = (d->in_d + dsplit - 1) / dsplit; sp.dsplit = (d->in_d + sp.dlen - 1) / sp.dlen;
+    sp.items = (int)(cols * sp.dsplit);
+    sp.w = (const act_t*)w_packed; sp.bias = bias; sp.act = d->act; sp.y_f32 = d->y_dtype == B200DM_F32; sp.y = y; sp.dbg = g_dbg_flag;
+    pl->grid = dim3((unsigned)(sp.items < ctas ? sp.items : ctas), 1, 1);
+    return B200DM_OK;
   }
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = pl->grid; cfg.blockDim = dim3(halo::kThreads); cfg.dynamicSmemBytes = pl->smem; cfg.stream = s;
-  cudaLaunchAttribute at[2];
-  at[0].id = cudaLaunchAttributeClusterDimension;
-  at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-  at[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[1].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at; cfg.numAttrs = b200dm_pdl_enabled() ? 2 : 1;
-  B2_CHECK_CUDA(cudaLaunchKernelEx(&cfg, kern, pl->mapA0, pl->mapA1, pl->mapB, pl->om.y[0], pl->om.y[1], pl->p));
+  if (k.family == Family::kSweep) {
+    const cuuint32_t boxy[5] = {32, 8, 16, 1, 1};
+    rc = encode_act(enc, &pl->mapS, "sweep X", x0, kTmapAct16, 32, d->in_w, d->in_h, d->in_d, d->batch, {32, 10, 18, 2, 1},
+                    CU_TENSOR_MAP_SWIZZLE_64B);
+    if (!rc) rc = encode_act(enc, &pl->om.y[0], "sweep Y", y, kTmapAct16, 32, d->in_w, d->in_h, d->in_d, d->batch, boxy, CU_TENSOR_MAP_SWIZZLE_64B);
+    if (!rc) rc = encode_weights3(enc, &pl->mapB, w_packed, g, v.wbox);
+    if (!rc && residual)
+      rc = encode_act(enc, &pl->om.r, "sweep residual", residual, kTmapAct16, 32, d->in_w, d->in_h, d->in_d, d->batch, boxy, CU_TENSOR_MAP_SWIZZLE_64B);
+    if (rc) return rc;
+    sweep::Params& wp = pl->wp;
+    wp.D = d->in_d; wp.H = d->in_h; wp.W = d->in_w; wp.batch = d->batch;
+    wp.tiles_w = (d->in_w + 7) / 8; wp.tiles_h = (d->in_h + 15) / 16;
+    const long long cols = (long long)d->batch * wp.tiles_w * wp.tiles_h, ctas = sms;
+    int dsplit = 1;
+    while (cols * dsplit < 6 * ctas && d->in_d / (dsplit * 2) >= 8) dsplit *= 2;   // >= ~6 items per CTA, d ranges of >= 8 planes
+    wp.dlen = (d->in_d + dsplit - 1) / dsplit; wp.dsplit = (d->in_d + wp.dlen - 1) / wp.dlen;
+    wp.items = (int)(cols * wp.dsplit);
+    p.batch = d->batch; p.in_d = p.out_d = d->in_d; p.in_h = p.out_h = d->in_h; p.in_w = p.out_w = d->in_w;
+    p.c_out = 32; p.n_pad = 32; p.act = d->act; p.post_act = d->reserved[0];
+    p.bias = bias; p.residual = (const act_t*)residual; p.y = y; p.dbg = g_dbg_flag; p.tma_epi = 1;
+    pl->grid = dim3((unsigned)(wp.items < ctas ? wp.items : ctas), 1, 1);
+    return B200DM_OK;
+  }
+  // per-tap GEMM and halo kernels
+  if (g.mtiles > 0x7fffffffLL) { b200dm_set_error("conv_plan_create: too many tiles"); return B200DM_ERR_INVALID; }
+  const bool halo = k.family != Family::kGemm, up = k.family == Family::kHaloUp, f32 = d->y_dtype == B200DM_F32;
+  const bool parity = d->mode == B200DM_CONV_PARITY;
+  const int st = d->mode == B200DM_CONV_DIRECT ? d->stride : 1;
+  {  // activations: the GEMM tile's box shifted per tap, or one halo d-plane slab (pair slab: {64, 10, 2, 10, 1} as rows [h][d][w])
+    const cuuint32_t box[5] = {64, (cuuint32_t)(k.pair ? 10 : halo ? 10 : g.box_w * st), (cuuint32_t)(k.pair ? 2 : halo ? 18 : g.box_h * st),
+                               (cuuint32_t)(k.pair ? 10 : halo ? 1 : g.box_d * st), (cuuint32_t)(halo ? 1 : g.box_n)};
+    rc = encode_act(enc, &pl->mapA0, "A", x0, kTmapAct16, d->c0, d->in_w, d->in_h, d->in_d, d->batch, box, CU_TENSOR_MAP_SWIZZLE_128B, 1,
+                    (cuuint32_t)st, k.pair);
+    if (!rc) rc = encode_act(enc, &pl->mapA1, "A", d->c1 > 0 ? x1 : x0, kTmapAct16, d->c1 > 0 ? d->c1 : d->c0, d->in_w, d->in_h, d->in_d,
+                             d->batch, box, CU_TENSOR_MAP_SWIZZLE_128B, 1, (cuuint32_t)st, k.pair);
+    if (rc) return rc;
+  }
+  if (halo) {
+    rc = encode_weights3(enc, &pl->mapB, w_packed, g, v.wbox);
+    if (rc) return rc;
+  } else {
+    // packed [group][n_pad rows][K]; batched GEMM: B is a raw activation tensor [batch][c_out rows][K = c0] whose rows beyond c_out
+    // of a sample alias the next sample (masked by the epilogue's col < c_out), K beyond c0 is zero-filled by TMA
+    const bool bg = d->mode == B200DM_CONV_BATCHED_GEMM;
+    const cuuint64_t dims[2] = {bg ? (cuuint64_t)d->c0 : (cuuint64_t)g.ktot, bg ? (cuuint64_t)d->batch * d->c_out : (cuuint64_t)g.groups * g.n_pad};
+    const cuuint64_t strides[1] = {dims[0] * 2};
+    const cuuint32_t box[2] = {(cuuint32_t)v.wbox[0], (cuuint32_t)v.wbox[1]}, es[2] = {1, 1};
+    const CUresult r = enc(&pl->mapB, kTmapAct16, 2, const_cast<void*>(w_packed), dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                           CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (r != CUDA_SUCCESS) { b200dm_set_error("cuTensorMapEncodeTiled(B) failed: %d", (int)r); return B200DM_ERR_CUDA; }
+  }
+  if (v.swap_ab) {
+    // per-sample transposed output [n][channel][voxel]: one box = 64 voxels x 128 channels.  Should the encode fail, the plan
+    // keeps the scalar transposed store.
+    const cuuint64_t Lv = (cuuint64_t)g.m_w * g.m_h * g.m_d;
+    const cuuint64_t dims[5] = {Lv, (cuuint64_t)d->c_out, 1, 1, (cuuint64_t)d->batch};
+    const cuuint64_t strides[4] = {Lv * 2, Lv * d->c_out * 2, Lv * d->c_out * 2, Lv * d->c_out * 2};
+    const cuuint32_t box[5] = {64, 128, 1, 1, 1}, es[5] = {1, 1, 1, 1, 1};
+    if (enc(&pl->om.y[0], kTmapAct16, 5, y, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
+            CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
+      v.swap_ab = v.staged_epi = false;
+  } else if (v.staged_epi) {
+    // output tile of the GEMM kernel, one output plane of the halo kernels (pair: 8w x 2d x 8h); 64-channel groups of 128-byte
+    // rows, fp32: 32-channel groups; C_out = 32 on the halo kernels: one group of 64-byte rows
+    const bool group32 = k.block_n == 32;
+    const CUtensorMapDataType dt = f32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : kTmapAct16;
+    const CUtensorMapSwizzle swz = group32 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B;
+    const cuuint32_t box[5] = {f32 || group32 ? 32u : 64u, (cuuint32_t)(halo ? 8 : g.box_w), (cuuint32_t)(k.pair ? 2 : halo ? 16 : g.box_h),
+                               (cuuint32_t)(k.pair ? 8 : halo ? 1 : g.box_d), (cuuint32_t)(halo ? 1 : g.box_n)};
+    const int ps = parity ? 2 : 1;   // output voxel stride of one M-space step; one map per output parity
+    for (int q = 0; q < (parity ? 8 : 1) && !rc; ++q) {
+      const size_t off = ((size_t)((q >> 2) & 1) * g.out_h * g.out_w + (size_t)((q >> 1) & 1) * g.out_w + (size_t)(q & 1)) * d->c_out * (f32 ? 4 : 2);
+      rc = encode_act(enc, &pl->om.y[q], "Y", (const char*)y + (parity ? off : 0), dt, d->c_out, g.out_w, g.out_h, g.out_d, d->batch, box,
+                      swz, ps, 1, k.pair);
+    }
+    if (!rc && residual && !halo)   // (the halo kernels read the residual into registers)
+      rc = encode_act(enc, &pl->om.r, "residual", residual, dt, d->c_out, g.out_w, g.out_h, g.out_d, d->batch, box, swz);
+    if (rc) return rc;
+  }
+  p.mode = d->mode; p.batch = d->batch;
+  p.in_d = d->in_d; p.in_h = d->in_h; p.in_w = d->in_w;
+  p.out_d = g.out_d; p.out_h = g.out_h; p.out_w = g.out_w;
+  p.m_d = g.m_d; p.m_h = g.m_h; p.m_w = g.m_w;
+  p.box_w = g.box_w; p.box_h = g.box_h; p.box_d = g.box_d; p.box_n = g.box_n;
+  p.tiles_w = g.tiles_w; p.tiles_h = g.tiles_h; p.tiles_d = g.tiles_d; p.tiles_n = g.tiles_n;
+  p.nch0 = g.nch0; p.nch1 = g.nch1; p.ntaps = g.ntaps; p.ksize = d->ksize; p.stride = st; p.pad = g.pad;
+  p.ksteps0_last = ((d->c0 - (g.nch0 - 1) * 64) + 15) / 16;
+  p.ksteps1_last = d->c1 > 0 ? ((d->c1 - (g.nch1 - 1) * 64) + 15) / 16 : 4;
+  p.c_out = d->c_out; p.n_pad = d->mode == B200DM_CONV_BATCHED_GEMM ? d->c_out : g.n_pad;
+  p.act = d->act; p.post_act = d->reserved[0]; p.y_f32 = f32; p.transposed_store = d->reserved[1];
+  p.chan_bias_rows = d->chan_bias_rows;
+  p.bias = bias; p.chan_bias = chan_bias; p.t_dev = t_dev;
+  p.residual = (const act_t*)residual; p.prelu_alpha = (const act_t*)prelu_alpha;
+  p.y = y; p.dbg = g_dbg_flag;
+  p.tma_epi = v.staged_epi; p.swap_ab = v.swap_ab; p.ksplit = v.ksplit;
+  const int ntiles = d->mode == B200DM_CONV_BATCHED_GEMM ? (d->c_out + k.block_n - 1) / k.block_n : g.n_pad / k.block_n;
+  if (!halo) {
+    pl->grid = dim3((unsigned)(g.mtiles * v.ksplit), (unsigned)ntiles, parity ? 8 : 1);
+    return B200DM_OK;
+  }
+  // persistent halo kernels: at most one CTA per SM (whole pairs) walks the tile list
+  p.tiles_w = (d->in_w + 7) / 8; p.tiles_h = k.pair ? (d->in_h + 7) / 8 : (d->in_h + 15) / 16; p.tiles_d = (d->in_d + v.dstep - 1) / v.dstep;
+  p.tiles_n = d->batch;
+  const long long per = (long long)p.tiles_w * p.tiles_h * p.tiles_d * p.tiles_n;
+  p.halo_td = v.dstep; p.halo_tiles_per_ntile = (int)per; p.halo_ntn = ntiles; p.halo_total_tiles = (int)(per * ntiles * (up ? 8 : 1));
+  int ctas = (int)sms;
+  if (ctas > p.halo_total_tiles) ctas = p.halo_total_tiles;
+  if (k.cg2) ctas &= ~1;
+  pl->grid = dim3((unsigned)ctas, 1, 1);
   return B200DM_OK;
 }
 
-constexpr int kHaloNSFused = 4;   // the 16-bit staging tiles of the fused update take the room of the fifth slab
-
-template <int TD>
-static int launch_halo_cg2_fused(const b200dm_conv_plan* pl, cudaStream_t s) {
-  auto kern = halo::conv_halo_kernel<128, TD, kHaloNSFused, 3, 3, true, false, true, true>;
-  static bool attr_set = false;
-  if (!attr_set) {
-    B2_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl->smem));
-    attr_set = true;
-  }
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = pl->grid; cfg.blockDim = dim3(halo::kThreadsFused); cfg.dynamicSmemBytes = pl->smem; cfg.stream = s;
-  cudaLaunchAttribute at[2];
-  at[0].id = cudaLaunchAttributeClusterDimension;
-  at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-  at[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[1].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at; cfg.numAttrs = b200dm_pdl_enabled() ? 2 : 1;
-  B2_CHECK_CUDA(cudaLaunchKernelEx(&cfg, kern, pl->mapA0, pl->mapA1, pl->mapB, pl->om.y[0], pl->om.y[1], pl->p));
-  return B200DM_OK;
-}
-
-template <int TD>
-static int launch_halo_wide(const b200dm_conv_plan* pl, cudaStream_t s) {
-  auto kern = halo::conv_halo_kernel<128, TD, kHaloNSWide, 2, 3, true>;
-  static bool attr_set = false;
-  if (!attr_set) {
-    B2_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl->smem));
-    attr_set = true;
-  }
-  B2_CHECK_CUDA(b2_launch(kern, pl->grid, dim3(halo::kThreads), pl->smem, s, pl->mapA0, pl->mapA1, pl->mapB, pl->om.y[0], pl->om.y[1], pl->p));
-  return B200DM_OK;
-}
-
-static int launch_halo_pair(const b200dm_conv_plan* pl, cudaStream_t s) {
-  auto kern = halo::conv_halo_kernel<64, 1, kHaloNSPair, 3, 3, true, true>;
-  static bool attr_set = false;
-  if (!attr_set) {
-    B2_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl->smem));
-    attr_set = true;
-  }
-  B2_CHECK_CUDA(b2_launch(kern, pl->grid, dim3(halo::kThreads), pl->smem, s, pl->mapA0, pl->mapA1, pl->mapB, pl->om.y[0], pl->om.y[1], pl->p));
-  return B200DM_OK;
-}
-
-// weight-ring depth / taps per stage by BLOCK_N (smem: 6 slabs x 23 KB + NB x TPS x BLOCK_N x 128 B <= 227 KB)
-static void halo_ring_config(int block_n, int* nb, int* tps) {
-  if (block_n >= 128) { *nb = 4; *tps = 1; }
-  else if (block_n == 64) { *nb = 3; *tps = 3; }
-  else { *nb = 4; *tps = 3; }
-}
-
-template <int BLOCK_N, int NB, int TPS>
-static int dispatch_halo(const b200dm_conv_plan* pl, cudaStream_t s) {
-  if constexpr (BLOCK_N >= 32) {
-    if (pl->p.tma_epi) return pl->halo_td == 2 ? launch_halo<BLOCK_N, 2, NB, TPS, true>(pl, s) : launch_halo<BLOCK_N, 1, NB, TPS, true>(pl, s);
-  }
-  return pl->halo_td == 2 ? launch_halo<BLOCK_N, 2, NB, TPS, false>(pl, s) : launch_halo<BLOCK_N, 1, NB, TPS, false>(pl, s);
-}
-
-static size_t halo_smem_bytes(const b200dm_conv_plan* pl) {
-  const bool st = pl->p.tma_epi != 0;
-  const int ns = pl->fuse ? kHaloNSFused : pl->halo_ns ? pl->halo_ns : (pl->pair ? kHaloNSPair : (pl->wide ? kHaloNSWide : halo_ns_for(pl->g.block_n, st)));   // (cg2: 5, or 4 for pair slabs)
-  return 1024 + (size_t)ns * (pl->pair ? 25 * 1024 : halo::kSlabBytes) +
-         (size_t)pl->halo_nb * pl->halo_tps * (pl->cg2 ? pl->g.block_n / 2 : pl->g.block_n) * 128 +
-         (size_t)halo::stage_bytes(pl->g.block_n, st) + (pl->fuse ? halo::kFuseStage16Bytes + 32 : 0) + (2 * ns + 2 * pl->halo_nb + 4) * 8 + 16 + 4 * pl->g.block_n * 4;
-}
+}  // namespace
 
 extern "C" int b200dm_conv_plan_create(const b200dm_conv_desc* d, const void* x0, const void* x1, const void* w_packed,
                                        const float* bias, const float* chan_bias, const int32_t* t_dev,
@@ -735,414 +1024,32 @@ extern "C" int b200dm_conv_plan_create(const b200dm_conv_desc* d, const void* x0
   B2_CHECK_ARG((d->c1 > 0) == (x1 != nullptr), "conv_plan_create: x1 must be given iff c1 > 0");
   B2_CHECK_ARG(d->y_dtype == B200DM_BF16 || d->y_dtype == B200DM_F32, "conv_plan_create: bad y dtype");
   B2_CHECK_ARG(((uintptr_t)x0 & 15) == 0 && ((uintptr_t)w_packed & 15) == 0 && ((uintptr_t)y & 15) == 0, "conv_plan_create: pointers must be 16-byte aligned");
-  EncodeTiledFn enc = get_encode_fn();
+  EncodeTiledFn enc = b2_encode_tiled_fn();
   if (!enc) { b200dm_set_error("conv_plan_create: cuTensorMapEncodeTiled unavailable (no CUDA driver?)"); return B200DM_ERR_CUDA; }
   rc = ensure_dbg_flag();
   if (rc) return rc;
 
-  b200dm_conv_plan* pl = new (std::nothrow) b200dm_conv_plan();
+  std::unique_ptr<b200dm_conv_plan> pl(new (std::nothrow) b200dm_conv_plan());
   B2_CHECK_ARG(pl, "conv_plan_create: out of memory");
   pl->desc = *d;
   pl->g = g;
-  const int st = d->mode == B200DM_CONV_DIRECT ? d->stride : 1;
-  // C_out = 1, C_in = 32, 3^3 stride 1 (the vqgan_attn_cp decoder's head): HBM-bound stencil-reduce kernel instead of an
-  // N = 16 tensor-core tile (conv_stencil.cuh); bias + activation epilogue only
-  if (d->mode == B200DM_CONV_DIRECT && d->ksize == 3 && d->stride == 1 && d->c_out == 1 && d->c0 == stencil::kC && d->c1 == 0 &&
-      !chan_bias && !residual && !prelu_alpha && d->reserved[0] == B200DM_ACT_NONE && d->reserved[1] == 0 && d->use_halo >= 0) {
-    cuuint64_t dims[5] = {(cuuint64_t)d->c0, (cuuint64_t)d->in_w, (cuuint64_t)d->in_h, (cuuint64_t)d->in_d, (cuuint64_t)d->batch};
-    cuuint64_t strides[4] = {(cuuint64_t)d->c0 * 2, (cuuint64_t)d->in_w * d->c0 * 2, (cuuint64_t)d->in_h * d->in_w * d->c0 * 2,
-                             (cuuint64_t)d->in_d * d->in_h * d->in_w * d->c0 * 2};
-    cuuint32_t box[5] = {(cuuint32_t)stencil::kC, (cuuint32_t)stencil::kHW, (cuuint32_t)stencil::kHH, 1, 1};
-    cuuint32_t es[5] = {1, 1, 1, 1, 1};
-    if (enc(&pl->mapS, kTmapAct16, 5, const_cast<void*>(x0), dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-            CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS) {
-      delete pl; b200dm_set_error("cuTensorMapEncodeTiled(stencil X) failed"); return B200DM_ERR_CUDA;
-    }
-    stencil::Params& sp = pl->sp;
-    memset(&sp, 0, sizeof(sp));
-    sp.batch = d->batch; sp.D = d->in_d; sp.H = d->in_h; sp.W = d->in_w;
-    sp.tiles_h = (d->in_h + stencil::kTH - 1) / stencil::kTH; sp.tiles_w = (d->in_w + stencil::kTW - 1) / stencil::kTW;
-    // d ranges: enough work items for ~6 per resident CTA (two CTAs per SM), each range >= 8 planes (2 halo planes per range)
-    const long long cols = (long long)d->batch * sp.tiles_h * sp.tiles_w, ctas = 2LL * b2_num_sms();
-    int dsplit = 1;
-    while (cols * dsplit < 6 * ctas && d->in_d / (dsplit * 2) >= 8) dsplit *= 2;
-    sp.dlen = (d->in_d + dsplit - 1) / dsplit; sp.dsplit = (d->in_d + sp.dlen - 1) / sp.dlen;
-    sp.items = (int)(cols * sp.dsplit);
-    sp.w = (const act_t*)w_packed; sp.bias = bias; sp.act = d->act; sp.y_f32 = d->y_dtype == B200DM_F32; sp.y = y; sp.dbg = g_dbg_flag;
-    pl->stencil = true;
-    pl->grid = dim3((unsigned)(sp.items < ctas ? sp.items : ctas), 1, 1);
-    pl->smem = stencil::kSmem;
-    pl->flops = 2.0 * 27 * d->c0 * (double)d->batch * d->in_d * d->in_h * d->in_w;
-    *out = pl;
-    return B200DM_OK;
-  }
-  // C_in = C_out = 32, 3^3 stride 1, 16-bit output (the decoders' 128^3 / 64^3 residual units): d-sweeping kernel with the three
-  // kd taps of an input plane as one N = 96 MMA and the weight set resident in shared memory (conv_sweep.cuh)
-  if (d->mode == B200DM_CONV_DIRECT && d->ksize == 3 && d->stride == 1 && d->c_out == 32 && d->c0 == 32 && d->c1 == 0 &&
-      d->y_dtype == B200DM_BF16 && !chan_bias && !prelu_alpha && d->reserved[1] == 0 && d->use_halo >= 0 && g.n_pad == 32 &&
-      g.ktot == 27 * 64 && d->in_w >= 8 && d->in_h >= 16 && d->in_d >= 2) {
-    const cuuint64_t C = 32;
-    cuuint64_t dims[5] = {C, (cuuint64_t)d->in_w, (cuuint64_t)d->in_h, (cuuint64_t)d->in_d, (cuuint64_t)d->batch};
-    cuuint64_t strides[4] = {C * 2, (cuuint64_t)d->in_w * C * 2, (cuuint64_t)d->in_h * d->in_w * C * 2,
-                             (cuuint64_t)d->in_d * d->in_h * d->in_w * C * 2};
-    cuuint32_t es[5] = {1, 1, 1, 1, 1};
-    cuuint32_t boxx[5] = {32, 10, 18, 2, 1}, boxy[5] = {32, 8, 16, 1, 1};
-    cuuint64_t wdims[3] = {64, 32, 27};
-    cuuint64_t wstrides[2] = {(cuuint64_t)g.ktot * 2, 128};
-    cuuint32_t wbox[3] = {32, 32, 1};
-    const bool okm =
-        enc(&pl->mapS, kTmapAct16, 5, const_cast<void*>(x0), dims, strides, boxx, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-            CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS &&
-        enc(&pl->om.y[0], kTmapAct16, 5, y, dims, strides, boxy, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-            CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS &&
-        enc(&pl->mapB, kTmapAct16, 3, const_cast<void*>(w_packed), wdims, wstrides, wbox, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-            CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-    const bool okr = !residual || enc(&pl->om.r, kTmapAct16, 5, const_cast<void*>(residual), dims, strides, boxy, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                                       CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-    if (!okm || !okr) { delete pl; b200dm_set_error("cuTensorMapEncodeTiled(sweep) failed"); return B200DM_ERR_CUDA; }
-    sweep::Params& wp = pl->wp;
-    memset(&wp, 0, sizeof(wp));
-    wp.D = d->in_d; wp.H = d->in_h; wp.W = d->in_w; wp.batch = d->batch;
-    wp.tiles_w = (d->in_w + 7) / 8; wp.tiles_h = (d->in_h + 15) / 16;
-    const long long cols = (long long)d->batch * wp.tiles_w * wp.tiles_h, ctas = b2_num_sms();
-    int dsplit = 1;
-    while (cols * dsplit < 6 * ctas && d->in_d / (dsplit * 2) >= 8) dsplit *= 2;   // >= ~6 items per CTA, d ranges of >= 8 planes
-    wp.dlen = (d->in_d + dsplit - 1) / dsplit; wp.dsplit = (d->in_d + wp.dlen - 1) / wp.dlen;
-    wp.items = (int)(cols * wp.dsplit);
-    ConvParams& p = pl->p;
-    memset(&p, 0, sizeof(p));
-    p.batch = d->batch; p.in_d = p.out_d = d->in_d; p.in_h = p.out_h = d->in_h; p.in_w = p.out_w = d->in_w;
-    p.c_out = 32; p.n_pad = 32; p.act = d->act; p.post_act = d->reserved[0];
-    p.bias = bias; p.residual = (const act_t*)residual; p.y = y; p.dbg = g_dbg_flag; p.tma_epi = 1;
-    pl->sweep = true; pl->halo = true;
-    pl->grid = dim3((unsigned)(wp.items < ctas ? wp.items : ctas), 1, 1);
-    pl->smem = sweep::kSmem;
-    pl->flops = 2.0 * 27 * 32 * 32 * (double)d->batch * d->in_d * d->in_h * d->in_w;
-    *out = pl;
-    return B200DM_OK;
-  }
-  // halo-reuse kernel: 3^3 stride-1 convs on volumes that fill its 8w x 16h tile (use_halo = -1 forces it off)
-  pl->halo = d->mode == B200DM_CONV_DIRECT && d->ksize == 3 && d->stride == 1 && d->in_w >= 8 && d->in_h >= 16 &&
-             d->reserved[1] == 0 && d->use_halo >= 0;
-  // 8 x 8 planes (the U-Net's deepest level): pair-slab tiles, 64 output channels per CTA so that >= 128 CTAs share the
-  // weight stream; bf16 staged output only
-  pl->pair = !pl->halo && d->mode == B200DM_CONV_DIRECT && d->ksize == 3 && d->stride == 1 && d->in_w == 8 && d->in_h == 8 &&
-             d->in_d >= 2 && d->reserved[1] == 0 && d->use_halo >= 0 && d->y_dtype == B200DM_BF16 && d->c_out % 64 == 0 &&
-             !prelu_alpha;
-  if (pl->pair) { pl->halo = true; g.block_n = 64; pl->g.block_n = 64; }
-  // x2 up-convolutions (nearest-upsample + conv3, ConvT k4 s2) on low-resolution planes that fill the 8 x 16 halo tile
-  {
-    const long long per_up = (long long)((d->in_w + 7) / 8) * ((d->in_h + 15) / 16) * ((d->in_d + 1) / 2) * d->batch;
-    // (C_out = 32 -- the decoders' last ConvT, 64 -> 32 at 64^3 -> 128^3 -- runs N = 32 tiles with 64-byte staged rows)
-    const bool up32 = d->c_out == 32 && g.block_n == 32;
-    pl->ups = d->mode == B200DM_CONV_PARITY && d->in_w >= 8 && d->in_h >= 16 && d->in_d >= 2 && (d->c_out % 64 == 0 || up32) &&
-              d->y_dtype == B200DM_BF16 && !residual && !prelu_alpha && d->reserved[1] == 0 && d->use_halo >= 0 && per_up % 2 == 0 &&
-              (g.block_n == 64 || g.block_n == 128 || up32);
-    if (pl->ups) pl->halo = true;
-    // the same on 8 x 8 low-resolution planes (8^3 -> 16^3): pair-slab tiles
-    const long long per_pair = (long long)((d->in_d + 1) / 2) * d->batch;
-    if (!pl->ups && d->mode == B200DM_CONV_PARITY && d->in_w == 8 && d->in_h == 8 && d->in_d >= 2 && d->in_d % 2 == 0 && d->c_out % 64 == 0 &&
-        d->y_dtype == B200DM_BF16 && !residual && !prelu_alpha && d->reserved[1] == 0 && d->use_halo >= 0 && per_pair % 2 == 0 &&
-        (g.block_n == 64 || g.block_n == 128)) {
-      pl->ups = true; pl->pair = true; pl->halo = true;
-    }
-  }
-  auto encodeA = [&](CUtensorMap* m, const void* ptr, int C) -> int {
-    cuuint64_t dims[5] = {(cuuint64_t)C, (cuuint64_t)d->in_w, (cuuint64_t)d->in_h, (cuuint64_t)d->in_d, (cuuint64_t)d->batch};
-    cuuint64_t strides[4] = {(cuuint64_t)C * 2, (cuuint64_t)d->in_w * C * 2, (cuuint64_t)d->in_h * d->in_w * C * 2,
-                             (cuuint64_t)d->in_d * d->in_h * d->in_w * C * 2};
-    cuuint32_t box[5] = {64, (cuuint32_t)(g.box_w * st), (cuuint32_t)(g.box_h * st), (cuuint32_t)(g.box_d * st), (cuuint32_t)g.box_n};
-    if (pl->pair) {   // dims listed as (C, W, D, H, N): the box {64, 10, 2, 10, 1} lands as rows [h][d][w]
-      dims[2] = (cuuint64_t)d->in_d; dims[3] = (cuuint64_t)d->in_h;
-      const cuuint64_t sh = strides[1], sd = strides[2];
-      strides[1] = sd; strides[2] = sh;
-      box[1] = 10; box[2] = 2; box[3] = 10; box[4] = 1;
-    } else if (pl->halo) { box[1] = 10; box[2] = 18; box[3] = 1; box[4] = 1; }   // one halo d-plane slab
-
-    cuuint32_t es[5] = {1, (cuuint32_t)st, (cuuint32_t)st, (cuuint32_t)st, 1};
-    CUresult r = enc(m, kTmapAct16, 5, const_cast<void*>(ptr), dims, strides, box, es,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) { b200dm_set_error("cuTensorMapEncodeTiled(A) failed: %d (C=%d dims %d,%d,%d,%d box %d,%d,%d,%d stride %d)", (int)r, C, d->in_w, d->in_h, d->in_d, d->batch, g.box_w, g.box_h, g.box_d, g.box_n, st); return B200DM_ERR_CUDA; }
-    return B200DM_OK;
-  };
-  rc = encodeA(&pl->mapA0, x0, d->c0);
-  if (rc) { delete pl; return rc; }
-  rc = encodeA(&pl->mapA1, d->c1 > 0 ? x1 : x0, d->c1 > 0 ? d->c1 : d->c0);
-  if (rc) { delete pl; return rc; }
-  {
-    cuuint64_t dims[2] = {(cuuint64_t)g.ktot, (cuuint64_t)g.groups * g.n_pad};
-    cuuint64_t strides[1] = {(cuuint64_t)g.ktot * 2};
-    if (d->mode == B200DM_CONV_BATCHED_GEMM) {
-      // B is a raw activation tensor [batch][c_out rows][K = c0]; rows beyond c_out of a sample alias the next sample
-      // (masked by the epilogue's col < c_out), K beyond c0 is zero-filled by TMA.
-      dims[0] = (cuuint64_t)d->c0; dims[1] = (cuuint64_t)d->batch * d->c_out; strides[0] = (cuuint64_t)d->c0 * 2;
-    }
-    cuuint32_t box[2] = {64, (cuuint32_t)g.block_n};
-    cuuint32_t es[3] = {1, 1, 1};
-    CUresult r;
-    if (pl->halo) {
-      const long long t1 = (long long)((d->in_w + 7) / 8) * ((d->in_h + 15) / 16) * ((d->in_d + 1) / 2) * d->batch;
-      {  // planes per tile: 2 (weight stage shared by two planes, two MMA issuer warps) unless that costs a wave
-        const long long sms = b2_num_sms(), nt = g.n_pad / g.block_n;
-        const long long t_one = (long long)((d->in_w + 7) / 8) * ((d->in_h + 15) / 16) * d->in_d * d->batch;
-        const long long cost2 = (t1 * nt + sms - 1) / sms * 2, cost1 = (t_one * nt + sms - 1) / sms;
-        pl->halo_td = d->in_d >= 2 && cost2 <= cost1 ? 2 : 1;
-        if (pl->pair) pl->halo_td = 2;   // d step of a pair tile (the kernel runs with one accumulator, TD = 1)
-      }
-      halo_ring_config(g.block_n, &pl->halo_nb, &pl->halo_tps);
-      // packed weights [n_pad rows][chunk*27 + tap][64] viewed as 3-D {64, rows, tap-chunks}: one box = TPS consecutive taps
-      cuuint64_t dims3[3] = {64, (cuuint64_t)g.n_pad, (cuuint64_t)(g.ktot / 64)};
-      cuuint64_t strides3[2] = {(cuuint64_t)g.ktot * 2, 128};
-      cuuint32_t box3[3] = {64, (cuuint32_t)g.block_n, (cuuint32_t)pl->halo_tps};
-      r = enc(&pl->mapB, kTmapAct16, 3, const_cast<void*>(w_packed), dims3, strides3, box3, es,
-              CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    } else {
-      r = enc(&pl->mapB, kTmapAct16, 2, const_cast<void*>(w_packed), dims, strides, box, es,
-              CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    }
-    if (r != CUDA_SUCCESS) { b200dm_set_error("cuTensorMapEncodeTiled(B) failed: %d (halo %d)", (int)r, (int)pl->halo); delete pl; return B200DM_ERR_CUDA; }
-  }
-  ConvParams& p = pl->p;
-  memset(&p, 0, sizeof(p));
-  p.mode = d->mode; p.batch = d->batch;
-  p.in_d = d->in_d; p.in_h = d->in_h; p.in_w = d->in_w;
-  p.out_d = g.out_d; p.out_h = g.out_h; p.out_w = g.out_w;
-  p.m_d = g.m_d; p.m_h = g.m_h; p.m_w = g.m_w;
-  p.box_w = g.box_w; p.box_h = g.box_h; p.box_d = g.box_d; p.box_n = g.box_n;
-  p.tiles_w = (g.m_w + g.box_w - 1) / g.box_w; p.tiles_h = (g.m_h + g.box_h - 1) / g.box_h;
-  p.tiles_d = (g.m_d + g.box_d - 1) / g.box_d; p.tiles_n = (d->batch + g.box_n - 1) / g.box_n;
-  p.nch0 = g.nch0; p.nch1 = g.nch1; p.ntaps = g.ntaps; p.ksize = d->ksize; p.stride = st; p.pad = g.pad;
-  p.ksteps0_last = ((d->c0 - (g.nch0 - 1) * 64) + 15) / 16;
-  p.ksteps1_last = d->c1 > 0 ? ((d->c1 - (g.nch1 - 1) * 64) + 15) / 16 : 4;
-  p.c_out = d->c_out; p.n_pad = d->mode == B200DM_CONV_BATCHED_GEMM ? d->c_out : g.n_pad;
-  p.act = d->act; p.post_act = d->reserved[0]; p.y_f32 = d->y_dtype == B200DM_F32; p.transposed_store = d->reserved[1];
-  p.chan_bias_rows = d->chan_bias_rows;
-  p.bias = bias; p.chan_bias = chan_bias; p.t_dev = t_dev;
-  p.residual = (const act_t*)residual; p.prelu_alpha = (const act_t*)prelu_alpha;
-  p.y = y; p.dbg = g_dbg_flag;
-  const long long mtiles = (long long)p.tiles_w * p.tiles_h * p.tiles_d * p.tiles_n;
-  if (mtiles > 0x7fffffffLL) { delete pl; b200dm_set_error("conv_plan_create: too many tiles"); return B200DM_ERR_INVALID; }
-  const int ntiles = d->mode == B200DM_CONV_BATCHED_GEMM ? (d->c_out + g.block_n - 1) / g.block_n : g.n_pad / g.block_n;
-  pl->grid = dim3((unsigned)mtiles, (unsigned)ntiles, d->mode == B200DM_CONV_PARITY ? 8 : 1);
-  // split-K: when the tile grid leaves most SMs idle and K is long, ksplit CTAs (one cluster) share a tile.  Each CTA
-  // streams its K range at the per-SM operand rate (~40 B/clk), so an under-filled grid is K-latency-bound otherwise.
-  p.ksplit = 1;
-  if (!pl->halo && d->reserved[1] == 0) {
-    const long long ctas = mtiles * ntiles * (d->mode == B200DM_CONV_PARITY ? 8 : 1);
-    const int nkb = (g.nch0 + g.nch1) * g.ntaps;
-    int ksp = 1;
-    while (ksp < 8 && ctas * (ksp * 2) <= b2_num_sms() && nkb / (ksp * 2) >= 13) ksp *= 2;   // >= 13 k-blocks per CTA: 3^3 convs only
-    if (ksp > 1) { p.ksplit = ksp; pl->grid.x = (unsigned)(mtiles * ksp); }
-  }
-  // pipeline depth 4; measured on B200: a deeper ring (6 stages at BLOCK_N=128, 8 below) does not help at BLOCK_N=128 (the
-  // operand stream is bandwidth-, not latency-bound) and hurts below 128, where 4 stages let two CTAs share an SM
-  pl->nstage = 4;
-  // short K loops (1^3 convs: 1-3 k-blocks) never fill four stages; two stages let 3-4 CTAs share an SM, which hides the
-  // per-CTA prologue / TMA latency / epilogue of these HBM-bound launches
-  if ((g.nch0 + g.nch1) * g.ntaps <= 3 && g.block_n >= 64) pl->nstage = 2;
-  // grids of several waves: two stages x three co-resident CTAs keep more operand bytes in flight per SM than one CTA with
-  // four stages, and hide every CTA's prologue / epilogue (measured: 16^3 128->128 parity conv 123 -> 77 us, 8^3 MLP GEMM
-  // 17.5 -> 12.7 us; a single-wave split-K grid gets slower, so it keeps four stages)
-  if (!pl->halo && (long long)pl->grid.x * pl->grid.y * pl->grid.z >= 2LL * b2_num_sms() && g.block_n >= 64 && p.ksplit <= 1)
-    pl->nstage = 2;
-  // split-K needs >= 26 k-blocks, the first two-stage rule <= 3: the split-K kernel is instantiated with four stages only
-  if (p.ksplit > 1 && pl->nstage != 4) {
-    delete pl; b200dm_set_error("conv_plan_create: internal: split-K plan with two stages"); return B200DM_ERR_UNSUPPORTED;
-  }
-  // staged (TMA-store) epilogue of the per-tap GEMM kernel: bf16 NDHWC output with whole 64-channel groups
-  memset(&pl->om, 0, sizeof(pl->om));
-  {
-    const bool f32 = d->y_dtype == B200DM_F32;   // fp32 output (the U-Net's eps): halo kernel only, 32-column groups
-    // (halo kernel, C_out = 32: one 32-channel group of 64-byte rows, SWIZZLE_64B -- the decoders' 128^3 convs)
-    const bool n32 = pl->halo && !pl->pair && d->c_out == 32 && g.block_n == 32 && !f32 && (pl->ups || d->mode == B200DM_CONV_DIRECT);
-    const bool want = (!f32 || pl->halo) && d->reserved[1] == 0 && !prelu_alpha &&
-                      ((d->c_out % 64 == 0 && g.block_n >= 64) || n32) && !(d->mode == B200DM_CONV_PARITY && residual);
-    if (want) {
-      const int par = d->mode == B200DM_CONV_PARITY ? 8 : 1;
-      const int ps = d->mode == B200DM_CONV_PARITY ? 2 : 1;   // output voxel stride of one M-space step
-      const cuuint64_t C = (cuuint64_t)d->c_out;
-      auto encodeY = [&](CUtensorMap* m, const void* base) -> bool {
-        cuuint64_t dims[5] = {C, (cuuint64_t)g.m_w, (cuuint64_t)g.m_h, (cuuint64_t)g.m_d, (cuuint64_t)d->batch};
-        const cuuint64_t eb = f32 ? 4 : 2;
-        cuuint64_t strides[4] = {C * eb * ps, (cuuint64_t)g.out_w * C * eb * ps, (cuuint64_t)g.out_h * g.out_w * C * eb * ps,
-                                 (cuuint64_t)g.out_d * g.out_h * g.out_w * C * eb};
-        cuuint32_t box[5] = {f32 || n32 ? 32u : 64u, (cuuint32_t)g.box_w, (cuuint32_t)g.box_h, (cuuint32_t)g.box_d, (cuuint32_t)g.box_n};
-        if (pl->pair) {   // (C, W, D, H, N) order, one 8w x 2d x 8h tile
-          dims[2] = (cuuint64_t)g.m_d; dims[3] = (cuuint64_t)g.m_h;
-          const cuuint64_t sh = strides[1], sd = strides[2];
-          strides[1] = sd; strides[2] = sh;
-          box[1] = 8; box[2] = 2; box[3] = 8; box[4] = 1;
-        } else if (pl->halo) { box[1] = 8; box[2] = 16; box[3] = 1; box[4] = 1; }   // one output plane of the halo kernel's tile
-        cuuint32_t es[5] = {1, 1, 1, 1, 1};
-        return enc(m, f32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : kTmapAct16, 5, const_cast<void*>(base), dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                   n32 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-      };
-      bool okm = true;
-      for (int q = 0; q < par && okm; ++q) {
-        const size_t off = d->mode == B200DM_CONV_PARITY
-                               ? ((size_t)((q >> 2) & 1) * g.out_h * g.out_w + (size_t)((q >> 1) & 1) * g.out_w + (size_t)(q & 1)) * d->c_out * 2
-                               : 0;
-        okm = encodeY(&pl->om.y[q], (const char*)y + off);
-      }
-      if (okm && residual && !pl->halo) okm = encodeY(&pl->om.r, residual);
-      if (!okm) { delete pl; b200dm_set_error("cuTensorMapEncodeTiled(Y) failed"); return B200DM_ERR_CUDA; }
-      p.tma_epi = 1;
-    }
-  }
-  // per-sample transposed store by operand swap (see the kernel): tiles of whole planes inside one sample, bias only
-  if (d->reserved[1] != 0 && !pl->halo && d->mode == B200DM_CONV_DIRECT && d->ksize == 1 && st == 1 &&
-      d->y_dtype == B200DM_BF16 && g.block_n == 128 && g.box_n == 1 && g.box_w == g.m_w && g.box_h == g.m_h && g.m_d % g.box_d == 0 &&
-      !residual && !prelu_alpha && !chan_bias && d->act == B200DM_ACT_NONE && d->reserved[0] == B200DM_ACT_NONE) {
-    const cuuint64_t Lv = (cuuint64_t)g.m_w * g.m_h * g.m_d;
-    cuuint64_t dims[5] = {Lv, (cuuint64_t)d->c_out, 1, 1, (cuuint64_t)d->batch};
-    cuuint64_t strides[4] = {Lv * 2, Lv * d->c_out * 2, Lv * d->c_out * 2, Lv * d->c_out * 2};
-    cuuint32_t box[5] = {64, 128, 1, 1, 1};
-    cuuint32_t es[5] = {1, 1, 1, 1, 1};
-    if (Lv % 8 == 0 && enc(&pl->om.y[0], kTmapAct16, 5, y, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                           CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS) {
-      p.swap_ab = 1;
-      p.tma_epi = 1;
-    }
-  }
-  pl->smem = conv_smem_bytes(g.block_n, pl->nstage, p.tma_epi && residual);
-  if (pl->smem > 232448) { p.tma_epi = 0; pl->smem = conv_smem_bytes(g.block_n, pl->nstage, false); }
-  // BLOCK_N = 128 with the staged epilogue: one-tap weight stages hold only 8 MMAs (4 per issuer warp) and the per-stage
-  // barrier round trip (~200 cycles) made those convs issue-bound (45 % of the MMA floor); 3-tap stages x 2 fit once the
-  // slab ring is the 4 slabs a channel chunk needs (the next chunk's slab i reloads as soon as slab i is released).
-  if (pl->halo && !pl->pair && g.block_n == 128 && p.tma_epi) {
-    cuuint64_t dims3[3] = {64, (cuuint64_t)g.n_pad, (cuuint64_t)(g.ktot / 64)};
-    cuuint64_t strides3[2] = {(cuuint64_t)g.ktot * 2, 128};
-    cuuint32_t box3[3] = {64, 128, 3};
-    cuuint32_t es3[3] = {1, 1, 1};
-    if (enc(&pl->mapB, kTmapAct16, 3, const_cast<void*>(w_packed), dims3, strides3, box3, es3,
-            CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-            CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS) { delete pl; b200dm_set_error("cuTensorMapEncodeTiled(B wide) failed"); return B200DM_ERR_CUDA; }
-    pl->wide = true; pl->halo_nb = 2; pl->halo_tps = 3;
-  }
-  // CTA pairs (cta_group::2) for every staged halo configuration with 64- or 128-channel tiles, and for N = 32 convs with at
-  // least two channel chunks (the U-Net's input conv, 256 -> 32, direct stores): needs an even tile count per n-tile so that the
-  // two CTAs of a pair always work on the same n-tile and run the same number of tiles.  Short-K N = 32 convs (one channel chunk)
-  // stay single-CTA: with direct stores pairing couples two epilogues (measured 4.18 -> 4.79 ms), staged it gained 3.79 -> 3.74 ms only.
-  const bool cg2_n32 = g.block_n == 32 && !pl->pair && !pl->ups && pl->halo_td == 2 && g.nch0 + g.nch1 >= 2;
-  if (pl->halo && (((g.block_n == 64 || g.block_n == 128) && p.tma_epi && (pl->pair || pl->halo_td == 2 || g.block_n == 128)) || cg2_n32)) {
-    const int td = pl->halo_td;   // (pair: d step 2)
-    const long long per = (long long)((d->in_w + 7) / 8) * (pl->pair ? (d->in_h + 7) / 8 : (d->in_h + 15) / 16) * ((d->in_d + td - 1) / td) * d->batch;
-    if (per % 2 == 0) {
-      cuuint64_t dims3[3] = {64, (cuuint64_t)g.n_pad, (cuuint64_t)(g.ktot / 64)};
-      cuuint64_t strides3[2] = {(cuuint64_t)g.ktot * 2, 128};
-      cuuint32_t box3[3] = {64, (cuuint32_t)(g.block_n / 2), 3};   // this CTA's half of the rows of a 3-tap weight stage
-      cuuint32_t es3[3] = {1, 1, 1};
-      if (enc(&pl->mapB, kTmapAct16, 3, const_cast<void*>(w_packed), dims3, strides3, box3, es3,
-              CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS) { delete pl; b200dm_set_error("cuTensorMapEncodeTiled(B cg2) failed"); return B200DM_ERR_CUDA; }
-      pl->cg2 = true; pl->wide = false; pl->halo_nb = cg2_n32 ? 4 : 3; pl->halo_tps = 3;
-    }
-  }
-  if (pl->ups) {
-    if (!p.tma_epi) { delete pl; b200dm_set_error("conv_plan_create: internal: up-conv plan without staged epilogue"); return B200DM_ERR_UNSUPPORTED; }
-    // packed [parity][n_pad rows][chunk*8 + tap][64]: one box = this CTA's half of the rows x the 4 in-plane taps of one td
-    cuuint64_t dims3[3] = {64, (cuuint64_t)g.groups * g.n_pad, (cuuint64_t)(g.ktot / 64)};
-    cuuint64_t strides3[2] = {(cuuint64_t)g.ktot * 2, 128};
-    cuuint32_t box3[3] = {64, (cuuint32_t)(g.block_n / 2), 4};
-    cuuint32_t es3[3] = {1, 1, 1};
-    if (enc(&pl->mapB, kTmapAct16, 3, const_cast<void*>(w_packed), dims3, strides3, box3, es3,
-            CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-            CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS) { delete pl; b200dm_set_error("cuTensorMapEncodeTiled(B up) failed"); return B200DM_ERR_CUDA; }
-    pl->cg2 = true; pl->wide = false; pl->halo_td = 2;
-    pl->halo_nb = g.block_n == 32 ? 4 : (g.block_n == 64 ? 3 : 2); pl->halo_tps = 4; pl->halo_ns = pl->pair ? 4 : 5;
-  }
-  if (pl->halo) {
-    const int td = pl->halo_td;
-    p.tiles_w = (d->in_w + 7) / 8; p.tiles_h = pl->pair ? (d->in_h + 7) / 8 : (d->in_h + 15) / 16; p.tiles_d = (d->in_d + td - 1) / td;
-    p.tiles_n = d->batch;
-    const long long per = (long long)p.tiles_w * p.tiles_h * p.tiles_d * p.tiles_n;
-    p.halo_td = td; p.halo_tiles_per_ntile = (int)per; p.halo_ntn = ntiles; p.halo_total_tiles = (int)(per * ntiles * (pl->ups ? 8 : 1));
-    int ctas = b2_num_sms();
-    if (ctas > p.halo_total_tiles) ctas = p.halo_total_tiles;
-    if (pl->cg2) ctas &= ~1;   // whole pairs
-    pl->grid = dim3((unsigned)ctas, 1, 1);
-    pl->smem = halo_smem_bytes(pl);
-  }
+  pl->v = select_variant(d, g, residual != nullptr, prelu_alpha != nullptr, chan_bias != nullptr);
+  rc = setup_plan(pl.get(), enc, x0, x1, w_packed, bias, chan_bias, t_dev, residual, prelu_alpha, y);
+  if (!rc) rc = bind_kernel(pl.get(), pl->v);
+  if (rc) return rc;
   // algorithmic FLOPs (SURVEY 8d): 2*k^3*Cin*Cout*B*out_voxels; convT: 2*64*Cin*Cout*B*in_voxels; GEMM: 2*M*N*K
   if (d->mode == B200DM_CONV_PARITY)
     pl->flops = d->ksize == 3 ? 2.0 * 27 * (d->c0 + d->c1) * d->c_out * (double)d->batch * g.out_d * g.out_h * g.out_w
                               : 2.0 * 64 * (d->c0 + d->c1) * d->c_out * (double)d->batch * d->in_d * d->in_h * d->in_w;
   else
     pl->flops = 2.0 * g.ntaps * (d->c0 + d->c1) * d->c_out * (double)d->batch * g.out_d * g.out_h * g.out_w;
-  *out = pl;
+  *out = pl.release();
   return B200DM_OK;
 }
 
 extern "C" int b200dm_conv_plan_run(b200dm_conv_plan* pl, void* stream) {
   B2_CHECK_ARG(pl, "conv_plan_run: null plan");
-  cudaStream_t s = (cudaStream_t)stream;
-  if (pl->stencil) {
-    auto kern = stencil::conv_stencil_c1_kernel;
-    static bool attr_set = false;
-    if (!attr_set) {
-      B2_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)stencil::kSmem));
-      attr_set = true;
-    }
-    B2_CHECK_CUDA(b2_launch(kern, pl->grid, dim3(stencil::kThreads), pl->smem, s, pl->mapS, pl->sp));
-    return B200DM_OK;
-  }
-  if (pl->sweep) {
-    auto kern = sweep::conv_sweep32_kernel;
-    static bool attr_set = false;
-    if (!attr_set) {
-      B2_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sweep::kSmem));
-      attr_set = true;
-    }
-    B2_CHECK_CUDA(b2_launch(kern, pl->grid, dim3(sweep::kThreads), pl->smem, s, pl->mapS, pl->mapB, pl->om.y[0], pl->residual_map(), pl->p, pl->wp));
-    return B200DM_OK;
-  }
-  if (pl->ups && pl->pair) return pl->g.block_n == 64 ? launch_halo_up<64, 4, 3, true>(pl, s) : launch_halo_up<128, 4, 2, true>(pl, s);
-  if (pl->ups && pl->g.block_n == 32) return launch_halo_up<32, 5, 4>(pl, s);
-  if (pl->ups) return pl->g.block_n == 64 ? launch_halo_up<64, 5, 3>(pl, s) : launch_halo_up<128, 5, 2>(pl, s);
-  if (pl->cg2) {
-    if (pl->fuse) return pl->halo_td == 2 ? launch_halo_cg2_fused<2>(pl, s) : launch_halo_cg2_fused<1>(pl, s);
-    if (pl->pair) return launch_halo_cg2<64, 1, kHaloNSPair, 3, true>(pl, s);
-    if (pl->g.block_n == 32) return pl->p.tma_epi ? launch_halo_cg2<32, 2, kHaloNS, 4, false, true>(pl, s)
-                                                  : launch_halo_cg2<32, 2, kHaloNS, 4, false, false>(pl, s);
-    if (pl->g.block_n == 64) return launch_halo_cg2<64, 2, kHaloNSStaged, 3, false>(pl, s);
-    return pl->halo_td == 2 ? launch_halo_cg2<128, 2, kHaloNSStaged, 3, false>(pl, s) : launch_halo_cg2<128, 1, kHaloNSStaged, 3, false>(pl, s);
-  }
-  if (pl->pair) return launch_halo_pair(pl, s);
-  if (pl->halo) {
-    switch (pl->g.block_n) {
-      case 16: return dispatch_halo<16, 4, 3>(pl, s);
-      case 32: return dispatch_halo<32, 4, 3>(pl, s);
-      case 64: return dispatch_halo<64, 3, 3>(pl, s);
-      case 128:
-        if (pl->wide) return pl->halo_td == 2 ? launch_halo_wide<2>(pl, s) : launch_halo_wide<1>(pl, s);
-        return dispatch_halo<128, 4, 1>(pl, s);
-    }
-  }
-  if (pl->nstage == 2) {
-    switch (pl->g.block_n) {
-      case 64: return launch_conv<64, 2, false>(pl, s);
-      case 128: return launch_conv<128, 2, false>(pl, s);
-    }
-  } else if (pl->p.ksplit > 1) {
-    switch (pl->g.block_n) {
-      case 16: return launch_conv<16, 4, true>(pl, s);
-      case 32: return launch_conv<32, 4, true>(pl, s);
-      case 64: return launch_conv<64, 4, true>(pl, s);
-      case 128: return launch_conv<128, 4, true>(pl, s);
-    }
-  } else {
-    switch (pl->g.block_n) {
-      case 16: return launch_conv<16, 4, false>(pl, s);
-      case 32: return launch_conv<32, 4, false>(pl, s);
-      case 64: return launch_conv<64, 4, false>(pl, s);
-      case 128: return launch_conv<128, 4, false>(pl, s);
-    }
-  }
-  b200dm_set_error("conv_plan_run: unsupported BLOCK_N %d", pl->g.block_n);
-  return B200DM_ERR_UNSUPPORTED;
+  return pl->inst->launch(pl, (cudaStream_t)stream);
 }
 
 extern "C" void b200dm_conv_plan_destroy(b200dm_conv_plan* p) { delete p; }
@@ -1161,10 +1068,10 @@ extern "C" int b200dm_conv_plan_set_fused_update(b200dm_conv_plan* pl, const b20
   B2_CHECK_ARG(pl && u && x_t && x_prev && x_prev_16, "conv_plan_set_fused_update: null argument");
   const b200dm_conv_desc* d = &pl->desc;
   const ConvParams& p = pl->p;
+  const KernelKey& k = pl->v.key;
   // the CTA-pair N = 128 halo kernel with the fp32 staged epilogue, no other epilogue term
-  if (!(pl->halo && pl->cg2 && !pl->pair && !pl->ups && !pl->sweep && !pl->stencil && pl->g.block_n == 128 &&
-        p.y_f32 && p.tma_epi && d->c_out % 128 == 0 && !p.residual && !p.prelu_alpha && p.act == B200DM_ACT_NONE &&
-        p.post_act == B200DM_ACT_NONE)) {
+  if (!(k.family == Family::kHalo && k.cg2 && !k.pair && k.block_n == 128 && p.y_f32 && k.staged && d->c_out % 128 == 0 &&
+        !p.residual && !p.prelu_alpha && p.act == B200DM_ACT_NONE && p.post_act == B200DM_ACT_NONE)) {
     b200dm_set_error("conv_plan_set_fused_update: only on the CTA-pair fp32-output 3^3 conv with C_out %% 128 == 0");
     return B200DM_ERR_UNSUPPORTED;
   }
@@ -1177,33 +1084,29 @@ extern "C" int b200dm_conv_plan_set_fused_update(b200dm_conv_plan* pl, const b20
   B2_CHECK_ARG(x_t == x_prev, "conv_plan_set_fused_update: x_prev must alias x_t (the tile is updated in place through one tensor map)");
   B2_CHECK_ARG(((uintptr_t)x_t & 15) == 0 && ((uintptr_t)x_prev & 15) == 0 && ((uintptr_t)x_prev_16 & 15) == 0,
                "conv_plan_set_fused_update: pointers must be 16-byte aligned");
-  EncodeTiledFn enc = get_encode_fn();
-  const cuuint64_t C = (cuuint64_t)d->c_out;
-  cuuint64_t dims[5] = {C, (cuuint64_t)d->in_w, (cuuint64_t)d->in_h, (cuuint64_t)d->in_d, (cuuint64_t)d->batch};
-  cuuint32_t box[5] = {16, 8, 16, 1, 1}, es[5] = {1, 1, 1, 1, 1};   // one round of the fused epilogue: 16 columns x one 8 x 16 plane tile
-  cuuint64_t st4[4] = {C * 4, (cuuint64_t)d->in_w * C * 4, (cuuint64_t)d->in_h * d->in_w * C * 4, (cuuint64_t)d->in_d * d->in_h * d->in_w * C * 4};
-  cuuint64_t st2[4] = {C * 2, (cuuint64_t)d->in_w * C * 2, (cuuint64_t)d->in_h * d->in_w * C * 2, (cuuint64_t)d->in_d * d->in_h * d->in_w * C * 2};
+  EncodeTiledFn enc = b2_encode_tiled_fn();
+  if (!enc) { b200dm_set_error("conv_plan_set_fused_update: cuTensorMapEncodeTiled unavailable"); return B200DM_ERR_CUDA; }
+  const cuuint32_t box[5] = {16, 8, 16, 1, 1};   // one round of the fused epilogue: 16 columns x one 8 x 16 plane tile
   CUtensorMap my, mz;
-  if (!enc ||
-      enc(&my, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 5, x_prev, dims, st4, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B,
-          CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS ||
-      enc(&mz, kTmapAct16, 5, x_prev_16, dims, st2, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_32B,
-          CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS) {
-    b200dm_set_error("conv_plan_set_fused_update: cuTensorMapEncodeTiled failed");
-    return B200DM_ERR_CUDA;
-  }
+  int rc = encode_act(enc, &my, "fused update x", x_prev, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, d->c_out, d->in_w, d->in_h, d->in_d,
+                      d->batch, box, CU_TENSOR_MAP_SWIZZLE_64B);
+  if (!rc) rc = encode_act(enc, &mz, "fused update x16", x_prev_16, kTmapAct16, d->c_out, d->in_w, d->in_h, d->in_d, d->batch, box,
+                           CU_TENSOR_MAP_SWIZZLE_32B);
+  Variant fused = pl->v;
+  fused.key.fuse = true;
+  fused.key.ns = kHaloNSFused;
+  if (!rc) rc = bind_kernel(pl, fused);
+  if (rc) return rc;
   pl->om.y[0] = my; pl->om.y[1] = mz;
   pl->p.upd = *u; pl->p.upd_x = x_t;
-  pl->fuse = true;
-  pl->smem = halo_smem_bytes(pl);
-  if (pl->smem > 232448) { b200dm_set_error("conv_plan_set_fused_update: shared memory"); return B200DM_ERR_UNSUPPORTED; }
   return B200DM_OK;
 }
 
 extern "C" int b200dm_conv_plan_info(const b200dm_conv_plan* p, int32_t* halo, int32_t* block_n, int32_t* ksplit) {
   B2_CHECK_ARG(p, "conv_plan_info: null plan");
-  if (halo) *halo = p->stencil ? 2 : (p->sweep ? 3 : (p->halo ? 1 : 0));   // 2 = HBM-bound stencil-reduce kernel (C_out = 1), 3 = d-sweeping N = 96 kernel
-  if (block_n) *block_n = p->g.block_n;
+  const Family f = p->v.key.family;
+  if (halo) *halo = f == Family::kStencil ? 2 : (f == Family::kSweep ? 3 : (f != Family::kGemm ? 1 : 0));   // 2 = HBM-bound stencil-reduce kernel (C_out = 1), 3 = d-sweeping N = 96 kernel
+  if (block_n) *block_n = p->v.key.block_n ? p->v.key.block_n : p->g.block_n;   // (stencil, sweep: the geometry's N tile)
   if (ksplit) *ksplit = p->p.ksplit;
   return B200DM_OK;
 }
@@ -1213,7 +1116,7 @@ extern "C" int b200dm_conv_plan_set_out_affine(b200dm_conv_plan* p, const float*
   B2_CHECK_ARG((scale == nullptr) == (shift == nullptr), "conv_plan_set_out_affine: give both scale and shift, or neither");
   B2_CHECK_ARG(!scale || !p->p.prelu_alpha, "conv_plan_set_out_affine: not combinable with PReLU");
   B2_CHECK_ARG(!scale || !p->p.swap_ab, "conv_plan_set_out_affine: not combinable with a transposed store");
-  B2_CHECK_ARG(!scale || !p->stencil, "conv_plan_set_out_affine: not available on the C_out = 1 stencil plan");
+  B2_CHECK_ARG(!scale || p->v.key.family != Family::kStencil, "conv_plan_set_out_affine: not available on the C_out = 1 stencil plan");
   p->p.out_scale = scale;
   p->p.out_shift = shift;
   return B200DM_OK;
@@ -1223,7 +1126,7 @@ extern "C" int b200dm_conv_plan_set_out_affine(b200dm_conv_plan* p, const float*
 // partial sums of the STORED values into `workspace` (float [rows][C][2], rows = batch * rows_per_sample); b200dm_gn_finalize
 // turns them into (mean, rstd) in a fixed order.  Returns the workspace size, 0 when the plan cannot produce partials.
 extern "C" size_t b200dm_conv_plan_gn_partials_bytes(const b200dm_conv_plan* p, int32_t* rows_per_sample) {
-  if (!p || !p->sweep) return 0;
+  if (!p || p->v.key.family != Family::kSweep) return 0;
   if (rows_per_sample) *rows_per_sample = p->wp.items / p->wp.batch * 2;
   return (size_t)p->wp.items * 2 * 32 * 2 * sizeof(float);
 }

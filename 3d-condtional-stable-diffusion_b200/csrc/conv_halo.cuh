@@ -59,6 +59,25 @@ constexpr int stage_group_bytes(int block_n) { return block_n >= 64 ? 16384 : 81
 constexpr int kFuseStage16Bytes = 2 * 8192;
 constexpr int stage_bytes(int block_n, bool staged) { return staged ? stage_bufs(block_n) * stage_groups(block_n) * stage_group_bytes(block_n) : 0; }
 
+// Shared-memory layout of conv_halo_kernel and conv_halo_up_kernel (TPS = 4, CG2, STAGED), offsets from the 1024-aligned base:
+// slab ring | weight ring | output staging | FUSE_UPD 16-bit staging | barriers | TMEM address | bias + scale [2][2][BLOCK_N].
+template <int BLOCK_N, int NS, int NB, int TPS, bool STAGED, bool PAIR, bool CG2, bool FUSE_UPD>
+struct Smem {
+  static constexpr int kSlabBytes = PAIR ? 25 * 1024 : halo::kSlabBytes;   // 200 (pair) / 180 rows of 128 B, 1 KB-rounded
+  static constexpr int kBRows = CG2 ? BLOCK_N / 2 : BLOCK_N;               // weight rows of one tap staged by THIS CTA
+  static constexpr int kTapBytes = kBRows * 128;
+  static constexpr int kBBytes = TPS * kTapBytes;                           // one weight stage
+  // slab full / empty, weight full / empty, TMEM full / empty x 2; FUSE_UPD: + x_t landed / tiles written x 2 staging sets
+  static constexpr int kBars = 2 * NS + 2 * NB + 4 + (FUSE_UPD ? 4 : 0);
+  static constexpr size_t kBRing = (size_t)NS * kSlabBytes;
+  static constexpr size_t kStage = kBRing + (size_t)NB * kBBytes;          // (1024-aligned: slabs and weight stages are multiples of 1 KB)
+  static constexpr size_t kStage16 = kStage + stage_bytes(BLOCK_N, STAGED);
+  static constexpr size_t kBarOff = kStage16 + (FUSE_UPD ? kFuseStage16Bytes : 0);
+  static constexpr size_t kTmemPtr = kBarOff + (size_t)kBars * 8;
+  static constexpr size_t kBias = kTmemPtr + 16;
+  static constexpr size_t kBytes = 1024 + kBias + 4 * BLOCK_N * 4;         // with the alignment slack
+};
+
 // PAIR (small planes, 8 x 8: the 8^3 level of the U-Net): the tile is 8 w x 8 h x 2 d.  The activation tensor map lists
 // its dims as (C, W, D, H, N), so one box {64, 10, 2, 10, 1} lands in smem as rows [h][d][w]: the 16 eight-row groups of
 // the M = 128 operand (group = h * 2 + d) are again a uniform 10 rows apart, the (kh, kw) tap shift is (kh * 20 + kw) rows,
@@ -78,13 +97,14 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constan
   static_assert(!STAGED || BLOCK_N >= 32, "staged epilogue works on whole 64-channel groups (or one 32-channel group)");
   static_assert(TPS == 1 || TPS == 3, "taps per weight stage: 1 or 3");
   static_assert(!PAIR || (STAGED && TD == 1), "pair-slab tiles: one accumulator, staged epilogue");
-  constexpr int kSlabBytes = PAIR ? 25 * 1024 : halo::kSlabBytes;   // 200 (pair) / 180 rows of 128 B, 1 KB-rounded
+  using L = Smem<BLOCK_N, NS, NB, TPS, STAGED, PAIR, CG2, FUSE_UPD>;
+  constexpr int kSlabBytes = L::kSlabBytes;
   constexpr int kSlabTx = PAIR ? 200 * 128 : halo::kSlabTx;
   constexpr int kKhUnits = PAIR ? 160 : 80;                          // one kh step in 16-byte units (20 / 10 rows)
   static_assert(!CG2 || BLOCK_N >= 32, "CTA-pair variant: each CTA stages BLOCK_N / 2 >= 16 weight rows");
-  constexpr int kBRows = CG2 ? BLOCK_N / 2 : BLOCK_N;   // weight rows of one tap staged by THIS CTA
-  constexpr int kTapBytes = kBRows * 128;
-  constexpr int kBBytes = TPS * kTapBytes;
+  constexpr int kBRows = L::kBRows;
+  constexpr int kTapBytes = L::kTapBytes;
+  constexpr int kBBytes = L::kBBytes;
   // MMA issuer warps: with TD = 2 each output plane (its own TMEM accumulator) is driven by its own warp.  Measured
   // (clock64 timeline): one issuing thread spends ~280 cycles per weight stage on barrier waits / commits / descriptor
   // arithmetic during which the shallow tcgen05 queue drains (59 cycles per N=64 MMA instead of the 48-cycle floor);
@@ -95,12 +115,12 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constan
   static_assert(kTmemCols <= 512 && (kTmemCols & (kTmemCols - 1)) == 0, "TMEM columns must be a power of two <= 512");
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint8_t* b_ring = smem + NS * kSlabBytes;
-  uint8_t* stg_base = b_ring + NB * kBBytes;   // (1024-aligned: slabs and weight stages are multiples of 1 KB)
-  uint8_t* stg16_base = stg_base + stage_bytes(BLOCK_N, STAGED);   // FUSE_UPD: two 8 KB tiles (128 rows x 32 x 16 bit)
-  uint64_t* bars = reinterpret_cast<uint64_t*>(stg16_base + (FUSE_UPD ? kFuseStage16Bytes : 0));
-  uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(bars + 2 * NS + 2 * NB + 4 + (FUSE_UPD ? 4 : 0));   // (+2 x_t barriers, +2 written barriers)
-  float* bias_s = reinterpret_cast<float*>(tmem_ptr_smem + 4);   // [2 acc stages][bias | scale][BLOCK_N]
+  uint8_t* b_ring = smem + L::kBRing;
+  uint8_t* stg_base = smem + L::kStage;
+  uint8_t* stg16_base = smem + L::kStage16;   // FUSE_UPD: two 8 KB tiles (128 rows x 32 x 16 bit)
+  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + L::kBarOff);
+  uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(smem + L::kTmemPtr);
+  float* bias_s = reinterpret_cast<float*>(smem + L::kBias);   // [2 acc stages][bias | scale][BLOCK_N]
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const uint32_t slab_base = ptx::smem_u32(smem);

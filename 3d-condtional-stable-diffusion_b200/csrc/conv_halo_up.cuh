@@ -20,6 +20,10 @@ namespace halo {
 // PAIR: 8 x 8 low-resolution planes (8^3 -> 16^3): the tile is 8 w x 8 h x 2 d from pair slabs (box {64, 10, 2, 10, 1} of a tensor map
 // whose dims are listed (C, W, D, H, N), rows [h][d][w] as in conv_halo_kernel's PAIR variant): one accumulator, one issuer warp,
 // two pair slabs per channel chunk (td = 0, 1), tap offset (th + ph) * 20 + (tw + pw) rows.
+// Shared memory: conv_halo_kernel's layout with 4-tap weight stages of half the rows and the staged epilogue.
+template <int BLOCK_N, int NS, int NB, bool PAIR>
+using UpSmem = Smem<BLOCK_N, NS, NB, 4, true, PAIR, true, false>;
+
 template <int BLOCK_N, int NS, int NB, bool PAIR = false>
 __global__ void __launch_bounds__(kThreads, 1)
 conv_halo_up_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant__ CUtensorMap mapA1,
@@ -29,19 +33,20 @@ conv_halo_up_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_cons
   constexpr int kSlabsPerChunk = PAIR ? 2 : 3;
   constexpr int kIss = PAIR ? 1 : 2;               // issuer warps
   constexpr int kKhUnits = PAIR ? 160 : 80;
-  constexpr int kSlabBytes = PAIR ? 25 * 1024 : halo::kSlabBytes, kSlabTx = PAIR ? 200 * 128 : halo::kSlabTx;
-  constexpr int kBRows = BLOCK_N / 2;
-  constexpr int kTapBytes = kBRows * 128;
-  constexpr int kBBytes = 4 * kTapBytes;
+  using L = UpSmem<BLOCK_N, NS, NB, PAIR>;
+  constexpr int kSlabBytes = L::kSlabBytes, kSlabTx = PAIR ? 200 * 128 : halo::kSlabTx;
+  constexpr int kBRows = L::kBRows;
+  constexpr int kTapBytes = L::kTapBytes;
+  constexpr int kBBytes = L::kBBytes;
   constexpr uint32_t kAccCols = TD * BLOCK_N;
   constexpr uint32_t kTmemCols = 2 * kAccCols;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint8_t* b_ring = smem + NS * kSlabBytes;
-  uint8_t* stg_base = b_ring + NB * kBBytes;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(stg_base + stage_bytes(BLOCK_N, true));
-  uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(bars + 2 * NS + 2 * NB + 4);
-  float* bias_s = reinterpret_cast<float*>(tmem_ptr_smem + 4);
+  uint8_t* b_ring = smem + L::kBRing;
+  uint8_t* stg_base = smem + L::kStage;
+  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + L::kBarOff);
+  uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(smem + L::kTmemPtr);
+  float* bias_s = reinterpret_cast<float*>(smem + L::kBias);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const uint32_t slab_base = ptx::smem_u32(smem);

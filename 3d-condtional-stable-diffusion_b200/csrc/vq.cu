@@ -305,27 +305,13 @@ extern "C" int b200dm_vq_argmin_gather(const b200dm_vq_desc* d, const void* x, c
 // ---- tensor-core candidate search + exact recheck (vq_tc.cuh): same indices as vq_kernel, bit for bit ----------------------
 namespace {
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn vq_encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* f = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &f, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(f);
-  }
-  return fn;
-}
-
 size_t vq_tc_smem_bytes(int k, int d) {
   const int dc = d / 64;
   return 1024 + (size_t)(2 * dc + vqtc::kNSB) * vqtc::kTile + (size_t)k * 4 + 128 * 4 * 2 + (size_t)256 * vqtc::kCap * 8 + 256 * 8 + 128 * 4 +
          (2 * vqtc::kNSB + 4) * 8 + 16;
 }
 bool vq_tc_supported(int k, int d) {
-  return k >= 128 && k % 128 == 0 && d >= 64 && d % 64 == 0 && d <= 256 && vq_tc_smem_bytes(k, d) <= 232448;
+  return k >= 128 && k % 128 == 0 && d >= 64 && d % 64 == 0 && d <= 256 && vq_tc_smem_bytes(k, d) <= kMaxDynamicSmem;
 }
 // workspace: [e_hi K*D fp16][e_lo K*D fp16][meta 4 fp32]
 size_t vq_tc_ws_bytes(int k, int d) { return (size_t)k * d * 4 + 16; }
@@ -357,7 +343,7 @@ extern "C" int b200dm_vq_argmin_gather_tc(const b200dm_vq_desc* d, const void* x
   B2_CHECK_ARG((reinterpret_cast<uintptr_t>(x) & 15) == 0, "vq_argmin_gather_tc: x must be 16-byte aligned");
   const int64_t blocks = (d->n + 127) / 128;
   B2_CHECK_ARG(blocks <= 0x7fffffff, "vq_argmin_gather_tc: too many rows");
-  EncodeTiledFn enc = vq_encode_fn();
+  EncodeTiledFn enc = b2_encode_tiled_fn();
   if (!enc) { b200dm_set_error("vq_argmin_gather_tc: cuTensorMapEncodeTiled unavailable"); return B200DM_ERR_CUDA; }
   CUtensorMap maps[2];
   for (int i = 0; i < 2; ++i) {

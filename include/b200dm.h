@@ -231,7 +231,7 @@ typedef struct {
   int32_t act;                      /* B200DM_ACT_* applied after bias adds, before the residual add */
   int32_t y_dtype;                  /* B200DM_BF16 or B200DM_F32 */
   int32_t chan_bias_rows;           /* rows in chan_bias per timestep (= batch) */
-  int32_t use_halo;                 /* 1: stage one halo tile per K-chunk and shift the A descriptor per tap */
+  int32_t use_halo;                 /* -1: per-tap GEMM kernel only; any other value: the kernel is chosen from the shape */
   int32_t reserved[4];
 } b200dm_conv_desc;
 
