@@ -130,6 +130,7 @@ _SIGS = {
     "b200dm_conv_plan_set_trace": (C.c_int, [C.c_void_p, C.c_void_p]),
     "b200dm_conv_plan_set_out_affine": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "b200dm_conv_plan_set_fused_update": (C.c_int, [C.c_void_p, C.POINTER(UpdateDesc), C.c_void_p, C.c_void_p, C.c_void_p]),
+    "b200dm_conv_plan_set_shortcut": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "b200dm_conv_plan_info": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     "b200dm_conv_plan_gn_partials_bytes": (C.c_size_t, [C.c_void_p, C.POINTER(C.c_int32)]),
     "b200dm_conv_plan_set_gn_partials": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t]),

@@ -645,10 +645,10 @@ int encode_act(EncodeTiledFn enc, CUtensorMap* m, const char* what, const void* 
 }
 
 // packed weights [groups * n_pad rows][ktot / 64 k-blocks][64] as the 3-D view {64, rows, k-blocks}; a box row of 64 (32)
-// channels is one 128-byte (64-byte) swizzle span
-int encode_weights3(EncodeTiledFn enc, CUtensorMap* m, const void* w, const Geometry& g, const int (&box)[3]) {
-  const cuuint64_t dims[3] = {64, (cuuint64_t)g.groups * g.n_pad, (cuuint64_t)(g.ktot / 64)};
-  const cuuint64_t strides[2] = {(cuuint64_t)g.ktot * 2, 128};
+// channels is one 128-byte (64-byte) swizzle span.  ktot: the row length (g.ktot, or longer with a folded shortcut's k-blocks)
+int encode_weights3(EncodeTiledFn enc, CUtensorMap* m, const void* w, const Geometry& g, const int (&box)[3], size_t ktot) {
+  const cuuint64_t dims[3] = {64, (cuuint64_t)g.groups * g.n_pad, (cuuint64_t)(ktot / 64)};
+  const cuuint64_t strides[2] = {(cuuint64_t)ktot * 2, 128};
   const cuuint32_t b[3] = {(cuuint32_t)box[0], (cuuint32_t)box[1], (cuuint32_t)box[2]}, es[3] = {1, 1, 1};
   const CUresult r = enc(m, kTmapAct16, 3, const_cast<void*>(w), dims, strides, b, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
                          box[0] == 64 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
@@ -670,6 +670,7 @@ struct b200dm_conv_plan {
   CUtensorMap mapA0, mapA1, mapB;
   ConvOutMaps om;
   CUtensorMap mapS;       // stencil / sweep kernels: the input (mapB = the sweep kernel's weights, om.y[0] its output)
+  CUtensorMap mapSc0, mapSc1;   // halo kernel: the two input segments of a folded 1^3 shortcut (b200dm_conv_plan_set_shortcut)
   stencil::Params sp;
   sweep::Params wp;
   dim3 grid;
@@ -773,10 +774,10 @@ cudaError_t launch_args(void (*k)(CUtensorMap, CUtensorMap, CUtensorMap, ConvOut
                         unsigned threads, cudaStream_t s) {
   return launch_plan(k, pl, threads, s, pl->mapA0, pl->mapA1, pl->mapB, pl->om, pl->p);
 }
-// halo kernel: output map (the fused update: x_{t-1}) and its 16-bit copy
-cudaError_t launch_args(void (*k)(CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, ConvParams),
+// halo kernel: output map (the fused update: x_{t-1}) and its 16-bit copy, shortcut input segments
+cudaError_t launch_args(void (*k)(CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, ConvParams),
                         const b200dm_conv_plan* pl, unsigned threads, cudaStream_t s) {
-  return launch_plan(k, pl, threads, s, pl->mapA0, pl->mapA1, pl->mapB, pl->om.y[0], pl->om.y[1], pl->p);
+  return launch_plan(k, pl, threads, s, pl->mapA0, pl->mapA1, pl->mapB, pl->om.y[0], pl->om.y[1], pl->mapSc0, pl->mapSc1, pl->p);
 }
 // sweep kernel: input, weights, output, residual (a valid map either way: unused without a residual)
 cudaError_t launch_args(void (*k)(CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, ConvParams, sweep::Params),
@@ -902,7 +903,7 @@ int setup_plan(b200dm_conv_plan* pl, EncodeTiledFn enc, const void* x0, const vo
     rc = encode_act(enc, &pl->mapS, "sweep X", x0, kTmapAct16, 32, d->in_w, d->in_h, d->in_d, d->batch, {32, 10, 18, 2, 1},
                     CU_TENSOR_MAP_SWIZZLE_64B);
     if (!rc) rc = encode_act(enc, &pl->om.y[0], "sweep Y", y, kTmapAct16, 32, d->in_w, d->in_h, d->in_d, d->batch, boxy, CU_TENSOR_MAP_SWIZZLE_64B);
-    if (!rc) rc = encode_weights3(enc, &pl->mapB, w_packed, g, v.wbox);
+    if (!rc) rc = encode_weights3(enc, &pl->mapB, w_packed, g, v.wbox, g.ktot);
     if (!rc && residual)
       rc = encode_act(enc, &pl->om.r, "sweep residual", residual, kTmapAct16, 32, d->in_w, d->in_h, d->in_d, d->batch, boxy, CU_TENSOR_MAP_SWIZZLE_64B);
     if (rc) return rc;
@@ -935,7 +936,7 @@ int setup_plan(b200dm_conv_plan* pl, EncodeTiledFn enc, const void* x0, const vo
     if (rc) return rc;
   }
   if (halo) {
-    rc = encode_weights3(enc, &pl->mapB, w_packed, g, v.wbox);
+    rc = encode_weights3(enc, &pl->mapB, w_packed, g, v.wbox, g.ktot);
     if (rc) return rc;
   } else {
     // packed [group][n_pad rows][K]; batched GEMM: B is a raw activation tensor [batch][c_out rows][K = c0] whose rows beyond c_out
@@ -1071,7 +1072,7 @@ extern "C" int b200dm_conv_plan_set_fused_update(b200dm_conv_plan* pl, const b20
   const KernelKey& k = pl->v.key;
   // the CTA-pair N = 128 halo kernel with the fp32 staged epilogue, no other epilogue term
   if (!(k.family == Family::kHalo && k.cg2 && !k.pair && k.block_n == 128 && p.y_f32 && k.staged && d->c_out % 128 == 0 &&
-        !p.residual && !p.prelu_alpha && p.act == B200DM_ACT_NONE && p.post_act == B200DM_ACT_NONE)) {
+        !p.residual && p.sc_nch0 == 0 && !p.prelu_alpha && p.act == B200DM_ACT_NONE && p.post_act == B200DM_ACT_NONE)) {
     b200dm_set_error("conv_plan_set_fused_update: only on the CTA-pair fp32-output 3^3 conv with C_out %% 128 == 0");
     return B200DM_ERR_UNSUPPORTED;
   }
@@ -1099,6 +1100,44 @@ extern "C" int b200dm_conv_plan_set_fused_update(b200dm_conv_plan* pl, const b20
   if (rc) return rc;
   pl->om.y[0] = my; pl->om.y[1] = mz;
   pl->p.upd = *u; pl->p.upd_x = x_t;
+  return B200DM_OK;
+}
+
+extern "C" int b200dm_conv_plan_set_shortcut(b200dm_conv_plan* pl, int32_t c0, int32_t c1, const void* x0, const void* x1,
+                                             const void* w_packed, const float* bias) {
+  B2_CHECK_ARG(pl && x0 && w_packed, "conv_plan_set_shortcut: null argument");
+  const b200dm_conv_desc* d = &pl->desc;
+  const KernelKey& k = pl->v.key;
+  // the halo-reuse 3^3 kernel carries the segment as a runtime option of every instantiation: the plan keeps its kernel
+  if (k.family != Family::kHalo || k.fuse) {
+    b200dm_set_error("conv_plan_set_shortcut: only on plans of the 3^3 halo-reuse kernel without the fused update");
+    return B200DM_ERR_UNSUPPORTED;
+  }
+  B2_CHECK_ARG(pl->p.sc_nch0 == 0, "conv_plan_set_shortcut: the plan already has a shortcut");
+  B2_CHECK_ARG(c0 > 0 && c0 % 8 == 0 && c1 >= 0 && c1 % 8 == 0, "conv_plan_set_shortcut: C_in segments must be multiples of 8 (got %d,%d)", c0, c1);
+  B2_CHECK_ARG((c1 > 0) == (x1 != nullptr), "conv_plan_set_shortcut: x1 must be given iff c1 > 0");
+  B2_CHECK_ARG(((uintptr_t)x0 & 15) == 0 && ((uintptr_t)x1 & 15) == 0 && ((uintptr_t)w_packed & 15) == 0,
+               "conv_plan_set_shortcut: pointers must be 16-byte aligned");
+  EncodeTiledFn enc = b2_encode_tiled_fn();
+  if (!enc) { b200dm_set_error("conv_plan_set_shortcut: cuTensorMapEncodeTiled unavailable"); return B200DM_ERR_CUDA; }
+  const int nch0 = (c0 + 63) / 64, nch1 = (c1 + 63) / 64;
+  const size_t ktot = pl->g.ktot + (size_t)(nch0 + nch1 + 2) / 3 * 3 * 64;   // + the shortcut's k-blocks, padded to whole 3-tap stages
+  // the 3^3 segments' halo slab box: the kernel reads the shortcut at its centre tap
+  const cuuint32_t box[5] = {64, 10, (cuuint32_t)(k.pair ? 2 : 18), (cuuint32_t)(k.pair ? 10 : 1), 1};
+  CUtensorMap m0, m1, mb;
+  int rc = encode_act(enc, &m0, "shortcut X", x0, kTmapAct16, c0, d->in_w, d->in_h, d->in_d, d->batch, box, CU_TENSOR_MAP_SWIZZLE_128B, 1,
+                      1, k.pair);
+  if (!rc) rc = encode_act(enc, &m1, "shortcut X", c1 > 0 ? x1 : x0, kTmapAct16, c1 > 0 ? c1 : c0, d->in_w, d->in_h, d->in_d, d->batch,
+                           box, CU_TENSOR_MAP_SWIZZLE_128B, 1, 1, k.pair);
+  if (!rc) rc = encode_weights3(enc, &mb, w_packed, pl->g, pl->v.wbox, ktot);
+  if (rc) return rc;
+  pl->mapSc0 = m0; pl->mapSc1 = m1; pl->mapB = mb;
+  ConvParams& p = pl->p;
+  p.sc_nch0 = nch0; p.sc_nch1 = nch1;
+  p.sc_ksteps0_last = ((c0 - (nch0 - 1) * 64) + 15) / 16;
+  p.sc_ksteps1_last = c1 > 0 ? ((c1 - (nch1 - 1) * 64) + 15) / 16 : 4;
+  p.bias = bias;
+  pl->flops += 2.0 * (c0 + c1) * d->c_out * (double)d->batch * pl->g.out_d * pl->g.out_h * pl->g.out_w;
   return B200DM_OK;
 }
 

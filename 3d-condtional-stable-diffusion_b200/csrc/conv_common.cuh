@@ -13,6 +13,9 @@ struct ConvParams {
   int tiles_w, tiles_h, tiles_d, tiles_n;
   int nch0, nch1, ntaps, ksize, stride, pad;
   int ksteps0_last, ksteps1_last;    // K=16 MMA steps that hold real channels in the LAST 64-channel chunk of each segment (1..4)
+  // halo kernel: a 1^3 conv of two more segments (the ResidualBlock shortcut of [x | skip]) accumulated after the 3^3 chunks,
+  // centre tap only (b200dm_conv_plan_set_shortcut); sc_nch0 = 0: none
+  int sc_nch0, sc_nch1, sc_ksteps0_last, sc_ksteps1_last;
   int c_out, n_pad;
   int act, post_act, y_f32, transposed_store;
   int chan_bias_rows;

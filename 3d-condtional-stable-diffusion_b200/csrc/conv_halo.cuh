@@ -16,6 +16,9 @@
 //             an mbarrier wait costs ~110 cycles and a commit ~45 on the single issuing thread, and an M128xN64xK16
 //             MMA only 48, so one tap per round trip is issue-bound; three are not.
 //   TMEM      2 accumulator stages x TD x BLOCK_N columns: the epilogue of tile i overlaps the MMAs of tile i+1.
+//   shortcut  optional 1^3 conv of two more tensors (mapS0 / mapS1: a ResidualBlock's [x | skip]) in the same accumulators, after
+//             the 3^3 chunks: per 64-channel chunk TD slabs (pair: the kd = 1 pair slab) of the same halo box, read at the
+//             centre tap only; its k-blocks follow the 3^3 ones in the weight rows (one tap each, padded to whole stages).
 //
 // Warps (384 threads): 0 = slab producer, 1 = weight producer, 2 = TMEM owner + MMA issuer, 3 = second MMA issuer (TD = 2), 4-11 = epilogue.
 // Every role loop is warp-uniform; a single elected lane (elect.sync) issues TMA / tcgen05 instructions.
@@ -92,7 +95,8 @@ template <int BLOCK_N, int TD, int NS, int NB, int TPS, bool STAGED, bool PAIR =
 __global__ void __launch_bounds__(FUSE_UPD ? kThreadsFused : kThreads, 1)
 conv_halo_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant__ CUtensorMap mapA1,
                  const __grid_constant__ CUtensorMap mapB, const __grid_constant__ CUtensorMap mapY,
-                 const __grid_constant__ CUtensorMap mapZ, const ConvParams p) {
+                 const __grid_constant__ CUtensorMap mapZ, const __grid_constant__ CUtensorMap mapS0,
+                 const __grid_constant__ CUtensorMap mapS1, const ConvParams p) {
   static_assert(!FUSE_UPD || (STAGED && BLOCK_N == 128 && !PAIR), "fused update: fp32 staged epilogue of the N = 128 tiles");
   static_assert(!STAGED || BLOCK_N >= 32, "staged epilogue works on whole 64-channel groups (or one 32-channel group)");
   static_assert(TPS == 1 || TPS == 3, "taps per weight stage: 1 or 3");
@@ -141,6 +145,7 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constan
 
   pdl_launch_dependents();
   const int nch = p.nch0 + p.nch1;
+  const int sc_nch = p.sc_nch0 + p.sc_nch1;
   const int first_tile = blockIdx.x, tile_step = gridDim.x;
   const uint32_t crank = CG2 ? ptx::cluster_ctarank() : 0u;
   const bool leader = crank == 0;
@@ -154,6 +159,7 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constan
     ptx::fence_barrier_init();
     ptx::prefetch_tmap(&mapA0);
     ptx::prefetch_tmap(&mapB);
+    if (sc_nch > 0) ptx::prefetch_tmap(&mapS0);
     if (STAGED) ptx::prefetch_tmap(&mapY);
     if (FUSE_UPD) ptx::prefetch_tmap(&mapZ);
   }
@@ -173,31 +179,37 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constan
     uint32_t s = 0, ph = 1;
     bool ok = true;
     int ti = 0;
+    // the next ring slot <- the slab of channels c0.. whose first input plane is d (pair slab: planes d, d + 1)
+    auto load_slab = [&](const Tile& t, const CUtensorMap* map, int c0, int d, int tag) {
+      ok = ptx::mbar_wait(slab_empty(s), ph, p.dbg, 11);
+      if (!ok) return;
+      if (lane == 0) trace_ev(p, 2, ti, tag);
+      if (ptx::elect_one()) {
+        if (CG2) {   // both CTAs' slabs complete on the LEADER's barrier, which expects both transfers
+          if (leader) ptx::mbar_expect_tx(slab_full(s), 2 * kSlabTx);
+          if (PAIR) ptx::tma_load_5d_cg2(slab_base + s * kSlabBytes, map, ptx::mapa_shared(slab_full(s), 0), c0, t.w0 - 1, d, t.h0 - 1, t.n);
+          else ptx::tma_load_5d_cg2(slab_base + s * kSlabBytes, map, ptx::mapa_shared(slab_full(s), 0), c0, t.w0 - 1, t.h0 - 1, d, t.n);
+        } else {
+          ptx::mbar_expect_tx(slab_full(s), kSlabTx);
+          if (PAIR) ptx::tma_load_5d(slab_base + s * kSlabBytes, map, slab_full(s), c0, t.w0 - 1, d, t.h0 - 1, t.n);
+          else ptx::tma_load_5d(slab_base + s * kSlabBytes, map, slab_full(s), c0, t.w0 - 1, t.h0 - 1, d, t.n);
+        }
+      }
+      __syncwarp();
+      if (++s == NS) { s = 0; ph ^= 1; }
+    };
     for (int id = first_tile; id < p.halo_total_tiles && ok; id += tile_step) {
       const Tile t = decode_tile<PAIR>(p, id);
       for (int j = 0; j < nch && ok; ++j) {
         const CUtensorMap* map = j < p.nch0 ? &mapA0 : &mapA1;
         const int c0 = (j < p.nch0 ? j : j - p.nch0) * 64;
-        for (int pl = 0; pl < TD + 2; ++pl) {
-          ok = ptx::mbar_wait(slab_empty(s), ph, p.dbg, 11);
-          if (!ok) break;
-          if (lane == 0) trace_ev(p, 2, ti, 20 + pl);
-          if (ptx::elect_one()) {
-            if (CG2) {   // both CTAs' slabs complete on the LEADER's barrier, which expects both transfers
-              if (leader) ptx::mbar_expect_tx(slab_full(s), 2 * kSlabTx);
-              if (PAIR) ptx::tma_load_5d_cg2(slab_base + s * kSlabBytes, map, ptx::mapa_shared(slab_full(s), 0), c0, t.w0 - 1,
-                                             t.d0 - 1 + pl, t.h0 - 1, t.n);
-              else ptx::tma_load_5d_cg2(slab_base + s * kSlabBytes, map, ptx::mapa_shared(slab_full(s), 0), c0, t.w0 - 1, t.h0 - 1,
-                                        t.d0 - 1 + pl, t.n);
-            } else {
-              ptx::mbar_expect_tx(slab_full(s), kSlabTx);
-              if (PAIR) ptx::tma_load_5d(slab_base + s * kSlabBytes, map, slab_full(s), c0, t.w0 - 1, t.d0 - 1 + pl, t.h0 - 1, t.n);
-              else ptx::tma_load_5d(slab_base + s * kSlabBytes, map, slab_full(s), c0, t.w0 - 1, t.h0 - 1, t.d0 - 1 + pl, t.n);
-            }
-          }
-          __syncwarp();
-          if (++s == NS) { s = 0; ph ^= 1; }
-        }
+        for (int pl = 0; pl < TD + 2 && ok; ++pl) load_slab(t, map, c0, t.d0 - 1 + pl, 20 + pl);
+      }
+      // shortcut: the output planes themselves (pair: the kd = 1 slab)
+      for (int j = 0; j < sc_nch && ok; ++j) {
+        const CUtensorMap* map = j < p.sc_nch0 ? &mapS0 : &mapS1;
+        const int c0 = (j < p.sc_nch0 ? j : j - p.sc_nch0) * 64;
+        for (int pl = 0; pl < TD && ok; ++pl) load_slab(t, map, c0, t.d0 + pl, 24 + pl);
       }
     }
   } else if (warp == 1) {
@@ -207,7 +219,7 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constan
     for (int id = first_tile; id < p.halo_total_tiles && ok; id += tile_step) {
       const Tile t = decode_tile<PAIR>(p, id);
       const int row0 = t.n_tile * BLOCK_N;
-      for (int kb = 0; kb < nch * 27; kb += TPS) {
+      for (int kb = 0; kb < nch * 27 + (sc_nch + TPS - 1) / TPS * TPS; kb += TPS) {
         ok = ptx::mbar_wait(b_empty(s), ph, p.dbg, 12);
         if (!ok) break;
         if (ptx::elect_one()) {
@@ -316,6 +328,37 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constan
         }
         qs += TD + 2;
         if (qs >= (uint32_t)NS) { qs -= NS; qph ^= 1; }
+      }
+      // shortcut: TPS chunks per weight stage, each one tap (the slab's centre) on its own TD slabs, released chunk by chunk
+      for (int j0 = 0; j0 < sc_nch && ok; j0 += TPS) {
+        ok = ptx::mbar_wait(b_full(sb), bph, p.dbg, 15);
+        if (!ok) break;
+        const uint64_t db0 = b_desc0 + (uint64_t)(sb * (kBBytes >> 4));
+#pragma unroll 1
+        for (int u = 0; u < TPS && j0 + u < sc_nch && ok; ++u) {
+          const int j = j0 + u;
+          const int ks = j == p.sc_nch0 - 1 ? p.sc_ksteps0_last : (j == sc_nch - 1 && p.sc_nch1 > 0 ? p.sc_ksteps1_last : 4);
+          uint32_t ph;
+          for (int pl = 0; pl < TD && ok; ++pl) { const uint32_t sl = slot(pl, ph); ok = ptx::mbar_wait(slab_full(sl), ph, p.dbg, 14); }
+          if (!ok) break;
+          ptx::tc_fence_after();
+#pragma unroll
+          for (int pl = 0; pl < TD; ++pl) {
+            if (pl < pl_lo || pl >= pl_hi) continue;
+            const uint64_t da = a_desc0 + (uint64_t)(slot(pl, ph) * (uint32_t)(kSlabBytes >> 4)) + (uint64_t)(kKhUnits + 8);   // kh = kw = 1
+            const uint64_t db = db0 + (uint64_t)(u * (kTapBytes >> 4));
+            mma(acc + pl * BLOCK_N, da, db, 1u);
+            if (ks > 1) mma(acc + pl * BLOCK_N, da + 2, db + 2, 1u);
+            if (ks > 2) mma(acc + pl * BLOCK_N, da + 4, db + 4, 1u);
+            if (ks > 3) mma(acc + pl * BLOCK_N, da + 6, db + 6, 1u);
+          }
+#pragma unroll
+          for (int pl = 0; pl < TD; ++pl) commit(slab_empty(slot(pl, ph)));
+          qs += TD;
+          if (qs >= (uint32_t)NS) { qs -= NS; qph ^= 1; }
+        }
+        commit(b_empty(sb));
+        if (++sb == NB) { sb = 0; bph ^= 1; }
       }
       commit(tmem_full(as));
     }

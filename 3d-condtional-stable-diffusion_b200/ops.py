@@ -225,6 +225,15 @@ def pack_conv_weights(desc: L.ConvDesc, keras_kernel: torch.Tensor, transposed=F
     return out
 
 
+def fold_shortcut_weights(w_packed: torch.Tensor, sc_desc: L.ConvDesc, sc_packed: torch.Tensor) -> torch.Tensor:
+    """Packed weights of a 3^3 conv with those of a 1^3 conv on the same output channels (``sc_desc``) appended to each row,
+    zero-padded to a multiple of 3 k-blocks: the layout ``ConvPlan.set_shortcut`` reads."""
+    kb = -(-sc_desc.c0 // 64) + -(-sc_desc.c1 // 64)
+    rows = sc_packed.numel() // (kb * 64)
+    pad = torch.zeros(rows, (-kb) % 3 * 64, dtype=w_packed.dtype, device=w_packed.device)
+    return torch.cat([w_packed.view(rows, -1), sc_packed.to(w_packed.device).view(rows, -1), pad], dim=1).reshape(-1)
+
+
 class ConvPlan:
     """One conv / GEMM invocation with fixed buffers (owns the TMA descriptors)."""
 
@@ -263,6 +272,20 @@ class ConvPlan:
             return False
         check(rc)
         self.keep = self.keep + (x_t, x_prev, x_prev_16, upd_desc)
+        return True
+
+    def set_shortcut(self, x0, x1, w_packed, bias):
+        """Fold a 1^3 conv of [x0 | x1] into this 3^3 conv's K loop (a ResidualBlock's shortcut): ``w_packed`` from
+        ``fold_shortcut_weights``, ``bias`` the two convs' biases summed.  False when the plan's kernel cannot (the caller then
+        runs the 1^3 conv on its own and passes its output as the residual)."""
+        rc = lib().b200dm_conv_plan_set_shortcut(self.h, x0.shape[-1], x1.shape[-1] if x1 is not None else 0, ptr(x0), ptr(x1),
+                                                 ptr(w_packed), ptr(bias))
+        if rc == L.ERR_UNSUPPORTED:
+            return False
+        check(rc)
+        nbytes = lambda t: float(t.numel() * t.element_size()) if t is not None else 0.0  # noqa: E731
+        self.alg_bytes += nbytes(x0) + nbytes(x1) + nbytes(w_packed) - nbytes(self.keep[2])
+        self.keep = self.keep + (x0, x1, w_packed, bias)
         return True
 
     def run(self):

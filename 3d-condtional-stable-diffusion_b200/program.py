@@ -41,9 +41,13 @@ class Program:
 
     # -- ops
     def conv(self, desc, x0, w_packed, y, x1=None, bias=None, chan_bias=None, t_dev=None, residual=None,
-             prelu_alpha=None, out_affine=None, note=""):
+             prelu_alpha=None, out_affine=None, shortcut=None, note=""):
+        """``shortcut``: (x0, x1, w_packed, bias) of ConvPlan.set_shortcut; returns None, adding nothing, when the plan's
+        kernel cannot carry it."""
         plan = ops.ConvPlan(desc, x0, w_packed, y, x1=x1, bias=bias, chan_bias=chan_bias, t_dev=t_dev,
                             residual=residual, prelu_alpha=prelu_alpha, out_affine=out_affine)
+        if shortcut is not None and not plan.set_shortcut(*shortcut):
+            return None
         check(lib().b200dm_program_add_conv(self.h, plan.h))
         plan.release()
         self.keep.extend(t for t in plan.keep if t is not None)

@@ -184,7 +184,9 @@ class UNet:
 
         def conv(x0, kname, cout, y=None, x1=None, k=3, stride=1, mode=L.CONV_DIRECT, act=None, bias=True, chan_bias=None,
                  residual=None, y_dtype=torch.bfloat16, transposed_store=False, dense=False, out_affine=None, note="",
-                 kern=None, bias_t=None):
+                 kern=None, bias_t=None, shortcut=None):
+            """``shortcut``: (x, skip, name) of a 1^3 conv folded into this conv's K loop; None (nothing launched) when the
+            conv's kernel cannot carry it."""
             Bx, D, H, Wd, c0 = x0.shape
             c1 = x1.shape[-1] if x1 is not None else 0
             desc = ops.make_conv_desc(mode, Bx, (D, H, Wd), c0, c1, cout, k, stride, act, None, y_dtype,
@@ -199,9 +201,15 @@ class UNet:
                 od, oh, ow = ops.conv_out_shape(mode, (D, H, Wd), stride)
                 y = pr.buf((Bx, cout, od * oh * ow) if transposed_store else (Bx, od, oh, ow, cout), y_dtype)
             bias_dev = None if not bias else (bias_t.to(dev).contiguous() if bias_t is not None else g(f"{kname}.bias"))
+            fold = None
+            if shortcut is not None:
+                sx, ss, sn = shortcut
+                sdesc = ops.make_conv_desc(L.CONV_DIRECT, Bx, (D, H, Wd), sx.shape[-1], ss.shape[-1] if ss is not None else 0, cout, 1)
+                fold = (sx, ss, ops.fold_shortcut_weights(wp, sdesc, ops.pack_conv_weights(sdesc, P[f"{sn}.kernel"])),
+                        (P[f"{kname}.bias"] + P[f"{sn}.bias"]).to(dev))   # the two biases summed once, in fp32
             return pr.conv(desc, x0, wp, y, x1=x1, bias=bias_dev, chan_bias=chan_bias,
                            t_dev=self.t_dev if (chan_bias is not None and not self.per_sample_t) else None, residual=residual,
-                           out_affine=out_affine, note=note or kname)
+                           out_affine=out_affine, shortcut=fold, note=note or kname)
 
         def bgemm(a, b, y_dtype, residual=None, note=""):
             Bx, M, K = a.shape
@@ -234,13 +242,10 @@ class UNet:
         def resblock(b, x, skip):
             n, w = b["name"], b["cout"]
             cin = b["cin"] + b["cskip"]
-            if cin != w:
-                # (norm1 as a side output of this conv, written from its A tiles, measured slower than the norm pass: 3.35 vs
-                # 3.15 ms/step on cfg-2 -- one-tile CTAs serialise load -> transform -> store)
-                res = conv(x, f"{n}.shortcut", w, x1=skip, k=1)
-            elif skip is None:
+            res = None      # width change: the 1^3 shortcut conv, with conv2 below
+            if cin == w and skip is None:
                 res = x
-            else:  # concat whose width equals w: materialise it once (identity affine)
+            elif cin == w:  # concat whose width equals w: materialise it once (identity affine)
                 one, zero = torch.ones(cin, device=dev), torch.zeros(cin, device=dev)
                 res = pr.norm_act(x, one, zero, pr.buf((*x.shape[:-1], cin)), x1=skip, note=f"{n}.concat")
             table = ops.dense_f32(temb, g(f"{n}.temb.kernel"), g(f"{n}.temb.bias"), act_in="silu")  # (T, w)
@@ -254,6 +259,16 @@ class UNet:
             sc2, sh2 = ops.bn_fold(g(f"{n}.norm2.gamma"), g(f"{n}.norm2.beta"), g(f"{n}.norm2.mean"), g(f"{n}.norm2.var"), 1e-3)
             h = conv(h, f"{n}.conv1", w, x1=h1, chan_bias=pr.hold(table), out_affine=(sc2, sh2), act="silu", note=f"{n}.conv1+norm2")
             pr.outputs[f"{n}.norm2"] = h
+            if cin != w:
+                # width change: the 1^3 shortcut of [x | skip] runs as the last K segment of conv2 (halo kernel), so its output is
+                # never stored and read back; where conv2's kernel cannot carry it, it is a conv of its own and conv2's residual.
+                # (norm1 as a side output of the shortcut conv, written from its A tiles, measured slower than the norm pass:
+                # 3.35 vs 3.15 ms/step on cfg-2 -- one-tile CTAs serialise load -> transform -> store)
+                y = pr.buf(h.shape)
+                if conv(h, f"{n}.conv2", w, y=y, shortcut=(x, skip, f"{n}.shortcut")) is not None:
+                    return y
+                res = conv(x, f"{n}.shortcut", w, x1=skip, k=1)
+                return conv(h, f"{n}.conv2", w, y=y, residual=res)
             return conv(h, f"{n}.conv2", w, residual=res)
 
         def attention_core(q, k, vT, scale, residual, note):

@@ -264,6 +264,14 @@ int b200dm_conv_plan_set_out_affine(b200dm_conv_plan* p, const float* scale, con
  * HBM and no separate update launch.  `u` is read as by b200dm_ddpm_update (tables, t_dev, seed, sample_id0, sampler; no injected
  * noise).  Returns B200DM_ERR_UNSUPPORTED unless the plan is the CTA-pair 3^3 conv with fp32 output and C_out % 128 == 0. */
 int b200dm_conv_plan_set_fused_update(b200dm_conv_plan* p, const b200dm_update_desc* u, const float* x_t, float* x_prev, void* x_prev_16);
+/* Fold a 1^3 conv of [x0 | x1] (c0 + c1 channels, the plan's input geometry: a ResidualBlock's shortcut) into
+ * this 3^3 conv's K loop: y = epilogue(conv(x) + W_sc [x0 | x1] + bias), so the shortcut is never stored and read back.
+ * w_packed: each of the plan's packed weight rows (b200dm_conv_pack_weights) followed by the same row of the 1^3 conv's packed
+ * weights, zero-padded to a multiple of 3 k-blocks of 64 channels; bias: the combined bias (the two convs' biases summed).
+ * Replaces the plan's weights and bias.  Returns B200DM_ERR_UNSUPPORTED unless the plan runs the halo-reuse 3^3 kernel
+ * without the fused update. */
+int b200dm_conv_plan_set_shortcut(b200dm_conv_plan* p, int32_t c0, int32_t c1, const void* x0, const void* x1, const void* w_packed,
+                                  const float* bias);
 /* which kernel / tile configuration the plan launches (profiling): halo 1 = persistent halo-reuse kernel */
 int b200dm_conv_plan_info(const b200dm_conv_plan* p, int32_t* halo, int32_t* block_n, int32_t* ksplit);
 /* GroupNorm statistics as a by-product of the producing conv (replaces a second read of the conv output by
