@@ -33,12 +33,6 @@ struct AttnParams {
   int* dbg;
 };
 
-__device__ __forceinline__ void tma_load_3d(uint32_t dst, const CUtensorMap* m, uint32_t bar, int c0, int c1, int c2) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];" ::"r"(dst),
-      "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1), "r"(c2)
-      : "memory");
-}
 __device__ __forceinline__ void tc_st_32x32b_x16(uint32_t taddr, const uint32_t (&r)[16]) {
   asm volatile(
       "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16};" ::"r"(taddr),
@@ -139,7 +133,7 @@ flash_attn_kernel(const __grid_constant__ CUtensorMap mapQ, const __grid_constan
     // ===================== TMA producer =====================
     if (ptx::elect_one()) {
       ptx::mbar_expect_tx(q_full, SM::kQ);
-      for (int c = 0; c < kDC; ++c) tma_load_3d(q_base + c * (128 * 128), &mapQ, q_full, c * 64, q0, n);
+      for (int c = 0; c < kDC; ++c) ptx::tma_load_3d(q_base + c * (128 * 128), &mapQ, q_full, c * 64, q0, n);
     }
     __syncwarp();
     uint32_t s = 0, ph = 1;
@@ -147,13 +141,13 @@ flash_attn_kernel(const __grid_constant__ CUtensorMap mapQ, const __grid_constan
       if (!ptx::mbar_wait(k_empty(s), ph, p.dbg, 21)) break;
       if (ptx::elect_one()) {
         ptx::mbar_expect_tx(k_full(s), SM::kK);
-        for (int c = 0; c < kDC; ++c) tma_load_3d(k_base + s * SM::kK + c * (BKV * 128), &mapK, k_full(s), c * 64, j * BKV, n);
+        for (int c = 0; c < kDC; ++c) ptx::tma_load_3d(k_base + s * SM::kK + c * (BKV * 128), &mapK, k_full(s), c * 64, j * BKV, n);
       }
       __syncwarp();
       if (!ptx::mbar_wait(v_empty(s), ph, p.dbg, 22)) break;
       if (ptx::elect_one()) {
         ptx::mbar_expect_tx(v_full(s), SM::kV);
-        for (int c = 0; c < kKC; ++c) tma_load_3d(v_base + s * SM::kV + c * (D * 128), &mapVt, v_full(s), j * BKV + c * 64, 0, n);
+        for (int c = 0; c < kKC; ++c) ptx::tma_load_3d(v_base + s * SM::kV + c * (D * 128), &mapVt, v_full(s), j * BKV + c * 64, 0, n);
       }
       __syncwarp();
       if (++s == NST) { s = 0; ph ^= 1; }
@@ -168,7 +162,7 @@ flash_attn_kernel(const __grid_constant__ CUtensorMap mapQ, const __grid_constan
       }
       if (okr && ptx::elect_one()) {
         ptx::mbar_expect_tx(res_full, SM::kQ);
-        for (int c = 0; c < kDC; ++c) tma_load_3d(k_base + c * (128 * 128), &mapR, res_full, c * 64, q0, n);
+        for (int c = 0; c < kDC; ++c) ptx::tma_load_3d(k_base + c * (128 * 128), &mapR, res_full, c * 64, q0, n);
       }
       __syncwarp();
     }

@@ -51,6 +51,24 @@ struct GemmSmem {
   static constexpr size_t bytes(bool staged_res) { return 1024 + bar_off(staged_res) + kTmemPtr + 16 + 2 * BLOCK_N * 4; }
 };
 
+// Split-K: adds the partial accumulators of the cluster's other ks - 1 CTAs (staged as fp32 [col / 4][row] float4 in their
+// shared memory, read through DSMEM) to NB blocks of 16 accumulator columns c0 + 16 b .. of row r.
+template <int NB>
+__device__ __forceinline__ void add_peer_partials(uint32_t (&rr)[NB][16], const float* stage_f, int c0, int r, int ks) {
+  for (int pr = 1; pr < ks; ++pr) {
+    const uint32_t remote = ptx::mapa_shared(ptx::smem_u32(stage_f + c0 * 128 + r * 4), (uint32_t)pr);
+#pragma unroll
+    for (int j = 0; j < 16; j += 4) {
+#pragma unroll
+      for (int b = 0; b < NB; ++b) {
+        const float4 a4 = ptx::ld_dsmem_f32x4(remote + (16 * b + j) * 512);
+        rr[b][j] = __float_as_uint(__uint_as_float(rr[b][j]) + a4.x); rr[b][j + 1] = __float_as_uint(__uint_as_float(rr[b][j + 1]) + a4.y);
+        rr[b][j + 2] = __float_as_uint(__uint_as_float(rr[b][j + 2]) + a4.z); rr[b][j + 3] = __float_as_uint(__uint_as_float(rr[b][j + 3]) + a4.w);
+      }
+    }
+  }
+}
+
 // KSPLIT: split-K cluster (K range per CTA, partial accumulators reduced through distributed shared memory by the cluster's
 // first CTA); four-stage instantiations only.
 // (two-stage instantiations: registers capped so that four CTAs share an SM -- see select_variant)
@@ -298,26 +316,14 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_consta
 #pragma unroll
             for (int h = 0; h < 2; ++h) {
               const int c0 = g * 64 + h * 32;
-              uint32_t ra[16], rb[16];
-              ptx::tc_ld_32x32b_x16(trow + (uint32_t)c0, ra);
-              ptx::tc_ld_32x32b_x16(trow + (uint32_t)c0 + 16, rb);
+              uint32_t rab[2][16];
+              ptx::tc_ld_32x32b_x16(trow + (uint32_t)c0, rab[0]);
+              ptx::tc_ld_32x32b_x16(trow + (uint32_t)c0 + 16, rab[1]);
               ptx::tc_wait_ld();
-              if (KSPLIT) {
-                for (int pr = 1; pr < ks; ++pr) {
-                  const uint32_t remote = ptx::mapa_shared(ptx::smem_u32(stage_f + c0 * 128 + r * 4), (uint32_t)pr);
-#pragma unroll
-                  for (int j = 0; j < 16; j += 4) {
-                    const float4 a4 = ptx::ld_dsmem_f32x4(remote + j * 512), b4 = ptx::ld_dsmem_f32x4(remote + (16 + j) * 512);
-                    ra[j] = __float_as_uint(__uint_as_float(ra[j]) + a4.x); ra[j + 1] = __float_as_uint(__uint_as_float(ra[j + 1]) + a4.y);
-                    ra[j + 2] = __float_as_uint(__uint_as_float(ra[j + 2]) + a4.z); ra[j + 3] = __float_as_uint(__uint_as_float(ra[j + 3]) + a4.w);
-                    rb[j] = __float_as_uint(__uint_as_float(rb[j]) + b4.x); rb[j + 1] = __float_as_uint(__uint_as_float(rb[j + 1]) + b4.y);
-                    rb[j + 2] = __float_as_uint(__uint_as_float(rb[j + 2]) + b4.z); rb[j + 3] = __float_as_uint(__uint_as_float(rb[j + 3]) + b4.w);
-                  }
-                }
-              }
-              conv_epilogue16_staged(p, ra, r, h * 32, n_tile * BLOCK_N + c0, has_bs ? bias_s + c0 : nullptr, cb,
+              if (KSPLIT) add_peer_partials(rab, stage_f, c0, r, ks);
+              conv_epilogue16_staged(p, rab[0], r, h * 32, n_tile * BLOCK_N + c0, has_bs ? bias_s + c0 : nullptr, cb,
                                      p.out_scale ? scale_s + c0 : nullptr, rs, stg);
-              conv_epilogue16_staged(p, rb, r, h * 32 + 16, n_tile * BLOCK_N + c0 + 16, has_bs ? bias_s + c0 + 16 : nullptr, cb,
+              conv_epilogue16_staged(p, rab[1], r, h * 32 + 16, n_tile * BLOCK_N + c0 + 16, has_bs ? bias_s + c0 + 16 : nullptr, cb,
                                      p.out_scale ? scale_s + c0 + 16 : nullptr, rs, stg);
             }
             ptx::fence_proxy_async();
@@ -334,22 +340,12 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_consta
         for (int c0 = 0; c0 < BLOCK_N; c0 += 16) {
           const int col0 = n_tile * BLOCK_N + c0;
           if (col0 >= p.c_out) break;  // warp-uniform
-          uint32_t rr[16];
-          ptx::tc_ld_32x32b_x16(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)c0, rr);
+          uint32_t rr[1][16];
+          ptx::tc_ld_32x32b_x16(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)c0, rr[0]);
           ptx::tc_wait_ld();
-          if (KSPLIT) {
-            for (int pr = 1; pr < ks; ++pr) {
-              const uint32_t remote = ptx::mapa_shared(ptx::smem_u32(stage_f + c0 * 128 + r * 4), (uint32_t)pr);
-#pragma unroll
-              for (int j = 0; j < 16; j += 4) {
-                const float4 a4 = ptx::ld_dsmem_f32x4(remote + j * 512);
-                rr[j] = __float_as_uint(__uint_as_float(rr[j]) + a4.x); rr[j + 1] = __float_as_uint(__uint_as_float(rr[j + 1]) + a4.y);
-                rr[j + 2] = __float_as_uint(__uint_as_float(rr[j + 2]) + a4.z); rr[j + 3] = __float_as_uint(__uint_as_float(rr[j + 3]) + a4.w);
-              }
-            }
-          }
+          if (KSPLIT) add_peer_partials(rr, stage_f, c0, r, ks);
           if (!valid) continue;
-          conv_epilogue16(p, rr, col0, n, vox, vox_per, row_off, has_bs ? bias_s + c0 : nullptr, cb,
+          conv_epilogue16(p, rr[0], col0, n, vox, vox_per, row_off, has_bs ? bias_s + c0 : nullptr, cb,
                           p.out_scale ? scale_s + c0 : nullptr);
         }
       }

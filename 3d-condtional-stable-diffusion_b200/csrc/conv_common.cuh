@@ -58,6 +58,40 @@ __device__ __forceinline__ void trace_ev(const ConvParams& p, int region, int& i
 
 __device__ __forceinline__ float bf(const act_t v) { return act_to_float(v); }
 
+// The epilogue's per-column terms on 16 values: + cb[col0 + j] (a global chan_bias row, only when a tile spans several
+// samples) -> * sc[j] -> + bs[j] (sc / bs: staged in shared memory once per tile, see conv_epilogue16).  nullptr = term absent.
+__device__ __forceinline__ void bias_scale16(float (&v)[16], const float* cb, int col0, const float* sc, const float* bs) {
+  if (cb) {
+#pragma unroll
+    for (int j = 0; j < 16; j += 4) {
+      const float4 b4 = __ldg(reinterpret_cast<const float4*>(cb + col0 + j));
+      v[j] += b4.x; v[j + 1] += b4.y; v[j + 2] += b4.z; v[j + 3] += b4.w;
+    }
+  }
+  if (sc) {
+#pragma unroll
+    for (int j = 0; j < 16; j += 4) {
+      const float4 s4 = *reinterpret_cast<const float4*>(sc + j);
+      v[j] *= s4.x; v[j + 1] *= s4.y; v[j + 2] *= s4.z; v[j + 3] *= s4.w;
+    }
+  }
+  if (bs) {
+#pragma unroll
+    for (int j = 0; j < 16; j += 4) {
+      const float4 b4 = *reinterpret_cast<const float4*>(bs + j);
+      v[j] += b4.x; v[j + 1] += b4.y; v[j + 2] += b4.z; v[j + 3] += b4.w;
+    }
+  }
+}
+
+
+// Byte offset of 16-byte unit `u` of row `r` in a tile of `row_bytes`-byte rows (128, 64 or 32) as a tensor map with
+// CU_TENSOR_MAP_SWIZZLE_128B / 64B / 32B lays it out in shared memory: the unit index is XORed with bits 7.. of the row's address.
+__device__ __forceinline__ uint32_t swizzle_off(uint32_t row_bytes, int r, int u) {
+  const int sw = row_bytes == 128 ? r & 7 : (row_bytes == 64 ? (r >> 1) & 3 : (r >> 2) & 1);
+  return (uint32_t)r * row_bytes + (uint32_t)((u ^ sw) << 4);
+}
+
 // Epilogue for 16 consecutive accumulator columns of one output voxel (thread = TMEM lane = GEMM row):
 //   + bias[co] + chan_bias[t][n][co]  ->  * out_scale[co] + out_shift[co]  ->  PReLU(alpha[voxel][co])  ->  act  ->
 //   + residual  ->  post_act  ->  store
@@ -74,27 +108,7 @@ __device__ __forceinline__ void conv_epilogue16(const ConvParams& p, const uint3
   const int ncol = (p.c_out - col0) < 16 ? (p.c_out - col0) : 16;
   if (ncol == 16 && !p.transposed_store) {
     // vector path: 16 channels = 32 B bf16 / 64 B fp32 per thread
-    if (cb) {
-#pragma unroll
-      for (int j = 0; j < 16; j += 4) {
-        const float4 b4 = __ldg(reinterpret_cast<const float4*>(cb + col0 + j));
-        v[j] += b4.x; v[j + 1] += b4.y; v[j + 2] += b4.z; v[j + 3] += b4.w;
-      }
-    }
-    if (sc) {
-#pragma unroll
-      for (int j = 0; j < 16; j += 4) {
-        const float4 s4 = *reinterpret_cast<const float4*>(sc + j);
-        v[j] *= s4.x; v[j + 1] *= s4.y; v[j + 2] *= s4.z; v[j + 3] *= s4.w;
-      }
-    }
-    if (bs) {
-#pragma unroll
-      for (int j = 0; j < 16; j += 4) {
-        const float4 b4 = *reinterpret_cast<const float4*>(bs + j);
-        v[j] += b4.x; v[j + 1] += b4.y; v[j + 2] += b4.z; v[j + 3] += b4.w;
-      }
-    }
+    bias_scale16(v, cb, col0, sc, bs);
     if (p.prelu_alpha) {
       float a[16];
       const act_t* ap = p.prelu_alpha + vox * p.c_out + col0;
@@ -164,34 +178,14 @@ __device__ __forceinline__ void conv_epilogue16_staged(const ConvParams& p, cons
   float v[16];
 #pragma unroll
   for (int j = 0; j < 16; ++j) v[j] = __uint_as_float(rr[j]);
-  if (cb) {
-#pragma unroll
-    for (int j = 0; j < 16; j += 4) {
-      const float4 b4 = __ldg(reinterpret_cast<const float4*>(cb + col0 + j));
-      v[j] += b4.x; v[j + 1] += b4.y; v[j + 2] += b4.z; v[j + 3] += b4.w;
-    }
-  }
-  if (sc) {
-#pragma unroll
-    for (int j = 0; j < 16; j += 4) {
-      const float4 s4 = *reinterpret_cast<const float4*>(sc + j);
-      v[j] *= s4.x; v[j + 1] *= s4.y; v[j + 2] *= s4.z; v[j + 3] *= s4.w;
-    }
-  }
-  if (bs) {
-#pragma unroll
-    for (int j = 0; j < 16; j += 4) {
-      const float4 b4 = *reinterpret_cast<const float4*>(bs + j);
-      v[j] += b4.x; v[j + 1] += b4.y; v[j + 2] += b4.z; v[j + 3] += b4.w;
-    }
-  }
+  bias_scale16(v, cb, col0, sc, bs);
   if (p.act != B200DM_ACT_NONE) {
     apply_act_vec(v, p.act);
   }
   // 128-byte rows (64 channels, SWIZZLE_128B: chunk ^ (row & 7)) or 64-byte rows (32 channels, SWIZZLE_64B: chunk ^ ((row >> 1) & 3))
-  const int ch = c_local >> 3, sw = row64 ? (r >> 1) & 3 : r & 7;
-  const uint32_t rb_ = (uint32_t)r * (row64 ? 64u : 128u);
-  const uint32_t o0 = rb_ + (uint32_t)(((ch) ^ sw) << 4), o1 = rb_ + (uint32_t)(((ch + 1) ^ sw) << 4);
+  const int ch = c_local >> 3;
+  const uint32_t row_bytes = row64 ? 64u : 128u;
+  const uint32_t o0 = swizzle_off(row_bytes, r, ch), o1 = swizzle_off(row_bytes, r, ch + 1);
   if (rs) {
     float a[16];
     unpack8(*reinterpret_cast<const bf16x8*>(rs + o0), *reinterpret_cast<float(*)[8]>(&a[0]));
@@ -220,20 +214,7 @@ __device__ __forceinline__ void conv_epilogue16_staged_f32(const ConvParams& p, 
   float v[16];
 #pragma unroll
   for (int j = 0; j < 16; ++j) v[j] = __uint_as_float(rr[j]);
-  if (sc) {
-#pragma unroll
-    for (int j = 0; j < 16; j += 4) {
-      const float4 s4 = *reinterpret_cast<const float4*>(sc + j);
-      v[j] *= s4.x; v[j + 1] *= s4.y; v[j + 2] *= s4.z; v[j + 3] *= s4.w;
-    }
-  }
-  if (bs) {
-#pragma unroll
-    for (int j = 0; j < 16; j += 4) {
-      const float4 b4 = *reinterpret_cast<const float4*>(bs + j);
-      v[j] += b4.x; v[j + 1] += b4.y; v[j + 2] += b4.z; v[j + 3] += b4.w;
-    }
-  }
+  bias_scale16(v, nullptr, 0, sc, bs);
   if (p.act != B200DM_ACT_NONE) {
     apply_act_vec(v, p.act);
   }
@@ -247,11 +228,9 @@ __device__ __forceinline__ void conv_epilogue16_staged_f32(const ConvParams& p, 
   if (p.post_act != B200DM_ACT_NONE) {
     apply_act_vec(v, p.post_act);
   }
-  const int u0 = c_local >> 2, sw = r & 7;
 #pragma unroll
   for (int u = 0; u < 4; ++u)
-    *reinterpret_cast<float4*>(stg + (uint32_t)r * 128u + (uint32_t)(((u0 + u) ^ sw) << 4)) =
-        make_float4(v[4 * u], v[4 * u + 1], v[4 * u + 2], v[4 * u + 3]);
+    *reinterpret_cast<float4*>(stg + swizzle_off(128, r, (c_local >> 2) + u)) = make_float4(v[4 * u], v[4 * u + 1], v[4 * u + 2], v[4 * u + 3]);
 }
 
 // Fused-update form of the fp32 staged epilogue: the 16 accumulator columns of this thread's row are eps_hat.  x_t of the same
@@ -266,20 +245,7 @@ __device__ __forceinline__ bool upd_epilogue16(const ConvParams& p, const uint32
   float v[16];
 #pragma unroll
   for (int j = 0; j < 16; ++j) v[j] = __uint_as_float(rr[j]);
-  if (sc) {
-#pragma unroll
-    for (int j = 0; j < 16; j += 4) {
-      const float4 s4 = *reinterpret_cast<const float4*>(sc + j);
-      v[j] *= s4.x; v[j + 1] *= s4.y; v[j + 2] *= s4.z; v[j + 3] *= s4.w;
-    }
-  }
-  if (bs) {
-#pragma unroll
-    for (int j = 0; j < 16; j += 4) {
-      const float4 b4 = *reinterpret_cast<const float4*>(bs + j);
-      v[j] += b4.x; v[j + 1] += b4.y; v[j + 2] += b4.z; v[j + 3] += b4.w;
-    }
-  }
+  bias_scale16(v, nullptr, 0, sc, bs);
   float z[16];
   if (gen) {
 #pragma unroll
@@ -289,18 +255,14 @@ __device__ __forceinline__ bool upd_epilogue16(const ConvParams& p, const uint32
     for (int j = 0; j < 16; ++j) z[j] = 0.0f;
   }
   if (!ptx::mbar_wait(xbar, xphase, p.dbg, 17)) return false;
-  const int sw = (r >> 1) & 3;
   float x[16], y[16];
 #pragma unroll
-  for (int u = 0; u < 4; ++u)
-    *reinterpret_cast<float4*>(&x[4 * u]) = *reinterpret_cast<const float4*>(stg + (uint32_t)r * 64u + (uint32_t)((u ^ sw) << 4));
+  for (int u = 0; u < 4; ++u) *reinterpret_cast<float4*>(&x[4 * u]) = *reinterpret_cast<const float4*>(stg + swizzle_off(64, r, u));
   upd::step_vec(k, p.upd.sampler, x, v, z, y);
 #pragma unroll
-  for (int u = 0; u < 4; ++u)
-    *reinterpret_cast<float4*>(stg + (uint32_t)r * 64u + (uint32_t)((u ^ sw) << 4)) = make_float4(y[4 * u], y[4 * u + 1], y[4 * u + 2], y[4 * u + 3]);
-  const int sw16 = (r >> 2) & 1;
-  *reinterpret_cast<bf16x8*>(stg16 + (uint32_t)r * 32u + (uint32_t)((0 ^ sw16) << 4)) = pack8(*reinterpret_cast<float(*)[8]>(&y[0]));
-  *reinterpret_cast<bf16x8*>(stg16 + (uint32_t)r * 32u + (uint32_t)((1 ^ sw16) << 4)) = pack8(*reinterpret_cast<float(*)[8]>(&y[8]));
+  for (int u = 0; u < 4; ++u) *reinterpret_cast<float4*>(stg + swizzle_off(64, r, u)) = make_float4(y[4 * u], y[4 * u + 1], y[4 * u + 2], y[4 * u + 3]);
+  *reinterpret_cast<bf16x8*>(stg16 + swizzle_off(32, r, 0)) = pack8(*reinterpret_cast<float(*)[8]>(&y[0]));
+  *reinterpret_cast<bf16x8*>(stg16 + swizzle_off(32, r, 1)) = pack8(*reinterpret_cast<float(*)[8]>(&y[8]));
   return true;
 }
 

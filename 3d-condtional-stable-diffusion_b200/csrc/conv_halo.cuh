@@ -32,13 +32,6 @@ constexpr int kThreadsFused = 416;         // FUSE_UPD: + one warp that owns the
 constexpr int kSlabBytes = 23 * 1024;      // 180 voxels x 128 B = 23040, rounded up to the 1024-B swizzle period
 constexpr int kSlabTx = 180 * 128;
 
-__device__ __forceinline__ void tma_load_3d(uint32_t dst, const CUtensorMap* m, uint32_t bar, int c0, int c1, int c2) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];" ::"r"(dst),
-      "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1), "r"(c2)
-      : "memory");
-}
-
 struct Tile {
   int w0, h0, d0, n, n_tile;
 };
@@ -80,6 +73,191 @@ struct Smem {
   static constexpr size_t kBias = kTmemPtr + 16;
   static constexpr size_t kBytes = 1024 + kBias + 4 * BLOCK_N * 4;         // with the alignment slack
 };
+
+// ---------------------------------------------------------------- pieces shared by conv_halo_kernel and conv_halo_up_kernel
+
+// Barriers from the base of the barrier area: slab full / empty [NS], weight full / empty [NB], accumulator (TMEM) full / empty [2].
+template <int NS, int NB>
+struct Bars {
+  uint32_t base;
+  __device__ __forceinline__ uint32_t slab_full(int s) const { return base + 8u * s; }
+  __device__ __forceinline__ uint32_t slab_empty(int s) const { return base + 8u * (NS + s); }
+  __device__ __forceinline__ uint32_t b_full(int s) const { return base + 8u * (2 * NS + s); }
+  __device__ __forceinline__ uint32_t b_empty(int s) const { return base + 8u * (2 * NS + NB + s); }
+  __device__ __forceinline__ uint32_t tmem_full(int s) const { return base + 8u * (2 * NS + 2 * NB + s); }
+  __device__ __forceinline__ uint32_t tmem_empty(int s) const { return base + 8u * (2 * NS + 2 * NB + 2 + s); }
+  // (thread 0) `issuers`: arrivals that release a slab / weight stage and fill an accumulator stage; `releasers`: arrivals
+  // that hand an accumulator stage back
+  __device__ __forceinline__ void init(uint32_t issuers, uint32_t releasers) const {
+    for (int s = 0; s < NS; ++s) { ptx::mbar_init(slab_full(s), 1); ptx::mbar_init(slab_empty(s), issuers); }
+    for (int s = 0; s < NB; ++s) { ptx::mbar_init(b_full(s), 1); ptx::mbar_init(b_empty(s), issuers); }
+    for (int s = 0; s < 2; ++s) { ptx::mbar_init(tmem_full(s), issuers); ptx::mbar_init(tmem_empty(s), releasers); }
+  }
+};
+
+// TMEM allocation by warp 2 (of both CTAs under CG2), permit relinquished at once
+template <bool CG2>
+__device__ __forceinline__ void tmem_alloc(uint32_t* tmem_ptr_smem, uint32_t cols) {
+  if (CG2) { ptx::tmem_alloc_cg2(ptx::smem_u32(tmem_ptr_smem), cols); ptx::tmem_relinquish_cg2(); }
+  else { ptx::tmem_alloc(ptx::smem_u32(tmem_ptr_smem), cols); ptx::tmem_relinquish(); }
+}
+
+// End of the set-up: every thread sees the barriers and the TMEM address (CG2: the peer's barriers exist -- fence_barrier_init --
+// before anything signals them); then wait for the previous kernel, whose tail the set-up overlapped.  Returns the TMEM base.
+template <bool CG2>
+__device__ __forceinline__ uint32_t setup_join(const uint32_t* tmem_ptr_smem) {
+  ptx::tc_fence_before();
+  __syncthreads();
+  if (CG2) ptx::cluster_sync_exit();
+  ptx::tc_fence_after();
+  const uint32_t tmem_base = *tmem_ptr_smem;
+  pdl_wait();
+  return tmem_base;
+}
+
+// Kernel tail: all roles are done; under CG2 the leader's MMAs read the peer's shared memory / write its TMEM until the cluster
+// barrier.  Warp 2 frees the TMEM.  `tp`: the launch's parameters when the tail is traced (timeline region 3), else nullptr.
+template <bool CG2>
+__device__ __forceinline__ void teardown(const ConvParams* tp, uint32_t tmem_base, uint32_t cols) {
+  int tx = 0;
+  if (tp && threadIdx.x == 128) trace_ev(*tp, 3, tx, 30);
+  ptx::tc_fence_before();
+  __syncthreads();
+  if (tp && threadIdx.x == 128) trace_ev(*tp, 3, tx, 31);
+  if (CG2) ptx::cluster_sync_exit();
+  if (tp && threadIdx.x == 128) trace_ev(*tp, 3, tx, 32);
+  if ((threadIdx.x >> 5) == 2) {
+    ptx::tc_fence_after();
+    if (CG2) ptx::tmem_dealloc_cg2(tmem_base, cols); else ptx::tmem_dealloc(tmem_base, cols);
+  }
+}
+
+// The MMA issuer's position in the slab ring: qs = slot of the current chunk's first slab, qph = its phase bit.  Carried
+// incrementally: the issuing thread is the pacing resource, and the integer divisions / modulos of a closed-form index cost
+// ~200 cycles per kd step during which the shallow MMA queue drains.
+template <int NS>
+struct SlabCursor {
+  uint32_t qs = 0, qph = 0;
+  __device__ __forceinline__ uint32_t slot(uint32_t i, uint32_t& ph) const {   // ring slot / phase of slab i of the chunk (i < NS)
+    uint32_t idx = qs + i;
+    const bool wrap = idx >= (uint32_t)NS;
+    ph = qph ^ (wrap ? 1u : 0u);
+    return wrap ? idx - NS : idx;
+  }
+  __device__ __forceinline__ void advance(uint32_t k) {
+    qs += k;
+    if (qs >= (uint32_t)NS) { qs -= NS; qph ^= 1; }
+  }
+};
+
+// Weight producer (warp 1): per tile, `stages` weight stages of `kps` consecutive k-blocks (the box depth of mapB) from weight
+// row row_of(tile id), for the tiles first_tile, first_tile + tile_step, ... (the kernel's schedule); under CG2 each CTA loads
+// its kBRows rows of the stage, completing on the leader's barrier.
+template <int NS, int NB, int kBRows, int kBBytes, bool CG2, class RowOf>
+__device__ __forceinline__ void produce_weights(const ConvParams& p, const Bars<NS, NB>& bar, const CUtensorMap* mapB, uint32_t bring_base,
+                                                uint32_t crank, int first_tile, int tile_step, int stages, int kps, int dbg_code,
+                                                RowOf&& row_of) {
+  uint32_t s = 0, ph = 1;
+  bool ok = true;
+  for (int id = first_tile; id < p.halo_total_tiles && ok; id += tile_step) {
+    const int row0 = row_of(id);
+    for (int kb = 0; kb < stages * kps; kb += kps) {
+      ok = ptx::mbar_wait(bar.b_empty(s), ph, p.dbg, dbg_code);
+      if (!ok) break;
+      if (ptx::elect_one()) {
+        if (CG2) {
+          if (crank == 0) ptx::mbar_expect_tx(bar.b_full(s), 2 * kBBytes);
+          ptx::tma_load_3d_cg2(bring_base + s * kBBytes, mapB, ptx::mapa_shared(bar.b_full(s), 0), 0, row0 + (int)crank * kBRows, kb);
+        } else {
+          ptx::mbar_expect_tx(bar.b_full(s), kBBytes);
+          ptx::tma_load_3d(bring_base + s * kBBytes, mapB, bar.b_full(s), 0, row0, kb);
+        }
+      }
+      __syncwarp();
+      if (++s == NB) { s = 0; ph ^= 1; }
+    }
+  }
+}
+
+// Bias + temb row of sample n for the tile's BLOCK_N columns from col_base -> bs / scs (the buffer of the tile's accumulator
+// stage), by the 256 epilogue threads BEFORE the accumulator is ready: the two dependent global round trips (t_dev, then the
+// table rows: ~1.5 k cycles) overlap the tile's MMAs instead of heading its epilogue.  The buffer was last read in tile it - 2;
+// every epilogue thread has passed a bar.sync of tile it - 1 since.  `ti`: the epilogue's trace index (event 20), or nullptr.
+template <int BLOCK_N>
+__device__ __forceinline__ void stage_tile_bias(const ConvParams& p, float* bs, float* scs, int n, int col_base, int* ti) {
+  const float* cbrow = nullptr;
+  if (p.chan_bias) {
+    const int tt = p.t_dev ? p.t_dev[0] : 0;
+    cbrow = p.chan_bias + ((int64_t)tt * p.chan_bias_rows + (p.chan_bias_rows > 1 ? n : 0)) * p.c_out;
+  }
+  stage_bias(p, bs, scs, col_base, BLOCK_N, cbrow, threadIdx.x - 128, 256);
+  if (ti && threadIdx.x == 128) trace_ev(p, 1, *ti, 20);
+  epilogue_bar_sync256();
+}
+
+// Staged 16-bit store of one output plane: wait until the staging buffer nstore % kBufs is free, run this thread's row of
+// TMEM columns [taddr, + BLOCK_N / 2) through conv_epilogue16_staged into it (whole 128-byte rows, SWIZZLE_128B; BLOCK_N = 32:
+// 64-byte rows, SWIZZLE_64B), then one TMA store per 64-channel group at (col_base + 64 g, w0, h0, od, n) -- PAIR: (.., w0, od,
+// h0, n) -- with the edges clipped by the TMA unit (row-per-thread 16-byte stores touch 32 lines per instruction).
+// bs / scs: the tile's staged bias and scale (used when has_bs / has_sc); `rpre`: this plane's residual rows in registers
+// (kChunks x 2 vectors), or nullptr; `ti`: the epilogue's trace index (events 13-15), or nullptr.
+template <int BLOCK_N, bool PAIR>
+__device__ __forceinline__ void store_plane16(const ConvParams& p, const CUtensorMap* map, uint8_t* stg_base, uint32_t nstore,
+                                              uint32_t taddr, int r, int cbase, int col_base, const float* bs, const float* scs,
+                                              bool has_bs, bool has_sc, int w0, int h0, int od, int n, bool pre,
+                                              const bf16x8 (*rpre)[2], int* ti) {
+  constexpr int kChunks = BLOCK_N / 32;   // 16-column chunks of this warp's column half
+  constexpr int kNG = stage_groups(BLOCK_N), kBufs = stage_bufs(BLOCK_N), kGB = stage_group_bytes(BLOCK_N);
+  constexpr bool kRow64 = BLOCK_N < 64;   // one 32-channel group: 64-byte rows, SWIZZLE_64B
+  const int grp = kRow64 ? 0 : cbase >> 6, cl0 = kRow64 ? cbase : cbase & 63;
+  const bool ev = ti && threadIdx.x == 128;
+  const int colt = col_base + cbase;
+  uint8_t* stg = stg_base + ((nstore % kBufs) * kNG + grp) * kGB;
+  if (threadIdx.x == 128) {   // the store that last used this buffer has finished reading it
+    if (kBufs == 2) ptx::bulk_wait_read_1(); else ptx::bulk_wait_read_all();
+  }
+  epilogue_bar_sync256();
+  if (ev) trace_ev(p, 1, *ti, 13);
+#pragma unroll
+  for (int c = 0; c < kChunks; c += 2) {
+    const int col0 = colt + c * 16;
+    uint32_t ra[16], rb[16];
+    ptx::tc_ld_32x32b_x16(taddr + c * 16, ra);
+    if (c + 1 < kChunks) ptx::tc_ld_32x32b_x16(taddr + c * 16 + 16, rb);
+    ptx::tc_wait_ld();
+    conv_epilogue16_staged(p, ra, r, cl0 + c * 16, col0, has_bs ? bs + cbase + c * 16 : nullptr, nullptr,
+                           has_sc ? scs + cbase + c * 16 : nullptr, nullptr, stg, pre, rpre ? rpre[c] : nullptr, kRow64);
+    if (c + 1 < kChunks)
+      conv_epilogue16_staged(p, rb, r, cl0 + c * 16 + 16, col0 + 16, has_bs ? bs + cbase + c * 16 + 16 : nullptr, nullptr,
+                             has_sc ? scs + cbase + c * 16 + 16 : nullptr, nullptr, stg, pre,
+                             rpre ? rpre[c + 1 < kChunks ? c + 1 : c] : nullptr, kRow64);
+  }
+  if (ev) trace_ev(p, 1, *ti, 14);
+  ptx::fence_proxy_async();
+  epilogue_bar_sync256();
+  if (ev) trace_ev(p, 1, *ti, 15);
+  if (threadIdx.x == 128) {
+    for (int g = 0; g < kNG; ++g)
+      if (col_base + g * 64 < p.c_out) {
+        const uint32_t src = ptx::smem_u32(stg_base + ((nstore % kBufs) * kNG + g) * kGB);
+        if (PAIR) ptx::tma_store_5d(map, src, col_base + g * 64, w0, od, h0, n);
+        else ptx::tma_store_5d(map, src, col_base + g * 64, w0, h0, od, n);
+      }
+    ptx::bulk_commit_group();
+  }
+}
+
+// Hand accumulator stage `as` back to the (leader's) MMA issuers, by lane 0 of each epilogue warp -- only for a tile that has a
+// successor two tiles on: nobody ever waits for the arrivals of a CTA's last two tiles, and the cluster-scope arrive costs the
+// arriving warp 2-2.5 k cycles (clock64 timeline) -- on the one-tile CTAs of the 16^3 / 8^3 levels that was the tail of a fully
+// exposed epilogue.
+template <bool CG2>
+__device__ __forceinline__ void release_acc(const ConvParams& p, uint32_t tmem_empty, int id, int tile_step) {
+  if ((threadIdx.x & 31) == 0 && id + 2 * tile_step < p.halo_total_tiles) {
+    if (CG2) ptx::mbar_arrive_cluster(ptx::mapa_shared(tmem_empty, 0));
+    else ptx::mbar_arrive(tmem_empty);
+  }
+}
 
 // PAIR (small planes, 8 x 8: the 8^3 level of the U-Net): the tile is 8 w x 8 h x 2 d.  The activation tensor map lists
 // its dims as (C, W, D, H, N), so one box {64, 10, 2, 10, 1} lands in smem as rows [h][d][w]: the 16 eight-row groups of
@@ -130,12 +308,7 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constan
   const uint32_t slab_base = ptx::smem_u32(smem);
   const uint32_t bring_base = ptx::smem_u32(b_ring);
   const uint32_t bar_base = ptx::smem_u32(bars);
-  auto slab_full = [&](int s) { return bar_base + 8u * s; };
-  auto slab_empty = [&](int s) { return bar_base + 8u * (NS + s); };
-  auto b_full = [&](int s) { return bar_base + 8u * (2 * NS + s); };
-  auto b_empty = [&](int s) { return bar_base + 8u * (2 * NS + NB + s); };
-  auto tmem_full = [&](int s) { return bar_base + 8u * (2 * NS + 2 * NB + s); };
-  auto tmem_empty = [&](int s) { return bar_base + 8u * (2 * NS + 2 * NB + 2 + s); };
+  const Bars<NS, NB> bar{bar_base};
   auto x_bar = [&](uint32_t set) { return bar_base + 8u * (2 * NS + 2 * NB + 4 + 2 * set); };   // FUSE_UPD: the x_t tiles of staging set `set` have landed
   // FUSE_UPD: the 256 epilogue threads have written the tiles of staging set `set`.  One barrier PER SET: the writers only arrive
   // (they never wait on it), so a fast warp may arrive for round r + 1 before a slow warp has arrived for round r -- on a single
@@ -151,10 +324,8 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constan
   const bool leader = crank == 0;
 
   if (threadIdx.x == 0) {
-    for (int s = 0; s < NS; ++s) { ptx::mbar_init(slab_full(s), 1); ptx::mbar_init(slab_empty(s), kIssuers); }
-    for (int s = 0; s < NB; ++s) { ptx::mbar_init(b_full(s), 1); ptx::mbar_init(b_empty(s), kIssuers); }
     // accumulator-stage release: one arrival per epilogue warp (both CTAs of a pair); FUSE_UPD: one per CTA, by the TMA agent
-    for (int s = 0; s < 2; ++s) { ptx::mbar_init(tmem_full(s), kIssuers); ptx::mbar_init(tmem_empty(s), FUSE_UPD ? (CG2 ? 2 : 1) : (CG2 ? 16 : 8)); }
+    bar.init(kIssuers, FUSE_UPD ? (CG2 ? 2 : 1) : (CG2 ? 16 : 8));
     if (FUSE_UPD) { ptx::mbar_init(x_bar(0), 4); ptx::mbar_init(x_bar(1), 4); ptx::mbar_init(w_bar(0), 256); ptx::mbar_init(w_bar(1), 256); }
     ptx::fence_barrier_init();
     ptx::prefetch_tmap(&mapA0);
@@ -163,16 +334,8 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constan
     if (STAGED) ptx::prefetch_tmap(&mapY);
     if (FUSE_UPD) ptx::prefetch_tmap(&mapZ);
   }
-  if (warp == 2) {
-    if (CG2) { ptx::tmem_alloc_cg2(ptx::smem_u32(tmem_ptr_smem), kTmemCols); ptx::tmem_relinquish_cg2(); }
-    else { ptx::tmem_alloc(ptx::smem_u32(tmem_ptr_smem), kTmemCols); ptx::tmem_relinquish(); }
-  }
-  ptx::tc_fence_before();
-  __syncthreads();
-  if (CG2) ptx::cluster_sync_exit();   // the peer's barriers exist (fence_barrier_init above) before anything signals them
-  ptx::tc_fence_after();
-  const uint32_t tmem_base = *tmem_ptr_smem;
-  pdl_wait();   // set-up above overlaps the previous kernel's tail
+  if (warp == 2) tmem_alloc<CG2>(tmem_ptr_smem, kTmemCols);
+  const uint32_t tmem_base = setup_join<CG2>(tmem_ptr_smem);
 
   if (warp == 0) {
     // ===================== slab producer =====================
@@ -181,18 +344,18 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constan
     int ti = 0;
     // the next ring slot <- the slab of channels c0.. whose first input plane is d (pair slab: planes d, d + 1)
     auto load_slab = [&](const Tile& t, const CUtensorMap* map, int c0, int d, int tag) {
-      ok = ptx::mbar_wait(slab_empty(s), ph, p.dbg, 11);
+      ok = ptx::mbar_wait(bar.slab_empty(s), ph, p.dbg, 11);
       if (!ok) return;
       if (lane == 0) trace_ev(p, 2, ti, tag);
       if (ptx::elect_one()) {
         if (CG2) {   // both CTAs' slabs complete on the LEADER's barrier, which expects both transfers
-          if (leader) ptx::mbar_expect_tx(slab_full(s), 2 * kSlabTx);
-          if (PAIR) ptx::tma_load_5d_cg2(slab_base + s * kSlabBytes, map, ptx::mapa_shared(slab_full(s), 0), c0, t.w0 - 1, d, t.h0 - 1, t.n);
-          else ptx::tma_load_5d_cg2(slab_base + s * kSlabBytes, map, ptx::mapa_shared(slab_full(s), 0), c0, t.w0 - 1, t.h0 - 1, d, t.n);
+          if (leader) ptx::mbar_expect_tx(bar.slab_full(s), 2 * kSlabTx);
+          if (PAIR) ptx::tma_load_5d_cg2(slab_base + s * kSlabBytes, map, ptx::mapa_shared(bar.slab_full(s), 0), c0, t.w0 - 1, d, t.h0 - 1, t.n);
+          else ptx::tma_load_5d_cg2(slab_base + s * kSlabBytes, map, ptx::mapa_shared(bar.slab_full(s), 0), c0, t.w0 - 1, t.h0 - 1, d, t.n);
         } else {
-          ptx::mbar_expect_tx(slab_full(s), kSlabTx);
-          if (PAIR) ptx::tma_load_5d(slab_base + s * kSlabBytes, map, slab_full(s), c0, t.w0 - 1, d, t.h0 - 1, t.n);
-          else ptx::tma_load_5d(slab_base + s * kSlabBytes, map, slab_full(s), c0, t.w0 - 1, t.h0 - 1, d, t.n);
+          ptx::mbar_expect_tx(bar.slab_full(s), kSlabTx);
+          if (PAIR) ptx::tma_load_5d(slab_base + s * kSlabBytes, map, bar.slab_full(s), c0, t.w0 - 1, d, t.h0 - 1, t.n);
+          else ptx::tma_load_5d(slab_base + s * kSlabBytes, map, bar.slab_full(s), c0, t.w0 - 1, t.h0 - 1, d, t.n);
         }
       }
       __syncwarp();
@@ -213,28 +376,9 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constan
       }
     }
   } else if (warp == 1) {
-    // ===================== weight producer =====================
-    uint32_t s = 0, ph = 1;
-    bool ok = true;
-    for (int id = first_tile; id < p.halo_total_tiles && ok; id += tile_step) {
-      const Tile t = decode_tile<PAIR>(p, id);
-      const int row0 = t.n_tile * BLOCK_N;
-      for (int kb = 0; kb < nch * 27 + (sc_nch + TPS - 1) / TPS * TPS; kb += TPS) {
-        ok = ptx::mbar_wait(b_empty(s), ph, p.dbg, 12);
-        if (!ok) break;
-        if (ptx::elect_one()) {
-          if (CG2) {   // this CTA's half of the rows; completion on the leader's barrier
-            if (leader) ptx::mbar_expect_tx(b_full(s), 2 * kBBytes);
-            ptx::tma_load_3d_cg2(bring_base + s * kBBytes, &mapB, ptx::mapa_shared(b_full(s), 0), 0, row0 + (int)crank * kBRows, kb);
-          } else {
-            ptx::mbar_expect_tx(b_full(s), kBBytes);
-            tma_load_3d(bring_base + s * kBBytes, &mapB, b_full(s), 0, row0, kb);
-          }
-        }
-        __syncwarp();
-        if (++s == NB) { s = 0; ph ^= 1; }
-      }
-    }
+    // ===================== weight producer: TPS taps per stage, the shortcut's k-blocks padded to whole stages =====================
+    produce_weights<NS, NB, kBRows, kBBytes, CG2>(p, bar, &mapB, bring_base, crank, first_tile, tile_step, nch * 27 / TPS + (sc_nch + TPS - 1) / TPS, TPS, 12,
+                                                  [&](int id) { return decode_tile<PAIR>(p, id).n_tile * BLOCK_N; });
   } else if (warp == 2 || (warp == 3 && kIssuers == 2)) {
     // ===================== MMA issuer(s) =====================
     const int pl_lo = kIssuers == 2 ? warp - 2 : 0, pl_hi = kIssuers == 2 ? warp - 1 : TD;   // planes this warp drives
@@ -248,23 +392,15 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constan
     auto commit = [&](uint32_t bar) { if (CG2) ptx::tc_commit_cg2(bar, (uint16_t)3); else ptx::tc_commit(bar); };
     const uint64_t a_desc0 = ptx::make_smem_desc(slab_base, 16, 1280, ptx::kLayoutSw128);
     const uint64_t b_desc0 = ptx::make_smem_desc(bring_base, 16, 1024, ptx::kLayoutSw128);
-    // Ring positions are carried incrementally (qs = slab slot of the chunk's first slab, qph = its phase bit): the
-    // issuing thread is the pacing resource, and the integer divisions / modulos of a closed-form index cost ~200 cycles
-    // per kd step during which the shallow MMA queue drains.
-    uint32_t it = 0, sb = 0, bph = 0, qs = 0, qph = 0;
+    uint32_t it = 0, sb = 0, bph = 0;
+    SlabCursor<NS> q;
     bool ok = true;
     int ti = 0;
-    auto slot = [&](uint32_t i, uint32_t& ph) -> uint32_t {   // ring slot / phase of slab i of the current chunk (i < NS)
-      uint32_t idx = qs + i;
-      const bool wrap = idx >= (uint32_t)NS;
-      ph = qph ^ (wrap ? 1u : 0u);
-      return wrap ? idx - NS : idx;
-    };
     if (ptx::elect_one()) {   // ONE lane runs the whole issue loop: no per-stage elect / warp reconvergence between MMAs
     for (int id = first_tile; id < p.halo_total_tiles && ok && leader; id += tile_step, ++it) {
       const uint32_t as = it & 1;
       if (tr) trace_ev(p, 0, ti, 1);
-      ok = ptx::mbar_wait(tmem_empty(as), ((it >> 1) & 1) ^ 1, p.dbg, 13);
+      ok = ptx::mbar_wait(bar.tmem_empty(as), ((it >> 1) & 1) ^ 1, p.dbg, 13);
       if (!ok) break;
       if (tr) trace_ev(p, 0, ti, 2);
       ptx::tc_fence_after();
@@ -277,24 +413,24 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constan
         for (int kd = 0; kd < 3 && ok; ++kd) {
           uint32_t ph;
           if (kd == 0) {
-            for (int pl = 0; pl < TD && ok; ++pl) { const uint32_t sl = slot(pl, ph); ok = ptx::mbar_wait(slab_full(sl), ph, p.dbg, 14); }
+            for (int pl = 0; pl < TD && ok; ++pl) { const uint32_t sl = q.slot(pl, ph); ok = ptx::mbar_wait(bar.slab_full(sl), ph, p.dbg, 14); }
           } else {
-            const uint32_t sl = slot(kd + TD - 1, ph);
-            ok = ptx::mbar_wait(slab_full(sl), ph, p.dbg, 14);
+            const uint32_t sl = q.slot(kd + TD - 1, ph);
+            ok = ptx::mbar_wait(bar.slab_full(sl), ph, p.dbg, 14);
           }
           if (!ok) break;
           if (tr) trace_ev(p, 0, ti, 3);
           uint64_t a_pl[TD];
 #pragma unroll
-          for (int pl = 0; pl < TD; ++pl) a_pl[pl] = a_desc0 + (uint64_t)(slot(pl + kd, ph) * (uint32_t)(kSlabBytes >> 4));
+          for (int pl = 0; pl < TD; ++pl) a_pl[pl] = a_desc0 + (uint64_t)(q.slot(pl + kd, ph) * (uint32_t)(kSlabBytes >> 4));
           const uint32_t first_kd = (j | kd) != 0 ? 1u : 0u;
           // slab released by this kd step: slab kd (last used at kd = min(index, 2)); after kd = 2 also slabs 3 .. TD+1
-          const uint32_t rel0 = slot(kd, ph), rel1 = TD == 2 ? slot(3, ph) : 0u;
+          const uint32_t rel0 = q.slot(kd, ph), rel1 = TD == 2 ? q.slot(3, ph) : 0u;
 #pragma unroll 1
           for (int kh = 0; kh < 3 && ok; ++kh) {
 #pragma unroll
             for (int g = 0; g < 3 / TPS; ++g) {   // TPS=3: one stage per kh row; TPS=1: three stages
-              ok = ptx::mbar_wait(b_full(sb), bph, p.dbg, 15);
+              ok = ptx::mbar_wait(bar.b_full(sb), bph, p.dbg, 15);
               if (!ok) break;
               ptx::tc_fence_after();
               {
@@ -314,10 +450,10 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constan
                     if (ks > 3) mma(acc + pl * BLOCK_N, da + 6, db + 6, 1u);
                   }
                 }
-                commit(b_empty(sb));
+                commit(bar.b_empty(sb));
                 if (kh == 2 && g == 3 / TPS - 1) {   // last stage of this kd step: release its slab(s) in the same breath
-                  commit(slab_empty(rel0));
-                  if (kd == 2 && TD == 2) commit(slab_empty(rel1));
+                  commit(bar.slab_empty(rel0));
+                  if (kd == 2 && TD == 2) commit(bar.slab_empty(rel1));
                 }
               }
               if (++sb == NB) { sb = 0; bph ^= 1; }
@@ -326,12 +462,11 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constan
           if (!ok) break;
           if (tr) trace_ev(p, 0, ti, 4);
         }
-        qs += TD + 2;
-        if (qs >= (uint32_t)NS) { qs -= NS; qph ^= 1; }
+        q.advance(TD + 2);
       }
       // shortcut: TPS chunks per weight stage, each one tap (the slab's centre) on its own TD slabs, released chunk by chunk
       for (int j0 = 0; j0 < sc_nch && ok; j0 += TPS) {
-        ok = ptx::mbar_wait(b_full(sb), bph, p.dbg, 15);
+        ok = ptx::mbar_wait(bar.b_full(sb), bph, p.dbg, 15);
         if (!ok) break;
         const uint64_t db0 = b_desc0 + (uint64_t)(sb * (kBBytes >> 4));
 #pragma unroll 1
@@ -339,13 +474,13 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constan
           const int j = j0 + u;
           const int ks = j == p.sc_nch0 - 1 ? p.sc_ksteps0_last : (j == sc_nch - 1 && p.sc_nch1 > 0 ? p.sc_ksteps1_last : 4);
           uint32_t ph;
-          for (int pl = 0; pl < TD && ok; ++pl) { const uint32_t sl = slot(pl, ph); ok = ptx::mbar_wait(slab_full(sl), ph, p.dbg, 14); }
+          for (int pl = 0; pl < TD && ok; ++pl) { const uint32_t sl = q.slot(pl, ph); ok = ptx::mbar_wait(bar.slab_full(sl), ph, p.dbg, 14); }
           if (!ok) break;
           ptx::tc_fence_after();
 #pragma unroll
           for (int pl = 0; pl < TD; ++pl) {
             if (pl < pl_lo || pl >= pl_hi) continue;
-            const uint64_t da = a_desc0 + (uint64_t)(slot(pl, ph) * (uint32_t)(kSlabBytes >> 4)) + (uint64_t)(kKhUnits + 8);   // kh = kw = 1
+            const uint64_t da = a_desc0 + (uint64_t)(q.slot(pl, ph) * (uint32_t)(kSlabBytes >> 4)) + (uint64_t)(kKhUnits + 8);   // kh = kw = 1
             const uint64_t db = db0 + (uint64_t)(u * (kTapBytes >> 4));
             mma(acc + pl * BLOCK_N, da, db, 1u);
             if (ks > 1) mma(acc + pl * BLOCK_N, da + 2, db + 2, 1u);
@@ -353,14 +488,13 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constan
             if (ks > 3) mma(acc + pl * BLOCK_N, da + 6, db + 6, 1u);
           }
 #pragma unroll
-          for (int pl = 0; pl < TD; ++pl) commit(slab_empty(slot(pl, ph)));
-          qs += TD;
-          if (qs >= (uint32_t)NS) { qs -= NS; qph ^= 1; }
+          for (int pl = 0; pl < TD; ++pl) commit(bar.slab_empty(q.slot(pl, ph)));
+          q.advance(TD);
         }
-        commit(b_empty(sb));
+        commit(bar.b_empty(sb));
         if (++sb == NB) { sb = 0; bph ^= 1; }
       }
-      commit(tmem_full(as));
+      commit(bar.tmem_full(as));
     }
     }   // elected lane
     __syncwarp();
@@ -418,26 +552,14 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constan
           }
         }
       }
-      // bias + temb row of this tile's sample -> smem once per tile (double-buffered by accumulator stage), BEFORE the
-      // accumulator is ready: the two dependent global round trips (t_dev, then the table rows: ~1.5 k cycles) overlap the
-      // tile's MMAs instead of heading its epilogue.  The buffer was last read in tile it - 2; every epilogue thread has
-      // passed a bar.sync of tile it - 1 since.
+      // bias + temb row of this tile's sample -> smem once per tile (double-buffered by accumulator stage)
       float* bs = bias_s + as * 2 * BLOCK_N;
       float* scs = bs + BLOCK_N;
       const bool has_bs = p.bias != nullptr || p.chan_bias != nullptr || p.out_scale != nullptr;
       const bool has_sc = p.out_scale != nullptr;
-      if (has_bs) {
-        const float* cbrow = nullptr;
-        if (p.chan_bias) {
-          const int tt = p.t_dev ? p.t_dev[0] : 0;
-          cbrow = p.chan_bias + ((int64_t)tt * p.chan_bias_rows + (p.chan_bias_rows > 1 ? t.n : 0)) * p.c_out;
-        }
-        stage_bias(p, bs, scs, t.n_tile * BLOCK_N, BLOCK_N, cbrow, threadIdx.x - 128, 256);
-        if (warp == 4 && lane == 0) trace_ev(p, 1, ti, 20);
-        epilogue_bar_sync256();
-      }
+      if (has_bs) stage_tile_bias<BLOCK_N>(p, bs, scs, t.n, t.n_tile * BLOCK_N, &ti);
       if (warp == 4 && lane == 0) trace_ev(p, 1, ti, 10);
-      const bool ok = ptx::mbar_wait(tmem_full(as), (it >> 1) & 1, p.dbg, 16);
+      const bool ok = ptx::mbar_wait(bar.tmem_full(as), (it >> 1) & 1, p.dbg, 16);
       ptx::tc_fence_after();
       if (!ok) break;
       if (warp == 4 && lane == 0) trace_ev(p, 1, ti, 11);
@@ -514,48 +636,13 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constan
         }
         nstore = 0;   // (buffer rotation is a bf16-path notion)
       } else if constexpr (STAGED) {
-        // bf16 plane tile -> swizzled smem -> one TMA store per 64-channel group (whole 128-byte rows, edges clipped by
-        // the TMA unit) instead of row-per-thread 16-byte stores that touch 32 lines per instruction
-        constexpr int kNG = stage_groups(BLOCK_N), kBufs = stage_bufs(BLOCK_N), kGB = stage_group_bytes(BLOCK_N);
-        constexpr bool kRow64 = BLOCK_N < 64;   // one 32-channel group: 64-byte rows, SWIZZLE_64B
-        const int grp = kRow64 ? 0 : cbase >> 6, cl0 = kRow64 ? cbase : cbase & 63;
 #pragma unroll
         for (int pl = 0; pl < TD; ++pl) {
           const int od = t.d0 + pl;
           if (od >= p.out_d) break;   // CTA-uniform
-          uint8_t* stg = stg_base + ((nstore % kBufs) * kNG + grp) * kGB;
-          if (warp == 4 && lane == 0) {   // the store that last used this buffer has finished reading it
-            if (kBufs == 2) ptx::bulk_wait_read_1(); else ptx::bulk_wait_read_all();
-          }
-          epilogue_bar_sync256();
-          if (warp == 4 && lane == 0) trace_ev(p, 1, ti, 13);
           const uint32_t taddr = tmem_base + ((uint32_t)(qd * 32) << 16) + as * kAccCols + pl * BLOCK_N + cbase;
-#pragma unroll
-          for (int c = 0; c < kChunks; c += 2) {
-            const int col0 = colt + c * 16;
-            uint32_t ra[16], rb[16];
-            ptx::tc_ld_32x32b_x16(taddr + c * 16, ra);
-            if (c + 1 < kChunks) ptx::tc_ld_32x32b_x16(taddr + c * 16 + 16, rb);
-            ptx::tc_wait_ld();
-            conv_epilogue16_staged(p, ra, r, cl0 + c * 16, col0, has_bs ? bs + cbase + c * 16 : nullptr, nullptr,
-                                   has_sc ? scs + cbase + c * 16 : nullptr, nullptr, stg, pre, rpre[pl][c], kRow64);
-            if (c + 1 < kChunks)
-              conv_epilogue16_staged(p, rb, r, cl0 + c * 16 + 16, col0 + 16, has_bs ? bs + cbase + c * 16 + 16 : nullptr, nullptr,
-                                     has_sc ? scs + cbase + c * 16 + 16 : nullptr, nullptr, stg, pre, rpre[pl][c + 1 < kChunks ? c + 1 : c], kRow64);
-          }
-          if (warp == 4 && lane == 0) trace_ev(p, 1, ti, 14);
-          ptx::fence_proxy_async();
-          epilogue_bar_sync256();
-          if (warp == 4 && lane == 0) trace_ev(p, 1, ti, 15);
-          if (warp == 4 && lane == 0) {
-            for (int g = 0; g < kNG; ++g)
-              if (t.n_tile * BLOCK_N + g * 64 < p.c_out) {
-                const uint32_t src = ptx::smem_u32(stg_base + ((nstore % kBufs) * kNG + g) * kGB);
-                if (PAIR) ptx::tma_store_5d(&mapY, src, t.n_tile * BLOCK_N + g * 64, t.w0, od, t.h0, t.n);
-                else ptx::tma_store_5d(&mapY, src, t.n_tile * BLOCK_N + g * 64, t.w0, t.h0, od, t.n);
-              }
-            ptx::bulk_commit_group();
-          }
+          store_plane16<BLOCK_N, PAIR>(p, &mapY, stg_base, nstore, taddr, r, cbase, t.n_tile * BLOCK_N, bs, scs, has_bs, has_sc,
+                                       t.w0, t.h0, od, t.n, pre, rpre[pl], &ti);
           ++nstore;
         }
       } else
@@ -590,13 +677,7 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constan
       if (warp == 4 && lane == 0) trace_ev(p, 1, ti, 12);
       // (FUSE_UPD: the agent warp releases the accumulator stage once the tile's last round is complete -- the cluster-scope
       // arrive costs the arriving warp ~2.5 k cycles, which these warps would pay at every tile boundary)
-      // Only a tile that has a successor two tiles on hands its accumulator stage back: nobody ever waits for the arrivals of a
-      // CTA's last two tiles, and the cluster-scope arrive costs the arriving warp 2-2.5 k cycles (clock64 timeline) -- on the
-      // one-tile CTAs of the 16^3 / 8^3 levels that was the tail of a fully exposed epilogue.
-      if (lane == 0 && !FUSE_UPD && id + 2 * tile_step < p.halo_total_tiles) {
-        if (CG2) ptx::mbar_arrive_cluster(ptx::mapa_shared(tmem_empty(as), 0));   // the leader's issuers own the accumulators
-        else ptx::mbar_arrive(tmem_empty(as));
-      }
+      if (!FUSE_UPD) release_acc<CG2>(p, bar.tmem_empty(as), id, tile_step);
     }
     if (STAGED && !FUSE_UPD && warp == 4 && lane == 0) ptx::bulk_wait_read_all();   // smem must outlive the last store's reads
   }
@@ -650,7 +731,7 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constan
             // hand the TMEM stage back to the (leader's) MMA issuers
             ptx::tc_fence_after();
             ptx::tc_fence_before();
-            if (CG2) ptx::mbar_arrive_cluster(ptx::mapa_shared(tmem_empty(atile & 1), 0)); else ptx::mbar_arrive(tmem_empty(atile & 1));
+            if (CG2) ptx::mbar_arrive_cluster(ptx::mapa_shared(bar.tmem_empty(atile & 1), 0)); else ptx::mbar_arrive(bar.tmem_empty(atile & 1));
           }
         }
         ++atile;
@@ -659,17 +740,7 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constan
     }
     if (warp == 12) __syncwarp();   // the agent's four lanes rejoin their warp before the block-wide barrier
   }
-  int tx = 0;   // (timeline region 3: kernel tail)
-  if (threadIdx.x == 128) trace_ev(p, 3, tx, 30);
-  ptx::tc_fence_before();
-  __syncthreads();
-  if (threadIdx.x == 128) trace_ev(p, 3, tx, 31);
-  if (CG2) ptx::cluster_sync_exit();   // the leader's MMAs read the peer's shared memory / write its TMEM until here
-  if (threadIdx.x == 128) trace_ev(p, 3, tx, 32);
-  if (warp == 2) {
-    ptx::tc_fence_after();
-    if (CG2) ptx::tmem_dealloc_cg2(tmem_base, kTmemCols); else ptx::tmem_dealloc(tmem_base, kTmemCols);
-  }
+  teardown<CG2>(&p, tmem_base, kTmemCols);
 }
 
 }  // namespace halo

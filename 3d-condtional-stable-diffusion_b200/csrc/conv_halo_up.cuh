@@ -52,12 +52,7 @@ conv_halo_up_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_cons
   const uint32_t slab_base = ptx::smem_u32(smem);
   const uint32_t bring_base = ptx::smem_u32(b_ring);
   const uint32_t bar_base = ptx::smem_u32(bars);
-  auto slab_full = [&](int s) { return bar_base + 8u * s; };
-  auto slab_empty = [&](int s) { return bar_base + 8u * (NS + s); };
-  auto b_full = [&](int s) { return bar_base + 8u * (2 * NS + s); };
-  auto b_empty = [&](int s) { return bar_base + 8u * (2 * NS + NB + s); };
-  auto tmem_full = [&](int s) { return bar_base + 8u * (2 * NS + 2 * NB + s); };
-  auto tmem_empty = [&](int s) { return bar_base + 8u * (2 * NS + 2 * NB + 2 + s); };
+  const Bars<NS, NB> bar{bar_base};
 
   pdl_launch_dependents();
   const int nch = p.nch0 + p.nch1;
@@ -85,20 +80,13 @@ conv_halo_up_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_cons
   };
 
   if (threadIdx.x == 0) {
-    for (int s = 0; s < NS; ++s) { ptx::mbar_init(slab_full(s), 1); ptx::mbar_init(slab_empty(s), kIss); }
-    for (int s = 0; s < NB; ++s) { ptx::mbar_init(b_full(s), 1); ptx::mbar_init(b_empty(s), kIss); }
-    for (int s = 0; s < 2; ++s) { ptx::mbar_init(tmem_full(s), kIss); ptx::mbar_init(tmem_empty(s), 16); }
+    bar.init(kIss, 16);
     ptx::fence_barrier_init();
     ptx::prefetch_tmap(&mapA0);
     ptx::prefetch_tmap(&mapB);
   }
-  if (warp == 2) { ptx::tmem_alloc_cg2(ptx::smem_u32(tmem_ptr_smem), kTmemCols); ptx::tmem_relinquish_cg2(); }
-  ptx::tc_fence_before();
-  __syncthreads();
-  ptx::cluster_sync_exit();
-  ptx::tc_fence_after();
-  const uint32_t tmem_base = *tmem_ptr_smem;
-  pdl_wait();
+  if (warp == 2) tmem_alloc<true>(tmem_ptr_smem, kTmemCols);
+  const uint32_t tmem_base = setup_join<true>(tmem_ptr_smem);
 
   if (warp == 0) {
     // ===================== slab producer: 3 slabs per channel chunk =====================
@@ -111,13 +99,13 @@ conv_halo_up_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_cons
         const CUtensorMap* map = j < p.nch0 ? &mapA0 : &mapA1;
         const int c0 = (j < p.nch0 ? j : j - p.nch0) * 64;
         for (int pl = 0; pl < kSlabsPerChunk; ++pl) {
-          ok = ptx::mbar_wait(slab_empty(s), ph, p.dbg, 41);
+          ok = ptx::mbar_wait(bar.slab_empty(s), ph, p.dbg, 41);
           if (!ok) break;
           if (ptx::elect_one()) {
-            if (leader) ptx::mbar_expect_tx(slab_full(s), 2 * kSlabTx);
-            if (PAIR) ptx::tma_load_5d_cg2(slab_base + s * kSlabBytes, map, ptx::mapa_shared(slab_full(s), 0), c0, t.w0 - 1,
+            if (leader) ptx::mbar_expect_tx(bar.slab_full(s), 2 * kSlabTx);
+            if (PAIR) ptx::tma_load_5d_cg2(slab_base + s * kSlabBytes, map, ptx::mapa_shared(bar.slab_full(s), 0), c0, t.w0 - 1,
                                            t.d0 - 1 + pd + pl, t.h0 - 1, t.n);
-            else ptx::tma_load_5d_cg2(slab_base + s * kSlabBytes, map, ptx::mapa_shared(slab_full(s), 0), c0, t.w0 - 1, t.h0 - 1,
+            else ptx::tma_load_5d_cg2(slab_base + s * kSlabBytes, map, ptx::mapa_shared(bar.slab_full(s), 0), c0, t.w0 - 1, t.h0 - 1,
                                       t.d0 - 1 + pd + pl, t.n);
           }
           __syncwarp();
@@ -127,22 +115,10 @@ conv_halo_up_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_cons
     }
   } else if (warp == 1) {
     // ===================== weight producer: one stage per (chunk, td) = 4 in-plane taps =====================
-    uint32_t s = 0, ph = 1;
-    bool ok = true;
-    for (int id = first_tile; id < p.halo_total_tiles && ok; id += tile_step) {
+    produce_weights<NS, NB, kBRows, kBBytes, true>(p, bar, &mapB, bring_base, crank, first_tile, tile_step, nch * 2, 4, 42, [&](int id) {
       const UTile t = decode(id);
-      const int row0 = t.par * p.n_pad + t.nt * BLOCK_N + (int)crank * kBRows;
-      for (int kb = 0; kb < nch * 2; ++kb) {
-        ok = ptx::mbar_wait(b_empty(s), ph, p.dbg, 42);
-        if (!ok) break;
-        if (ptx::elect_one()) {
-          if (leader) ptx::mbar_expect_tx(b_full(s), 2 * kBBytes);
-          ptx::tma_load_3d_cg2(bring_base + s * kBBytes, &mapB, ptx::mapa_shared(b_full(s), 0), 0, row0, kb * 4);
-        }
-        __syncwarp();
-        if (++s == NB) { s = 0; ph ^= 1; }
-      }
-    }
+      return t.par * p.n_pad + t.nt * BLOCK_N;
+    });
   } else if (warp == 2 || (warp == 3 && kIss == 2)) {
     // ===================== MMA issuers (leader CTA): warp 2 -> output plane 0, warp 3 -> plane 1 =====================
     const int pl = warp - 2;
@@ -150,19 +126,14 @@ conv_halo_up_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_cons
     const uint64_t a_desc0 = ptx::make_smem_desc(slab_base, 16, 1280, ptx::kLayoutSw128);
     const uint64_t b_desc0 = ptx::make_smem_desc(bring_base, 16, 1024, ptx::kLayoutSw128);
     if (leader && ptx::elect_one()) {
-      uint32_t it = 0, sb = 0, bph = 0, qs = 0, qph = 0;
+      uint32_t it = 0, sb = 0, bph = 0;
+      SlabCursor<NS> q;
       bool ok = true;
-      auto slot = [&](uint32_t i, uint32_t& phs) -> uint32_t {
-        uint32_t idx = qs + i;
-        const bool wrap = idx >= (uint32_t)NS;
-        phs = qph ^ (wrap ? 1u : 0u);
-        return wrap ? idx - NS : idx;
-      };
       for (int id = first_tile; id < p.halo_total_tiles && ok; id += tile_step, ++it) {
         const UTile t = decode(id);
         const int ph_ = (t.par >> 1) & 1, pw_ = t.par & 1;
         const uint32_t as = it & 1;
-        ok = ptx::mbar_wait(tmem_empty(as), ((it >> 1) & 1) ^ 1, p.dbg, 43);
+        ok = ptx::mbar_wait(bar.tmem_empty(as), ((it >> 1) & 1) ^ 1, p.dbg, 43);
         if (!ok) break;
         ptx::tc_fence_after();
         const uint32_t acc = tmem_base + as * kAccCols + pl * BLOCK_N;
@@ -172,17 +143,17 @@ conv_halo_up_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_cons
           for (int td = 0; td < 2 && ok; ++td) {
             uint32_t phs;
             if (PAIR) {   // pair slab td
-              const uint32_t sl = slot(td, phs);
-              ok = ptx::mbar_wait(slab_full(sl), phs, p.dbg, 44);
+              const uint32_t sl = q.slot(td, phs);
+              ok = ptx::mbar_wait(bar.slab_full(sl), phs, p.dbg, 44);
             } else if (td == 0) {
-              for (int i = 0; i < TD && ok; ++i) { const uint32_t sl = slot(i, phs); ok = ptx::mbar_wait(slab_full(sl), phs, p.dbg, 44); }
+              for (int i = 0; i < TD && ok; ++i) { const uint32_t sl = q.slot(i, phs); ok = ptx::mbar_wait(bar.slab_full(sl), phs, p.dbg, 44); }
             } else {
-              const uint32_t sl = slot(TD, phs);
-              ok = ptx::mbar_wait(slab_full(sl), phs, p.dbg, 44);
+              const uint32_t sl = q.slot(TD, phs);
+              ok = ptx::mbar_wait(bar.slab_full(sl), phs, p.dbg, 44);
             }
             if (!ok) break;
-            const uint64_t a_pl = a_desc0 + (uint64_t)(slot(pl + td, phs) * (uint32_t)(kSlabBytes >> 4));
-            ok = ptx::mbar_wait(b_full(sb), bph, p.dbg, 45);
+            const uint64_t a_pl = a_desc0 + (uint64_t)(q.slot(pl + td, phs) * (uint32_t)(kSlabBytes >> 4));
+            ok = ptx::mbar_wait(bar.b_full(sb), bph, p.dbg, 45);
             if (!ok) break;
             ptx::tc_fence_after();
             const uint64_t db0 = b_desc0 + (uint64_t)(sb * (kBBytes >> 4));
@@ -195,107 +166,56 @@ conv_halo_up_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_cons
               if (ks > 2) ptx::tc_mma_f16_cg2(acc, da + 4, db + 4, idesc, 1u);
               if (ks > 3) ptx::tc_mma_f16_cg2(acc, da + 6, db + 6, idesc, 1u);
             }
-            ptx::tc_commit_cg2(b_empty(sb), (uint16_t)3);
+            ptx::tc_commit_cg2(bar.b_empty(sb), (uint16_t)3);
             if (PAIR) {
-              ptx::tc_commit_cg2(slab_empty(slot(td, phs)), (uint16_t)3);
+              ptx::tc_commit_cg2(bar.slab_empty(q.slot(td, phs)), (uint16_t)3);
             } else if (td == 0) {
-              ptx::tc_commit_cg2(slab_empty(slot(0, phs)), (uint16_t)3);
+              ptx::tc_commit_cg2(bar.slab_empty(q.slot(0, phs)), (uint16_t)3);
             } else {
-              ptx::tc_commit_cg2(slab_empty(slot(1, phs)), (uint16_t)3);
-              ptx::tc_commit_cg2(slab_empty(slot(2, phs)), (uint16_t)3);
+              ptx::tc_commit_cg2(bar.slab_empty(q.slot(1, phs)), (uint16_t)3);
+              ptx::tc_commit_cg2(bar.slab_empty(q.slot(2, phs)), (uint16_t)3);
             }
             if (++sb == NB) { sb = 0; bph ^= 1; }
           }
-          qs += kSlabsPerChunk;
-          if (qs >= (uint32_t)NS) { qs -= NS; qph ^= 1; }
+          q.advance(kSlabsPerChunk);
         }
-        ptx::tc_commit_cg2(tmem_full(as), (uint16_t)3);
+        ptx::tc_commit_cg2(bar.tmem_full(as), (uint16_t)3);
       }
     }
     __syncwarp();
   } else if (warp >= 4) {
     // ===================== epilogue: 8 warps; lane quarter = warp % 4, column half = (warp - 4) / 4 =====================
-    constexpr int kHalfCols = BLOCK_N / 2;
-    constexpr int kChunks = kHalfCols / 16;
-    constexpr int kNG = stage_groups(BLOCK_N), kBufs = stage_bufs(BLOCK_N), kGB = stage_group_bytes(BLOCK_N);
-    constexpr bool kRow64 = BLOCK_N < 64;   // C_out = 32 (the decoders' last ConvT): 64-byte rows, SWIZZLE_64B (conv_halo.cuh)
     const int qd = warp & 3;
-    const int half = (warp - 4) >> 2;
-    const int cbase = half * kHalfCols;
+    const int cbase = ((warp - 4) >> 2) * (BLOCK_N / 2);   // column half
     const int r = qd * 32 + lane;
-    const int grp = kRow64 ? 0 : cbase >> 6, cl0 = kRow64 ? cbase : cbase & 63;
     uint32_t it = 0, nstore = 0;
     for (int id = first_tile; id < p.halo_total_tiles; id += tile_step, ++it) {
       const UTile t = decode(id);
       const uint32_t as = it & 1;
-      const int colt = t.nt * BLOCK_N + cbase;
-      // bias staging before the accumulator is ready (see conv_halo.cuh): its global round trips overlap the tile's MMAs
       float* bs = bias_s + as * 2 * BLOCK_N;
       float* scs = bs + BLOCK_N;
       const bool has_bs = p.bias != nullptr || p.chan_bias != nullptr || p.out_scale != nullptr;
       const bool has_sc = p.out_scale != nullptr;
-      if (has_bs) {
-        const float* cbrow = nullptr;
-        if (p.chan_bias) {
-          const int tt = p.t_dev ? p.t_dev[0] : 0;
-          cbrow = p.chan_bias + ((int64_t)tt * p.chan_bias_rows + (p.chan_bias_rows > 1 ? t.n : 0)) * p.c_out;
-        }
-        stage_bias(p, bs, scs, t.nt * BLOCK_N, BLOCK_N, cbrow, threadIdx.x - 128, 256);
-        epilogue_bar_sync256();
-      }
-      const bool ok = ptx::mbar_wait(tmem_full(as), (it >> 1) & 1, p.dbg, 46);
+      if (has_bs) stage_tile_bias<BLOCK_N>(p, bs, scs, t.n, t.nt * BLOCK_N, nullptr);
+      const bool ok = ptx::mbar_wait(bar.tmem_full(as), (it >> 1) & 1, p.dbg, 46);
       ptx::tc_fence_after();
       if (!ok) break;
 #pragma unroll
       for (int pl = 0; pl < TD; ++pl) {
         const int od = t.d0 + pl;            // low-resolution (M-space) plane; the parity map places it at 2 * od + pd
         if (od >= p.m_d) break;              // CTA-uniform
-        uint8_t* stg = stg_base + ((nstore % kBufs) * kNG + grp) * kGB;
-        if (warp == 4 && lane == 0) {
-          if (kBufs == 2) ptx::bulk_wait_read_1(); else ptx::bulk_wait_read_all();
-        }
-        epilogue_bar_sync256();
         const uint32_t taddr = tmem_base + ((uint32_t)(qd * 32) << 16) + as * kAccCols + pl * BLOCK_N + cbase;
-#pragma unroll
-        for (int c = 0; c < kChunks; c += 2) {
-          const int col0 = colt + c * 16;
-          uint32_t ra[16], rb[16];
-          ptx::tc_ld_32x32b_x16(taddr + c * 16, ra);
-          if (c + 1 < kChunks) ptx::tc_ld_32x32b_x16(taddr + c * 16 + 16, rb);
-          ptx::tc_wait_ld();
-          conv_epilogue16_staged(p, ra, r, cl0 + c * 16, col0, has_bs ? bs + cbase + c * 16 : nullptr, nullptr,
-                                 has_sc ? scs + cbase + c * 16 : nullptr, nullptr, stg, false, nullptr, kRow64);
-          if (c + 1 < kChunks)
-            conv_epilogue16_staged(p, rb, r, cl0 + c * 16 + 16, col0 + 16, has_bs ? bs + cbase + c * 16 + 16 : nullptr, nullptr,
-                                   has_sc ? scs + cbase + c * 16 + 16 : nullptr, nullptr, stg, false, nullptr, kRow64);
-        }
-        ptx::fence_proxy_async();
-        epilogue_bar_sync256();
-        if (warp == 4 && lane == 0) {
-          for (int g = 0; g < kNG; ++g)
-            if (t.nt * BLOCK_N + g * 64 < p.c_out)
-              if (PAIR) ptx::tma_store_5d(&om.y[t.par], ptx::smem_u32(stg_base + ((nstore % kBufs) * kNG + g) * kGB), t.nt * BLOCK_N + g * 64,
-                                          t.w0, od, t.h0, t.n);
-              else ptx::tma_store_5d(&om.y[t.par], ptx::smem_u32(stg_base + ((nstore % kBufs) * kNG + g) * kGB), t.nt * BLOCK_N + g * 64,
-                                     t.w0, t.h0, od, t.n);
-          ptx::bulk_commit_group();
-        }
+        store_plane16<BLOCK_N, PAIR>(p, &om.y[t.par], stg_base, nstore, taddr, r, cbase, t.nt * BLOCK_N, bs, scs, has_bs, has_sc,
+                                     t.w0, t.h0, od, t.n, false, nullptr, nullptr);
         ++nstore;
       }
       ptx::tc_fence_before();
       __syncwarp();
-      // (nobody waits for the release of a CTA's last two tiles; the cluster-scope arrive costs 2-2.5 k cycles: see conv_halo.cuh)
-      if (lane == 0 && id + 2 * tile_step < p.halo_total_tiles) ptx::mbar_arrive_cluster(ptx::mapa_shared(tmem_empty(as), 0));
+      release_acc<true>(p, bar.tmem_empty(as), id, tile_step);
     }
     if (warp == 4 && lane == 0) ptx::bulk_wait_read_all();
   }
-  ptx::tc_fence_before();
-  __syncthreads();
-  ptx::cluster_sync_exit();
-  if (warp == 2) {
-    ptx::tc_fence_after();
-    ptx::tmem_dealloc_cg2(tmem_base, kTmemCols);
-  }
+  teardown<true>(nullptr, tmem_base, kTmemCols);
 }
 
 }  // namespace halo

@@ -55,12 +55,6 @@ __device__ __forceinline__ Item decode(const Params& q, int item) {
   return it;
 }
 
-__device__ __forceinline__ void tma_load_3d(uint32_t dst, const CUtensorMap* m, uint32_t bar, int c0, int c1, int c2) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];" ::"r"(dst),
-      "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1), "r"(c2)
-      : "memory");
-}
 __device__ __forceinline__ void group_bar_sync(int g) { asm volatile("bar.sync %0, 256;" ::"r"(g + 1) : "memory"); }
 
 constexpr uint64_t kLayoutSw64 = 4;
@@ -173,7 +167,7 @@ conv_sweep32_kernel(const __grid_constant__ CUtensorMap mapX, const __grid_const
     if (ptx::elect_one()) {
       ptx::mbar_expect_tx(w_full, kWBytes);
       for (int kd = 0; kd < 3; ++kd)
-        for (int k9 = 0; k9 < 9; ++k9) tma_load_3d(w_base + (k9 * 3 + kd) * 2048, &mapW, w_full, 0, 0, kd * 9 + k9);
+        for (int k9 = 0; k9 < 9; ++k9) ptx::tma_load_3d(w_base + (k9 * 3 + kd) * 2048, &mapW, w_full, 0, 0, kd * 9 + k9);
     }
     __syncwarp();
   } else if (warp == 2) {

@@ -56,11 +56,6 @@ struct Params {
 __host__ __device__ constexpr uint32_t idesc_f16(int m, int n) {   // kind::f16, A/B = IEEE fp16 (format 0), D = fp32, K-major both
   return (1u << 4) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(m >> 4) << 24);
 }
-__device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* m, uint32_t bar, int c0, int c1) {
-  asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];" ::"r"(dst),
-               "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1)
-               : "memory");
-}
 __device__ __forceinline__ void scan_bar_sync() { asm volatile("bar.sync 1, 256;" ::: "memory"); }   // the 8 scan warps
 
 template <bool kX16>
@@ -258,7 +253,7 @@ vq_tc_kernel(const __grid_constant__ CUtensorMap mapHi, const __grid_constant__ 
           if (!ok) break;
           if (ptx::elect_one()) {
             ptx::mbar_expect_tx(b_full(s), kTile);
-            tma_load_2d(b_base + s * kTile, part == 0 ? &mapHi : &mapLo, b_full(s), c * 64, t * 128);
+            ptx::tma_load_2d(b_base + s * kTile, part == 0 ? &mapHi : &mapLo, b_full(s), c * 64, t * 128);
           }
           __syncwarp();
           if (++s == kNSB) { s = 0; ph ^= 1; }
