@@ -102,10 +102,17 @@ _SIGS = {
     "b200dm_step_advance": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p]),
     "b200dm_step_advance_seq": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "b200dm_gather_rows_f32": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p]),
+    "b200dm_q_sample": (C.c_int, [C.c_void_p] * 5 + [C.c_int64, C.c_int32, C.c_uint64, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "b200dm_noise_loss_workspace": (C.c_size_t, [C.c_int32]),
+    "b200dm_noise_loss": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_double, C.c_uint64, C.c_int64,
+                                    C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "b200dm_vq_distances": (C.c_int, [C.POINTER(VqDesc)] + [C.c_void_p] * 5),
     "b200dm_bn_fold": (C.c_int, [C.c_void_p] * 4 + [C.c_float, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
     "b200dm_gn_stats": (C.c_int, [C.POINTER(NormDesc), C.c_void_p, C.c_float, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "b200dm_gn_stats_workspace": (C.c_size_t, [C.POINTER(NormDesc)]),
+    "b200dm_bn_stats_workspace": (C.c_size_t, [C.c_int32]),
+    "b200dm_bn_stats": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p, C.c_float, C.c_void_p, C.c_void_p, C.c_void_p,
+                                  C.c_size_t, C.c_void_p]),
     "b200dm_norm_act_fwd": (C.c_int, [C.POINTER(NormDesc)] + [C.c_void_p] * 7),
     "b200dm_norm_act_ex": (C.c_int, [C.POINTER(NormExDesc)] + [C.c_void_p] * 8),
     "b200dm_stats_f32_workspace": (C.c_size_t, [C.c_int32]),
@@ -147,6 +154,8 @@ _SIGS = {
     "b200dm_program_add_conv": (C.c_int, [C.c_void_p, C.c_void_p]),
     "b200dm_program_add_norm_act": (C.c_int, [C.c_void_p, C.POINTER(NormDesc)] + [C.c_void_p] * 6),
     "b200dm_program_add_gn_stats": (C.c_int, [C.c_void_p, C.POINTER(NormDesc), C.c_void_p, C.c_float, C.c_void_p, C.c_void_p, C.c_size_t]),
+    "b200dm_program_add_bn_stats": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p, C.c_float,
+                                              C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t]),
     "b200dm_program_add_layernorm": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_float, C.c_int32, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_void_p)]),
     "b200dm_program_add_softmax": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_float]),
     "b200dm_program_add_update": (C.c_int, [C.c_void_p, C.POINTER(UpdateDesc)] + [C.c_void_p] * 5),

@@ -118,8 +118,11 @@ __global__ void __launch_bounds__(256, 4) norm_act_kernel(b200dm_norm_desc d, co
 // grid = (chunks, batch).  Thread (row r, octet o) keeps per-channel sum / sumsq for its octet over
 // voxels r, r+R, ... of the block's chunk; the block reduces in a fixed order and writes one
 // (sum, sumsq) pair per group to partial[n][chunk][g].  gn_final combines chunks in fp64.
+// kCentered: the sums are of x - center[c] (BatchNorm's second pass, groups == C; see bn_final_kernel).
+template <bool kCentered>
 __global__ void __launch_bounds__(256) gn_partial_kernel(const act_t* __restrict__ x, int64_t voxels, int C,
-                                                         int groups, int chunks, float* __restrict__ partial) {
+                                                         int groups, int chunks, float* __restrict__ partial,
+                                                         const float* __restrict__ center) {
   pdl_launch_dependents();
   pdl_wait();
   __shared__ float ssum[256 * 8];
@@ -135,10 +138,17 @@ __global__ void __launch_bounds__(256) gn_partial_kernel(const act_t* __restrict
 #pragma unroll
   for (int i = 0; i < 8; ++i) s[i] = q[i] = 0.f;
   const act_t* xs = x + (int64_t)n * voxels * C + (o << 3);
+  float k[8];
+#pragma unroll
+  for (int i = 0; i < 8; ++i) k[i] = kCentered ? center[(o << 3) + i] : 0.f;
   if (r < rows) {
     for (int64_t v = v0 + r; v < v1; v += rows) {
       float f[8];
       unpack8(*reinterpret_cast<const bf16x8*>(xs + v * C), f);
+      if (kCentered) {
+#pragma unroll
+        for (int i = 0; i < 8; ++i) f[i] -= k[i];
+      }
 #pragma unroll
       for (int i = 0; i < 8; ++i) { s[i] += f[i]; q[i] = fmaf(f[i], f[i], q[i]); }
     }
@@ -183,6 +193,36 @@ __global__ void gn_final_kernel(const float* __restrict__ partial, int batch, in
   mean_rstd[i * 2] = (float)mean;
   mean_rstd[i * 2 + 1] = (float)(1.0 / sqrt(var + (double)eps));
 }
+
+// BatchNormalization with batch statistics (training=True): per-channel mean and biased variance over all B*D*H*W rows,
+// from gn_partial_kernel's per-chunk sums with groups == C, combined in fixed chunk order in fp64 (bit-reproducible).
+// Two passes over x: pass 1 (scale == nullptr) writes center[c] = mean; pass 2 gets the sums of d = x - center and
+// forms var = E[d^2] - E[d]^2 -- the corrected two-pass form, so a channel whose |mean| >> std loses nothing to
+// cancellation -- then scale = gamma * rsqrt(var + eps), shift = beta - mean * scale: the coefficients norm_act_kernel
+// and the conv epilogue's affine read.
+__global__ void bn_final_kernel(const float* __restrict__ partial, int C, int chunks, double count, float eps,
+                                float* __restrict__ center, const float* __restrict__ gamma, const float* __restrict__ beta,
+                                float* __restrict__ scale, float* __restrict__ shift) {
+  pdl_launch_dependents();
+  pdl_wait();
+  const int c = blockIdx.x * blockDim.x + threadIdx.x;
+  if (c >= C) return;
+  double a = 0.0, b = 0.0;
+  for (int k = 0; k < chunks; ++k) {
+    const float* p = partial + ((int64_t)k * C + c) * 2;
+    a += (double)p[0]; b += (double)p[1];
+  }
+  const double d = a / count;
+  if (!scale) { center[c] = (float)d; return; }
+  double var = b / count - d * d;
+  if (var < 0.0) var = 0.0;
+  const double mean = (double)center[c] + d;
+  const float sc = (float)((double)gamma[c] / sqrt(var + (double)eps));
+  scale[c] = sc;
+  shift[c] = (float)((double)beta[c] - mean * (double)sc);
+}
+
+constexpr int kBnChunks = 256;
 
 // ------------------------------------------------------------------ LayerNorm over C (one warp per row)
 template <int kVecPerLane>
@@ -387,11 +427,37 @@ extern "C" int b200dm_gn_stats(const b200dm_norm_desc* d, const void* x, float e
   B2_CHECK_ARG(C <= 512 && 256 % (C / 8) == 0, "gn_stats: C=%d unsupported (need C/8 to divide 256, C<=512)", C);
   const int chunks = 64;
   cudaStream_t s = (cudaStream_t)stream;
-  B2_CHECK_CUDA(b2_launch(gn_partial_kernel, dim3(chunks, d->batch), dim3(256), 0, s, (const act_t*)x, d->voxels, C, d->groups, chunks, workspace));
+  B2_CHECK_CUDA(b2_launch(gn_partial_kernel<false>, dim3(chunks, d->batch), dim3(256), 0, s, (const act_t*)x, d->voxels, C, d->groups, chunks,
+                          workspace, (const float*)nullptr));
   B2_CHECK_LAUNCH();
   const int tot = d->batch * d->groups;
   B2_CHECK_CUDA(b2_launch(gn_final_kernel, dim3((tot + 127) / 128), dim3(128), 0, s, workspace, d->batch, d->groups, chunks,
                                                     (double)d->voxels * (double)(C / d->groups), eps, mean_rstd));
+  B2_CHECK_LAUNCH();
+  return B200DM_OK;
+}
+
+extern "C" size_t b200dm_bn_stats_workspace(int32_t c) {
+  return c > 0 ? ((size_t)kBnChunks * c * 2 + c) * sizeof(float) : 0;
+}
+
+extern "C" int b200dm_bn_stats(const void* x, int64_t rows, int32_t c, const float* gamma, const float* beta, float eps,
+                               float* scale, float* shift, float* workspace, size_t ws_bytes, void* stream) {
+  B2_CHECK_ARG(x && gamma && beta && scale && shift && workspace && rows > 0, "bn_stats: bad arguments");
+  B2_CHECK_ARG(c >= 8 && c <= 512 && c % 8 == 0 && 256 % (c / 8) == 0, "bn_stats: C=%d unsupported (need C/8 to divide 256, 8 <= C <= 512)", c);
+  B2_CHECK_ARG(ws_bytes >= b200dm_bn_stats_workspace(c), "bn_stats: workspace too small");
+  cudaStream_t s = (cudaStream_t)stream;
+  float* center = workspace + (size_t)kBnChunks * c * 2;
+  const act_t* xb = (const act_t*)x;
+  const dim3 fgrid((c + 127) / 128);
+  B2_CHECK_CUDA(b2_launch(gn_partial_kernel<false>, dim3(kBnChunks), dim3(256), 0, s, xb, rows, (int)c, (int)c, kBnChunks, workspace,
+                          (const float*)nullptr));
+  B2_CHECK_CUDA(b2_launch(bn_final_kernel, fgrid, dim3(128), 0, s, (const float*)workspace, (int)c, kBnChunks, (double)rows, eps, center,
+                          (const float*)nullptr, (const float*)nullptr, (float*)nullptr, (float*)nullptr));
+  B2_CHECK_CUDA(b2_launch(gn_partial_kernel<true>, dim3(kBnChunks), dim3(256), 0, s, xb, rows, (int)c, (int)c, kBnChunks, workspace,
+                          (const float*)center));
+  B2_CHECK_CUDA(b2_launch(bn_final_kernel, fgrid, dim3(128), 0, s, (const float*)workspace, (int)c, kBnChunks, (double)rows, eps, center,
+                          gamma, beta, scale, shift));
   B2_CHECK_LAUNCH();
   return B200DM_OK;
 }

@@ -12,7 +12,7 @@
 #include "common.cuh"
 
 namespace {
-enum OpKind { OP_CONV, OP_NORM, OP_GNSTATS, OP_LN, OP_SOFTMAX, OP_UPDATE, OP_ADVANCE, OP_ATTN, OP_NORM_EX, OP_STATS_F32, OP_SYNC, OP_GN_FINAL };
+enum OpKind { OP_CONV, OP_NORM, OP_GNSTATS, OP_LN, OP_SOFTMAX, OP_UPDATE, OP_ADVANCE, OP_ATTN, OP_NORM_EX, OP_STATS_F32, OP_SYNC, OP_GN_FINAL, OP_BN_STATS };
 constexpr int kMaxLanes = 10;
 struct Op {
   OpKind kind;
@@ -108,6 +108,15 @@ extern "C" int b200dm_program_add_gn_stats(b200dm_program* p, const b200dm_norm_
   B2_CHECK_ARG(p && d && x && mean_rstd && workspace, "program_add_gn_stats: null argument");
   Op op; op.kind = OP_GNSTATS; op.nd = *d; op.p0 = x; op.f0 = eps; op.out = mean_rstd; op.out2 = workspace; op.ws = ws_bytes;
   op.launches = 2;
+  p->push(op);
+  return B200DM_OK;
+}
+
+extern "C" int b200dm_program_add_bn_stats(b200dm_program* p, const void* x, int64_t rows, int32_t c, const float* gamma,
+                                           const float* beta, float eps, float* scale, float* shift, float* workspace, size_t ws_bytes) {
+  B2_CHECK_ARG(p && x && gamma && beta && scale && shift && workspace, "program_add_bn_stats: null argument");
+  Op op; op.kind = OP_BN_STATS; op.p0 = x; op.i0 = rows; op.i1 = c; op.p1 = gamma; op.p2 = beta; op.f0 = eps; op.out = scale;
+  op.out2 = shift; op.p3 = workspace; op.ws = ws_bytes; op.launches = 4;
   p->push(op);
   return B200DM_OK;
 }
@@ -249,6 +258,10 @@ static int run_op(Op& op, void* stream) {
       case OP_SYNC: break;
       case OP_GN_FINAL:
         rc = b200dm_gn_finalize((const float*)op.p0, op.i1, op.i2, op.nd.c0, op.nd.groups, op.i0, op.f0, (float*)op.out, stream);
+        break;
+      case OP_BN_STATS:
+        rc = b200dm_bn_stats(op.p0, op.i0, op.i1, (const float*)op.p1, (const float*)op.p2, op.f0, (float*)op.out, (float*)op.out2,
+                             (float*)op.p3, op.ws, stream);
         break;
       case OP_STATS_F32: rc = b200dm_stats_f32((const float*)op.p0, op.i1, op.i0, op.f0, (float*)op.out, op.out2, op.ws, stream); break;
     }

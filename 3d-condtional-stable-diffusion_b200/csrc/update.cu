@@ -10,6 +10,8 @@ namespace {
 
 using namespace upd;
 
+constexpr uint32_t kTrainNoiseStream = 2;   // Philox stream id of train_step's noise
+
 // 8 elements per thread per trip (two Philox counters), two trips in flight: 4x LDG.128 x_t, 2-4x LDG.128 eps issued before
 // any use; grid = (blocks, batch) so the loop has no index division.
 template <bool kEpsBf16>
@@ -94,6 +96,73 @@ __global__ void __launch_bounds__(256) philox_normal_kernel(float* __restrict__ 
   }
 }
 
+// Forward diffusion of train_step (conditional_dm3d.py:481-490): x_t = sqrt(abar_t) * z + sqrt(1 - abar_t) * noise for a
+// per-sample t, in the reference's fp32 op order (two rounded products, one rounded sum).  The noise is Philox stream 2,
+// counter (element / 4, 0, global sample index, 2) -- streams 0 (update) and 1 (x_T) belong to the sampler -- or injected.
+// grid = (blocks, batch); 4 elements per thread per trip.
+__global__ void __launch_bounds__(256) q_sample_kernel(const float* __restrict__ z, const float* __restrict__ sqrt_ab,
+                                                       const float* __restrict__ sqrt_1mab, const int32_t* __restrict__ t,
+                                                       const float* __restrict__ noise, int64_t n_per_sample, uint64_t seed,
+                                                       int64_t sample_id0, act_t* __restrict__ x16, float* __restrict__ x32) {
+  pdl_launch_dependents();
+  pdl_wait();
+  const int64_t b = blockIdx.y, base = b * n_per_sample;
+  const int tb = t[b];
+  const float a = sqrt_ab[tb], s = sqrt_1mab[tb];
+  for (int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; j < (n_per_sample >> 2); j += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t off = base + (j << 2);
+    float x[4], e[4];
+    *reinterpret_cast<float4*>(x) = __ldg(reinterpret_cast<const float4*>(z + off));
+    if (noise) *reinterpret_cast<float4*>(e) = __ldg(reinterpret_cast<const float4*>(noise + off));
+    else normal4((uint32_t)j, 0u, (uint32_t)(sample_id0 + b), kTrainNoiseStream, seed, e);
+#pragma unroll
+    for (int q = 0; q < 4; ++q) x[q] = __fadd_rn(__fmul_rn(a, x[q]), __fmul_rn(s, e[q]));
+    *reinterpret_cast<act2_t*>(x16 + off) = floats_to_act2(x[0], x[1]);
+    *reinterpret_cast<act2_t*>(x16 + off + 2) = floats_to_act2(x[2], x[3]);
+    if (x32) *reinterpret_cast<float4*>(x32 + off) = *reinterpret_cast<float4*>(x);
+  }
+}
+
+// sum over all elements of (noise - eps_hat)^2, per block in fixed order (fp64), one partial per block: the numerator of
+// train_step's MSE(reduction=SUM) (conditional_dm3d.py:496-499).  The noise is regenerated from q_sample_kernel's stream (or
+// read when injected).  grid = (blocks, batch)
+constexpr int kLossBlocks = 64;
+__global__ void __launch_bounds__(256) sq_err_partial_kernel(const float* __restrict__ eps, const float* __restrict__ noise,
+                                                             int64_t n_per_sample, uint64_t seed, int64_t sample_id0,
+                                                             double* __restrict__ partial) {
+  pdl_launch_dependents();
+  pdl_wait();
+  const int64_t b = blockIdx.y, base = b * n_per_sample;
+  double acc = 0.0;
+  for (int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; j < (n_per_sample >> 2); j += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t off = base + (j << 2);
+    float y[4], e[4];
+    *reinterpret_cast<float4*>(y) = __ldg(reinterpret_cast<const float4*>(eps + off));
+    if (noise) *reinterpret_cast<float4*>(e) = __ldg(reinterpret_cast<const float4*>(noise + off));
+    else normal4((uint32_t)j, 0u, (uint32_t)(sample_id0 + b), kTrainNoiseStream, seed, e);
+    float s = 0.f;
+#pragma unroll
+    for (int q = 0; q < 4; ++q) { const float d = __fsub_rn(e[q], y[q]); s = __fadd_rn(s, __fmul_rn(d, d)); }
+    acc += (double)s;
+  }
+  __shared__ double red[256];
+  red[threadIdx.x] = acc;
+  __syncthreads();
+  for (int o = 128; o > 0; o >>= 1) {
+    if ((int)threadIdx.x < o) red[threadIdx.x] += red[threadIdx.x + o];
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) partial[b * gridDim.x + blockIdx.x] = red[0];
+}
+
+__global__ void sq_err_final_kernel(const double* __restrict__ partial, int n, double inv_divisor, float* __restrict__ loss) {
+  pdl_launch_dependents();
+  pdl_wait();
+  double a = 0.0;
+  for (int i = 0; i < n; ++i) a += partial[i];
+  *loss = (float)(a * inv_divisor);
+}
+
 __global__ void step_advance_kernel(int32_t* t_dev, int32_t delta) {
   pdl_launch_dependents();
   pdl_wait();
@@ -160,6 +229,39 @@ extern "C" int b200dm_step_advance_seq(int32_t* t_dev, const int32_t* seq, void*
 extern "C" int b200dm_step_advance(int32_t* t_dev, int32_t delta, void* stream) {
   B2_CHECK_ARG(t_dev, "step_advance: null t_dev");
   B2_CHECK_CUDA(b2_launch(step_advance_kernel, dim3(1), dim3(1), 0, (cudaStream_t)stream, t_dev, delta));
+  B2_CHECK_LAUNCH();
+  return B200DM_OK;
+}
+
+extern "C" int b200dm_q_sample(const float* z, const float* sqrt_alpha_bar, const float* sqrt_one_minus_alpha_bar,
+                               const int32_t* t, const float* noise, int64_t n_per_sample, int32_t batch, uint64_t seed,
+                               int64_t sample_id0, void* x_t16, float* x_t32, void* stream) {
+  B2_CHECK_ARG(z && sqrt_alpha_bar && sqrt_one_minus_alpha_bar && t && x_t16, "q_sample: null argument");
+  B2_CHECK_ARG(n_per_sample > 0 && n_per_sample % 4 == 0 && batch > 0 && batch <= 65535, "q_sample: bad shape");
+  const int64_t want = ((n_per_sample >> 2) + 255) / 256;
+  int64_t cap = ((int64_t)b2_num_sms() * 8 + batch - 1) / batch;
+  if (cap < 1) cap = 1;
+  B2_CHECK_CUDA(b2_launch(q_sample_kernel, dim3((unsigned)(want < cap ? want : cap), (unsigned)batch), dim3(256), 0, (cudaStream_t)stream,
+                          z, sqrt_alpha_bar, sqrt_one_minus_alpha_bar, t, noise, n_per_sample, seed, sample_id0, (act_t*)x_t16, x_t32));
+  B2_CHECK_LAUNCH();
+  return B200DM_OK;
+}
+
+extern "C" size_t b200dm_noise_loss_workspace(int32_t batch) { return batch > 0 ? (size_t)batch * kLossBlocks * sizeof(double) : 0; }
+
+extern "C" int b200dm_noise_loss(const float* eps_hat, const float* noise, int64_t n_per_sample, int32_t batch, int32_t channels,
+                                 double divisor, uint64_t seed, int64_t sample_id0, float* loss, void* workspace, size_t ws_bytes,
+                                 void* stream) {
+  B2_CHECK_ARG(eps_hat && loss && workspace, "noise_loss: null argument");
+  B2_CHECK_ARG(n_per_sample > 0 && n_per_sample % 4 == 0 && batch > 0 && batch <= 65535 && channels > 0 && divisor > 0.0,
+               "noise_loss: bad arguments");
+  B2_CHECK_ARG(ws_bytes >= b200dm_noise_loss_workspace(batch), "noise_loss: workspace too small");
+  cudaStream_t s = (cudaStream_t)stream;
+  B2_CHECK_CUDA(b2_launch(sq_err_partial_kernel, dim3(kLossBlocks, (unsigned)batch), dim3(256), 0, s, eps_hat, noise, n_per_sample, seed,
+                          sample_id0, (double*)workspace));
+  // Keras MSE: mean over the channel axis, then the SUM reduction over (B, D, H, W); then / divisor
+  B2_CHECK_CUDA(b2_launch(sq_err_final_kernel, dim3(1), dim3(1), 0, s, (const double*)workspace, (int)(batch * kLossBlocks),
+                          1.0 / ((double)channels * divisor), loss));
   B2_CHECK_LAUNCH();
   return B200DM_OK;
 }

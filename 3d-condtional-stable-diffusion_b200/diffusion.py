@@ -8,7 +8,8 @@ timesteps / num_gpus / kernel_resize / bs), same attributes (.timesteps .b .netw
 .vqvae_trainer) and the same ``sample(x_t, pred_noise, t, shape) -> (mean, var)`` and
 ``generate(shape, last_step[, context_value]) -> latents`` contracts.  Build additions (explicit extensions,
 SURVEY 8b): ``x_T=``, ``noise=`` (inject), ``seed=``, ``sample_id0=`` (multi-GPU sharding), ``sampler="ddim"``,
-``steps=``, per-sample ``context=`` ids, and ``decode(latents, quantize=False)``.
+``steps=``, per-sample ``context=`` ids, ``decode(latents, quantize=False)`` and ``train_loss`` (the forward half of
+train_step and its loss, without gradients).
 
 The reverse loop is one captured CUDA graph per step: U-Net program + fused posterior update + a device-side
 timestep decrement, replayed T times with zero host work in between.  Samples are independent (BatchNorm in inference
@@ -72,11 +73,13 @@ class DiffusionModel:
                                    context_dim=1 if self.conditional else None,
                                    first_conv_channels=self.first_conv_channels, conditional=self.conditional)
         self._step = None
+        self._train = None
 
     # ------------------------------------------------------------------ reference API
     def load_weights(self, path):
         self.network.load_weights(path)
         self._step = None
+        self._train = None
 
     def sample(self, x_t, pred_noise, curr_time_step, shape=None):
         """-> (posterior_mean, variance); the reference returns the variance under the name log-variance
@@ -262,14 +265,72 @@ class DiffusionModel:
         latents, _ = self.quantizer(self.encoder(images))
         return latents
 
+    def _t_dev(self, t, B):
+        t = torch.as_tensor(t).reshape(-1).long().cpu()
+        if t.numel() == 1:
+            t = t.expand(B)
+        if t.numel() != B or int(t.min()) < 0 or int(t.max()) >= self.timesteps:
+            raise ValueError(f"t must hold {B} timesteps in [0, {self.timesteps})")
+        return t, t.to(torch.int32).cuda()
+
     def q_sample(self, latents, t, noise):
         """Forward diffusion of train_step (conditional_dm3d.py:484-490): sqrt(abar_t) * latents + sqrt(1 - abar_t) * noise,
-        t (B,) int.  A host-side helper over the fp32 schedule tables (not on the sampling path)."""
-        t = torch.as_tensor(t).long().reshape(-1).cpu()
-        h = self.b.host
-        sqb = torch.from_numpy(h["sqrt_alpha_bar"])[t].reshape(-1, 1, 1, 1, 1).to(latents.device, torch.float32)
-        osqb = torch.from_numpy(h["sqrt_one_minus_alpha_bar"])[t].reshape(-1, 1, 1, 1, 1).to(latents.device, torch.float32)
-        return sqb * latents.float() + osqb * noise.to(latents.device, torch.float32)
+        t (B,) int, in the reference's fp32 op order -> fp32 x_t on the device (the q-sample kernel of train_loss)."""
+        L.require_gpu()
+        self.b.to(torch.device("cuda", torch.cuda.current_device()))
+        z = latents.cuda().float().contiguous()
+        _, t_dev = self._t_dev(t, z.shape[0])
+        return ops.q_sample(self.b, z, t_dev, noise=noise.to(z.device, torch.float32).contiguous(), want_f32=True)[1]
+
+    @staticmethod
+    def draw_timesteps(seed, batch, timesteps):
+        """t ~ U{0..T-1} per sample (conditional_dm3d.py:474) from a host generator seeded with ``seed``: reproducible."""
+        g = torch.Generator().manual_seed(int(seed))
+        return torch.randint(0, timesteps, (batch,), generator=g, dtype=torch.int64)
+
+    def loss_divisor(self):
+        """global_bs * lc^4: train_step divides the summed MSE by this literal (conditional_dm3d.py:496-499, SURVEY 3.5)."""
+        return float(self.global_bs) * float(self.lc) ** 4
+
+    def train_loss(self, images=None, *, latents=None, context=None, t=None, noise=None, seed=None):
+        """The loss train_step computes (conditional_dm3d.py:471-499), without the gradient step: ``latents`` (or the frozen
+        ``encode(images)``) -> t ~ U{0..T-1} per sample from a host generator seeded with ``seed`` (unless ``t`` is given) ->
+        x_t = q_sample(latents, t, noise) with the noise from Philox stream 2 of ``seed`` (unless ``noise`` is injected) ->
+        eps_hat = network([x_t, t, ctx], training=True) (batch-statistics BatchNorm, moving statistics not updated) ->
+        MSE(reduction=SUM)(noise, eps_hat) / (global_bs * lc^4).  BatchNorm statistics are those of this process's batch, as on a
+        MirroredStrategy replica; ``global_bs`` is ``args.bs``.  ``seed=None`` draws a fresh seed (kept in ``last_seed``; the t
+        used in ``last_t``).  Returns the loss as a 0-d fp32 tensor on the device."""
+        if latents is None:
+            if images is None:
+                raise ValueError("train_loss: give images or latents")
+            latents = self.encode(images)
+        L.require_gpu()
+        dev = torch.device("cuda", torch.cuda.current_device())
+        z = latents.to(dev, torch.float32).contiguous()
+        B = z.shape[0]
+        if tuple(z.shape[1:]) != (self.latent_size,) * 3 + (self.lc,):
+            raise ValueError(f"train_loss: latents {tuple(z.shape)} do not match the latent geometry")
+        if seed is None:
+            seed = int.from_bytes(os.urandom(7), "little")
+        self.last_seed = seed
+        if t is None:
+            t = self.draw_timesteps(seed, B, self.timesteps)
+        t, t_dev = self._t_dev(t, B)
+        self.last_t = t.clone()
+        key = (B, self.network.weights_version)
+        if self._train is None or self._train["key"] != key:
+            self.b.to(dev)
+            self._train = dict(key=key, net=copy.copy(self.network).compile(B, self.timesteps, dev, training=True))
+        net = self._train["net"]
+        if self.conditional:
+            ctx = torch.as_tensor(0 if context is None else context).reshape(-1)
+            net.set_context(ctx.expand(B) if ctx.numel() == 1 else ctx)
+        if noise is not None:
+            noise = noise.to(dev, torch.float32).contiguous()
+        net.set_timesteps(t)
+        ops.q_sample(self.b, z, t_dev, noise=noise, seed=seed, out16=net.x_in)
+        net.forward_inplace()
+        return ops.noise_loss(net.eps, self.loss_divisor(), noise=noise, seed=seed)[0]
 
     def decode(self, latents, quantize=False):
         """latents -> volumes through the first-stage decoder; ``quantize=True`` snaps latents to the codebook first

@@ -73,6 +73,32 @@ def ddpm_update(tables, x_t, eps, t, noise=None, seed=0, sample_id0=0, sampler=0
     return (out, out_b) if want_bf16 else out
 
 
+def q_sample(tables, z, t_dev, noise=None, seed=0, sample_id0=0, want_f32=False, out16=None):
+    """x_t = sqrt(abar_t) z + sqrt(1 - abar_t) noise (train_step, conditional_dm3d.py:481-490) for per-sample ``t_dev`` (B,) int32
+    on the device; the noise is Philox stream 2 of ``seed`` unless injected.  -> 16-bit x_t (and fp32 x_t when ``want_f32``)."""
+    _dev()
+    assert z.dtype == torch.float32 and z.is_contiguous() and t_dev.dtype == torch.int32
+    if out16 is None:
+        out16 = torch.empty(z.shape, dtype=L.ACT_DTYPE, device=z.device)
+    x32 = torch.empty_like(z) if want_f32 else None
+    check(lib().b200dm_q_sample(ptr(z), ptr(tables.dev["sqrt_alpha_bar"]), ptr(tables.dev["sqrt_one_minus_alpha_bar"]), ptr(t_dev),
+                                ptr(noise), z[0].numel(), z.shape[0], seed, sample_id0, ptr(out16), ptr(x32), stream()))
+    return (out16, x32) if want_f32 else out16
+
+
+def noise_loss(eps_hat, divisor, noise=None, seed=0, sample_id0=0):
+    """MSE(reduction=SUM)(noise, eps_hat) / divisor (conditional_dm3d.py:496-499): mean over the last axis, sum over the rest.
+    The noise is regenerated from q_sample's stream unless injected.  -> fp32 (1,) on the device."""
+    _dev()
+    assert eps_hat.dtype == torch.float32 and eps_hat.is_contiguous()
+    B = eps_hat.shape[0]
+    ws = torch.empty(lib().b200dm_noise_loss_workspace(B) // 8, dtype=torch.float64, device=eps_hat.device)
+    loss = torch.empty(1, dtype=torch.float32, device=eps_hat.device)
+    check(lib().b200dm_noise_loss(ptr(eps_hat), ptr(noise), eps_hat[0].numel(), B, eps_hat.shape[-1], float(divisor), seed, sample_id0,
+                                  ptr(loss), ptr(ws), ws.numel() * 8, stream()))
+    return loss
+
+
 def philox_normal(shape, seed, sample_id0=0, step=0, stream_id=1, want_bf16=False):
     dev = _dev()
     x = torch.empty(shape, dtype=torch.float32, device=dev)
@@ -86,6 +112,19 @@ def bn_fold(gamma, beta, mean, var, eps=1e-3):
     _dev()
     scale, shift = torch.empty_like(gamma), torch.empty_like(gamma)
     check(lib().b200dm_bn_fold(ptr(gamma), ptr(beta), ptr(mean), ptr(var), eps, gamma.numel(), ptr(scale), ptr(shift), stream()))
+    return scale, shift
+
+
+def bn_stats(x, gamma, beta, eps=1e-3, scale=None, shift=None):
+    """BatchNormalization with the batch's own statistics (training=True): x (..., C) 16-bit -> (scale, shift) fp32 (C,), the
+    per-channel affine of norm_act / the conv epilogue."""
+    _dev()
+    c = x.shape[-1]
+    scale = torch.empty(c, dtype=torch.float32, device=x.device) if scale is None else scale
+    shift = torch.empty(c, dtype=torch.float32, device=x.device) if shift is None else shift
+    ws = torch.empty(lib().b200dm_bn_stats_workspace(c) // 4, dtype=torch.float32, device=x.device)
+    check(lib().b200dm_bn_stats(ptr(x), x.numel() // c, c, ptr(gamma), ptr(beta), eps, ptr(scale), ptr(shift), ptr(ws), ws.numel() * 4,
+                                stream()))
     return scale, shift
 
 

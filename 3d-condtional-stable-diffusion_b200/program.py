@@ -98,6 +98,19 @@ class Program:
         self.log.append(("gn_stats", note, x.numel() * 2.0))
         return mr
 
+    def bn_stats(self, x, gamma, beta, scale, shift, eps=1e-3, note=""):
+        """scale / shift (fp32 (C,) views) <- BatchNorm coefficients from the batch statistics of x (training=True); two reads
+        of x."""
+        c = x.shape[-1]
+        ws_bytes = lib().b200dm_bn_stats_workspace(c)
+        ws = self.buf((ws_bytes // 4,), torch.float32)
+        check(lib().b200dm_program_add_bn_stats(self.h, ptr(x), x.numel() // c, c, ptr(gamma), ptr(beta), eps, ptr(scale), ptr(shift),
+                                                ptr(ws), ws_bytes))
+        self.hold(x, gamma, beta, scale, shift)
+        self.bytes += x.numel() * 4.0
+        self.log.append(("bn_stats", note, x.numel() * 4.0))
+        return scale, shift
+
     def norm_act_ex(self, x, a, b, y, kind=0, groups=1, mean_rstd=None, prelu_alpha=None, residual=None, act=None, post_act=None,
                     upsample=False, note=""):
         """y = post_act(residual + act(PReLU(norm(x)))), x optionally nearest-upsampled x2; y (B,D,H,W,C) bf16 | fp32."""

@@ -125,6 +125,8 @@ class UNet:
         self.prog = None
         self.weights_version = 0   # bumped by set_weights: compiled copies held elsewhere (DiffusionModel._step) key on it
         self._per_sample = None    # lazily compiled variant for a (B,) vector of distinct timesteps
+        self._training = None      # lazily compiled training-mode variant (batch-statistics BatchNorm)
+        self.training = False
 
     @property
     def params(self):
@@ -138,6 +140,7 @@ class UNet:
         self._params = {k: torch.as_tensor(np.asarray(v) if not torch.is_tensor(v) else v).float().cpu() for k, v in params.items()}
         self.prog = None
         self._per_sample = None
+        self._training = None
         self.weights_version += 1
 
     def load_weights(self, path, name_map=None, assume_creation_order=False):
@@ -157,11 +160,16 @@ class UNet:
         return sum(int(np.prod(s)) for _, s, _ in self.spec)
 
     # ---- compilation ------------------------------------------------------------------------
-    def compile(self, batch: int, timesteps: int, device=None, t_dev=None, per_sample_t=False):
+    def compile(self, batch: int, timesteps: int, device=None, t_dev=None, per_sample_t=False, training=False):
         """Pack weights, precompute the t-only tables, allocate every activation buffer and record the launches.
         ``per_sample_t``: the ResidualBlock time-embedding rows come from per-sample (B, w) buffers (filled by
-        ``_set_timesteps`` from the hoisted tables) instead of one device-side timestep for the whole batch -- the form
-        train_step calls the network in (t ~ U{0..T-1} per sample, conditional_dm3d.py:474,493)."""
+        ``set_timesteps`` from the hoisted tables) instead of one device-side timestep for the whole batch -- the form
+        train_step calls the network in (t ~ U{0..T-1} per sample, conditional_dm3d.py:474,493).
+        ``training``: the program of ``network(..., training=True)`` (conditional_dm3d.py:493), on the per-sample-t form: every
+        BatchNormalization normalises with the statistics of the current batch (a statistics op writes its scale / shift on the
+        device before the apply pass), so none of the folds that assume constant statistics is used -- conv1 stores
+        conv + temb and norm2 is a pass of its own, proj_in reads the normalised tensor, no shadow-lane norm1 halves.  The
+        moving statistics are not updated: that belongs to a step that also applies gradients."""
         L.require_gpu()
         cfg, P = self.cfg, self.params
         dev = device or torch.device("cuda", torch.cuda.current_device())
@@ -170,7 +178,8 @@ class UNet:
         pr = Program(dev)
         self.prog = pr
         self.t_dev = t_dev if t_dev is not None else torch.zeros(4, dtype=torch.int32, device=dev)   # [t, t_prev, seq idx, -]
-        self.per_sample_t, self._temb_rows = bool(per_sample_t), []
+        self.training = bool(training)
+        self.per_sample_t, self._temb_rows = bool(per_sample_t) or self.training, []
         g = lambda n: P[n].to(dev).contiguous()  # noqa: E731
 
         # --- K12: time embedding MLP for every t, then per-ResidualBlock Dense(swish(temb)) tables (T, w)
@@ -218,12 +227,26 @@ class UNet:
             y = pr.buf((Bx, M, N), y_dtype)
             return pr.conv(desc, a, b, y, residual=residual, note=note)
 
+        def bn_affine(name, x0, x1=None):
+            """(scale, shift) of BatchNorm ``name`` over [x0 | x1]: folded from the moving statistics, or -- training -- written
+            on the device by statistics ops, each concat half from its own tensor (the statistics are per channel)."""
+            if not self.training:
+                return ops.bn_fold(g(f"{name}.gamma"), g(f"{name}.beta"), g(f"{name}.mean"), g(f"{name}.var"), 1e-3)
+            gam, bet = g(f"{name}.gamma"), g(f"{name}.beta")
+            sc, sh = pr.buf(gam.shape, torch.float32), pr.buf(gam.shape, torch.float32)
+            c0 = x0.shape[-1]
+            pr.bn_stats(x0, gam[:c0], bet[:c0], sc[:c0], sh[:c0], note=f"{name}.stats")
+            if x1 is not None:
+                pr.bn_stats(x1, gam[c0:], bet[c0:], sc[c0:], sh[c0:], note=f"{name}.stats.skip")
+            pr.hold(gam, bet)
+            return sc, sh
+
         def bn_act(x0, name, act, x1=None, note=""):
             """BatchNorm(inference) [+ swish] of x0 (or of the concat [x0, x1]) -> (y0, y1|None): the conv that reads it takes
             the two channel segments separately.  One fused norm(+concat) pass, or the x half only when the skip half was
             normalised in the shadow of the 8^3 phase.  (Writing the normalised copies from the producers' epilogues instead
             measured slower: 5.47 vs 5.08 ms/step on cfg-2, the conv epilogues are on the critical path.)"""
-            sc, sh = ops.bn_fold(g(f"{name}.gamma"), g(f"{name}.beta"), g(f"{name}.mean"), g(f"{name}.var"), 1e-3)
+            sc, sh = bn_affine(name, x0, x1)
             c0 = x0.shape[-1]
             if x1 is not None and id(x1) in self.shadow_norms:
                 # the skip half was normalised with this block's parameters in the shadow of the 8^3 phase (lane 4, see below):
@@ -254,10 +277,14 @@ class UNet:
                 self._temb_rows.append((pr.hold(table), rows))
                 table = rows
             h, h1 = bn_act(x, f"{n}.norm1", "silu", x1=skip)
-            # conv1 + temb -> BN(norm2) -> swish (dm3d.py:237-244): conv1's output has no other reader, so norm2 and the
-            # activation run in conv1's epilogue on the fp32 accumulator (one HBM pass and one bf16 rounding fewer)
-            sc2, sh2 = ops.bn_fold(g(f"{n}.norm2.gamma"), g(f"{n}.norm2.beta"), g(f"{n}.norm2.mean"), g(f"{n}.norm2.var"), 1e-3)
-            h = conv(h, f"{n}.conv1", w, x1=h1, chan_bias=pr.hold(table), out_affine=(sc2, sh2), act="silu", note=f"{n}.conv1+norm2")
+            if self.training:   # norm2's statistics are those of conv1's output: it is stored, then normalised
+                h = conv(h, f"{n}.conv1", w, x1=h1, chan_bias=pr.hold(table))
+                h, _ = bn_act(h, f"{n}.norm2", "silu")
+            else:
+                # conv1 + temb -> BN(norm2) -> swish (dm3d.py:237-244): conv1's output has no other reader, so norm2 and the
+                # activation run in conv1's epilogue on the fp32 accumulator (one HBM pass and one bf16 rounding fewer)
+                sc2, sh2 = ops.bn_fold(g(f"{n}.norm2.gamma"), g(f"{n}.norm2.beta"), g(f"{n}.norm2.mean"), g(f"{n}.norm2.var"), 1e-3)
+                h = conv(h, f"{n}.conv1", w, x1=h1, chan_bias=pr.hold(table), out_affine=(sc2, sh2), act="silu", note=f"{n}.conv1+norm2")
             pr.outputs[f"{n}.norm2"] = h
             if cin != w:
                 # width change: the 1^3 shortcut of [x | skip] runs as the last K segment of conv2 (halo kernel), so its output is
@@ -305,11 +332,15 @@ class UNet:
             scale = float(c) ** -0.5
             # inference BatchNorm followed by the 1^3 proj_in conv is one affine map: fold it into proj_in's kernel and bias
             # (W' = diag(a) W, b' = b + shift . W; conditional_dm3d.py:187-188) -- no normalisation pass
-            sc_n, sh_n = ops.bn_fold(g(f"{n}.norm.gamma"), g(f"{n}.norm.beta"), g(f"{n}.norm.mean"), g(f"{n}.norm.var"), 1e-3)
-            w_in = P[f"{n}.proj_in.kernel"].reshape(c, c)
-            w_fold = (sc_n.cpu()[:, None] * w_in).reshape(1, 1, 1, c, c)
-            b_fold = P[f"{n}.proj_in.bias"] + sh_n.cpu() @ w_in
-            h = conv(x, f"{n}.proj_in", c, k=1, act="relu", kern=w_fold, bias_t=b_fold)
+            if self.training:   # batch statistics: normalise, then the plain proj_in
+                nrm, _ = bn_act(x, f"{n}.norm", None)
+                h = conv(nrm, f"{n}.proj_in", c, k=1, act="relu")
+            else:
+                sc_n, sh_n = ops.bn_fold(g(f"{n}.norm.gamma"), g(f"{n}.norm.beta"), g(f"{n}.norm.mean"), g(f"{n}.norm.var"), 1e-3)
+                w_in = P[f"{n}.proj_in.kernel"].reshape(c, c)
+                w_fold = (sc_n.cpu()[:, None] * w_in).reshape(1, 1, 1, c, c)
+                b_fold = P[f"{n}.proj_in.bias"] + sh_n.cpu() @ w_in
+                h = conv(x, f"{n}.proj_in", c, k=1, act="relu", kern=w_fold, bias_t=b_fold)
             gam = [g(f"{n}.norm{i}.gamma") for i in (1, 2, 3)]
             bet = [g(f"{n}.norm{i}.beta") for i in (1, 2, 3)]
             ln = pr.layernorm(h, gam, bet, [pr.buf(h.shape) for _ in range(3)], 1e-3, note=f"{n}.ln")
@@ -351,7 +382,7 @@ class UNet:
         # (BN + swish with the CONSUMER block's parameters, dm3d.py:235-236) are therefore run on lane 4 while the 8^3 phase
         # executes on the other lanes, and the up-path passes shrink to the x half.
         self.shadow_norms, self.shadow_joined = {}, False
-        use_shadow = len(cfg.widths) >= 2
+        use_shadow = len(cfg.widths) >= 2 and not self.training   # training: the norm1 halves wait for their statistics on lane 0
         consumer, stack = {}, []          # push index -> the up-path ResidualBlock that pops it
         npush = 0
         for b in self.blocks:
@@ -443,8 +474,28 @@ class UNet:
         self.prog.run()
         return self.eps
 
-    def __call__(self, inputs):
-        """network([x (B,S,S,S,C) fp32|bf16, t (B,) int (, ctx (B,)|(B,1,1) int)]) -> eps_hat fp32 (new tensor)."""
+    def set_timesteps(self, t):
+        """Per-sample-t programs: gather the (B, w) time-embedding rows of ``t`` (B,) from the hoisted tables."""
+        tidx = torch.as_tensor(t).reshape(-1).to(torch.int32).to(self.device)
+        for table, rows in self._temb_rows:
+            L.check(L.lib().b200dm_gather_rows_f32(L.ptr(table), table.shape[0], L.ptr(tidx), L.ptr(rows), rows.shape[0],
+                                                  rows.shape[1], L.stream()))
+
+    def training_program(self):
+        """The training-mode compiled copy (``compile(..., training=True)``) of this compiled network, built on first use: same
+        weights, own activation buffers; ``self`` and its inference program are untouched by it."""
+        if self.training:
+            return self
+        if self._training is None:
+            import copy
+            self._training = copy.copy(self).compile(self.batch, self.timesteps, self.device, training=True)
+        return self._training
+
+    def __call__(self, inputs, training=False):
+        """network([x (B,S,S,S,C) fp32|bf16, t (B,) int (, ctx (B,)|(B,1,1) int)], training=False) -> eps_hat fp32 (new tensor).
+        ``training=True`` (train_step's call, conditional_dm3d.py:493): every BatchNormalization uses the statistics of this
+        batch, so a sample's eps_hat depends on the others; the moving statistics are NOT updated (that side effect belongs to a
+        step that also applies gradients).  ``training=False`` runs the inference program, unchanged by training calls."""
         x, t = inputs[0], inputs[1]
         if self.prog is None or self.batch != x.shape[0]:
             raise L.B200dmError("UNet: call compile(batch, timesteps) first (batch must match)")
@@ -453,6 +504,10 @@ class UNet:
             tvec = tvec.expand(x.shape[0])
         if tvec.numel() != x.shape[0] or int(tvec.min()) < 0 or int(tvec.max()) >= self.timesteps:
             raise L.B200dmError(f"UNet: t must hold {x.shape[0]} timesteps in [0, {self.timesteps})")
+        if bool(training) != self.training:
+            if not training:
+                raise L.B200dmError("UNet: this is the training-mode program; call the network it was built from")
+            return self.training_program()(inputs, training=True)
         tv = int(tvec[0])
         if not bool((tvec == tv).all()) and not self.per_sample_t:
             # distinct timesteps per sample (train_step's call, conditional_dm3d.py:493): a second compiled program whose conv
@@ -464,10 +519,7 @@ class UNet:
         if len(inputs) > 2 and self.cfg.conditional:
             self.set_context(torch.as_tensor(inputs[2]).reshape(-1))
         if self.per_sample_t:
-            tidx = tvec.to(torch.int32).to(self.device)
-            for table, rows in self._temb_rows:
-                L.check(L.lib().b200dm_gather_rows_f32(L.ptr(table), table.shape[0], L.ptr(tidx), L.ptr(rows), rows.shape[0],
-                                                      rows.shape[1], L.stream()))
+            self.set_timesteps(tvec)
         self.t_dev.copy_(torch.tensor([tv, tv - 1, 0, 0], dtype=torch.int32))
         x = x.to(self.device)
         self.x_in.copy_(x if x.dtype == L.ACT_DTYPE else ops.cast(x.contiguous().float(), L.ACT_DTYPE))

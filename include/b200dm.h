@@ -97,6 +97,19 @@ int b200dm_step_advance_seq(int32_t* t_dev, const int32_t* seq, void* stream);
  * with distinct t per sample (train_step, conditional_dm3d.py:474,493) */
 int b200dm_gather_rows_f32(const float* table, int32_t table_rows, const int32_t* idx, float* out, int32_t rows, int32_t cols,
                            void* stream);
+/* Forward diffusion of train_step (conditional_dm3d.py:481-490): x_t = sqrt_alpha_bar[t[b]] * z + sqrt_one_minus_alpha_bar[t[b]]
+ * * noise in the reference's fp32 op order, t device int32[batch].  noise_or_null NULL: Philox4x32-10 stream 2, counter
+ * (element/4, 0, sample_id0 + b, 2) (streams 0 / 1 are the sampler's).  Writes x_t as the 16-bit network input and, when
+ * x_t32_or_null is given, as fp32. */
+int b200dm_q_sample(const float* z, const float* sqrt_alpha_bar, const float* sqrt_one_minus_alpha_bar, const int32_t* t,
+                    const float* noise_or_null, int64_t n_per_sample, int32_t batch, uint64_t seed, int64_t sample_id0,
+                    void* x_t16, float* x_t32_or_null, void* stream);
+/* train_step's loss (conditional_dm3d.py:496-499): MSE(reduction=SUM)(noise, eps_hat) / divisor = sum over (B,D,H,W) of the
+ * mean over `channels` of (noise - eps_hat)^2, / divisor -> loss fp32[1] (device).  The noise is regenerated from
+ * b200dm_q_sample's stream with the same seed / sample_id0, or read from noise_or_null.  Fixed reduction order: bit-reproducible. */
+size_t b200dm_noise_loss_workspace(int32_t batch);
+int b200dm_noise_loss(const float* eps_hat, const float* noise_or_null, int64_t n_per_sample, int32_t batch, int32_t channels,
+                      double divisor, uint64_t seed, int64_t sample_id0, float* loss, void* workspace, size_t ws_bytes, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * K6/K7  fused normalisation + activation (+ channel concat, + per-voxel PReLU) in one HBM pass.
@@ -123,6 +136,13 @@ int b200dm_bn_fold(const float* gamma, const float* beta, const float* mean, con
 int b200dm_gn_stats(const b200dm_norm_desc* d, const void* x, float eps, float* mean_rstd /* [B][G][2] */,
                     float* workspace, size_t ws_bytes, void* stream);
 size_t b200dm_gn_stats_workspace(const b200dm_norm_desc* d);
+/* BatchNormalization with the statistics of the batch (training=True): x (rows = B*D*H*W, c) 16-bit, per-channel mean and
+ * biased variance (tf.nn.moments) -> scale[c] = gamma[c] * rsqrt(var + eps), shift[c] = beta[c] - mean * scale: the
+ * coefficients of b200dm_norm_act_fwd kind 0 and of b200dm_conv_plan_set_out_affine.  Deterministic two-pass reduction
+ * (fixed-order fp64 combine of per-CTA partials; the second pass sums x - mean).  c in 8..512 with c/8 dividing 256. */
+size_t b200dm_bn_stats_workspace(int32_t c);
+int b200dm_bn_stats(const void* x, int64_t rows, int32_t c, const float* gamma, const float* beta, float eps, float* scale,
+                    float* shift, float* workspace, size_t ws_bytes, void* stream);
 int b200dm_norm_act_fwd(const b200dm_norm_desc* d, const void* x0, const void* x1_or_null,
                         const float* scale_or_gamma, const float* shift_or_beta,
                         const float* mean_rstd_or_null, void* y, void* stream);
@@ -320,6 +340,8 @@ int b200dm_program_add_conv(b200dm_program* p, b200dm_conv_plan* plan /* ownersh
 int b200dm_program_add_norm_act(b200dm_program* p, const b200dm_norm_desc* d, const void* x0,
                                 const void* x1_or_null, const float* a, const float* b,
                                 const float* mean_rstd_or_null, void* y);
+int b200dm_program_add_bn_stats(b200dm_program* p, const void* x, int64_t rows, int32_t c, const float* gamma, const float* beta,
+                                float eps, float* scale, float* shift, float* workspace, size_t ws_bytes);
 int b200dm_program_add_gn_stats(b200dm_program* p, const b200dm_norm_desc* d, const void* x, float eps,
                                 float* mean_rstd, float* workspace, size_t ws_bytes);
 int b200dm_program_add_gn_finalize(b200dm_program* p, const float* partials, int32_t batch, int32_t rows_per_sample, int32_t c,
