@@ -213,6 +213,14 @@ def stream():
     return C.c_void_p(torch.cuda.current_stream().cuda_stream)
 
 
+def check_storage(*ts):
+    """Raise when a 16-bit tensor is not the library's storage type: the kernels take raw pointers and would read bf16 bits as
+    fp16 (or the reverse) without a word.  None and non-16-bit tensors pass."""
+    for t in ts:
+        if t is not None and t.dtype in (torch.bfloat16, torch.float16) and t.dtype != ACT_DTYPE:
+            raise B200dmError(f"libb200dm ({_precision} build) stores {ACT_DTYPE}; got a {t.dtype} tensor")
+
+
 def dt(t):
     if t.dtype == torch.float32:
         return F32

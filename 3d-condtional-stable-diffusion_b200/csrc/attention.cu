@@ -277,15 +277,25 @@ flash_attn_kernel(const __grid_constant__ CUtensorMap mapQ, const __grid_constan
         tc_wait_st();
         ptx::tc_fence_before();
       }
-      // ---- p = exp2(s*c - m_ref) -> bf16 (in place: two per register)
+      // ---- p = exp2(s*c - m_ref) -> 16-bit (in place: two per register)
       float ls4[4] = {0.f, 0.f, 0.f, 0.f};
       const float nm = -m_ref;
 #pragma unroll
       for (int i = 0; i < BKV; i += 2) {
         const float p0 = ex2(fmaf(__uint_as_float(sv[i]), p.scale_log2e, nm));
         const float p1 = ex2(fmaf(__uint_as_float(sv[i + 1]), p.scale_log2e, nm));
+#ifdef B200DM_ACT_FP16
+        // l sums the ROUNDED p, the weights P.V consumes, so that they are normalised exactly: in fp16, p < 2^-25 rounds to
+        // 0, and summing the unrounded p would shrink the output by (sum of the flushed p) / l -- 2.8e-3 for 131072 keys 25.5
+        // binades below the row maximum.  (Shifting p up instead does not help: the tensor cores' fp32 accumulation of P.V
+        // drops products that far below the running O.)  bf16 has fp32's exponent range; its p do not underflow.
+        const act2_t h = floats_to_act2(p0, p1);
+        const float2 hf = act2_to_float2(h);
+        ls4[(i >> 1) & 3] += hf.x + hf.y;
+#else
         ls4[(i >> 1) & 3] += p0 + p1;
         const act2_t h = floats_to_act2(p0, p1);
+#endif
         memcpy(&sv[i >> 1], &h, 4);
       }
       l += (ls4[0] + ls4[1]) + (ls4[2] + ls4[3]);

@@ -76,6 +76,7 @@ def ddpm_update(tables, x_t, eps, t, noise=None, seed=0, sample_id0=0, sampler=0
 def q_sample(tables, z, t_dev, noise=None, seed=0, sample_id0=0, want_f32=False, out16=None):
     """x_t = sqrt(abar_t) z + sqrt(1 - abar_t) noise (train_step, conditional_dm3d.py:481-490) for per-sample ``t_dev`` (B,) int32
     on the device; the noise is Philox stream 2 of ``seed`` unless injected.  -> 16-bit x_t (and fp32 x_t when ``want_f32``)."""
+    L.check_storage(z, noise, out16)
     _dev()
     assert z.dtype == torch.float32 and z.is_contiguous() and t_dev.dtype == torch.int32
     if out16 is None:
@@ -89,6 +90,7 @@ def q_sample(tables, z, t_dev, noise=None, seed=0, sample_id0=0, want_f32=False,
 def noise_loss(eps_hat, divisor, noise=None, seed=0, sample_id0=0):
     """MSE(reduction=SUM)(noise, eps_hat) / divisor (conditional_dm3d.py:496-499): mean over the last axis, sum over the rest.
     The noise is regenerated from q_sample's stream unless injected.  -> fp32 (1,) on the device."""
+    L.check_storage(eps_hat, noise)
     _dev()
     assert eps_hat.dtype == torch.float32 and eps_hat.is_contiguous()
     B = eps_hat.shape[0]
@@ -118,6 +120,7 @@ def bn_fold(gamma, beta, mean, var, eps=1e-3):
 def bn_stats(x, gamma, beta, eps=1e-3, scale=None, shift=None):
     """BatchNormalization with the batch's own statistics (training=True): x (..., C) 16-bit -> (scale, shift) fp32 (C,), the
     per-channel affine of norm_act / the conv epilogue."""
+    L.check_storage(x)
     _dev()
     c = x.shape[-1]
     scale = torch.empty(c, dtype=torch.float32, device=x.device) if scale is None else scale
@@ -137,6 +140,7 @@ def make_norm_desc(x0, x1=None, kind=0, groups=1, act=None) -> L.NormDesc:
 
 
 def gn_stats(x, groups, eps):
+    L.check_storage(x)
     _dev()
     d = make_norm_desc(x, None, 1, groups)
     ws = torch.empty(lib().b200dm_gn_stats_workspace(C.byref(d)) // 4, dtype=torch.float32, device=x.device)
@@ -146,7 +150,8 @@ def gn_stats(x, groups, eps):
 
 
 def norm_act(x0, a, b, act=None, x1=None, kind=0, groups=1, mean_rstd=None, out=None):
-    """y = act(affine(x)) over [x0, x1] concatenated on channels (bf16 in, bf16 out)."""
+    """y = act(affine(x)) over [x0, x1] concatenated on channels (16-bit in, 16-bit out)."""
+    L.check_storage(x0, x1, out)
     _dev()
     d = make_norm_desc(x0, x1, kind, groups, act)
     if out is None:
@@ -163,6 +168,7 @@ def _ptr_array(ts):
 
 
 def layernorm(x, gammas, betas, eps=1e-3):
+    L.check_storage(x)
     _dev()
     c = x.shape[-1]
     rows = x.numel() // c
@@ -278,6 +284,7 @@ class ConvPlan:
 
     def __init__(self, desc, x0, w_packed, y, x1=None, bias=None, chan_bias=None, t_dev=None, residual=None, prelu_alpha=None,
                  out_affine=None):
+        L.check_storage(x0, x1, w_packed, residual, prelu_alpha, y)
         _dev()
         self.keep = (x0, x1, w_packed, bias, chan_bias, t_dev, residual, prelu_alpha, y) + tuple(out_affine or ())  # keep buffers alive
         # algorithmic HBM bytes of one launch: every operand read once, the output written once
@@ -381,7 +388,8 @@ def conv3d(x0, keras_kernel, bias=None, x1=None, mode=L.CONV_DIRECT, stride=1, a
 
 
 def batched_gemm(a, b, y_dtype=torch.float32, residual=None):
-    """y[n] = a[n] (M,K) @ b[n] (N,K)^T, bf16 operands, fp32 accumulate (attention matmuls)."""
+    """y[n] = a[n] (M,K) @ b[n] (N,K)^T, 16-bit operands, fp32 accumulate (attention matmuls)."""
+    L.check_storage(a, b, residual)
     dev = _dev()
     B, M, K = a.shape
     N = b.shape[1]

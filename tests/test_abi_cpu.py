@@ -150,3 +150,42 @@ def test_fp16_storage_build_exports_the_same_abi(L):
             "import pytest\ntry:\n    L.set_precision('bf16'); raise SystemExit(3)\nexcept L.B200dmError:\n    pass") % ROOT
     r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True)
     assert r.returncode == 0, r.stderr
+
+
+@pytest.mark.parametrize("precision,other", [("fp16", "bfloat16"), ("bf16", "float16")])
+def test_other_16bit_type_is_rejected_before_the_device(precision, other):
+    """A 16-bit tensor of the type the loaded build does not store is an error naming both types, raised before any device
+    check: the kernels take raw pointers and would otherwise read bf16 bits as fp16 (or the reverse)."""
+    code = f"""
+import os, sys
+os.environ['B200DM_PRECISION'] = {precision!r}
+sys.path.insert(0, {ROOT!r})
+import torch, b200dm
+from b200dm import ops, _lib as L
+bad = torch.zeros(1, 4, 4, 4, 64, dtype=torch.{other})
+f32 = torch.zeros(1, 4, 4, 4, 64)
+one = torch.ones(64)
+desc = ops.make_conv_desc(L.CONV_DIRECT, 1, (4, 4, 4), 64, 0, 64, 1, 1)
+calls = dict(
+    ConvPlan=lambda: ops.ConvPlan(desc, bad, torch.zeros(64 * 64, dtype=L.ACT_DTYPE), torch.zeros(1, 4, 4, 4, 64, dtype=L.ACT_DTYPE)),
+    norm_act=lambda: ops.norm_act(bad, one, one),
+    gn_stats=lambda: ops.gn_stats(bad, 8, 1e-6),
+    layernorm=lambda: ops.layernorm(bad, [one], [one]),
+    bn_stats=lambda: ops.bn_stats(bad, one, one),
+    q_sample=lambda: ops.q_sample(ops.ScheduleTables(4), f32, torch.zeros(1, dtype=torch.int32), out16=bad),
+    noise_loss=lambda: ops.noise_loss(bad, 1.0),
+    batched_gemm=lambda: ops.batched_gemm(bad[0, 0], bad[0, 0]),
+)
+for name, call in calls.items():
+    try:
+        call()
+    except L.B200dmError as e:
+        msg = str(e)
+        assert str(L.ACT_DTYPE) in msg and 'torch.{other}' in msg, (name, msg)
+    else:
+        raise SystemExit(name + ': no error')
+print('rejected', len(calls))
+"""
+    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True)
+    assert r.returncode == 0, r.stdout + r.stderr
+    assert "rejected 8" in r.stdout

@@ -1,20 +1,24 @@
 """GPU parity of the flash-style tcgen05 attention kernel (csrc/attention.cu) vs the oracle's attention_core
 (softmax(q k^T * scale) v over flattened voxel tokens; networks/dm3d.py:51-61, conditional_dm3d.py:162-184).
 
-Tolerance (stated): q, k, v are bf16 on both sides, scores / softmax statistics / accumulation are fp32 on both sides; the
-kernel rounds the UNNORMALISED probabilities to bf16 before P.V (the oracle's bf16-emulation rounds the normalised ones) and
-writes bf16 outputs: rel-L2 <= 5e-3, max-abs <= 2e-2 * max|ref|."""
+Tolerance (stated): q, k, v are 16-bit on both sides, scores / softmax statistics / accumulation are fp32 on both sides; the
+kernel rounds the UNNORMALISED probabilities to the storage type before P.V (the oracle does not round them) and writes 16-bit
+outputs: rel-L2 <= 1.28 U, max-abs <= 5.12 U * max|ref|, U the unit roundoff of the storage type (2^-8 bf16, 2^-11 fp16)."""
 import numpy as np
 import pytest
 import torch
 
+from b200dm import _lib
 from oracle import ops as O
 
 pytestmark = pytest.mark.gpu
 
+ACT = _lib.ACT_DTYPE
+U = 2 ** -8 if _lib.precision() == "bf16" else 2 ** -11   # unit roundoff of the storage type: its largest relative rounding error
+
 
 def _r(t):
-    return t.to(torch.bfloat16).to(torch.float32)
+    return t.to(ACT).to(torch.float32)
 
 
 def _rand(shape, seed, scale=1.0):
@@ -24,8 +28,8 @@ def _rand(shape, seed, scale=1.0):
 def _run(cuda, q, k, v, scale, residual=None):
     from b200dm import ops, _lib
     vt = v.transpose(1, 2).contiguous()
-    o = ops.attention(q.to(cuda, torch.bfloat16), k.to(cuda, torch.bfloat16), vt.to(cuda, torch.bfloat16), scale,
-                      residual=None if residual is None else residual.to(cuda, torch.bfloat16))
+    o = ops.attention(q.to(cuda, ACT), k.to(cuda, ACT), vt.to(cuda, ACT), scale,
+                      residual=None if residual is None else residual.to(cuda, ACT))
     torch.cuda.synchronize()
     assert _lib.debug_flag() == 0, "tcgen05/TMA pipeline watchdog fired"
     return o.float().cpu()
@@ -55,7 +59,7 @@ def test_flash_attention_matches_oracle(cuda, B, Lq, Lk, D, res):
     rel = ((o - ref).norm() / ref.norm()).item()
     mx = (o - ref).abs().max().item() / ref.abs().max().item()
     print(f"attention B{B} Lq{Lq} Lk{Lk} D{D}: rel-L2 {rel:.3e} max-abs/max {mx:.3e}")
-    assert rel <= 5e-3 and mx <= 2e-2, (rel, mx)
+    assert rel <= 1.28 * U and mx <= 5.12 * U, (rel, mx)
 
 
 def test_flash_attention_peaked_scores(cuda):
@@ -66,7 +70,8 @@ def test_flash_attention_peaked_scores(cuda):
     ref = O.attention_core(q, k, v, scale)
     o = _run(cuda, q, k, v, scale)
     rel = ((o - ref).norm() / ref.norm()).item()
-    assert rel <= 8e-3, rel
+    print(f"peaked scores: rel-L2 {rel:.3e}")
+    assert rel <= 2.05 * U, rel
 
 
 def test_flash_attention_full_size_properties(cuda):
@@ -78,11 +83,11 @@ def test_flash_attention_full_size_properties(cuda):
     k = _rand((B, L, D), 2)
     v0 = _rand((1, 1, D), 3)
     o = _run(cuda, q, k, v0.expand(B, L, D).contiguous(), D ** -0.5)
-    assert (o - v0).abs().max().item() <= 2e-2 * v0.abs().max().item()
+    assert (o - v0).abs().max().item() <= 5.12 * U * v0.abs().max().item()
     v = _rand((B, L, D), 4)
     o = _run(cuda, q, torch.zeros(B, L, D), v, D ** -0.5)
     mean = v.mean(1, keepdim=True)
-    assert (o - mean).abs().max().item() <= 2e-3 + 2e-2 * mean.abs().max().item()
+    assert (o - mean).abs().max().item() <= 2e-3 + 5.12 * U * mean.abs().max().item()
 
 
 def test_flash_attention_strided_q_k(cuda):
@@ -91,10 +96,10 @@ def test_flash_attention_strided_q_k(cuda):
     B, L, D = 2, 512, 256
     qk = _rand((B, L, 2 * D), 1)
     v = _rand((B, L, D), 2)
-    dqk = qk.to(cuda, torch.bfloat16)
-    o = ops.attention(dqk[..., :D], dqk[..., D:], v.transpose(1, 2).contiguous().to(cuda, torch.bfloat16), D ** -0.5)
+    dqk = qk.to(cuda, ACT)
+    o = ops.attention(dqk[..., :D], dqk[..., D:], v.transpose(1, 2).contiguous().to(cuda, ACT), D ** -0.5)
     torch.cuda.synchronize()
     assert _lib.debug_flag() == 0
     ref = O.attention_core(qk[..., :D], qk[..., D:], v, D ** -0.5)
     o = o.float().cpu()
-    assert ((o - ref).norm() / ref.norm()).item() <= 5e-3
+    assert ((o - ref).norm() / ref.norm()).item() <= 1.28 * U

@@ -1,20 +1,25 @@
 """GPU parity: tcgen05 implicit-GEMM conv (all variants) vs the oracle's Keras-semantics conv.
 
-Inputs and weights are bf16-representable, accumulation is fp32 on both sides, so the only
-difference is summation order: tolerance 2e-3 * max|y| absolute on fp32 outputs (stated), and one
-bf16 ulp (2^-8 relative) on bf16 outputs.
+Inputs and weights are representable in the 16-bit storage type, accumulation is fp32 on both sides, so the only
+difference on fp32 outputs is summation order: tolerance A * max|y| absolute (A set from the measured spread, 4x margin),
+plus U (the storage type's unit roundoff, its largest relative rounding error) per 16-bit rounding on 16-bit outputs.
 """
 import numpy as np
 import pytest
 import torch
 
+from b200dm import _lib
 from oracle import ops as O
 
 pytestmark = pytest.mark.gpu
 
+ACT = _lib.ACT_DTYPE
+U = 2 ** -8 if _lib.precision() == "bf16" else 2 ** -11   # unit roundoff of the storage type: its largest relative rounding error
+A = 2e-5   # fp32 accumulation in another order: measured <= 3.6e-6 of max|y| in either build (B200)
 
-def _r(t):  # bf16-representable fp32
-    return t.to(torch.bfloat16).to(torch.float32)
+
+def _r(t):  # storage-representable fp32
+    return t.to(ACT).to(torch.float32)
 
 
 def _rand(shape, seed, scale=1.0):
@@ -22,10 +27,11 @@ def _rand(shape, seed, scale=1.0):
     return _r(torch.randn(shape, generator=g) * scale)
 
 
-def _close(y, ref, tol=2e-3, what=""):
+def _close(y, ref, tol=A, what=""):
     y = y.float().cpu()
     err = (y - ref).abs().max().item()
     den = ref.abs().max().item() + 1e-12
+    print(f"{what}: rel max err {err / den:.3e} (bound {tol:.3e})")
     assert err <= tol * den, f"{what}: max abs err {err:.4e} vs max|ref| {den:.4e} (rel {err/den:.3e})"
 
 
@@ -54,7 +60,7 @@ def test_conv3_same(cuda, B, S, cin, cout):
     w = _rand((3, 3, 3, cin, cout), 2, 1.0 / np.sqrt(27 * cin))
     b = torch.randn(cout, generator=torch.Generator().manual_seed(3))
     ref = O.conv3d(x, w, b)
-    y = ops.conv3d(x.to(cuda, torch.bfloat16), w, bias=b.to(cuda), y_dtype=torch.float32)
+    y = ops.conv3d(x.to(cuda, ACT), w, bias=b.to(cuda), y_dtype=torch.float32)
     _check_flag()
     _close(y, ref, what=f"conv3 B{B} S{S} {cin}->{cout}")
 
@@ -68,11 +74,11 @@ def test_conv3_bf16_out_and_epilogue(cuda):
     cbias = torch.randn(B, cout, generator=torch.Generator().manual_seed(4))
     res = _rand((B, S, S, S, cout), 5)
     ref = O.swish(O.conv3d(x, w, b) + cbias[:, None, None, None, :]) + res
-    y = ops.conv3d(x.to(cuda, torch.bfloat16), w, bias=b.to(cuda), chan_bias=cbias.to(cuda), act="silu",
-                   residual=res.to(cuda, torch.bfloat16))
+    y = ops.conv3d(x.to(cuda, ACT), w, bias=b.to(cuda), chan_bias=cbias.to(cuda), act="silu",
+                   residual=res.to(cuda, ACT))
     _check_flag()
-    assert y.dtype == torch.bfloat16
-    _close(y, ref, tol=6e-3, what="conv3 + bias + temb + silu + residual (bf16 out)")
+    assert y.dtype == ACT
+    _close(y, ref, tol=A + U, what="conv3 + bias + temb + silu + residual (16-bit out)")
 
 
 def test_conv3_pair_slab_tiles(cuda):
@@ -86,10 +92,10 @@ def test_conv3_pair_slab_tiles(cuda):
         res = _rand((B, D, 8, 8, cout), 5)
         xin = x0 if x1 is None else torch.cat([x0, x1], -1)
         ref = O.conv3d(xin, w, b) + res
-        y = ops.conv3d(x0.to(cuda, torch.bfloat16), w, bias=b.to(cuda), residual=res.to(cuda, torch.bfloat16),
-                       x1=None if x1 is None else x1.to(cuda, torch.bfloat16))
+        y = ops.conv3d(x0.to(cuda, ACT), w, bias=b.to(cuda), residual=res.to(cuda, ACT),
+                       x1=None if x1 is None else x1.to(cuda, ACT))
         _check_flag()
-        _close(y, ref, tol=6e-3, what=f"pair-slab conv3 B{B} D{D} {c0}+{c1}->{cout}")
+        _close(y, ref, tol=A + U, what=f"pair-slab conv3 B{B} D{D} {c0}+{c1}->{cout}")
 
 
 def test_conv3_two_segments(cuda):
@@ -98,7 +104,7 @@ def test_conv3_two_segments(cuda):
     x0, x1 = _rand((B, S, S, S, c0), 1), _rand((B, S, S, S, c1), 6)
     w = _rand((3, 3, 3, c0 + c1, cout), 2, 1.0 / np.sqrt(27 * (c0 + c1)))
     ref = O.conv3d(torch.cat([x0, x1], -1), w)
-    y = ops.conv3d(x0.to(cuda, torch.bfloat16), w, x1=x1.to(cuda, torch.bfloat16), y_dtype=torch.float32)
+    y = ops.conv3d(x0.to(cuda, ACT), w, x1=x1.to(cuda, ACT), y_dtype=torch.float32)
     _check_flag()
     _close(y, ref, what="conv3 over [x, skip] K-segments")
 
@@ -109,7 +115,7 @@ def test_conv1(cuda):
     x = _rand((B, S, S, S, cin), 1)
     w = _rand((1, 1, 1, cin, cout), 2, 1.0 / np.sqrt(cin))
     ref = torch.relu(O.conv3d(x, w))
-    y = ops.conv3d(x.to(cuda, torch.bfloat16), w, act="relu", y_dtype=torch.float32)
+    y = ops.conv3d(x.to(cuda, ACT), w, act="relu", y_dtype=torch.float32)
     _check_flag()
     _close(y, ref, what="conv1 + relu")
 
@@ -121,7 +127,7 @@ def test_conv_head_cout1(cuda):
     w = _rand((3, 3, 3, cin, 1), 2, 1.0 / np.sqrt(27 * cin))
     b = torch.tensor([0.25])
     ref = O.conv3d(x, w, b)
-    y = ops.conv3d(x.to(cuda, torch.bfloat16), w, bias=b.to(cuda), y_dtype=torch.float32)
+    y = ops.conv3d(x.to(cuda, ACT), w, bias=b.to(cuda), y_dtype=torch.float32)
     _check_flag()
     _close(y, ref, what="conv3 32->1 head")
 
@@ -133,7 +139,7 @@ def test_conv3_stride2_tf_same(cuda, S, c):
     x = _rand((2, S, S, S, c), 1)
     w = _rand((3, 3, 3, c, c), 2, 1.0 / np.sqrt(27 * c))
     ref = O.conv3d(x, w, stride=2)
-    y = ops.conv3d(x.to(cuda, torch.bfloat16), w, stride=2, y_dtype=torch.float32)
+    y = ops.conv3d(x.to(cuda, ACT), w, stride=2, y_dtype=torch.float32)
     _check_flag()
     assert tuple(y.shape) == tuple(ref.shape)
     _close(y, ref, what="conv3 stride 2")
@@ -146,10 +152,10 @@ def test_upsample_conv_parity_fold(cuda, S, c):
     w = _rand((3, 3, 3, c, c), 2, 1.0 / np.sqrt(27 * c))
     b = torch.randn(c, generator=torch.Generator().manual_seed(3))
     ref = O.conv3d(O.upsample_nearest2(x), w, b)
-    y = ops.conv3d(x.to(cuda, torch.bfloat16), w, bias=b.to(cuda), mode=_lib.CONV_PARITY, y_dtype=torch.float32)
+    y = ops.conv3d(x.to(cuda, ACT), w, bias=b.to(cuda), mode=_lib.CONV_PARITY, y_dtype=torch.float32)
     _check_flag()
-    # folded taps are summed in fp32 then rounded to bf16 once: error bound is one bf16 ulp of a weight
-    _close(y, ref, tol=8e-3, what="UpSampling3D(2)+Conv3 as 8 parity sub-convs")
+    # folded taps are summed in fp32 then rounded to the storage type once: the reference's taps are not; two ulps of a weight
+    _close(y, ref, tol=A + 2 * U, what="UpSampling3D(2)+Conv3 as 8 parity sub-convs")
 
 
 @pytest.mark.parametrize("S,cin,cout", [(4, 128, 64), (8, 64, 32)])
@@ -159,7 +165,7 @@ def test_conv_transpose_k4s2(cuda, S, cin, cout):
     w = _rand((4, 4, 4, cout, cin), 2, 1.0 / np.sqrt(8 * cin))
     b = torch.randn(cout, generator=torch.Generator().manual_seed(3))
     ref = O.conv3d_transpose(x, w, b)
-    y = ops.conv3d(x.to(cuda, torch.bfloat16), w, bias=b.to(cuda), mode=_lib.CONV_PARITY, transposed=True, y_dtype=torch.float32)
+    y = ops.conv3d(x.to(cuda, ACT), w, bias=b.to(cuda), mode=_lib.CONV_PARITY, transposed=True, y_dtype=torch.float32)
     _check_flag()
     _close(y, ref, what="Conv3DTranspose k4 s2")
 
@@ -169,19 +175,19 @@ def test_conv_transpose_k4s2(cuda, S, cin, cout):
 def test_up_conv_halo_kernel_bf16(cuda, S, cin, cout, transposed):
     """bf16-output x2 up-convolutions on planes that fill the 8 x 16 halo tile run conv_halo_up_kernel (CTA pairs, staged
     TMA stores through the parity maps); C_out = 32 takes the N = 32 tiles with 64-byte staged rows (the decoders' last
-    ConvT, vqgan_attn_cp.py:404-412).  Tolerance: one bf16 ulp of the output (2^-8) on top of the fp32 bound."""
+    ConvT, vqgan_attn_cp.py:404-412).  Tolerance: one output rounding (U) on top of the fp32 bound."""
     from b200dm import ops, _lib
     x = _rand((2, S, S, S, cin), 1)
     b = torch.randn(cout, generator=torch.Generator().manual_seed(3))
     if transposed:
         w = _rand((4, 4, 4, cout, cin), 2, 1.0 / np.sqrt(8 * cin))
         ref = O.conv3d_transpose(x, w, b)
-        tol = 2e-3 + 2.0 ** -8
+        tol = A + U
     else:
         w = _rand((3, 3, 3, cin, cout), 2, 1.0 / np.sqrt(27 * cin))
         ref = O.conv3d(O.upsample_nearest2(x), w, b)
-        tol = 8e-3 + 2.0 ** -8
-    y = ops.conv3d(x.to(cuda, torch.bfloat16), w, bias=b.to(cuda), mode=_lib.CONV_PARITY, transposed=transposed, y_dtype=torch.bfloat16)
+        tol = A + 3 * U   # + the folded taps' weight rounding (test_upsample_conv_parity_fold)
+    y = ops.conv3d(x.to(cuda, ACT), w, bias=b.to(cuda), mode=_lib.CONV_PARITY, transposed=transposed, y_dtype=ACT)
     _check_flag()
     assert tuple(y.shape) == tuple(ref.shape)
     _close(y, ref, tol=tol, what="x2 up-conv (halo up kernel), bf16 out")
@@ -195,8 +201,8 @@ def test_prelu_postact_epilogue(cuda):
     w = _rand((3, 3, 3, c, c), 2, 1.0 / np.sqrt(27 * c))
     alpha = _r(torch.rand(S, S, S, c, generator=torch.Generator().manual_seed(8)) * 0.3)
     ref = torch.relu(x + O.prelu(O.conv3d(h, w), alpha))
-    y = ops.conv3d(h.to(cuda, torch.bfloat16), w, prelu_alpha=alpha.to(cuda, torch.bfloat16),
-                   residual=x.to(cuda, torch.bfloat16), post_act="relu", y_dtype=torch.float32)
+    y = ops.conv3d(h.to(cuda, ACT), w, prelu_alpha=alpha.to(cuda, ACT),
+                   residual=x.to(cuda, ACT), post_act="relu", y_dtype=torch.float32)
     _check_flag()
     _close(y, ref, what="PReLU + residual + ReLU epilogue")
 
@@ -205,30 +211,30 @@ def test_batched_gemm_and_transposed_store(cuda):
     from b200dm import ops, _lib
     B, L, Cc = 2, 512, 256
     q, k = _rand((B, L, Cc), 1), _rand((B, L, Cc), 2)
-    s = ops.batched_gemm(q.to(cuda, torch.bfloat16), k.to(cuda, torch.bfloat16))
+    s = ops.batched_gemm(q.to(cuda, ACT), k.to(cuda, ACT))
     _check_flag()
     _close(s, torch.einsum("blc,bLc->blL", q, k), what="Q K^T")
     # V^T via a transposed-store 1^3 conv
     x = _rand((B, 8, 8, 8, Cc), 3)
     w = _rand((1, 1, 1, Cc, Cc), 4, 1.0 / 16)
-    desc = ops.make_conv_desc(_lib.CONV_DIRECT, B, (8, 8, 8), Cc, 0, Cc, 1, 1, y_dtype=torch.bfloat16, transposed_store=True)
+    desc = ops.make_conv_desc(_lib.CONV_DIRECT, B, (8, 8, 8), Cc, 0, Cc, 1, 1, y_dtype=ACT, transposed_store=True)
     wp = ops.pack_conv_weights(desc, w).to(cuda)
-    vt = torch.empty(B, Cc, L, dtype=torch.bfloat16, device=cuda)
+    vt = torch.empty(B, Cc, L, dtype=ACT, device=cuda)
     bv = _rand((Cc,), 6)
-    plan = ops.ConvPlan(desc, x.to(cuda, torch.bfloat16), wp, vt, bias=bv.to(cuda))
+    plan = ops.ConvPlan(desc, x.to(cuda, ACT), wp, vt, bias=bv.to(cuda))
     plan.run()
     _check_flag()
     ref = (O.conv3d(x, w) + bv).reshape(B, L, Cc).transpose(1, 2)
-    _close(vt, ref, tol=6e-3, what="transposed store (operand swap)")
+    _close(vt, ref, tol=A + U, what="transposed store (operand swap)")
     # small volume (tile spans samples): the scalar transposed path
     xs = _rand((B, 4, 4, 4, Cc), 7)
-    descs = ops.make_conv_desc(_lib.CONV_DIRECT, B, (4, 4, 4), Cc, 0, Cc, 1, 1, y_dtype=torch.bfloat16, transposed_store=True)
-    vts = torch.empty(B, Cc, 64, dtype=torch.bfloat16, device=cuda)
-    ops.ConvPlan(descs, xs.to(cuda, torch.bfloat16), ops.pack_conv_weights(descs, w).to(cuda), vts, bias=bv.to(cuda)).run()
+    descs = ops.make_conv_desc(_lib.CONV_DIRECT, B, (4, 4, 4), Cc, 0, Cc, 1, 1, y_dtype=ACT, transposed_store=True)
+    vts = torch.empty(B, Cc, 64, dtype=ACT, device=cuda)
+    ops.ConvPlan(descs, xs.to(cuda, ACT), ops.pack_conv_weights(descs, w).to(cuda), vts, bias=bv.to(cuda)).run()
     _check_flag()
-    _close(vts, (O.conv3d(xs, w) + bv).reshape(B, 64, Cc).transpose(1, 2), tol=6e-3, what="transposed store (scalar path)")
+    _close(vts, (O.conv3d(xs, w) + bv).reshape(B, 64, Cc).transpose(1, 2), tol=A + U, what="transposed store (scalar path)")
     p = _r(torch.softmax(torch.randn(B, L, L, generator=torch.Generator().manual_seed(5)), -1))
-    o = ops.batched_gemm(p.to(cuda, torch.bfloat16), vt)
+    o = ops.batched_gemm(p.to(cuda, ACT), vt)
     _check_flag()
     _close(o, torch.einsum("blL,bcL->blc", p, vt.float().cpu()), what="P V")
 
@@ -265,8 +271,8 @@ def test_conv3_halo_kernel(cuda, B, dhw, c0, c1, cout):
         desc = ops.make_conv_desc(_lib.CONV_DIRECT, B, dhw, c0, c1, cout, 3, 1, y_dtype=torch.float32, use_halo=m)
         wp = ops.pack_conv_weights(desc, w).to(cuda)
         y = torch.empty(B, D, H, W, cout, dtype=torch.float32, device=cuda)
-        ops.ConvPlan(desc, x0.to(cuda, torch.bfloat16), wp, y, x1=x1.to(cuda, torch.bfloat16) if c1 else None,
-                     bias=b.to(cuda), residual=res.to(cuda, torch.bfloat16)).run()
+        ops.ConvPlan(desc, x0.to(cuda, ACT), wp, y, x1=x1.to(cuda, ACT) if c1 else None,
+                     bias=b.to(cuda), residual=res.to(cuda, ACT)).run()
         _check_flag()
         ys[m] = y.cpu()
     d = (ys[0] - ys[-1]).abs().max().item() / ys[-1].abs().max().item()
@@ -291,7 +297,7 @@ def test_conv_out_affine_fuses_consumer_batchnorm(cuda, B, S, cin, cout, halo):
     mean, var = torch.randn(cout, generator=g) * 0.1, torch.rand(cout, generator=g) + 0.5
     ref = O.swish(O.batchnorm_infer(O.conv3d(x, w, b) + temb[:, None, None, None, :], gamma, beta, mean, var))
     sc, sh = ops.bn_fold(gamma.to(cuda), beta.to(cuda), mean.to(cuda), var.to(cuda), 1e-3)
-    y = ops.conv3d(x.to(cuda, torch.bfloat16), w, bias=b.to(cuda), chan_bias=temb.to(cuda), act="silu", out_affine=(sc, sh),
+    y = ops.conv3d(x.to(cuda, ACT), w, bias=b.to(cuda), chan_bias=temb.to(cuda), act="silu", out_affine=(sc, sh),
                    y_dtype=torch.float32, use_halo=halo)
     _check_flag()
     _close(y, ref, what=f"conv3 + temb + BN + swish fused, B{B} S{S} {cin}->{cout}")
@@ -320,7 +326,7 @@ def test_conv3_head_stencil_kernel(cuda, shape):
     _close(y, y2.float().cpu(), tol=2e-5, what="stencil vs per-tap GEMM kernel")
     y16 = ops.conv3d(xd, w, bias=b.to(cuda), act="silu")
     _check_flag()
-    _close(y16, O.swish(ref), tol=6e-3, what="stencil head + silu (16-bit out)")
+    _close(y16, O.swish(ref), tol=A + U, what="stencil head + silu (16-bit out)")
 
 
 @pytest.mark.parametrize("shape,extras", [((2, 20, 16, 8), False), ((1, 35, 24, 12), True), ((3, 9, 48, 40), True)])
@@ -349,11 +355,11 @@ def test_conv3_sweep32_kernel(cuda, shape, extras):
     ref = O.conv3d(x, w, b)
     if extras:
         ref = O.swish(ref * sc + sh) + res
-    _close(y, ref, tol=6e-3, what=f"sweep32 {shape}")
+    _close(y, ref, tol=A + U, what=f"sweep32 {shape}")
     # the same layer on the halo kernel (tuning switch off -> use_halo = -1 selects the per-tap GEMM): agree to one 16-bit ulp
     y2 = ops.conv3d(xd, w, bias=b.to(cuda), use_halo=-1, act="silu" if extras else None,
                     residual=None if res is None else res.to(cuda, L.ACT_DTYPE), out_affine=(sc.to(cuda), sh.to(cuda)) if extras else None)
-    _close(y, y2.float().cpu(), tol=8e-3, what="sweep32 vs per-tap GEMM kernel")
+    _close(y, y2.float().cpu(), tol=A + 2 * U, what="sweep32 vs per-tap GEMM kernel")
     # GroupNorm statistics from the epilogue's partial sums (of the stored values) vs a direct evaluation, 8 groups
     mr = torch.empty(B, 8, 2, dtype=torch.float32, device=cuda)
     L.check(L.lib().b200dm_gn_finalize(L.ptr(ws), B, rows, 32, 8, D * H * W, 1e-6, L.ptr(mr), L.stream()))

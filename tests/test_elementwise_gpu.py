@@ -5,13 +5,17 @@ import pytest
 import torch
 
 from oracle import ops as O, sampler as OS, philox as OP, first_stage as OF, init as OI
+from b200dm import _lib
 from oracle.schedule import Betas
 
 pytestmark = pytest.mark.gpu
 
+ACT = _lib.ACT_DTYPE
+U = 2 ** -8 if _lib.precision() == "bf16" else 2 ** -11   # unit roundoff of the storage type: its largest relative rounding error
+
 
 def _r(t):
-    return t.to(torch.bfloat16).to(torch.float32)
+    return t.to(ACT).to(torch.float32)
 
 
 @pytest.mark.parametrize("t", [999, 500, 1, 0])
@@ -32,12 +36,12 @@ def test_ddpm_update_injected_noise_bit_exact(cuda, t):
     assert err <= 4e-7 * max(1.0, ref.abs().max().item()), err
     if t == 0:
         assert torch.equal(y.cpu(), torch.clamp(OS.sample(b, x, eps, 0)[0], -1, 1))
-    # bf16 eps input + bf16 copy of the output
+    # 16-bit eps input + 16-bit copy of the output
     eb = _r(eps)
-    y2, y2b = ops.ddpm_update(tabs, x.to(cuda), eb.to(cuda, torch.bfloat16), t, noise=z.to(cuda), want_bf16=True)
+    y2, y2b = ops.ddpm_update(tabs, x.to(cuda), eb.to(cuda, ACT), t, noise=z.to(cuda), want_bf16=True)
     ref2 = OS.ddpm_step(b, x, eb, t, z)
     assert (y2.cpu() - ref2).abs().max().item() <= 4e-7 * max(1.0, ref2.abs().max().item())
-    assert torch.equal(y2b.cpu(), y2.cpu().to(torch.bfloat16))
+    assert torch.equal(y2b.cpu(), y2.cpu().to(ACT))
 
 
 def test_ddim_update(cuda):
@@ -84,9 +88,9 @@ def test_bn_act_concat(cuda, act):
     ref = O.batchnorm_infer(torch.cat([x0, x1], -1), gamma, beta, mean, var)
     ref = O.swish(ref) if act == "silu" else (torch.relu(ref) if act == "relu" else ref)
     sc, sh = ops.bn_fold(gamma.to(cuda), beta.to(cuda), mean.to(cuda), var.to(cuda), 1e-3)
-    y = ops.norm_act(x0.to(cuda, torch.bfloat16), sc, sh, act=act, x1=x1.to(cuda, torch.bfloat16))
+    y = ops.norm_act(x0.to(cuda, ACT), sc, sh, act=act, x1=x1.to(cuda, ACT))
     err = (y.float().cpu() - ref).abs().max().item()
-    assert err <= 2 ** -8 * ref.abs().max().item() + 1e-6, err
+    assert err <= U * ref.abs().max().item() + 1e-6, err
 
 
 @pytest.mark.parametrize("C,G,S", [(32, 32, 16), (64, 32, 8), (128, 32, 8), (64, 8, 8)])
@@ -97,13 +101,13 @@ def test_groupnorm_silu(cuda, C, G, S):
     x = _r(torch.randn(B, S, S, S, C, generator=g) * 2 + 0.3)
     gamma, beta = torch.rand(C, generator=g) + 0.5, torch.randn(C, generator=g) * 0.1
     ref = O.swish(O.groupnorm(x, gamma, beta, G, 1e-6))
-    xb = x.to(cuda, torch.bfloat16)
+    xb = x.to(cuda, ACT)
     mr = ops.gn_stats(xb, G, 1e-6)
     xg = x.reshape(B, -1, G, C // G)
     assert (mr[..., 0].cpu() - xg.mean(dim=(1, 3))).abs().max().item() < 1e-5
     y = ops.norm_act(xb, gamma.to(cuda), beta.to(cuda), act="silu", kind=1, groups=G, mean_rstd=mr)
     err = (y.float().cpu() - ref).abs().max().item()
-    assert err <= 2 ** -8 * ref.abs().max().item() + 1e-5, err
+    assert err <= U * ref.abs().max().item() + 1e-5, err
 
 
 def test_layernorm3(cuda):
@@ -112,10 +116,10 @@ def test_layernorm3(cuda):
     x = _r(torch.randn(2, 8, 8, 8, 256, generator=g))
     gs = [torch.rand(256, generator=g) + 0.5 for _ in range(3)]
     bs = [torch.randn(256, generator=g) * 0.1 for _ in range(3)]
-    ys = ops.layernorm(x.to(cuda, torch.bfloat16), [t.to(cuda) for t in gs], [t.to(cuda) for t in bs], 1e-3)
+    ys = ops.layernorm(x.to(cuda, ACT), [t.to(cuda) for t in gs], [t.to(cuda) for t in bs], 1e-3)
     for y, ga, be in zip(ys, gs, bs):
         ref = O.layernorm(x, ga, be)
-        assert (y.float().cpu() - ref).abs().max().item() <= 2 ** -8 * ref.abs().max().item() + 1e-5
+        assert (y.float().cpu() - ref).abs().max().item() <= U * ref.abs().max().item() + 1e-5
 
 
 def test_softmax_and_dense(cuda):
@@ -124,7 +128,7 @@ def test_softmax_and_dense(cuda):
     s = torch.randn(64, 512, generator=g) * 3
     p = ops.softmax_rows(s.to(cuda), 0.25)
     ref = torch.softmax(s * 0.25, -1)
-    assert (p.float().cpu() - ref).abs().max().item() <= 2 ** -8 * ref.max().item()
+    assert (p.float().cpu() - ref).abs().max().item() <= U * ref.max().item()
     x, w, b = torch.randn(37, 128, generator=g), torch.randn(128, 1000, generator=g) * 0.1, torch.randn(1000, generator=g)
     y = ops.dense_f32(x.to(cuda), w.to(cuda), b.to(cuda), act_in="silu", act_out="silu")
     ref = O.swish(O.dense(O.swish(x), w, b))
@@ -194,12 +198,15 @@ def test_vq_tensor_core_search_is_bit_identical(cuda, N, D, K, x16):
     x[:64] = cb[torch.randint(0, K, (64,), generator=g)]  # rows equal to codes
     x[64:96] = cb[[3, 5, 9, K // 2 + 1] * 8] + torch.randn(32, D, generator=g) * 1e-6
     x[96:128] = 0.5 * (cb[3] + cb[11]) + torch.randn(32, D, generator=g) * 1e-7   # equidistant to two codes up to noise
-    x[128:160] *= 1e-9
-    x[160:192] *= 1e9
+    # tiny / huge but finite in the input type: 1e-9 / 1e9 are 0 / inf in fp16
+    tiny, huge = (2.0 ** -12, 2.0 ** 12) if x16 and ACT == torch.float16 else (1e-9, 1e9)
+    x[128:160] *= tiny
+    x[160:192] *= huge
     x[192:200] = 0
     x[200:232] = cb[torch.randint(0, K, (32,), generator=g)] * 40   # large ||x||: fl(||x||^2 + ||e||^2) is coarse, many fp32 ties
     if x16:
-        x = x.to(L.storage(torch.bfloat16))
+        x = x.to(ACT)
+        assert torch.isfinite(x).all() and (x[128:160] != 0).any()
     (i0, q0, h0, _), (i1, q1, h1, st) = _vq_both(x, cb, cuda)
     assert L.debug_flag() == 0
     assert torch.equal(i0, i1), f"{(i0 != i1).sum().item()} of {N} indices differ (first rows {torch.nonzero(i0 != i1)[:8].flatten().tolist()})"

@@ -10,9 +10,13 @@ import numpy as np
 import pytest
 import torch
 
+from b200dm import _lib
 from oracle import init as OI, first_stage as OF
 
 pytestmark = pytest.mark.gpu
+
+ACT = _lib.ACT_DTYPE
+U = 2 ** -8 if _lib.precision() == "bf16" else 2 ** -11   # unit roundoff of the storage type: its largest relative rounding error
 
 
 def _flag_ok():
@@ -45,7 +49,9 @@ def test_cfg2_chain_is_batch_permutation_equivariant(cuda):
 @pytest.mark.parametrize("case", ["halo64", "halo128", "halo32", "halo32s", "pair", "gemm1", "down", "up", "up8", "up32"])
 def test_fullsize_convs_are_exactly_homogeneous(cuda, case):
     """y(4 x) == 4 y(x) bit for bit (no bias): every product and partial sum scales by an exact power of two, so any
-    dropped / duplicated tap, tile or K chunk at the full cfg-2 shapes shows up, without an oracle run."""
+    dropped / duplicated tap, tile or K chunk at the full cfg-2 shapes shows up, without an oracle run.  Exact where y is a
+    normal number of the storage type; a subnormal y (1 in ~2e4 outputs in fp16, none in bf16) is rounded on a grid that
+    does not scale, so 4 y(x) and y(4 x) may differ there by up to one quantum of the scaled grid."""
     from b200dm import ops, _lib
     B = 8
     cfg = dict(halo64=(32, 64, 64, 3, 1, _lib.CONV_DIRECT), halo128=(16, 128, 128, 3, 1, _lib.CONV_DIRECT),
@@ -55,13 +61,15 @@ def test_fullsize_convs_are_exactly_homogeneous(cuda, case):
                up8=(8, 256, 256, 3, 1, _lib.CONV_PARITY), up32=(32, 64, 32, 3, 1, _lib.CONV_PARITY))[case]
     S, cin, cout, k, stride, mode = cfg
     g = torch.Generator().manual_seed(1)
-    x = torch.randn(B, S, S, S, cin, generator=g).to(torch.bfloat16)
-    w = (torch.randn(k, k, k, cin, cout, generator=g) / np.sqrt(k ** 3 * cin)).to(torch.bfloat16).float()
-    y1 = ops.conv3d(x.to(cuda), w, mode=mode, stride=stride, y_dtype=torch.bfloat16).float()
-    y4 = ops.conv3d((x.float() * 4).to(torch.bfloat16).to(cuda), w, mode=mode, stride=stride, y_dtype=torch.bfloat16).float()
+    x = torch.randn(B, S, S, S, cin, generator=g).to(ACT)
+    w = (torch.randn(k, k, k, cin, cout, generator=g) / np.sqrt(k ** 3 * cin)).to(ACT).float()
+    y1 = ops.conv3d(x.to(cuda), w, mode=mode, stride=stride, y_dtype=ACT).float()
+    y4 = ops.conv3d((x.float() * 4).to(ACT).to(cuda), w, mode=mode, stride=stride, y_dtype=ACT).float()
     _flag_ok()
     assert torch.isfinite(y1).all() and y1.abs().max() > 0.1
-    assert torch.equal(y4, y1 * 4)
+    normal = y1.abs() >= torch.finfo(ACT).tiny
+    assert torch.equal(y4[normal], y1[normal] * 4)
+    assert bool(((y4 - y1 * 4).abs()[~normal] <= 4 * torch.finfo(ACT).tiny * torch.finfo(ACT).eps).all())
     # spot-check 64 output voxels against a direct fp64 evaluation of the Keras 'same' / upsample+conv definition
     xs, idx = x.float(), torch.randint(0, y1.shape[1], (64, 3), generator=g)
     for (d, h, ww) in idx.tolist():
@@ -83,7 +91,7 @@ def test_fullsize_convs_are_exactly_homogeneous(cuda, case):
                         src = xs[n, pd, ph, pw]
                     acc += src.double() @ w[kd, kh, kw].double()
         got = y1[n, d, h, ww].cpu().double()
-        assert (got - acc).abs().max() <= 2e-2 * acc.abs().max() + 1e-3, (case, d, h, ww)
+        assert (got - acc).abs().max() <= 5 * U * acc.abs().max() + 1e-3, (case, d, h, ww)
 
 
 def test_cfg3_vq_fullsize_properties(cuda):

@@ -4,7 +4,7 @@ reverse chain with injected noise -- product (CUDA, through the C ABI) vs oracle
 Tolerances (stated, and why):
   * every kernel accumulates in fp32, so on IDENTICAL inputs a layer matches the oracle to ~1e-6 (tests/test_conv_gpu.py);
     test_unet_layer_trace pins that inside the assembled network: 'in' conv rel-L2 <= 1e-5 and the first ResidualBlock
-    <= 1e-3 (4e-3 behind the fused conv1+norm2 epilogue, which skips one bf16 rounding) against the oracle that rounds to bf16 at the same storage points (Emu(True)).
+    <= 1e-3 (4e-3 behind the fused conv1+norm2 epilogue, which skips one 16-bit rounding) against the oracle that rounds to the storage type at the same storage points (emu16()).
   * activations are STORED in bf16 (north_star).  A network of ~100 bf16 storage points is chaotic at the ulp level:
     one rounding flip (4e-3 of an element) perturbs 27*C downstream sums and flips more, so after ~10 layers the
     product and the emulating oracle are decorrelated at the bf16 noise floor.  The whole-network bound is therefore
@@ -12,6 +12,8 @@ Tolerances (stated, and why):
     (measured 1.4e-2; the two oracles differ from each other by 1.5e-2 with these stress-initialised weights).
   * chain (T steps, injected noise): latents rel-L2 <= 1e-2, max-abs <= 5e-2 against the emulating oracle
     (measured 3e-3 / 1.5e-2 at T=12: the posterior update damps eps_hat error, it does not compound it).
+  * the fp16 storage build (tests/test_fp16_build_gpu.py runs this file there) has 8x smaller storage rounding: each storage-floor
+    bound is tol(bf16, fp16), the fp16 value set from the error measured in that build with the margin the bf16 bound has.
 """
 import types
 
@@ -26,6 +28,18 @@ from oracle.unet import UNet as OUNet
 from oracle import first_stage as OF
 
 pytestmark = pytest.mark.gpu
+
+
+def tol(bf16, fp16):
+    """A storage-floor bound: its value in the bf16 build and in the fp16 build (8x smaller storage rounding)."""
+    from b200dm import _lib
+    return bf16 if _lib.precision() == "bf16" else fp16
+
+
+def emu16():
+    """The oracle that rounds to the build's 16-bit storage type where the CUDA path stores."""
+    from b200dm import _lib
+    return Emu(True, dtype=_lib.ACT_DTYPE)
 
 
 def rel(a, b):
@@ -52,12 +66,12 @@ def test_unet_uncond_forward(cuda, S, C_lat, B):
         y = net([x.to(cuda), tt])
         from b200dm import _lib
         assert _lib.debug_flag() == 0
-        ref_e = ou.forward(P, x, tt, emu=Emu(True))
+        ref_e = ou.forward(P, x, tt, emu=emu16())
         ref_x = ou.forward(P, x, tt)
         r_e, r_x = rel(y, ref_e), rel(y, ref_x)
         print(f"uncond S={S} t={t}: rel-L2 vs bf16-emulating oracle {r_e:.3e}, vs fp32 oracle {r_x:.3e}")
-        assert r_e <= 2.5e-2, r_e
-        assert r_x <= 2.5e-2, r_x
+        assert r_e <= tol(2.5e-2, 3.2e-3), r_e
+        assert r_x <= tol(2.5e-2, 3.2e-3), r_x
 
 
 def test_unet_layer_trace(cuda):
@@ -69,14 +83,17 @@ def test_unet_layer_trace(cuda):
     tt = torch.full((B,), 37)
     net([x.to(cuda), tt])
     tr = {}
-    ou.forward(P, x, tt, emu=Emu(True, tr))
+    ou.forward(P, x, tt, emu=Emu(True, tr, dtype=emu16().dtype))
     errs = {k: rel(v.reshape(tr[k].shape), tr[k]) for k, v in net.prog.outputs.items() if k in tr}
-    assert errs["in"] <= 1e-5, errs["in"]
+    print("layer trace:", {k: f"{errs[k]:.2e}" for k in ("in", "down.0.res.0.norm1", "down.0.res.0.norm2", "down.0.res.0.conv2")},
+          f"max {max(errs.values()):.2e}")
+    assert errs["in"] <= tol(1e-5, 5e-5), errs["in"]   # fp16: rounding flips of the stored output (~1 in 2e3 elements)
     # conv1 -> norm2 -> swish is ONE kernel (BN applied to the fp32 accumulator): the emulating oracle rounds conv1's
     # output to bf16 first, so that tensor differs by one extra bf16 rounding (<= 2^-8 per element)
-    for k, tol in (("down.0.res.0.norm1", 1e-3), ("down.0.res.0.norm2", 4e-3), ("down.0.res.0.conv2", 4e-3)):
-        assert errs[k] <= tol, (k, errs[k])
-    assert max(errs.values()) <= 2.5e-2
+    for k, bound in (("down.0.res.0.norm1", tol(1e-3, 1e-4)), ("down.0.res.0.norm2", tol(4e-3, 5e-4)),
+                     ("down.0.res.0.conv2", tol(4e-3, 5e-4))):
+        assert errs[k] <= bound, (k, errs[k])
+    assert max(errs.values()) <= tol(2.5e-2, 3.2e-3)
 
 
 def test_unet_cond_forward(cuda):
@@ -87,11 +104,11 @@ def test_unet_cond_forward(cuda):
     ctx = torch.tensor([0, 1])
     tt = torch.full((B,), 21)
     y = net([x.to(cuda), tt, ctx])
-    ref_e = ou.forward(P, x, tt, ctx=ctx, emu=Emu(True))
+    ref_e = ou.forward(P, x, tt, ctx=ctx, emu=emu16())
     ref_x = ou.forward(P, x, tt, ctx=ctx)
     r_e, r_x = rel(y, ref_e), rel(y, ref_x)
     print(f"cond: rel-L2 vs bf16-emulating oracle {r_e:.3e}, vs fp32 oracle {r_x:.3e}")
-    assert r_e <= 2.5e-2 and r_x <= 2.5e-2
+    assert r_e <= tol(2.5e-2, 3.2e-3) and r_x <= tol(2.5e-2, 3.2e-3)
     # context must matter and be per-sample
     y2 = net([x.to(cuda), tt, torch.tensor([1, 1])])
     assert rel(y2[1:], y[1:].cpu()) < 1e-6 and rel(y2[:1], y[:1].cpu()) > 1e-4
@@ -111,12 +128,12 @@ def test_full_chain_injected_noise(cuda):
     noises = {i: OI.normal(shape, 100 + i) for i in range(1, T)}
     lat = dm.generate(shape, x_T=x_T, noise=noises)
     ob = OBetas(T)
-    emu = Emu(True)
+    emu = emu16()
     ref = OS.generate(lambda x, i: ou.forward(P, x, torch.full((B,), i), emu=emu), ob, x_T, noises=noises)
     r = rel(lat, ref)
     ma = (lat.cpu() - ref).abs().max().item()
     print(f"chain T={T}: rel-L2 {r:.3e} max-abs {ma:.3e}")
-    assert r <= 1e-2 and ma <= 5e-2, (r, ma)
+    assert r <= tol(1e-2, 1.2e-3) and ma <= tol(5e-2, 6e-3), (r, ma)
     # graph path with the Philox stream == eager path with the oracle's Philox noise injected
     lat_g = dm.generate(shape, x_T=x_T, seed=77)
     from oracle import philox
@@ -124,12 +141,14 @@ def test_full_chain_injected_noise(cuda):
     inj = {i: torch.from_numpy(philox.normal(77, i, np.arange(B), n_elem)).reshape(shape) for i in range(1, T)}
     lat_e = dm.generate(shape, x_T=x_T, noise=inj)
     # (the two noise streams agree to ~1e-6; the chain amplifies that like any other ulp-level perturbation)
-    assert rel(lat_g, lat_e.cpu()) <= 5e-3, rel(lat_g, lat_e.cpu())
+    print(f"graph + Philox vs eager + injected: rel-L2 {rel(lat_g, lat_e.cpu()):.3e}")
+    assert rel(lat_g, lat_e.cpu()) <= tol(5e-3, 8e-4), rel(lat_g, lat_e.cpu())
     # sharding invariance: sample 1 generated alone with sample_id0=1 equals row 1 of the batch
     dm1 = b200dm.DiffusionModel(S, 256, C_lat, None, args)
     dm1.network.set_weights(P)
     lat_1 = dm1.generate((1,) + shape[1:], x_T=x_T[1:], seed=77, sample_id0=1)
-    assert rel(lat_1, lat_g[1:].cpu()) <= 5e-3, rel(lat_1, lat_g[1:].cpu())
+    print(f"sample 1 alone vs in the batch: rel-L2 {rel(lat_1, lat_g[1:].cpu()):.3e}")
+    assert rel(lat_1, lat_g[1:].cpu()) <= tol(5e-3, 8e-4), rel(lat_1, lat_g[1:].cpu())
 
 
 def test_monai_decoder(cuda):
@@ -141,9 +160,9 @@ def test_monai_decoder(cuda):
     z = OI.normal((2, 4, 4, 4, 64), 11)
     y = dec(z.to(cuda))
     assert tuple(y.shape) == (2, 16, 16, 16, 1) and y.dtype == torch.float32
-    r_e, r_x = rel(y, od.forward(P, z, Emu(True))), rel(y, od.forward(P, z))
+    r_e, r_x = rel(y, od.forward(P, z, emu16())), rel(y, od.forward(P, z))
     print(f"monai decoder: rel-L2 vs emu {r_e:.3e}, vs fp32 {r_x:.3e}")
-    assert r_e <= 8e-3 and r_x <= 3e-2
+    assert r_e <= tol(8e-3, 1.2e-3) and r_x <= tol(3e-2, 4e-3)
 
 
 def test_monai_encoder_and_quantize(cuda):
@@ -157,9 +176,9 @@ def test_monai_encoder_and_quantize(cuda):
     vol = OI.normal((2, 16, 16, 16, 1), 12)
     z = enc(vol.to(cuda))
     assert tuple(z.shape) == (2, 4, 4, 4, 8) and z.dtype == torch.float32
-    r_e, r_x = rel(z, oe.forward(P, vol, Emu(True))), rel(z, oe.forward(P, vol))
+    r_e, r_x = rel(z, oe.forward(P, vol, emu16())), rel(z, oe.forward(P, vol))
     print(f"monai encoder: rel-L2 vs emu {r_e:.3e}, vs fp32 {r_x:.3e}")
-    assert r_e <= 8e-3 and r_x <= 3e-2
+    assert r_e <= tol(8e-3, 1.2e-3) and r_x <= tol(3e-2, 4e-3)
     # quantise the SAME latents on both sides: indices bit-exact (the encoder's own rounding noise is tested above)
     vq = b200dm.VectorQuantizer(64, 8, layout="DK")
     cb = OI.codebook(64, 8, "DK", seed=3)
@@ -196,9 +215,9 @@ def test_attn_cp_decoder_and_quantize(cuda):
     assert abs(perp - perp_ref.item()) <= 1e-3 * perp_ref.item()
     y = vq.decoder(q)
     assert tuple(y.shape) == (2, 16, 16, 16, 1)
-    r_e, r_x = rel(y, od.forward(P, q_ref, Emu(True))), rel(y, od.forward(P, q_ref))
+    r_e, r_x = rel(y, od.forward(P, q_ref, emu16())), rel(y, od.forward(P, q_ref))
     print(f"attn_cp decoder: rel-L2 vs emu {r_e:.3e}, vs fp32 {r_x:.3e}")
-    assert r_e <= 8e-3 and r_x <= 3e-2
+    assert r_e <= tol(8e-3, 1.2e-3) and r_x <= tol(3e-2, 4e-3)
 
 
 @pytest.mark.parametrize("variant", ["vqgan", "gnorm", "stride"])
@@ -220,9 +239,9 @@ def test_vqgan_family_decoders(cuda, variant, channels):
     from b200dm import _lib
     assert _lib.debug_flag() == 0
     assert tuple(y.shape) == (2, 16, 16, 16, 2) and y.dtype == torch.float32
-    r_e, r_x = rel(y, od.forward(P, z, Emu(True))), rel(y, od.forward(P, z))
+    r_e, r_x = rel(y, od.forward(P, z, emu16())), rel(y, od.forward(P, z))
     print(f"{variant} {channels} decoder: rel-L2 vs emu {r_e:.3e}, vs fp32 {r_x:.3e}")
-    assert r_e <= 1e-2 and r_x <= 3e-2
+    assert r_e <= tol(1e-2, 1.3e-3) and r_x <= tol(3e-2, 4e-3)
 
 
 @pytest.mark.parametrize("sampler,cond,S,C_lat,B", [("ddpm", False, 16, 128, 2), ("ddim", False, 16, 128, 2), ("ddpm", True, 32, 256, 2),

@@ -101,14 +101,17 @@ def test_folded_matches_two_launch_form(cuda, S, w, c0, c1):
 
 @pytest.mark.parametrize("S,w,c0,c1", CASES)
 def test_folded_is_exactly_homogeneous(cuda, S, w, c0, c1):
-    """y(4 h, 4 x) == 4 y(h, x) bit for bit without bias: a dropped or duplicated shortcut chunk, slab or tap shows up."""
+    """y(4 h, 4 x) == 4 y(h, x) bit for bit without bias: a dropped or duplicated shortcut chunk, slab or tap shows up.  Exact
+    where y is a normal number of the storage type; a subnormal y (fp16 only) may differ by one quantum of the scaled grid."""
     from b200dm import _lib as L
     h, x, skip, w2, wsc, _, _ = _operands(S, w, c0, c1, seed=3 * S + c0)
     four = lambda t: (t.float() * 4).to(L.ACT_DTYPE) if t is not None else None  # noqa: E731
     y1 = _folded(cuda, h, x, skip, w2, wsc, None, None)
     y4 = _folded(cuda, four(h), four(x), four(skip), w2, wsc, None, None)
     assert y1.abs().max() > 0.5
-    assert torch.equal(y4, y1 * 4)
+    normal = y1.abs() >= torch.finfo(L.ACT_DTYPE).tiny
+    assert torch.equal(y4[normal], y1[normal] * 4)
+    assert bool(((y4 - y1 * 4).abs()[~normal] <= 4 * torch.finfo(L.ACT_DTYPE).tiny * torch.finfo(L.ACT_DTYPE).eps).all())
 
 
 def test_cfg2_program_folds_every_width_change(cuda, monkeypatch):

@@ -8,9 +8,9 @@ from b200dm import ops, _lib
 B, L, D = [int(v) for v in sys.argv[1:4]]
 iters = int(sys.argv[4]) if len(sys.argv) > 4 else 10
 dev = torch.device("cuda", 0)
-q = torch.randn(B, L, D, device=dev).bfloat16()
-k = torch.randn(B, L, D, device=dev).bfloat16()
-vt = torch.randn(B, D, L, device=dev).bfloat16()
+q = torch.randn(B, L, D, device=dev).to(_lib.ACT_DTYPE)
+k = torch.randn(B, L, D, device=dev).to(_lib.ACT_DTYPE)
+vt = torch.randn(B, D, L, device=dev).to(_lib.ACT_DTYPE)
 o = torch.empty_like(q)
 plan = ops.AttnPlan(q, k, vt, o, D ** -0.5)
 for _ in range(3):
