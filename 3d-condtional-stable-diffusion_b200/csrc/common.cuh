@@ -6,6 +6,8 @@
 #include <cuda_fp16.h>
 #include <stdint.h>
 #include <stdio.h>
+#include <functional>
+#include <vector>
 #include "../../include/b200dm.h"
 
 void b200dm_set_error(const char* fmt, ...);
@@ -97,6 +99,53 @@ template <typename... KArgs, typename... Args>
 static inline cudaError_t b2_launch(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, Args... args) {
   return b2_launch_cluster(kern, grid, block, 1u, smem, s, args...);
 }
+
+// ---- bound ops ------------------------------------------------------------------------------------------------------
+// An op ready to launch: kernel launches with grid, block, dynamic shared memory and arguments fixed.  bind_X(args..., op)
+// does all of b200dm_X(args..., stream) that comes before its first launch -- argument checks (same codes and messages), grid
+// and shared-memory sizing -- without a stream; b200dm_X is bind_X + run(), and a step program records and replays the op.
+struct BoundOp {
+  std::vector<std::function<int(cudaStream_t)>> launches;   // each returns a B200DM_* code
+  int run(cudaStream_t s) const {
+    for (const auto& launch : launches)
+      if (const int rc = launch(s)) return rc;
+    B2_CHECK_LAUNCH();
+    return B200DM_OK;
+  }
+};
+
+// static: the closure may capture a kernel argument type of a .cu file's anonymous namespace
+template <typename... KArgs, typename... Args>
+static void bind_launch(BoundOp* op, void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, Args... args) {
+  op->launches.push_back([=](cudaStream_t s) -> int {
+    B2_CHECK_CUDA(b2_launch(kern, grid, block, smem, s, args...));
+    return B200DM_OK;
+  });
+}
+
+template <typename Bind, typename... Args>
+int bind_and_run(Bind bind, void* stream, Args... args) {
+  BoundOp op;
+  const int rc = bind(args..., &op);
+  return rc ? rc : op.run((cudaStream_t)stream);
+}
+
+int bind_norm_act_fwd(const b200dm_norm_desc* d, const void* x0, const void* x1, const float* a, const float* b,
+                      const float* mean_rstd, void* y, BoundOp* op);
+int bind_gn_stats(const b200dm_norm_desc* d, const void* x, float eps, float* mean_rstd, float* workspace, size_t ws_bytes, BoundOp* op);
+int bind_bn_stats(const void* x, int64_t rows, int32_t c, const float* gamma, const float* beta, float eps, float* scale,
+                  float* shift, float* workspace, size_t ws_bytes, BoundOp* op);
+int bind_gn_finalize(const float* partials, int32_t batch, int32_t rows_per_sample, int32_t c, int32_t groups,
+                     int64_t voxels_per_sample, float eps, float* mean_rstd, BoundOp* op);
+int bind_layernorm_fwd(const void* x, int64_t rows, int32_t c, float eps, int32_t n_out, const float* const* gammas,
+                       const float* const* betas, void* const* ys, BoundOp* op);
+int bind_norm_act_ex(const b200dm_norm_ex_desc* d, const void* x, const float* a, const float* b, const float* mean_rstd,
+                     const void* prelu_alpha, const void* residual, void* y, BoundOp* op);
+int bind_stats_f32(const float* x, int32_t batch, int64_t per_sample, float eps, float* mean_rstd, void* workspace, size_t ws_bytes, BoundOp* op);
+int bind_softmax_rows(const float* s, void* p_bf16, int64_t rows, int32_t cols, float scale, BoundOp* op);
+int bind_ddpm_update(const b200dm_update_desc* d, const float* x_t, const void* eps, const float* noise, float* x_prev,
+                     void* x_prev_bf16, BoundOp* op);
+int bind_step_advance(int32_t* t_dev, int32_t delta, BoundOp* op);
 
 // ---- TMA descriptors ----------------------------------------------------------------------------------------------
 // Opt-in limit of one block's dynamic shared memory on sm_100 (227 KB).

@@ -1175,12 +1175,17 @@ extern "C" int b200dm_conv_plan_set_gn_partials(b200dm_conv_plan* p, float* work
   return B200DM_OK;
 }
 
-extern "C" int b200dm_gn_finalize(const float* partials, int32_t batch, int32_t rows_per_sample, int32_t c, int32_t groups,
-                                  int64_t voxels_per_sample, float eps, float* mean_rstd, void* stream) {
+int bind_gn_finalize(const float* partials, int32_t batch, int32_t rows_per_sample, int32_t c, int32_t groups,
+                     int64_t voxels_per_sample, float eps, float* mean_rstd, BoundOp* op) {
   B2_CHECK_ARG(partials && mean_rstd && batch > 0 && rows_per_sample > 0 && c > 0 && groups > 0 && c % groups == 0 && voxels_per_sample > 0,
                "gn_finalize: bad argument");
   const double count = (double)voxels_per_sample * (c / groups);
-  B2_CHECK_CUDA(b2_launch(sweep::gn_finalize_kernel, dim3((unsigned)(batch * groups)), dim3(128), 0, (cudaStream_t)stream, partials,
-                          rows_per_sample, 1, c, groups, count, eps, mean_rstd));
+  bind_launch(op, sweep::gn_finalize_kernel, dim3((unsigned)(batch * groups)), dim3(128), 0, partials, rows_per_sample, 1, c, groups, count, eps,
+                  mean_rstd);
   return B200DM_OK;
+}
+
+extern "C" int b200dm_gn_finalize(const float* partials, int32_t batch, int32_t rows_per_sample, int32_t c, int32_t groups,
+                                  int64_t voxels_per_sample, float eps, float* mean_rstd, void* stream) {
+  return bind_and_run(bind_gn_finalize, stream, partials, batch, rows_per_sample, c, groups, voxels_per_sample, eps, mean_rstd);
 }

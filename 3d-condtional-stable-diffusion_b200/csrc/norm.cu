@@ -416,8 +416,8 @@ extern "C" size_t b200dm_gn_stats_workspace(const b200dm_norm_desc* d) {
   return (size_t)d->batch * chunks * d->groups * 2 * sizeof(float);
 }
 
-extern "C" int b200dm_gn_stats(const b200dm_norm_desc* d, const void* x, float eps, float* mean_rstd, float* workspace,
-                               size_t ws_bytes, void* stream) {
+int bind_gn_stats(const b200dm_norm_desc* d, const void* x, float eps, float* mean_rstd, float* workspace, size_t ws_bytes,
+                  BoundOp* op) {
   int rc = check_norm_desc(d, "gn_stats");
   if (rc) return rc;
   B2_CHECK_ARG(d->kind == 1 && d->c1 == 0, "gn_stats: kind must be 1 with a single source");
@@ -426,44 +426,47 @@ extern "C" int b200dm_gn_stats(const b200dm_norm_desc* d, const void* x, float e
   const int C = d->c0;
   B2_CHECK_ARG(C <= 512 && 256 % (C / 8) == 0, "gn_stats: C=%d unsupported (need C/8 to divide 256, C<=512)", C);
   const int chunks = 64;
-  cudaStream_t s = (cudaStream_t)stream;
-  B2_CHECK_CUDA(b2_launch(gn_partial_kernel<false>, dim3(chunks, d->batch), dim3(256), 0, s, (const act_t*)x, d->voxels, C, d->groups, chunks,
-                          workspace, (const float*)nullptr));
-  B2_CHECK_LAUNCH();
+  bind_launch(op, gn_partial_kernel<false>, dim3(chunks, d->batch), dim3(256), 0, (const act_t*)x, d->voxels, C, d->groups, chunks, workspace,
+                  (const float*)nullptr);
   const int tot = d->batch * d->groups;
-  B2_CHECK_CUDA(b2_launch(gn_final_kernel, dim3((tot + 127) / 128), dim3(128), 0, s, workspace, d->batch, d->groups, chunks,
-                                                    (double)d->voxels * (double)(C / d->groups), eps, mean_rstd));
-  B2_CHECK_LAUNCH();
+  bind_launch(op, gn_final_kernel, dim3((tot + 127) / 128), dim3(128), 0, workspace, d->batch, d->groups, chunks,
+                  (double)d->voxels * (double)(C / d->groups), eps, mean_rstd);
   return B200DM_OK;
+}
+
+extern "C" int b200dm_gn_stats(const b200dm_norm_desc* d, const void* x, float eps, float* mean_rstd, float* workspace,
+                               size_t ws_bytes, void* stream) {
+  return bind_and_run(bind_gn_stats, stream, d, x, eps, mean_rstd, workspace, ws_bytes);
 }
 
 extern "C" size_t b200dm_bn_stats_workspace(int32_t c) {
   return c > 0 ? ((size_t)kBnChunks * c * 2 + c) * sizeof(float) : 0;
 }
 
-extern "C" int b200dm_bn_stats(const void* x, int64_t rows, int32_t c, const float* gamma, const float* beta, float eps,
-                               float* scale, float* shift, float* workspace, size_t ws_bytes, void* stream) {
+int bind_bn_stats(const void* x, int64_t rows, int32_t c, const float* gamma, const float* beta, float eps, float* scale,
+                  float* shift, float* workspace, size_t ws_bytes, BoundOp* op) {
   B2_CHECK_ARG(x && gamma && beta && scale && shift && workspace && rows > 0, "bn_stats: bad arguments");
   B2_CHECK_ARG(c >= 8 && c <= 512 && c % 8 == 0 && 256 % (c / 8) == 0, "bn_stats: C=%d unsupported (need C/8 to divide 256, 8 <= C <= 512)", c);
   B2_CHECK_ARG(ws_bytes >= b200dm_bn_stats_workspace(c), "bn_stats: workspace too small");
-  cudaStream_t s = (cudaStream_t)stream;
   float* center = workspace + (size_t)kBnChunks * c * 2;
   const act_t* xb = (const act_t*)x;
   const dim3 fgrid((c + 127) / 128);
-  B2_CHECK_CUDA(b2_launch(gn_partial_kernel<false>, dim3(kBnChunks), dim3(256), 0, s, xb, rows, (int)c, (int)c, kBnChunks, workspace,
-                          (const float*)nullptr));
-  B2_CHECK_CUDA(b2_launch(bn_final_kernel, fgrid, dim3(128), 0, s, (const float*)workspace, (int)c, kBnChunks, (double)rows, eps, center,
-                          (const float*)nullptr, (const float*)nullptr, (float*)nullptr, (float*)nullptr));
-  B2_CHECK_CUDA(b2_launch(gn_partial_kernel<true>, dim3(kBnChunks), dim3(256), 0, s, xb, rows, (int)c, (int)c, kBnChunks, workspace,
-                          (const float*)center));
-  B2_CHECK_CUDA(b2_launch(bn_final_kernel, fgrid, dim3(128), 0, s, (const float*)workspace, (int)c, kBnChunks, (double)rows, eps, center,
-                          gamma, beta, scale, shift));
-  B2_CHECK_LAUNCH();
+  bind_launch(op, gn_partial_kernel<false>, dim3(kBnChunks), dim3(256), 0, xb, rows, (int)c, (int)c, kBnChunks, workspace, (const float*)nullptr);
+  bind_launch(op, bn_final_kernel, fgrid, dim3(128), 0, (const float*)workspace, (int)c, kBnChunks, (double)rows, eps, center,
+                  (const float*)nullptr, (const float*)nullptr, (float*)nullptr, (float*)nullptr);
+  bind_launch(op, gn_partial_kernel<true>, dim3(kBnChunks), dim3(256), 0, xb, rows, (int)c, (int)c, kBnChunks, workspace, (const float*)center);
+  bind_launch(op, bn_final_kernel, fgrid, dim3(128), 0, (const float*)workspace, (int)c, kBnChunks, (double)rows, eps, center, gamma, beta,
+                  scale, shift);
   return B200DM_OK;
 }
 
-extern "C" int b200dm_norm_act_fwd(const b200dm_norm_desc* d, const void* x0, const void* x1, const float* a,
-                                   const float* b, const float* mean_rstd, void* y, void* stream) {
+extern "C" int b200dm_bn_stats(const void* x, int64_t rows, int32_t c, const float* gamma, const float* beta, float eps,
+                               float* scale, float* shift, float* workspace, size_t ws_bytes, void* stream) {
+  return bind_and_run(bind_bn_stats, stream, x, rows, c, gamma, beta, eps, scale, shift, workspace, ws_bytes);
+}
+
+int bind_norm_act_fwd(const b200dm_norm_desc* d, const void* x0, const void* x1, const float* a, const float* b,
+                      const float* mean_rstd, void* y, BoundOp* op) {
   int rc = check_norm_desc(d, "norm_act_fwd");
   if (rc) return rc;
   B2_CHECK_ARG(x0 && a && b && y, "norm_act_fwd: null pointer");
@@ -491,15 +494,18 @@ extern "C" int b200dm_norm_act_fwd(const b200dm_norm_desc* d, const void* x0, co
     const int m = c8n / g;   // gridDim.x must be a multiple of m for the fixed-octet path
     if (m > 1 && (int64_t)gx * 256 < items) gx = (gx + m - 1) / m * m;
   }
-  B2_CHECK_CUDA(b2_launch(kern, dim3(gx, d->batch), dim3(256), 2 * C * sizeof(float), (cudaStream_t)stream,
-      *d, (const act_t*)x0, (const act_t*)x1, a, b, mean_rstd, (act_t*)y));
-  B2_CHECK_LAUNCH();
+  bind_launch(op, kern, dim3(gx, d->batch), dim3(256), 2 * C * sizeof(float), *d, (const act_t*)x0, (const act_t*)x1, a, b, mean_rstd,
+                  (act_t*)y);
   return B200DM_OK;
 }
 
-extern "C" int b200dm_layernorm_fwd(const void* x, int64_t rows, int32_t c, float eps, int32_t n_out,
-                                    const float* const* gammas, const float* const* betas, void* const* ys,
-                                    void* stream) {
+extern "C" int b200dm_norm_act_fwd(const b200dm_norm_desc* d, const void* x0, const void* x1, const float* a,
+                                   const float* b, const float* mean_rstd, void* y, void* stream) {
+  return bind_and_run(bind_norm_act_fwd, stream, d, x0, x1, a, b, mean_rstd, y);
+}
+
+int bind_layernorm_fwd(const void* x, int64_t rows, int32_t c, float eps, int32_t n_out, const float* const* gammas,
+                       const float* const* betas, void* const* ys, BoundOp* op) {
   B2_CHECK_ARG(x && rows > 0 && gammas && betas && ys, "layernorm_fwd: bad arguments");
   B2_CHECK_ARG(c > 0 && c % 8 == 0 && c <= 1024, "layernorm_fwd: C=%d unsupported (multiple of 8, <= 1024)", c);
   B2_CHECK_ARG(n_out >= 1 && n_out <= 3, "layernorm_fwd: n_out must be 1..3");
@@ -512,22 +518,27 @@ extern "C" int b200dm_layernorm_fwd(const void* x, int64_t rows, int32_t c, floa
     B2_CHECK_ARG(((uintptr_t)g[i] & 15) == 0 && ((uintptr_t)b[i] & 15) == 0, "layernorm_fwd: gamma/beta %d must be 16-byte aligned", i);
   }
   const int grid = grid_for(rows * 32, 256, 8);
-  cudaStream_t s = (cudaStream_t)stream;
-  const act_t* xb = (const act_t*)x;
-  if (c <= 256) B2_CHECK_CUDA(b2_launch(layernorm_kernel<1>, dim3(grid), dim3(256), 0, s, xb, rows, c, eps, n_out, g[0], b[0], g[1], b[1], g[2], b[2], y[0], y[1], y[2]));
-  else if (c <= 512) B2_CHECK_CUDA(b2_launch(layernorm_kernel<2>, dim3(grid), dim3(256), 0, s, xb, rows, c, eps, n_out, g[0], b[0], g[1], b[1], g[2], b[2], y[0], y[1], y[2]));
-  else B2_CHECK_CUDA(b2_launch(layernorm_kernel<4>, dim3(grid), dim3(256), 0, s, xb, rows, c, eps, n_out, g[0], b[0], g[1], b[1], g[2], b[2], y[0], y[1], y[2]));
-  B2_CHECK_LAUNCH();
+  auto kern = c <= 256 ? layernorm_kernel<1> : (c <= 512 ? layernorm_kernel<2> : layernorm_kernel<4>);
+  bind_launch(op, kern, dim3(grid), dim3(256), 0, (const act_t*)x, rows, c, eps, n_out, g[0], b[0], g[1], b[1], g[2], b[2], y[0], y[1], y[2]);
+  return B200DM_OK;
+}
+
+extern "C" int b200dm_layernorm_fwd(const void* x, int64_t rows, int32_t c, float eps, int32_t n_out,
+                                    const float* const* gammas, const float* const* betas, void* const* ys,
+                                    void* stream) {
+  return bind_and_run(bind_layernorm_fwd, stream, x, rows, c, eps, n_out, gammas, betas, ys);
+}
+
+int bind_softmax_rows(const float* s, void* p_bf16, int64_t rows, int32_t cols, float scale, BoundOp* op) {
+  B2_CHECK_ARG(s && p_bf16 && rows > 0 && cols > 0, "softmax_rows: bad arguments");
+  const int64_t cap = (int64_t)b2_num_sms() * 8;
+  const int grid = (int)(rows < cap ? rows : cap);
+  bind_launch(op, softmax_rows_kernel, dim3(grid), dim3(256), 0, s, (act_t*)p_bf16, rows, cols, scale);
   return B200DM_OK;
 }
 
 extern "C" int b200dm_softmax_rows(const float* s, void* p_bf16, int64_t rows, int32_t cols, float scale, void* stream) {
-  B2_CHECK_ARG(s && p_bf16 && rows > 0 && cols > 0, "softmax_rows: bad arguments");
-  const int64_t cap = (int64_t)b2_num_sms() * 8;
-  const int grid = (int)(rows < cap ? rows : cap);
-  B2_CHECK_CUDA(b2_launch(softmax_rows_kernel, dim3(grid), dim3(256), 0, (cudaStream_t)stream, s, (act_t*)p_bf16, rows, cols, scale));
-  B2_CHECK_LAUNCH();
-  return B200DM_OK;
+  return bind_and_run(bind_softmax_rows, stream, s, p_bf16, rows, cols, scale);
 }
 
 extern "C" int b200dm_cast(const void* x, int32_t x_dtype, void* y, int32_t y_dtype, int64_t n, void* stream) {

@@ -154,8 +154,8 @@ static int check_ex(const b200dm_norm_ex_desc* d, const char* who) {
   return B200DM_OK;
 }
 
-extern "C" int b200dm_norm_act_ex(const b200dm_norm_ex_desc* d, const void* x, const float* a, const float* b,
-                                  const float* mean_rstd, const void* prelu_alpha, const void* residual, void* y, void* stream) {
+int bind_norm_act_ex(const b200dm_norm_ex_desc* d, const void* x, const float* a, const float* b, const float* mean_rstd,
+                     const void* prelu_alpha, const void* residual, void* y, BoundOp* op) {
   int rc = check_ex(d, "norm_act_ex");
   if (rc) return rc;
   B2_CHECK_ARG(x && a && b && y, "norm_act_ex: null pointer");
@@ -172,21 +172,29 @@ extern "C" int b200dm_norm_act_ex(const b200dm_norm_ex_desc* d, const void* x, c
   const int64_t cap = (int64_t)b2_num_sms() * 8;
   int gx = (int)((want < cap ? want : cap) / d->batch);
   if (gx < 1) gx = 1;
-  cudaStream_t s = (cudaStream_t)stream;
-  if (vec) B2_CHECK_CUDA(b2_launch(norm_ex_vec_kernel, dim3(gx, d->batch), dim3(256), 2 * d->c * sizeof(float), s, p));
-  else B2_CHECK_CUDA(b2_launch(norm_ex_scalar_kernel, dim3(gx, d->batch), dim3(256), 0, s, p));
+  if (vec) bind_launch(op, norm_ex_vec_kernel, dim3(gx, d->batch), dim3(256), 2 * d->c * sizeof(float), p);
+  else bind_launch(op, norm_ex_scalar_kernel, dim3(gx, d->batch), dim3(256), 0, p);
   return B200DM_OK;
+}
+
+extern "C" int b200dm_norm_act_ex(const b200dm_norm_ex_desc* d, const void* x, const float* a, const float* b,
+                                  const float* mean_rstd, const void* prelu_alpha, const void* residual, void* y, void* stream) {
+  return bind_and_run(bind_norm_act_ex, stream, d, x, a, b, mean_rstd, prelu_alpha, residual, y);
 }
 
 extern "C" size_t b200dm_stats_f32_workspace(int32_t batch) { return (size_t)batch * kStatChunks * 2 * sizeof(double); }
 
-extern "C" int b200dm_stats_f32(const float* x, int32_t batch, int64_t per_sample, float eps, float* mean_rstd, void* workspace,
-                                size_t ws_bytes, void* stream) {
+int bind_stats_f32(const float* x, int32_t batch, int64_t per_sample, float eps, float* mean_rstd, void* workspace,
+                   size_t ws_bytes, BoundOp* op) {
   B2_CHECK_ARG(x && mean_rstd && workspace && batch > 0 && per_sample > 0, "stats_f32: bad argument");
   B2_CHECK_ARG(ws_bytes >= b200dm_stats_f32_workspace(batch), "stats_f32: workspace too small");
-  cudaStream_t s = (cudaStream_t)stream;
-  B2_CHECK_CUDA(b2_launch(stats_f32_partial_kernel, dim3(kStatChunks, batch), dim3(256), 0, s, x, per_sample, kStatChunks, (double*)workspace));
-  B2_CHECK_CUDA(b2_launch(stats_f32_final_kernel, dim3((batch + 63) / 64), dim3(64), 0, s, (const double*)workspace, batch, kStatChunks,
-                          (double)per_sample, eps, mean_rstd));
+  bind_launch(op, stats_f32_partial_kernel, dim3(kStatChunks, batch), dim3(256), 0, x, per_sample, kStatChunks, (double*)workspace);
+  bind_launch(op, stats_f32_final_kernel, dim3((batch + 63) / 64), dim3(64), 0, (const double*)workspace, batch, kStatChunks,
+                  (double)per_sample, eps, mean_rstd);
   return B200DM_OK;
+}
+
+extern "C" int b200dm_stats_f32(const float* x, int32_t batch, int64_t per_sample, float eps, float* mean_rstd, void* workspace,
+                                size_t ws_bytes, void* stream) {
+  return bind_and_run(bind_stats_f32, stream, x, batch, per_sample, eps, mean_rstd, workspace, ws_bytes);
 }

@@ -184,8 +184,8 @@ __global__ void step_advance_seq_kernel(int32_t* t_dev, const int32_t* __restric
 
 }  // namespace
 
-extern "C" int b200dm_ddpm_update(const b200dm_update_desc* d, const float* x_t, const void* eps,
-                                  const float* noise, float* x_prev, void* x_prev_bf16, void* stream) {
+int bind_ddpm_update(const b200dm_update_desc* d, const float* x_t, const void* eps, const float* noise, float* x_prev,
+                     void* x_prev_bf16, BoundOp* op) {
   B2_CHECK_ARG(d && x_t && eps && x_prev, "ddpm_update: null argument");
   B2_CHECK_ARG(d->n_per_sample > 0 && d->n_per_sample % 8 == 0, "ddpm_update: n_per_sample must be a positive multiple of 8");
   B2_CHECK_ARG(d->batch > 0, "ddpm_update: batch must be > 0");
@@ -198,13 +198,14 @@ extern "C" int b200dm_ddpm_update(const b200dm_update_desc* d, const float* x_t,
   int64_t cap = ((int64_t)b2_num_sms() * 4 + d->batch - 1) / d->batch;   // one resident wave: 4 blocks per SM (62 registers)
   if (cap < 1) cap = 1;
   const dim3 grid((unsigned)(want < cap ? want : cap), (unsigned)d->batch);
-  cudaStream_t s = (cudaStream_t)stream;
-  if (d->eps_dtype == B200DM_BF16)
-    B2_CHECK_CUDA(b2_launch(update_kernel<true>, grid, dim3(256), 0, s, *d, x_t, eps, noise, x_prev, (act_t*)x_prev_bf16));
-  else
-    B2_CHECK_CUDA(b2_launch(update_kernel<false>, grid, dim3(256), 0, s, *d, x_t, eps, noise, x_prev, (act_t*)x_prev_bf16));
-  B2_CHECK_LAUNCH();
+  bind_launch(op, d->eps_dtype == B200DM_BF16 ? update_kernel<true> : update_kernel<false>, grid, dim3(256), 0, *d, x_t, eps, noise, x_prev,
+                  (act_t*)x_prev_bf16);
   return B200DM_OK;
+}
+
+extern "C" int b200dm_ddpm_update(const b200dm_update_desc* d, const float* x_t, const void* eps,
+                                  const float* noise, float* x_prev, void* x_prev_bf16, void* stream) {
+  return bind_and_run(bind_ddpm_update, stream, d, x_t, eps, noise, x_prev, x_prev_bf16);
 }
 
 extern "C" int b200dm_philox_normal(float* x, void* x_bf16, int64_t n_per_sample, int32_t batch, uint64_t seed,
@@ -226,11 +227,14 @@ extern "C" int b200dm_step_advance_seq(int32_t* t_dev, const int32_t* seq, void*
   return B200DM_OK;
 }
 
-extern "C" int b200dm_step_advance(int32_t* t_dev, int32_t delta, void* stream) {
+int bind_step_advance(int32_t* t_dev, int32_t delta, BoundOp* op) {
   B2_CHECK_ARG(t_dev, "step_advance: null t_dev");
-  B2_CHECK_CUDA(b2_launch(step_advance_kernel, dim3(1), dim3(1), 0, (cudaStream_t)stream, t_dev, delta));
-  B2_CHECK_LAUNCH();
+  bind_launch(op, step_advance_kernel, dim3(1), dim3(1), 0, t_dev, delta);
   return B200DM_OK;
+}
+
+extern "C" int b200dm_step_advance(int32_t* t_dev, int32_t delta, void* stream) {
+  return bind_and_run(bind_step_advance, stream, t_dev, delta);
 }
 
 extern "C" int b200dm_q_sample(const float* z, const float* sqrt_alpha_bar, const float* sqrt_one_minus_alpha_bar,

@@ -332,6 +332,9 @@ double b200dm_attention_plan_flops(const b200dm_attn_plan* p);
 /* ---------------------------------------------------------------------------------------------
  * Step program: an ordered list of the above ops with fixed buffers, launched natively in one
  * call (one ctypes crossing per U-Net forward instead of ~250), CUDA-graph capturable.
+ * Every op is checked and sized when it is recorded: add_X returns the code and b200dm_last_error() text that the
+ * direct entry point X returns for the same arguments, and records nothing on error (add_conv / add_attention take
+ * the plan only on success).  run / run_timed replay the recorded launches and fail only on a CUDA error.
  * --------------------------------------------------------------------------------------------- */
 typedef struct b200dm_program b200dm_program;
 int b200dm_program_create(b200dm_program** out);
