@@ -135,7 +135,7 @@ int bind_norm_act_fwd(const b200dm_norm_desc* d, const void* x0, const void* x1,
 int bind_gn_stats(const b200dm_norm_desc* d, const void* x, float eps, float* mean_rstd, float* workspace, size_t ws_bytes, BoundOp* op);
 int bind_bn_stats(const void* x, int64_t rows, int32_t c, const float* gamma, const float* beta, float eps, float* scale,
                   float* shift, float* workspace, size_t ws_bytes, BoundOp* op);
-int bind_gn_finalize(const float* partials, int32_t batch, int32_t rows_per_sample, int32_t c, int32_t groups,
+int bind_gn_finalize(const double* partials, int32_t batch, int32_t rows_per_sample, int32_t c, int32_t groups,
                      int64_t voxels_per_sample, float eps, float* mean_rstd, BoundOp* op);
 int bind_layernorm_fwd(const void* x, int64_t rows, int32_t c, float eps, int32_t n_out, const float* const* gammas,
                        const float* const* betas, void* const* ys, BoundOp* op);

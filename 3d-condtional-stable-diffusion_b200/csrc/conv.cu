@@ -1158,16 +1158,17 @@ extern "C" int b200dm_conv_plan_set_out_affine(b200dm_conv_plan* p, const float*
 }
 
 // GroupNorm statistics as a by-product of the producing conv (d-sweeping kernel only): the epilogue accumulates per-(item, channel)
-// partial sums of the STORED values into `workspace` (float [rows][C][2], rows = batch * rows_per_sample); b200dm_gn_finalize
+// partial sums of the STORED values into `workspace` (double [rows][C][2], rows = batch * rows_per_sample); b200dm_gn_finalize
 // turns them into (mean, rstd) in a fixed order.  Returns the workspace size, 0 when the plan cannot produce partials.
 extern "C" size_t b200dm_conv_plan_gn_partials_bytes(const b200dm_conv_plan* p, int32_t* rows_per_sample) {
   if (!p || p->v.key.family != Family::kSweep) return 0;
   if (rows_per_sample) *rows_per_sample = p->wp.items / p->wp.batch * 2;
-  return (size_t)p->wp.items * 2 * 32 * 2 * sizeof(float);
+  return (size_t)p->wp.items * 2 * 32 * 2 * sizeof(double);
 }
 
-extern "C" int b200dm_conv_plan_set_gn_partials(b200dm_conv_plan* p, float* workspace, size_t ws_bytes) {
+extern "C" int b200dm_conv_plan_set_gn_partials(b200dm_conv_plan* p, double* workspace, size_t ws_bytes) {
   B2_CHECK_ARG(p && workspace, "conv_plan_set_gn_partials: null argument");
+  B2_CHECK_ARG(((uintptr_t)workspace & 7) == 0, "conv_plan_set_gn_partials: workspace must be 8-byte aligned");
   const size_t need = b200dm_conv_plan_gn_partials_bytes(p, nullptr);
   if (need == 0) { b200dm_set_error("conv_plan_set_gn_partials: this plan cannot produce GroupNorm partial sums"); return B200DM_ERR_UNSUPPORTED; }
   B2_CHECK_ARG(ws_bytes >= need, "conv_plan_set_gn_partials: workspace too small (%zu < %zu)", ws_bytes, need);
@@ -1175,7 +1176,7 @@ extern "C" int b200dm_conv_plan_set_gn_partials(b200dm_conv_plan* p, float* work
   return B200DM_OK;
 }
 
-int bind_gn_finalize(const float* partials, int32_t batch, int32_t rows_per_sample, int32_t c, int32_t groups,
+int bind_gn_finalize(const double* partials, int32_t batch, int32_t rows_per_sample, int32_t c, int32_t groups,
                      int64_t voxels_per_sample, float eps, float* mean_rstd, BoundOp* op) {
   B2_CHECK_ARG(partials && mean_rstd && batch > 0 && rows_per_sample > 0 && c > 0 && groups > 0 && c % groups == 0 && voxels_per_sample > 0,
                "gn_finalize: bad argument");
@@ -1185,7 +1186,7 @@ int bind_gn_finalize(const float* partials, int32_t batch, int32_t rows_per_samp
   return B200DM_OK;
 }
 
-extern "C" int b200dm_gn_finalize(const float* partials, int32_t batch, int32_t rows_per_sample, int32_t c, int32_t groups,
+extern "C" int b200dm_gn_finalize(const double* partials, int32_t batch, int32_t rows_per_sample, int32_t c, int32_t groups,
                                   int64_t voxels_per_sample, float eps, float* mean_rstd, void* stream) {
   return bind_and_run(bind_gn_finalize, stream, partials, batch, rows_per_sample, c, groups, voxels_per_sample, eps, mean_rstd);
 }

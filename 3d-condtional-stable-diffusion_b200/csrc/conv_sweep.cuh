@@ -35,12 +35,12 @@ constexpr int kR = 16;                      // TMEM ring: 16 slots x 32 columns 
 constexpr int kWBytes = 27 * 2048;          // [kh*3+kw][kd][32 co][32 ci] bf16, one 2 KB SWIZZLE_64B tile per tap
 constexpr int kStgBytes = 8192;             // one plane tile: 128 rows x 64 B
 constexpr size_t kSmem = 1024 + (size_t)kNS * kSlabBytes + kWBytes + 4 * kStgBytes + (2 * kNS + 1 + 2 * kR + 2) * 8 + 8 + 2 * 32 * 4 +
-                         2 * 4 * 2 * 32 * 4;
+                         2 * 4 * 2 * 32 * 4 + 2 * 32 * 4;
 
 struct Params {
   int D, H, W, batch;
   int tiles_w, tiles_h, dsplit, dlen, items;
-  float* gn_part;   // optional [items][2 groups][32 channels][2] partial (sum, sum of squares) of the STORED values, else null
+  double* gn_part;   // optional [items][2 groups][32 channels][2] partial (sum, sum of squares) of the STORED values, else null
 };
 
 struct Item { int n, h0, w0, d0, d1; };
@@ -108,6 +108,7 @@ conv_sweep32_kernel(const __grid_constant__ CUtensorMap mapX, const __grid_const
   uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(bars + 2 * kNS + 1 + 2 * kR + 2);
   float* bias_s = reinterpret_cast<float*>(tmem_ptr_smem + 2);   // [bias | scale][32] (16-byte aligned)
   float* red_s = bias_s + 64;                                     // [group][quarter][half][16 columns][2]
+  float* piv_s = red_s + 2 * 4 * 2 * 32;                          // [group][32 channels]: GroupNorm pivots of the current item
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const uint32_t slab_base = ptx::smem_u32(smem), w_base = ptx::smem_u32(w_s), bar_base = ptx::smem_u32(bars);
@@ -257,6 +258,7 @@ conv_sweep32_kernel(const __grid_constant__ CUtensorMap mapX, const __grid_const
       const int ow = it.w0 + iw, oh = it.h0 + ih;
       const bool inb = ow < q.W && oh < q.H;
       float sacc = 0.f;   // GroupNorm partial of (channel, statistic) pair `lane` over this warp's rows and planes (see below)
+      bool first = true;  // this group's first plane of the item: its row 0 (always inside the volume) gives the pivots
       for (int pq = 0; pq < nout && ok; ++pq) {
         const uint32_t G = gbase + (uint32_t)pq;
         if ((int)(G & 1) != e) continue;
@@ -310,26 +312,14 @@ conv_sweep32_kernel(const __grid_constant__ CUtensorMap mapX, const __grid_const
           apply_act_vec(v, p.post_act);
         }
         const bf16x8 o0 = pack8(*reinterpret_cast<float(*)[8]>(&v[0])), o1 = pack8(*reinterpret_cast<float(*)[8]>(&v[8]));
-        if (q.gn_part) {
-          // GroupNorm statistics of the tensor as STORED (rounded).  32 values per row (16 sums, 16 squares) are reduce-SCATTERED
-          // over the warp's 32 rows: after 5 exchange steps (16 + 8 + 4 + 2 + 1 shuffles) lane L holds the total of value L, so the
-          // running sums take ONE register per thread instead of 32 (640 threads share the register file).
-          float w[32];
+        if (q.gn_part && first && r == 0) {
+          float w[16];
           unpack8(o0, *reinterpret_cast<float(*)[8]>(&w[0]));
           unpack8(o1, *reinterpret_cast<float(*)[8]>(&w[8]));
 #pragma unroll
-          for (int j = 0; j < 16; ++j) { w[j] = inb ? w[j] : 0.f; w[16 + j] = w[j] * w[j]; }
-#pragma unroll
-          for (int o = 16; o >= 1; o >>= 1) {
-            const bool up = (lane & o) != 0;
-#pragma unroll
-            for (int j = 0; j < o; ++j) {
-              const float send = up ? w[j] : w[j + o], keep = up ? w[j + o] : w[j];
-              w[j] = keep + __shfl_xor_sync(0xffffffffu, send, o);
-            }
-          }
-          sacc += w[0];
+          for (int j = 0; j < 16; ++j) piv_s[e * 32 + 16 * half + j] = w[j];   // read after the group barrier below
         }
+        first = false;
         if (!res) {   // (with a residual the buffer was claimed before its tile was loaded, and every thread has seen that load land)
           if (gtid == 0) ptx::bulk_wait_read_1();   // the store that last used this buffer has finished reading it
           group_bar_sync(e);
@@ -342,6 +332,28 @@ conv_sweep32_kernel(const __grid_constant__ CUtensorMap mapX, const __grid_const
           ptx::tma_store_5d(&mapY, ptx::smem_u32(stg), 0, it.w0, it.h0, od, it.n);
           ptx::bulk_commit_group();
         }
+        if (q.gn_part) {
+          // GroupNorm statistics of the tensor as STORED (rounded), as sums of d = y - K[channel] (pivots of this item, so the fp32
+          // sums do not carry the channel's offset: see gn_partial_kernel).  32 values per row (16 sums, 16 squares) are reduce-SCATTERED
+          // over the warp's 32 rows: after 5 exchange steps (16 + 8 + 4 + 2 + 1 shuffles) lane L holds the total of value L, so the
+          // running sums take ONE register per thread instead of 32 (640 threads share the register file).
+          float w[32];
+          unpack8(o0, *reinterpret_cast<float(*)[8]>(&w[0]));
+          unpack8(o1, *reinterpret_cast<float(*)[8]>(&w[8]));
+          const float* pv = piv_s + e * 32 + 16 * half;
+#pragma unroll
+          for (int j = 0; j < 16; ++j) { w[j] = inb ? w[j] - pv[j] : 0.f; w[16 + j] = w[j] * w[j]; }
+#pragma unroll
+          for (int o = 16; o >= 1; o >>= 1) {
+            const bool up = (lane & o) != 0;
+#pragma unroll
+            for (int j = 0; j < o; ++j) {
+              const float send = up ? w[j] : w[j + o], keep = up ? w[j + o] : w[j];
+              w[j] = keep + __shfl_xor_sync(0xffffffffu, send, o);
+            }
+          }
+          sacc += w[0];
+        }
         if (trw) trace_ev(p, 1, ti, 12);
         ++nstore;
       }
@@ -349,12 +361,20 @@ conv_sweep32_kernel(const __grid_constant__ CUtensorMap mapX, const __grid_const
         // column sums of this group's planes: 4 lane quarters -> shared memory -> one value per (channel, statistic), fixed order
         red_s[((e * 4 + qd) * 2 + half) * 32 + lane] = sacc;   // lane < 16: sum of channel 16*half + lane; else sum of squares
         group_bar_sync(e);
-        if (gtid < 64) {   // (channel, stat) pair gtid: channel = gtid / 2
+        if (gtid < 64) {   // (channel, stat) pair gtid: channel = gtid / 2; fp64 (sum, sum of squares) of y rebuilt from the pivot
           const int c = gtid >> 1, st = gtid & 1, hf = c >> 4, cj = c & 15;
-          float acc = 0.f;
+          float s1 = 0.f, s2 = 0.f;
 #pragma unroll
-          for (int k = 0; k < 4; ++k) acc += red_s[((e * 4 + k) * 2 + hf) * 32 + cj + 16 * st];
-          q.gn_part[(((size_t)item * 2 + e) * 32 + c) * 2 + st] = acc;
+          for (int k = 0; k < 4; ++k) {
+            s1 += red_s[((e * 4 + k) * 2 + hf) * 32 + cj];
+            s2 += red_s[((e * 4 + k) * 2 + hf) * 32 + cj + 16];
+          }
+          const int f = (e - (int)gbase) & 1;                      // this group's first plane of the item
+          const int planes = nout > f ? (nout - f + 1) >> 1 : 0;
+          const double cnt = (double)planes * min(8, q.W - it.w0) * min(16, q.H - it.h0);
+          const double K = planes ? (double)piv_s[e * 32 + c] : 0.0;
+          q.gn_part[(((size_t)item * 2 + e) * 32 + c) * 2 + st] =
+              st ? cnt * K * K + 2.0 * K * (double)s1 + (double)s2 : cnt * K + (double)s1;
         }
         group_bar_sync(e);
       }
@@ -369,7 +389,7 @@ conv_sweep32_kernel(const __grid_constant__ CUtensorMap mapX, const __grid_const
 
 // mean / rstd of GroupNorm from the conv's per-item partial sums: one block per (sample, group), fixed summation order
 // (items ascending, then channels) in double precision -> the chain stays bit-reproducible.
-__global__ void __launch_bounds__(128) gn_finalize_kernel(const float* __restrict__ part, int items_per_sample, int parts, int C,
+__global__ void __launch_bounds__(128) gn_finalize_kernel(const double* __restrict__ part, int items_per_sample, int parts, int C,
                                                           int groups, double count, float eps, float* __restrict__ mean_rstd) {
   pdl_launch_dependents();
   pdl_wait();
@@ -378,8 +398,8 @@ __global__ void __launch_bounds__(128) gn_finalize_kernel(const float* __restric
   double a = 0.0, b = 0.0;
   const int rows = items_per_sample * parts;
   for (int i = threadIdx.x; i < rows; i += 128) {
-    const float* pr = part + (((size_t)n * rows + i) * C + (size_t)g * cpg) * 2;
-    for (int c = 0; c < cpg; ++c) { a += (double)pr[2 * c]; b += (double)pr[2 * c + 1]; }
+    const double* pr = part + (((size_t)n * rows + i) * C + (size_t)g * cpg) * 2;
+    for (int c = 0; c < cpg; ++c) { a += pr[2 * c]; b += pr[2 * c + 1]; }
   }
   s_sum[threadIdx.x] = a; s_sq[threadIdx.x] = b;
   __syncthreads();

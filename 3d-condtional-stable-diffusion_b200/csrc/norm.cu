@@ -118,10 +118,16 @@ __global__ void __launch_bounds__(256, 4) norm_act_kernel(b200dm_norm_desc d, co
 // grid = (chunks, batch).  Thread (row r, octet o) keeps per-channel sum / sumsq for its octet over
 // voxels r, r+R, ... of the block's chunk; the block reduces in a fixed order and writes one
 // (sum, sumsq) pair per group to partial[n][chunk][g].  gn_final combines chunks in fp64.
-// kCentered: the sums are of x - center[c] (BatchNorm's second pass, groups == C; see bn_final_kernel).
-template <bool kCentered>
+// kSums: float sums of x (BatchNorm's first pass, groups == C).
+// kCentered: float sums of x - center[c] (BatchNorm's second pass, groups == C; see bn_final_kernel).
+// kPivot (GroupNorm): the fp32 sums are of d = x - K_g, K_g the chunk's first value of group g's first channel, so they never
+// carry the group's offset; the block writes the fp64 sums of x rebuilt from them, sum x = n K + sum d and
+// sum x^2 = n K^2 + 2 K sum d + sum d^2 (products of a 16-bit K and fp32 sums: exact in fp64), into double partial[n][chunk][g][2].
+// One-pass fp32 sums of x and x^2 would cancel in var = E[x^2] - E[x]^2 once |mean| >> std (at 150 std in fp16: 4e-3 of rstd).
+enum GnSums { kSums, kCentered, kPivot };
+template <int kMode>
 __global__ void __launch_bounds__(256) gn_partial_kernel(const act_t* __restrict__ x, int64_t voxels, int C,
-                                                         int groups, int chunks, float* __restrict__ partial,
+                                                         int groups, int chunks, void* __restrict__ partial,
                                                          const float* __restrict__ center) {
   pdl_launch_dependents();
   pdl_wait();
@@ -140,17 +146,39 @@ __global__ void __launch_bounds__(256) gn_partial_kernel(const act_t* __restrict
   const act_t* xs = x + (int64_t)n * voxels * C + (o << 3);
   float k[8];
 #pragma unroll
-  for (int i = 0; i < 8; ++i) k[i] = kCentered ? center[(o << 3) + i] : 0.f;
+  for (int i = 0; i < 8; ++i) k[i] = kMode == kCentered ? center[(o << 3) + i] : 0.f;
+  if (kMode == kPivot && v0 < v1) {
+    const int cg = C / groups;
+#pragma unroll
+    for (int i = 0; i < 8; ++i) k[i] = act_to_float(xs[v0 * C - (o << 3) + ((o << 3) + i) / cg * cg]);
+  }
   if (r < rows) {
-    for (int64_t v = v0 + r; v < v1; v += rows) {
-      float f[8];
-      unpack8(*reinterpret_cast<const bf16x8*>(xs + v * C), f);
-      if (kCentered) {
+    if constexpr (kMode == kPivot) {
+      // the 8 pivots cost a resident block per SM (48 registers instead of 40): two loads in flight per thread make up for it
+      for (int64_t v = v0 + r; v < v1; v += 2 * rows) {
+        bf16x8 pk[2];
+        pk[0] = *reinterpret_cast<const bf16x8*>(xs + v * C);
+        if (v + rows < v1) pk[1] = *reinterpret_cast<const bf16x8*>(xs + (v + rows) * C);
 #pragma unroll
-        for (int i = 0; i < 8; ++i) f[i] -= k[i];
+        for (int u = 0; u < 2; ++u) {
+          if (v + u * rows >= v1) break;
+          float f[8];
+          unpack8(pk[u], f);
+#pragma unroll
+          for (int i = 0; i < 8; ++i) { f[i] -= k[i]; s[i] += f[i]; q[i] = fmaf(f[i], f[i], q[i]); }
+        }
       }
+    } else {
+      for (int64_t v = v0 + r; v < v1; v += rows) {
+        float f[8];
+        unpack8(*reinterpret_cast<const bf16x8*>(xs + v * C), f);
+        if (kMode == kCentered) {
 #pragma unroll
-      for (int i = 0; i < 8; ++i) { s[i] += f[i]; q[i] = fmaf(f[i], f[i], q[i]); }
+          for (int i = 0; i < 8; ++i) f[i] -= k[i];
+        }
+#pragma unroll
+        for (int i = 0; i < 8; ++i) { s[i] += f[i]; q[i] = fmaf(f[i], f[i], q[i]); }
+      }
     }
   }
 #pragma unroll
@@ -170,12 +198,21 @@ __global__ void __launch_bounds__(256) gn_partial_kernel(const act_t* __restrict
   for (int g = threadIdx.x; g < groups; g += blockDim.x) {
     float a = 0.f, b = 0.f;
     for (int c = g * cg; c < (g + 1) * cg; ++c) { a += csum[c]; b += csq[c]; }
-    float* p = partial + (((int64_t)n * chunks + chunk) * groups + g) * 2;
-    p[0] = a; p[1] = b;
+    const int64_t i = ((int64_t)n * chunks + chunk) * groups + g;
+    if (kMode == kPivot) {
+      const double cnt = v0 < v1 ? (double)(v1 - v0) * cg : 0.0;
+      const double K = v0 < v1 ? (double)act_to_float(xs[v0 * C - (o << 3) + g * cg]) : 0.0;
+      double* p = static_cast<double*>(partial) + i * 2;
+      p[0] = cnt * K + (double)a;
+      p[1] = cnt * K * K + 2.0 * K * (double)a + (double)b;
+    } else {
+      float* p = static_cast<float*>(partial) + i * 2;
+      p[0] = a; p[1] = b;
+    }
   }
 }
 
-__global__ void gn_final_kernel(const float* __restrict__ partial, int batch, int groups, int chunks, double count,
+__global__ void gn_final_kernel(const double* __restrict__ partial, int batch, int groups, int chunks, double count,
                                 float eps, float* __restrict__ mean_rstd) {
   pdl_launch_dependents();
   pdl_wait();
@@ -184,8 +221,8 @@ __global__ void gn_final_kernel(const float* __restrict__ partial, int batch, in
   const int n = i / groups, g = i % groups;
   double a = 0.0, b = 0.0;
   for (int c = 0; c < chunks; ++c) {
-    const float* p = partial + (((int64_t)n * chunks + c) * groups + g) * 2;
-    a += (double)p[0]; b += (double)p[1];
+    const double* p = partial + (((int64_t)n * chunks + c) * groups + g) * 2;
+    a += p[0]; b += p[1];
   }
   const double mean = a / count;
   double var = b / count - mean * mean;
@@ -195,7 +232,7 @@ __global__ void gn_final_kernel(const float* __restrict__ partial, int batch, in
 }
 
 // BatchNormalization with batch statistics (training=True): per-channel mean and biased variance over all B*D*H*W rows,
-// from gn_partial_kernel's per-chunk sums with groups == C, combined in fixed chunk order in fp64 (bit-reproducible).
+// from gn_partial_kernel's per-chunk float sums with groups == C, combined in fixed chunk order in fp64 (bit-reproducible).
 // Two passes over x: pass 1 (scale == nullptr) writes center[c] = mean; pass 2 gets the sums of d = x - center and
 // forms var = E[d^2] - E[d]^2 -- the corrected two-pass form, so a channel whose |mean| >> std loses nothing to
 // cancellation -- then scale = gamma * rsqrt(var + eps), shift = beta - mean * scale: the coefficients norm_act_kernel
@@ -413,7 +450,7 @@ static int check_norm_desc(const b200dm_norm_desc* d, const char* who) {
 extern "C" size_t b200dm_gn_stats_workspace(const b200dm_norm_desc* d) {
   if (!d || d->groups <= 0) return 0;
   const int chunks = 64;
-  return (size_t)d->batch * chunks * d->groups * 2 * sizeof(float);
+  return (size_t)d->batch * chunks * d->groups * 2 * sizeof(double);
 }
 
 int bind_gn_stats(const b200dm_norm_desc* d, const void* x, float eps, float* mean_rstd, float* workspace, size_t ws_bytes,
@@ -422,14 +459,15 @@ int bind_gn_stats(const b200dm_norm_desc* d, const void* x, float eps, float* me
   if (rc) return rc;
   B2_CHECK_ARG(d->kind == 1 && d->c1 == 0, "gn_stats: kind must be 1 with a single source");
   B2_CHECK_ARG(x && mean_rstd && workspace, "gn_stats: null pointer");
+  B2_CHECK_ARG(((uintptr_t)workspace & 7) == 0, "gn_stats: workspace must be 8-byte aligned");
   B2_CHECK_ARG(ws_bytes >= b200dm_gn_stats_workspace(d), "gn_stats: workspace too small");
   const int C = d->c0;
   B2_CHECK_ARG(C <= 512 && 256 % (C / 8) == 0, "gn_stats: C=%d unsupported (need C/8 to divide 256, C<=512)", C);
   const int chunks = 64;
-  bind_launch(op, gn_partial_kernel<false>, dim3(chunks, d->batch), dim3(256), 0, (const act_t*)x, d->voxels, C, d->groups, chunks, workspace,
-                  (const float*)nullptr);
+  bind_launch(op, gn_partial_kernel<kPivot>, dim3(chunks, d->batch), dim3(256), 0, (const act_t*)x, d->voxels, C, d->groups, chunks,
+                  (void*)workspace, (const float*)nullptr);
   const int tot = d->batch * d->groups;
-  bind_launch(op, gn_final_kernel, dim3((tot + 127) / 128), dim3(128), 0, workspace, d->batch, d->groups, chunks,
+  bind_launch(op, gn_final_kernel, dim3((tot + 127) / 128), dim3(128), 0, (const double*)workspace, d->batch, d->groups, chunks,
                   (double)d->voxels * (double)(C / d->groups), eps, mean_rstd);
   return B200DM_OK;
 }
@@ -451,10 +489,12 @@ int bind_bn_stats(const void* x, int64_t rows, int32_t c, const float* gamma, co
   float* center = workspace + (size_t)kBnChunks * c * 2;
   const act_t* xb = (const act_t*)x;
   const dim3 fgrid((c + 127) / 128);
-  bind_launch(op, gn_partial_kernel<false>, dim3(kBnChunks), dim3(256), 0, xb, rows, (int)c, (int)c, kBnChunks, workspace, (const float*)nullptr);
+  bind_launch(op, gn_partial_kernel<kSums>, dim3(kBnChunks), dim3(256), 0, xb, rows, (int)c, (int)c, kBnChunks, (void*)workspace,
+                  (const float*)nullptr);
   bind_launch(op, bn_final_kernel, fgrid, dim3(128), 0, (const float*)workspace, (int)c, kBnChunks, (double)rows, eps, center,
                   (const float*)nullptr, (const float*)nullptr, (float*)nullptr, (float*)nullptr);
-  bind_launch(op, gn_partial_kernel<true>, dim3(kBnChunks), dim3(256), 0, xb, rows, (int)c, (int)c, kBnChunks, workspace, (const float*)center);
+  bind_launch(op, gn_partial_kernel<kCentered>, dim3(kBnChunks), dim3(256), 0, xb, rows, (int)c, (int)c, kBnChunks, (void*)workspace,
+                  (const float*)center);
   bind_launch(op, bn_final_kernel, fgrid, dim3(128), 0, (const float*)workspace, (int)c, kBnChunks, (double)rows, eps, center, gamma, beta,
                   scale, shift);
   return B200DM_OK;

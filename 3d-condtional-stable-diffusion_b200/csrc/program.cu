@@ -99,7 +99,7 @@ extern "C" int b200dm_program_add_bn_stats(b200dm_program* p, const void* x, int
   return record(p, "program_add_bn_stats", bind_bn_stats, x, rows, c, gamma, beta, eps, scale, shift, workspace, ws_bytes);
 }
 
-extern "C" int b200dm_program_add_gn_finalize(b200dm_program* p, const float* partials, int32_t batch, int32_t rows_per_sample,
+extern "C" int b200dm_program_add_gn_finalize(b200dm_program* p, const double* partials, int32_t batch, int32_t rows_per_sample,
                                               int32_t c, int32_t groups, int64_t voxels_per_sample, float eps, float* mean_rstd) {
   return record(p, "program_add_gn_finalize", bind_gn_finalize, partials, batch, rows_per_sample, c, groups, voxels_per_sample, eps,
                 mean_rstd);

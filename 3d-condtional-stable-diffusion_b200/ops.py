@@ -339,13 +339,13 @@ class ConvPlan:
         return self.y
 
     def gn_partials(self):
-        """GroupNorm partial sums as a by-product of this conv: -> (workspace fp32 (B * rows, C, 2), rows per sample), or None
+        """GroupNorm partial sums as a by-product of this conv: -> (workspace fp64 (B * rows, C, 2), rows per sample), or None
         when the plan's kernel cannot produce them (the caller then runs a statistics pass over y)."""
         rows = C.c_int32(0)
         nbytes = lib().b200dm_conv_plan_gn_partials_bytes(self.h, C.byref(rows))
         if nbytes == 0:
             return None
-        ws = torch.zeros(nbytes // 4, dtype=torch.float32, device=self.y.device)
+        ws = torch.zeros(nbytes // 8, dtype=torch.float64, device=self.y.device)
         check(lib().b200dm_conv_plan_set_gn_partials(self.h, ptr(ws), nbytes))
         self.keep = self.keep + (ws,)
         return ws, rows.value

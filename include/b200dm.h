@@ -296,12 +296,13 @@ int b200dm_conv_plan_set_shortcut(b200dm_conv_plan* p, int32_t c0, int32_t c1, c
 int b200dm_conv_plan_info(const b200dm_conv_plan* p, int32_t* halo, int32_t* block_n, int32_t* ksplit);
 /* GroupNorm statistics as a by-product of the producing conv (replaces a second read of the conv output by
  * tfa GroupNormalization's moments, vqgan_attn_cp.py:258-275): plans that support it (the d-sweeping C_in = C_out = 32 kernel)
- * accumulate per-(work item, channel) partial sums of the STORED values into `workspace` = float[batch * rows_per_sample][C][2];
+ * accumulate per-(work item, channel) partial sums of the STORED values into `workspace` = double[batch * rows_per_sample][C][2]
+ * (fp32 sums about a per-item pivot, rebuilt in fp64: exact enough when |mean| >> std);
  * b200dm_gn_finalize reduces them in a fixed order (bit-reproducible) to (mean, rstd) per (sample, group).
  * _bytes returns 0 when the plan cannot produce partials. */
 size_t b200dm_conv_plan_gn_partials_bytes(const b200dm_conv_plan* plan, int32_t* rows_per_sample);
-int b200dm_conv_plan_set_gn_partials(b200dm_conv_plan* plan, float* workspace, size_t ws_bytes);
-int b200dm_gn_finalize(const float* partials, int32_t batch, int32_t rows_per_sample, int32_t c, int32_t groups,
+int b200dm_conv_plan_set_gn_partials(b200dm_conv_plan* plan, double* workspace, size_t ws_bytes);
+int b200dm_gn_finalize(const double* partials, int32_t batch, int32_t rows_per_sample, int32_t c, int32_t groups,
                        int64_t voxels_per_sample, float eps, float* mean_rstd, void* stream);
 /* tuning aid: device int64[4*2048] receiving CTA 0's per-role timeline ((clock64 << 8) | tag); NULL switches it off */
 int b200dm_conv_plan_set_trace(b200dm_conv_plan* p, void* trace);
@@ -347,7 +348,7 @@ int b200dm_program_add_bn_stats(b200dm_program* p, const void* x, int64_t rows, 
                                 float eps, float* scale, float* shift, float* workspace, size_t ws_bytes);
 int b200dm_program_add_gn_stats(b200dm_program* p, const b200dm_norm_desc* d, const void* x, float eps,
                                 float* mean_rstd, float* workspace, size_t ws_bytes);
-int b200dm_program_add_gn_finalize(b200dm_program* p, const float* partials, int32_t batch, int32_t rows_per_sample, int32_t c,
+int b200dm_program_add_gn_finalize(b200dm_program* p, const double* partials, int32_t batch, int32_t rows_per_sample, int32_t c,
                                    int32_t groups, int64_t voxels_per_sample, float eps, float* mean_rstd);
 int b200dm_program_add_layernorm(b200dm_program* p, const void* x, int64_t rows, int32_t c, float eps,
                                  int32_t n_out, const float* const* gammas, const float* const* betas,

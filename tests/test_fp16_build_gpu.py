@@ -13,7 +13,7 @@ pytestmark = pytest.mark.gpu
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 FILES = ["test_conv_gpu.py", "test_attention_gpu.py", "test_elementwise_gpu.py", "test_fullsize_gpu.py", "test_shortcut_fold_gpu.py",
-         "test_model_gpu.py", "test_train_forward_gpu.py", "test_storage_edges_gpu.py"]
+         "test_model_gpu.py", "test_train_forward_gpu.py", "test_storage_edges_gpu.py", "test_norm_gpu.py"]
 
 
 @pytest.mark.skipif(os.environ.get("B200DM_PRECISION", "bf16") != "bf16", reason="already the fp16 child run")
